@@ -2,6 +2,7 @@
 """bench.py — Mpaths/s (pixels x spp / s) of the path-tracing hot path.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1|2|3|4a|4b|5]
+                  [--dump-outputs DIR]
 
 A step is one frame of the chosen BASELINE.json configuration (default 3, the one the metric is quoted on:
 scenes/cornell_box.json + seeded random spheres = 492 shapes, 1024 x 1024, 256 spp, max depth 8); config 2 is the
@@ -17,6 +18,11 @@ renderer (C++ restatement of the reference, BVH like Scene::new builds) on a bou
 
 `--impl reference` runs ONLY the oracle (liboracle.so) on the flattened scene files under oracle/scenes/ -- it
 imports nothing of the product package and loads none of its libraries.
+
+`--dump-outputs DIR` writes what the timed path returned in its last timed step as DIR/<name>.npy (float64, see
+dump_outputs): the frame of configs 1, 3, 4a, 4b, 5 or the nearest-hit records of config 2.  Scenes, rays and RNG
+seeds are fixed, so two builds run with the same arguments can be compared output for output.  Nothing is written
+to the source tree.
 """
 from __future__ import annotations
 
@@ -28,6 +34,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True   # the benchmark runs from a tree it must leave as it found it (possibly read-only)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -138,8 +145,8 @@ def cpu_reference_run(cfg: str, steps: int, warmup: int):
     n_paths = c["w"] * c["h"] * spp
     secs, counters = [], None
     for i in range(warmup + steps):
-        _, info = osc.render(cam, c["w"], c["h"], spp, DEPTH, seed=RNG_SEED + i, rng="xoshiro", use_bvh=True,
-                             threads=threads, counters=(i == warmup + steps - 1))
+        frame, info = osc.render(cam, c["w"], c["h"], spp, DEPTH, seed=RNG_SEED + i, rng="xoshiro", use_bvh=True,
+                                 threads=threads, counters=(i == warmup + steps - 1))
         if i >= warmup:
             secs.append(info["seconds"])
         counters = info.get("counters", counters)
@@ -148,7 +155,7 @@ def cpu_reference_run(cfg: str, steps: int, warmup: int):
             f"{n_paths} paths per step; C++ restatement of the reference's threaded renderer with its BVH, {threads} "
             f"worker threads + 1 serial dispatcher (not the Rust binary: no Rust toolchain in the image)")
     return {"value": n_paths / mean_s / 1e6, "unit": "Mpaths/s", "ms": mean_s * 1e3, "cores": threads, "sample": desc,
-            "n_units": n_paths, "counters": counters}
+            "n_units": n_paths, "counters": counters, "outputs": {"frame": frame}}
 
 
 def bench_rays(n, seed=42, target_radius=3.0):
@@ -182,7 +189,30 @@ def cpu_rays_run(po, threads, steps, warmup):
     mean_s = sum(secs) / len(secs)
     return {"value": len(rays) / mean_s / 1e6, "unit": "Mrays/s", "ms": mean_s * 1e3, "cores": threads,
             "sample": f"all {len(rays)} rays per step, ShapeCollection loop (no BVH), {threads} threads; C++ restatement "
-                      "of the reference (not the Rust binary)", "n_units": len(rays), "counters": None}
+                      "of the reference (not the Rust binary)", "n_units": len(rays), "counters": None,
+            "outputs": {k: out[k] for k in ("index", "t", "normal")}}
+
+
+DUMP_LIMIT = 64_000_000    # bytes --dump-outputs writes at most
+DUMP_SEED = 20240601
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """--dump-outputs: every array as out_dir/<name>.npy in float64 (shape indices are exact in it).  The arrays share
+    their first axis (image rows, rays); when together they exceed DUMP_LIMIT, the same fixed, seeded sample of that
+    axis is kept from each, in increasing order, and its indices are written as out_dir/sample_index.npy."""
+    import numpy as np
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    per_item = sum(a.nbytes for a in arrays.values()) // n
+    if n * per_item > DUMP_LIMIT:
+        keep = (DUMP_LIMIT - 4096) // (per_item + 8)      # (+ the index array, + the .npy headers)
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, keep, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        arrays["sample_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def emit(line: dict) -> None:
@@ -226,7 +256,11 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="3", choices=sorted(CONFIGS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
 
     in_torchrun = "WORLD_SIZE" in os.environ
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -261,6 +295,8 @@ def main():
         assert "rs_pathtracing_b200" not in sys.modules
         r = cpu_reference_run(cfg, args.steps, args.warmup)
         assert "rs_pathtracing_b200" not in sys.modules   # the reference arm runs the oracle alone
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, r["outputs"])
         line = {"impl": "reference", "metric": unit, "value": r["value"], "unit": unit, "n_gpus": args.gpus,
                 "steps": args.steps, "warmup": args.warmup, "ms_per_step": r["ms"], "higher_is_better": True,
                 "scaling": "strong", "vs_baseline": None, "dtype": "f64", "data": "synthetic", "config": config,
@@ -359,11 +395,13 @@ def run_frames(ctx, cfg):
     t0 = time.perf_counter()
     # the K steps as ONE pipelined sequence: every step renders and assembles a complete frame; step n's exchange to
     # rank 0 and its k_assemble overlap step n+1's render (DistributedRenderer.render_jobs_device)
-    dr.render_many_device(cam, WIDTH, HEIGHT, SPP, args.steps,
-                          on_rendered=lambda i: frame_ms.append(sc.stats(local_rank).last_frame_ms))   # CUDA events on the library's stream
+    last_frame = dr.render_many_device(cam, WIDTH, HEIGHT, SPP, args.steps,
+                                       on_rendered=lambda i: frame_ms.append(sc.stats(local_rank).last_frame_ms))   # CUDA events on the library's stream
     barrier()
     wall_s = time.perf_counter() - t0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:   # (the passes below reuse the frame buffer)
+        dump_outputs(args.dump_outputs, {"frame": last_frame.cpu().numpy()})
     launches = sc.stats(local_rank).kernel_launches
     # per-kernel device time: the same K steps again with one CUDA event pair around every launch on the
     # library's stream (the event pairs serialise the two stream lanes, so they stay out of the pass `value` comes from)
@@ -574,6 +612,8 @@ def run_rays(ctx):
         evs.append((a, b))
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:   # rank 0's rays
+        dump_outputs(args.dump_outputs, {"index": d_idx.cpu().numpy(), "t": d_t.cpu().numpy(), "normal": d_n.cpu().numpy()})
     ms = max_over_ranks(sum(a.elapsed_time(b) for a, b in evs) / args.steps)
     value = n_all / (ms * 1e-3) / 1e6
     # end to end: host rays in, host hit records out through rt_intersect_batch

@@ -1,10 +1,11 @@
 """Builds rust/patch/describe.patch: the edits to the reference crate that make `GpuRenderer` a drop-in
 (`Describe` hooks on Shape / ShapeFunction / Material / Texture, `Scene::flat()`, `#[repr(C)] Vector3d`,
-`pub mod gpu`).  Works on a scratch copy of /root/reference/src (authoring container only), inserts the additions
-below at anchors found in the reference text, and writes `diff -U1` of the result -- one line of context, so the
-patch carries our additions and next to nothing of the reference.
+`pub mod gpu`).  Works on a scratch copy of the reference crate (a checkout of dkarpushkin/rs-pathtracing: the
+directory holding its Cargo.toml and src/, named by RS_PATHTRACING_SRC), inserts the additions below at anchors found
+in the reference text, and writes `diff -U1` of the result -- one line of context, so the patch carries our additions
+and next to nothing of the reference.
 
-  python tools/make_rust_patch.py          # rewrites rust/patch/describe.patch
+  RS_PATHTRACING_SRC=<checkout> python tools/make_rust_patch.py [OUT]   # OUT defaults to rust/patch/describe.patch
 """
 import os
 import shutil
@@ -13,7 +14,7 @@ import sys
 import tempfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+REF = os.environ.get("RS_PATHTRACING_SRC", "")
 
 
 def insert_after(text, anchor, addition, occurrence=1):
@@ -160,8 +161,8 @@ def fn_describe(body, ret):
 
 
 def main():
-    if not os.path.isdir(REF):
-        sys.exit("needs /root/reference (authoring container)")
+    if not os.path.isdir(os.path.join(REF, "src")):
+        sys.exit("RS_PATHTRACING_SRC must name a checkout of the reference crate")
     tmp = tempfile.mkdtemp()
     a, b = os.path.join(tmp, "a"), os.path.join(tmp, "b")
     for d in (a, b):
@@ -240,7 +241,7 @@ def main():
     diff = subprocess.run(["diff", "-U1", "-r", "-N", "a", "b"], cwd=tmp, capture_output=True).stdout   # bytes: keep CRLF
     # no timestamps in the file headers: the patch is reproducible
     diff = b"\n".join(l.split(b"\t")[0] if l.startswith((b"--- ", b"+++ ")) else l for l in diff.split(b"\n"))
-    out = os.path.join(ROOT, "rust", "patch", "describe.patch")
+    out = sys.argv[1] if len(sys.argv) > 1 else os.path.join(ROOT, "rust", "patch", "describe.patch")
     with open(out, "wb") as f:
         f.write(diff)
     shutil.rmtree(tmp)
