@@ -11,6 +11,7 @@
  *   ThreadPoolRenderer::new(scene, thread_number, depth)                  src/renderer/step_by_step.rs:37
  *   Scene::closest_hit(&Ray, min_t, max_t)                                src/world/mod.rs:42-44
  *   renderer::trace_pixel_samples(&(idx, rays), &Scene, depth)            src/renderer/mod.rs:151-155
+ *   renderer::trace_pixel_samples_group(&[(idx, rays)], &Scene, depth)    src/renderer/mod.rs:127-149
  *
  * Conventions
  *   - every entry point returns 0 (RT_OK) or a negative rt_status; nothing unwinds or aborts
@@ -185,7 +186,7 @@ void rt_scene_destroy(rt_scene* scene);
  * is assembled there.  rt_render_poll / rt_render_wait deliver the assembled frame (no partial delivery: *done
  * flips when the whole frame is there), rt_render_device_frame exposes it on device_ids[0].  The frame is the one a
  * single device renders, bit for bit (the RNG is keyed per pixel, the accumulators are f64 sums).  Every other
- * entry point (rt_intersect_batch, rt_trace_pixel_samples, statistics, an explicitly sharded rt_render_start)
+ * entry point (rt_intersect_batch, rt_trace_pixel_samples[_group], statistics, an explicitly sharded rt_render_start)
  * addresses device_ids[0].  n_devices = 1 is rt_scene_create. */
 int rt_scene_create_multi(const rt_scene_desc* desc, int n_devices, const int* device_ids, rt_scene** out);
 /* number of devices behind the handle (1 for rt_scene_create) */
@@ -307,9 +308,35 @@ int rt_tonemap_rgba8_device(rt_scene* scene, const uint8_t** d_rgba, uint8_t* rg
 /* ---- pixel probe (replaces renderer::trace_pixel_samples, src/renderer/mod.rs:151-155) */
 
 /* Traces caller-supplied primary rays (host buffer) as samples of ONE pixel and returns their
- * mean radiance; RNG keyed by (seed, pixel_index, sample = ray number). */
+ * mean radiance; RNG keyed by (seed, pixel_index, sample = ray number).  The one-group case of
+ * rt_trace_pixel_samples_group; n_rays = 0 is rejected. */
 int rt_trace_pixel_samples(rt_scene* scene, const rt_ray* rays, uint32_t n_rays, uint32_t max_depth,
                            uint64_t seed, uint32_t pixel_index, rt_vec3* mean_out);
+
+/* renderer::trace_pixel_samples_group, src/renderer/mod.rs:127-149: many pixels in one wavefront.
+ * Group g is rays[offsets[g] .. offsets[g+1]), samples 0, 1, ... of pixel pixel_index[g]; means[g] = the sum of
+ * their ray_color / n_g with the arithmetic of rt_trace_pixel_samples (RNG keyed by (seed, pixel_index[g], sample),
+ * per-path radiance rounded to float, f64 sum in sample order, one division).  So group g gives what
+ * rt_trace_pixel_samples gives for its rays alone, and the camera's own primary rays with pixel_index = x + y*width
+ * give the pixels of the rt_render_start frame of the same seed, depth and samples -- bit for bit, whatever the
+ * batch size, the lanes, the order of the groups or their split into calls.  An empty group gives NaN (the
+ * reference's Vector3d / 0.0); pixel indices may repeat; rays are never renormalised; n_groups = 0 does nothing.
+ * RT_ERR_INVALID: offsets[0] != 0, decreasing offsets, offsets[n_groups] != n_rays, a group of 2^32 rays or more,
+ * a NULL array that is needed, max_depth > 62.  RT_ERR_STATE while a frame is in flight.  The frame, its
+ * accumulator and the progressive accumulation are left alone; rt_stats.paths grows by n_rays.  Addresses
+ * device_ids[0] of a multi-device handle.  Blocks until means[] is written. */
+int rt_trace_pixel_samples_group(rt_scene* scene, const rt_ray* rays, uint64_t n_rays,
+                                 const uint64_t* offsets /* n_groups + 1 */, const uint32_t* pixel_index /* n_groups */,
+                                 uint32_t n_groups, uint32_t max_depth, uint64_t seed, rt_vec3* means /* n_groups */);
+/* The same with d_rays and d_means DEVICE pointers on the scene's (first) device; offsets and pixel_index stay HOST
+ * arrays (the batches are planned from them; they are read before the call returns, pinned or pageable).  Ordered after the work queued
+ * on `stream` before the call, and work queued on `stream` after it runs after d_rays has been read and d_means
+ * written; returns without waiting (except while rt_set_kernel_timing is on).  stream: a cudaStream_t as void*;
+ * NULL = the library's own non-blocking stream; the legacy default stream (handle 0, e.g. torch's default stream) is
+ * named by cudaStreamLegacy = 0x1. */
+int rt_trace_pixel_samples_group_device(rt_scene* scene, const rt_ray* d_rays, uint64_t n_rays,
+                                        const uint64_t* offsets, const uint32_t* pixel_index, uint32_t n_groups,
+                                        uint32_t max_depth, uint64_t seed, rt_vec3* d_means, void* stream);
 
 /* ---- instrumentation ---------------------------------------------------------------- */
 

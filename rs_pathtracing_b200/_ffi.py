@@ -150,6 +150,10 @@ CORE_SYMBOLS = {
     "rt_tonemap_rgba8_device": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.c_void_p, C.POINTER(C.c_uint64)]),
     "rt_trace_pixel_samples": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint64, C.c_uint32,
                                          C.POINTER(Vec3)]),
+    "rt_trace_pixel_samples_group": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint32,
+                                               C.c_uint32, C.c_uint64, C.c_void_p]),
+    "rt_trace_pixel_samples_group_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
+                                                      C.c_uint32, C.c_uint32, C.c_uint64, C.c_void_p, C.c_void_p]),
     "rt_get_stats": (C.c_int, [C.c_void_p, C.POINTER(Stats)]),
     "rt_reset_stats": (C.c_int, [C.c_void_p]),
     "rt_set_counters": (C.c_int, [C.c_void_p, C.c_int]),

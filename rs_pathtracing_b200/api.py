@@ -197,6 +197,40 @@ class Scene:
                                                   rays.shape[0], depth, seed, pixel_index, C.byref(mean)))
         return np.array(mean.tuple())
 
+    def trace_pixel_samples_group(self, rays, offsets, pixel_index, depth: int, seed: int = 0,
+                                  device: Optional[int] = None):
+        """renderer::trace_pixel_samples_group (src/renderer/mod.rs:127-149): group g = rays[offsets[g]:offsets[g+1]],
+        the samples of pixel pixel_index[g]; returns the (g, 3) per-group means (NaN for an empty group).
+        rays: numpy (n, 6) float64 -> numpy result after the host round trip; or a contiguous float64 CUDA torch tensor
+        (n, 6) on the scene's device -> a torch tensor on that device, queued on torch's current stream without a host
+        synchronisation.  offsets / pixel_index are host arrays in both cases."""
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64).reshape(-1)
+        pixel_index = np.ascontiguousarray(pixel_index, dtype=np.uint32).reshape(-1)
+        n_groups = pixel_index.shape[0]
+        if offsets.shape[0] != n_groups + 1:
+            raise ValueError(f"offsets needs n_groups + 1 = {n_groups + 1} entries, got {offsets.shape[0]}")
+        p = lambda a: a.ctypes.data_as(C.c_void_p)
+        if type(rays).__module__.split(".")[0] == "torch":
+            import torch
+            if not (rays.is_cuda and rays.dtype == torch.float64 and rays.dim() == 2 and rays.shape[1] == 6
+                    and rays.is_contiguous()):
+                raise ValueError("rays: a contiguous float64 CUDA tensor of shape (n, 6)")
+            h = self.device_scene(device)
+            if rays.device.index != self._device:
+                raise ValueError(f"rays are on {rays.device}, the scene's device is cuda:{self._device}")
+            means = torch.empty((n_groups, 3), dtype=torch.float64, device=rays.device)
+            # torch's default stream is the legacy default stream (handle 0), which the ABI names cudaStreamLegacy = 0x1
+            stream = torch.cuda.current_stream(rays.device).cuda_stream or 1
+            _check(_ffi.core().rt_trace_pixel_samples_group_device(h, rays.data_ptr(), rays.shape[0], p(offsets),
+                                                                   p(pixel_index), n_groups, depth, seed,
+                                                                   means.data_ptr(), stream))
+            return means
+        rays = np.ascontiguousarray(rays, dtype=np.float64).reshape(-1, 6)
+        means = np.empty((n_groups, 3), np.float64)
+        _check(_ffi.core().rt_trace_pixel_samples_group(self.device_scene(device), p(rays), rays.shape[0], p(offsets),
+                                                        p(pixel_index), n_groups, depth, seed, p(means)))
+        return means
+
     def stats(self, device: Optional[int] = None) -> Stats:
         s = Stats()
         _check(_ffi.core().rt_get_stats(self.device_scene(device), C.byref(s)))

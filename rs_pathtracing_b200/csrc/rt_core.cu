@@ -6,6 +6,8 @@
 //   k_bounce            one segment of ray_color for every live path: nearest hit, scatter / emit /
 //                       sky, survivors compacted into the next queue (ballot + popc + one atomic per warp)
 //   k_resolve           per-pixel mean (trace_pixel_samples) -> (f64 sums, samples) accumulator + f64 frame
+//   k_load_groups       caller-supplied rays of groups of any size -> level-0 queue + RNG keys (trace_pixel_samples_group)
+//   k_group_resolve     per-group mean of caller-supplied rays, continued across the batches of a large group
 //   k_assemble          multi-GPU: gathered tile-packed shards -> frame
 //   k_tonemap           the bins' sqrt / clamp / *256 -> RGBA8
 // Compile with -fmad=false (see rt_math.cuh).
@@ -260,8 +262,8 @@ k_raygen(RayCasterDev rc, ShardMap map, unsigned long long first_owned, uint32_t
 template <bool COUNT>
 __global__ void __launch_bounds__(256)
 k_bounce(DevScene S, bool use_smem, PathQueue in, const uint32_t* __restrict__ count_in, PathQueue out,
-         uint32_t* count_out, uint32_t level, uint32_t max_depth, ShardMap map, unsigned long long first_owned,
-         uint32_t spp, uint32_t k0, uint32_t k1, float4* __restrict__ radiance, DevCounters* g_counters) {
+         uint32_t* count_out, uint32_t level, uint32_t max_depth, const uint2* __restrict__ path_key, uint32_t k0,
+         uint32_t k1, float4* __restrict__ radiance, DevCounters* g_counters) {
     Staged st = stage_scene(S, use_smem);
     DevCounters c = {};
     const uint32_t n = *count_in;
@@ -287,12 +289,11 @@ k_bounce(DevScene S, bool use_smem, PathQueue in, const uint32_t* __restrict__ c
             } else {
                 HitRec h;
                 finalize_hit(S, bi, bt, ro, rd, h);
-                uint32_t pl = pid / spp, s = pid % spp, x, y;
-                map.pixel_of(first_owned + pl, x, y);
+                const uint2 key = path_key[pid];   // written by k_raygen / k_load_groups, as k_shade reads it
                 PathRng rng;
                 rng.k0 = k0; rng.k1 = k1;
-                rng.pixel = x + y * map.width;
-                rng.sample = s;
+                rng.pixel = key.x;
+                rng.sample = key.y;
                 rng.begin_event(level + 1);
                 D3 ndir, atten;
                 if (scatter_or_emit(S, h, rd, rng, ndir, atten)) {  // :29-32
@@ -520,6 +521,8 @@ __global__ void __launch_bounds__(256, 3)
 k_shade(DevScene S, PathQueue in, const uint32_t* __restrict__ count_in, HitQueue hq, PathQueue out, uint32_t* count_out,
         uint32_t level, uint32_t max_depth, ShardMap map, unsigned long long first_owned, uint32_t spp, uint32_t k0,
         uint32_t k1, float4* __restrict__ radiance) {
+    // (map / first_owned / spp are not read -- the RNG key comes from hq.key -- but stay in the signature: dropping them
+    // moves the other parameters in the constant bank and changes the generated code; measured -0.8 % on the frame)
     const uint32_t n = *count_in;
     // random_in_unit_sphere is drawn by the whole warp for its rejected lanes (coop_random_in_unit_sphere)
     __shared__ uint4 s_ball_id[256];
@@ -614,6 +617,47 @@ k_resolve(const float4* __restrict__ radiance, uint32_t n_pixels, uint32_t spp, 
     frame_owned[first_owned + pl] = rt_vec3{sx / ln, sy / ln, sz / ln};
 }
 
+// K5b: per-group mean of caller rays (trace_pixel_samples, src/renderer/mod.rs:151-155, per group of :127-149), one
+// thread per group of the batch (rays [r0, r1), group slice as in k_load_groups).  The same arithmetic as k_resolve:
+// f64 sums in sample order from 0.0, then one division by the group's ray count -- an empty group gives 0 / 0 = NaN,
+// what the reference's Vector3d / 0.0 gives.  A group larger than a batch is traced in consecutive batches of ONE
+// stream: its running f64 sum waits in means[k] between them, and the batch that holds its last ray divides.
+__global__ void __launch_bounds__(256)
+k_group_resolve(const float4* __restrict__ radiance, unsigned long long r0, unsigned long long r1,
+                const unsigned long long* __restrict__ offsets, uint32_t n_groups, rt_vec3* __restrict__ means) {
+    const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n_groups) return;
+    const unsigned long long first = offsets[k], end = offsets[k + 1];
+    double sx = 0.0, sy = 0.0, sz = 0.0;
+    if (first < r0) {   // continued from the previous batch
+        const rt_vec3 prev = means[k];
+        sx = prev.x; sy = prev.y; sz = prev.z;
+    }
+    const unsigned long long a = first > r0 ? first : r0, b = end < r1 ? end : r1;
+    // the sum is serial (its order is the contract); the loads of 16 samples are issued together so that a large group
+    // waits for memory once per 16 samples instead of once per sample
+    unsigned long long r = a;
+    for (; r + 16 <= b; r += 16) {
+        float4 v[16];
+#pragma unroll
+        for (int j = 0; j < 16; j++) v[j] = radiance[r - r0 + j];
+#pragma unroll
+        for (int j = 0; j < 16; j++) {
+            sx += (double)v[j].x; sy += (double)v[j].y; sz += (double)v[j].z;
+        }
+    }
+    for (; r < b; r++) {
+        const float4 v = radiance[r - r0];
+        sx += (double)v.x; sy += (double)v.y; sz += (double)v.z;
+    }
+    if (end > r1) {
+        means[k] = rt_vec3{sx, sy, sz};
+        return;
+    }
+    const double n = (double)(end - first);
+    means[k] = rt_vec3{sx / n, sy / n, sz / n};
+}
+
 // K7: de-interleave gathered shards into the frame (x + y*w, f64 linear mean)
 struct ShardPtrs {
     const Acc* p[16];
@@ -647,20 +691,29 @@ k_tonemap(const rt_vec3* __restrict__ frame, unsigned long long n, uchar4* __res
     rgba[i] = make_uchar4(q(r), q(g), q(b), 255);
 }
 
-// scatter owned-order pixels into a full frame (host path of a sharded render keeps it simple and
-// does this on the host; this kernel serves rt_trace_pixel_samples' ray upload)
+// K6: caller-supplied rays (trace_pixel_samples_group, src/renderer/mod.rs:127-149).  The batch is rays [r0, r0 + n)
+// of the call; `offsets` is the batch's slice of the call's group offsets (offsets[k] = first ray of group k, global
+// ray numbers, n_groups + 1 entries, offsets[0] <= r0 and offsets[n_groups] >= r0 + n).  Path i is ray r0 + i: its
+// group is found by binary search, its RNG key is (pixel_index[group], ray number inside the group).
 __global__ void __launch_bounds__(256)
-k_load_rays(const rt_ray* __restrict__ rays, uint32_t n, PathQueue q, uint32_t* count_out, uint2* __restrict__ path_key,
-            uint32_t pixel_index) {
-    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+k_load_groups(const rt_ray* __restrict__ rays, uint32_t n, unsigned long long r0, const unsigned long long* __restrict__ offsets,
+              const uint32_t* __restrict__ pixel_index, uint32_t n_groups, PathQueue q, uint32_t* count_out,
+              uint2* __restrict__ path_key) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i == 0) *count_out = n;
     if (i >= n) return;
-    rt_ray r = rays[i];
-    q.ox[i] = r.origin.x; q.oy[i] = r.origin.y; q.oz[i] = r.origin.z;
-    q.dx[i] = r.direction.x; q.dy[i] = r.direction.y; q.dz[i] = r.direction.z;
+    const unsigned long long r = r0 + i;
+    uint32_t lo = 0, hi = n_groups;   // the last group that starts at or before r (empty groups before it start there too)
+    while (hi - lo > 1) {
+        const uint32_t mid = lo + (hi - lo) / 2;
+        if (offsets[mid] <= r) lo = mid; else hi = mid;
+    }
+    const rt_ray ray = rays[i];
+    q.ox[i] = ray.origin.x; q.oy[i] = ray.origin.y; q.oz[i] = ray.origin.z;
+    q.dx[i] = ray.direction.x; q.dy[i] = ray.direction.y; q.dz[i] = ray.direction.z;
     q.bx[i] = 1.0; q.by[i] = 1.0; q.bz[i] = 1.0;
     q.pid[i] = i;
-    path_key[i] = make_uint2(pixel_index, i);  // sample i of the pixel
+    path_key[i] = make_uint2(pixel_index[lo], (uint32_t)(r - offsets[lo]));   // (groups have fewer than 2^32 rays)
 }
 
 // FMA micro-benchmarks: 8 independent chains per thread, FMA counted as 2 flop
@@ -791,6 +844,19 @@ struct rt_scene {
     cudaEvent_t ev_multi_done = nullptr;
     bool multi_active = false;            // the frame in flight / last completed was rendered by all devices
     rt_render_params multi_rp{};
+    // rt_trace_pixel_samples_group: the call's group offsets and pixel indices on the device, the host form's rays and
+    // means (persistent buffers, grown on demand), and the events that order a call against the caller's stream
+    unsigned long long* d_group_off = nullptr;
+    uint32_t* d_group_pix = nullptr;
+    rt_vec3* d_group_means = nullptr;
+    rt_ray* d_group_rays = nullptr;
+    uint64_t group_off_cap = 0, group_pix_cap = 0, group_means_cap = 0, group_rays_cap = 0;
+    // host copies of the caller's offsets / pixel indices: pageable memory the library owns, so that the upload has read
+    // them when cudaMemcpyAsync returns even if the caller's arrays are pinned (an upload from pinned memory is only
+    // read when the stream gets there, after the caller may have reused them)
+    std::vector<uint64_t> h_group_off;
+    std::vector<uint32_t> h_group_pix;
+    cudaEvent_t ev_group_in = nullptr, ev_group_start = nullptr, ev_group_done = nullptr;
 };
 
 template <class T>
@@ -801,6 +867,17 @@ static int upload(rt_scene* sc, const T* src, size_t count, const T** out) {
     sc->allocs.push_back(d);
     if (count) CU(cudaMemcpy(d, src, count * sizeof(T), cudaMemcpyHostToDevice));
     *out = (const T*)d;
+    return RT_OK;
+}
+
+template <class T>
+static int ensure_device_array(T*& p, uint64_t& cap, uint64_t n) {   // persistent buffer, grown on demand
+    if (cap >= n) return RT_OK;
+    cudaFree(p);
+    p = nullptr;
+    cap = 0;
+    CU(cudaMalloc(&p, std::max<uint64_t>(n, 1) * sizeof(T)));
+    cap = n;
     return RT_OK;
 }
 
@@ -894,6 +971,10 @@ int rt_scene_create(const rt_scene_desc* d, int device, rt_scene** out) {
     cudaEventCreate(&sc->ev_b);
     cudaEventCreate(&sc->ev_frame_start);
     cudaEventCreate(&sc->ev_frame_stop);
+    if (cudaEventCreateWithFlags(&sc->ev_group_in, cudaEventDisableTiming) != cudaSuccess ||
+        cudaEventCreateWithFlags(&sc->ev_group_start, cudaEventDisableTiming) != cudaSuccess ||
+        cudaEventCreateWithFlags(&sc->ev_group_done, cudaEventDisableTiming) != cudaSuccess)
+        return bail(fail(RT_ERR_CUDA, "cudaEventCreate failed"));
 
     const uint32_t n = d->n_shapes;
     sc->ds.n_shapes = (int)n;
@@ -1154,6 +1235,10 @@ void rt_scene_destroy(rt_scene* sc) {
     cudaFree(sc->d_full_frame);
     cudaFree(sc->d_tone_in);
     cudaFree(sc->d_tone_out);
+    cudaFree(sc->d_group_off);
+    cudaFree(sc->d_group_pix);
+    cudaFree(sc->d_group_means);
+    cudaFree(sc->d_group_rays);
     if (sc->host_stage) cudaFreeHost(sc->host_stage);
     bind_lane(sc, 0);
     for (int l = 0; l < RT_MAX_LANES; l++)
@@ -1171,6 +1256,9 @@ void rt_scene_destroy(rt_scene* sc) {
     if (sc->ev_b) cudaEventDestroy(sc->ev_b);
     if (sc->ev_frame_start) cudaEventDestroy(sc->ev_frame_start);
     if (sc->ev_frame_stop) cudaEventDestroy(sc->ev_frame_stop);
+    if (sc->ev_group_in) cudaEventDestroy(sc->ev_group_in);
+    if (sc->ev_group_start) cudaEventDestroy(sc->ev_group_start);
+    if (sc->ev_group_done) cudaEventDestroy(sc->ev_group_done);
     if (sc->stream) cudaStreamDestroy(sc->stream);
     if (sc->copy_stream) cudaStreamDestroy(sc->copy_stream);
     delete sc;
@@ -1334,8 +1422,7 @@ static int alloc_queue(rt_scene* sc, PathQueue& q, uint64_t cap) {
 
 
 // enqueue the bounce loop for paths already in q[0] (count in d_counts[0]); no host sync
-static void launch_bounces(rt_scene* sc, uint32_t max_depth, unsigned long long first_owned, uint32_t spp, uint64_t seed,
-                           const RaygenArgs* raygen = nullptr) {
+static void launch_bounces(rt_scene* sc, uint32_t max_depth, uint64_t seed, const RaygenArgs* raygen = nullptr) {
     uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
     for (uint32_t level = 0; level <= max_depth; level++) {
         PathQueue& in = sc->q[level & 1];
@@ -1348,12 +1435,12 @@ static void launch_bounces(rt_scene* sc, uint32_t max_depth, unsigned long long 
             KernelSpan span(sc, RT_KCLASS_EXTEND);
             if (sc->counters_on)
                 k_bounce<true><<<sc->grid, 256, sc->smem_bytes, sc->stream>>>(sc->ds, sc->use_smem, in, cnt_in, out, cnt_out, level,
-                                                                              max_depth, sc->map, first_owned, spp, k0, k1,
-                                                                              sc->d_radiance, sc->d_counters);
+                                                                              max_depth, sc->hq.key, k0, k1, sc->d_radiance,
+                                                                              sc->d_counters);
             else
                 k_bounce<false><<<sc->grid, 256, sc->smem_bytes, sc->stream>>>(sc->ds, sc->use_smem, in, cnt_in, out, cnt_out, level,
-                                                                               max_depth, sc->map, first_owned, spp, k0, k1,
-                                                                               sc->d_radiance, sc->d_counters);
+                                                                               max_depth, sc->hq.key, k0, k1, sc->d_radiance,
+                                                                               sc->d_counters);
             continue;
         }
         {
@@ -1415,7 +1502,7 @@ static void launch_bounces(rt_scene* sc, uint32_t max_depth, unsigned long long 
             const bool binned = sc->shade_binned && level < max_depth;
 #define RT_LAUNCH_SHADE(C_, B_)                                                                                              \
     k_shade<C_, B_><<<sc->grid_shade, 256, 0, sc->stream>>>(sc->ds, in, cnt_in, sc->hq, out, cnt_out, level, max_depth, sc->map, \
-                                                            first_owned, spp, k0, k1, sc->d_radiance)
+                                                            0ull, 1u, k0, k1, sc->d_radiance)
             if (sc->counters_on) {
                 if (binned) RT_LAUNCH_SHADE(true, true); else RT_LAUNCH_SHADE(true, false);
             } else {
@@ -1546,13 +1633,13 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
                 RaygenArgs rg;
                 rg.rc = rcd; rg.map = sc->map; rg.first_owned = first; rg.n_paths = npx * spp; rg.spp = spp;
                 rg.k0 = k0; rg.k1 = k1; rg.sample_base = sample_base; rg.radiance = sc->d_radiance; rg.count_out = sc->d_counts;
-                launch_bounces(sc, p->max_depth, first, spp, p->seed, &rg);
+                launch_bounces(sc, p->max_depth, p->seed, &rg);
             } else {
                 {
                     KernelSpan span(sc, RT_KCLASS_RAYGEN);
                     k_raygen<<<sc->grid, 256, 0, sc->stream>>>(rcd, sc->map, first, npx, spp, k0, k1, sc->q[0], sc->d_counts, sc->d_radiance, sc->hq.key, sample_base);
                 }
-                launch_bounces(sc, p->max_depth, first, spp, p->seed);
+                launch_bounces(sc, p->max_depth, p->seed);
             }
             {
                 KernelSpan span(sc, RT_KCLASS_RESOLVE);
@@ -1918,43 +2005,160 @@ int rt_tonemap_rgba8_device(rt_scene* sc, const uint8_t** d_rgba, uint8_t* rgba_
     return RT_OK;
 }
 
+// ---- caller-supplied rays of many pixels (renderer::trace_pixel_samples_group, src/renderer/mod.rs:127-149) -------
+static int check_groups(rt_scene* sc, const rt_ray* rays, uint64_t n_rays, const uint64_t* offsets,
+                        const uint32_t* pixel_index, uint32_t n_groups, uint32_t max_depth, const rt_vec3* means) {
+    if (!sc) return fail(RT_ERR_INVALID, "null scene");
+    if (max_depth > RT_MAX_LEVELS - 2) return fail(RT_ERR_INVALID, "max_depth too large (limit 62)");
+    if (n_groups == 0) return n_rays == 0 ? RT_OK : fail(RT_ERR_INVALID, "rays without groups");
+    if (!offsets || !pixel_index || !means || (n_rays && !rays)) return fail(RT_ERR_INVALID, "null argument");
+    if (offsets[0] != 0) return fail(RT_ERR_INVALID, "offsets[0] must be 0");
+    for (uint32_t g = 0; g < n_groups; g++) {
+        if (offsets[g + 1] < offsets[g]) return fail(RT_ERR_INVALID, "offsets decrease");
+        if (offsets[g + 1] - offsets[g] > 0xFFFFFFFFull) return fail(RT_ERR_INVALID, "a group has 2^32 rays or more");
+    }
+    if (offsets[n_groups] != n_rays) return fail(RT_ERR_INVALID, "offsets[n_groups] must be n_rays");
+    if (sc->rendering) return fail(RT_ERR_STATE, "a frame is in flight");
+    return RT_OK;
+}
+
+struct GroupBatch {
+    uint64_t r0, r1;   // rays [r0, r1) of the call
+    uint32_t g0, g1;   // groups [g0, g1): every group with a ray in the batch (and the empty ones between them)
+    int lane;
+};
+
+// Enqueue a validated call (n_groups > 0) on the library's streams; the main stream ends after every lane.  No host
+// synchronisation.  Whole groups are packed in order into batches of at most RT_B200_BATCH_PATHS paths that alternate
+// over the lanes like a frame's; a group larger than a batch is cut into batch-sized pieces that all run on ONE lane, so
+// its running sum (k_group_resolve) passes from piece to piece in stream order and no lane reads another's partial sum.
+static int trace_groups(rt_scene* sc, const rt_ray* d_rays, uint64_t n_rays, const uint64_t* offsets,
+                        const uint32_t* pixel_index, uint32_t n_groups, uint32_t max_depth, uint64_t seed, rt_vec3* d_means) {
+    uint64_t cap = std::min<uint64_t>(std::max<uint64_t>(env_size("RT_B200_BATCH_PATHS", (size_t)1 << 23), 1), 0xFFFFFFF0ull);
+    int lanes_used = sc->ktiming ? 1 : sc->n_lanes;   // the lane policy of render_start_single
+    if (!sc->lanes_from_env && lanes_used > 2 && (n_rays + cap - 1) / cap < 6) lanes_used = 2;
+    if (lanes_used > 1) {
+        const uint64_t split = (n_rays + lanes_used - 1) / lanes_used;
+        if (split >= ((uint64_t)1 << 20)) cap = std::min(cap, split);
+    }
+    std::vector<GroupBatch> plan;
+    uint64_t lane_paths[RT_MAX_LANES] = {0, 0, 0};
+    uint64_t unit = 0;
+    for (uint32_t g = 0; g < n_groups; unit++) {
+        const int lane = (int)(unit % (uint64_t)lanes_used);
+        const uint32_t g0 = g;
+        const uint64_t r0 = offsets[g];
+        if (offsets[g + 1] - r0 > cap) {
+            for (uint64_t r = r0; r < offsets[g + 1]; r += cap)
+                plan.push_back({r, std::min(r + cap, offsets[g + 1]), g, g + 1, lane});
+            g++;
+        } else {
+            while (g < n_groups && offsets[g + 1] - r0 <= cap) g++;
+            plan.push_back({r0, offsets[g], g0, g, lane});
+        }
+        lane_paths[lane] = std::max(lane_paths[lane], std::min<uint64_t>(offsets[g] - r0, cap));
+    }
+    lanes_used = (int)std::min<uint64_t>((uint64_t)lanes_used, unit);
+    int rc = RT_OK;
+    for (int l = 0; l < lanes_used && rc == RT_OK; l++) {
+        bind_lane(sc, l);
+        rc = ensure_path_buffers(sc, std::max<uint64_t>(lane_paths[l], 1024));
+    }
+    bind_lane(sc, 0);
+    if (rc != RT_OK) return rc;
+    if ((rc = ensure_device_array(sc->d_group_off, sc->group_off_cap, (uint64_t)n_groups + 1)) != RT_OK) return rc;
+    if ((rc = ensure_device_array(sc->d_group_pix, sc->group_pix_cap, n_groups)) != RT_OK) return rc;
+    auto enqueue = [&]() -> int {
+        // the main stream is past the previous call (it waited for every lane) when it overwrites the offsets
+        sc->h_group_off.assign(offsets, offsets + (uint64_t)n_groups + 1);
+        sc->h_group_pix.assign(pixel_index, pixel_index + n_groups);
+        CU(cudaMemcpyAsync(sc->d_group_off, sc->h_group_off.data(), ((uint64_t)n_groups + 1) * sizeof(uint64_t),
+                           cudaMemcpyHostToDevice, sc->stream));
+        CU(cudaMemcpyAsync(sc->d_group_pix, sc->h_group_pix.data(), (uint64_t)n_groups * sizeof(uint32_t),
+                           cudaMemcpyHostToDevice, sc->stream));
+        CU(cudaEventRecord(sc->ev_group_start, sc->stream));
+        for (int l = 1; l < lanes_used; l++) CU(cudaStreamWaitEvent(sc->lanes[l].stream, sc->ev_group_start, 0));
+        for (const GroupBatch& b : plan) {
+            bind_lane(sc, b.lane);
+            const uint32_t n = (uint32_t)(b.r1 - b.r0), ng = b.g1 - b.g0;
+            if (n > 0) {
+                CU(cudaMemsetAsync(sc->d_counts, 0, RT_CNT_WORDS * sizeof(uint32_t), sc->stream));
+                {
+                    KernelSpan span(sc, RT_KCLASS_RAYGEN);
+                    k_load_groups<<<(unsigned)(((uint64_t)n + 255) / 256), 256, 0, sc->stream>>>(
+                        d_rays + b.r0, n, b.r0, sc->d_group_off + b.g0, sc->d_group_pix + b.g0, ng, sc->q[0], sc->d_counts, sc->hq.key);
+                }
+                launch_bounces(sc, max_depth, seed);
+            }
+            {
+                KernelSpan span(sc, RT_KCLASS_RESOLVE);
+                k_group_resolve<<<(unsigned)(((uint64_t)ng + 255) / 256), 256, 0, sc->stream>>>(
+                    sc->d_radiance, b.r0, b.r1, sc->d_group_off + b.g0, ng, d_means + b.g0);
+            }
+        }
+        bind_lane(sc, 0);
+        for (int l = 1; l < lanes_used; l++) {
+            CU(cudaEventRecord(sc->lanes[l].done, sc->lanes[l].stream));
+            CU(cudaStreamWaitEvent(sc->stream, sc->lanes[l].done, 0));
+        }
+        CU(cudaGetLastError());
+        return RT_OK;
+    };
+    rc = enqueue();
+    bind_lane(sc, 0);
+    if (rc != RT_OK) return rc;
+    sc->paths += n_rays;
+    return RT_OK;
+}
+
+int rt_trace_pixel_samples_group_device(rt_scene* sc, const rt_ray* d_rays, uint64_t n_rays, const uint64_t* offsets,
+                                        const uint32_t* pixel_index, uint32_t n_groups, uint32_t max_depth, uint64_t seed,
+                                        rt_vec3* d_means, void* stream) {
+    int rc = check_groups(sc, d_rays, n_rays, offsets, pixel_index, n_groups, max_depth, d_means);
+    if (rc != RT_OK || n_groups == 0) return rc;
+    CU(cudaSetDevice(sc->device));
+    cudaStream_t caller = (cudaStream_t)stream;   // NULL: the library's stream
+    if (caller) {
+        CU(cudaEventRecord(sc->ev_group_in, caller));
+        CU(cudaStreamWaitEvent(sc->stream, sc->ev_group_in, 0));
+    }
+    if ((rc = trace_groups(sc, d_rays, n_rays, offsets, pixel_index, n_groups, max_depth, seed, d_means)) != RT_OK) return rc;
+    if (caller) {   // work the caller queues next (e.g. freeing the rays) runs after the last read of d_rays / write of d_means
+        CU(cudaEventRecord(sc->ev_group_done, sc->stream));
+        CU(cudaStreamWaitEvent(caller, sc->ev_group_done, 0));
+    }
+    if (sc->ktiming) {   // the event pairs of the kernel timing are read once the work has run
+        CU(cudaStreamSynchronize(sc->stream));
+        resolve_spans(sc);
+    }
+    return RT_OK;
+}
+
+int rt_trace_pixel_samples_group(rt_scene* sc, const rt_ray* rays, uint64_t n_rays, const uint64_t* offsets,
+                                 const uint32_t* pixel_index, uint32_t n_groups, uint32_t max_depth, uint64_t seed,
+                                 rt_vec3* means) {
+    int rc = check_groups(sc, rays, n_rays, offsets, pixel_index, n_groups, max_depth, means);
+    if (rc != RT_OK || n_groups == 0) return rc;
+    CU(cudaSetDevice(sc->device));
+    if ((rc = ensure_device_array(sc->d_group_rays, sc->group_rays_cap, n_rays)) != RT_OK) return rc;
+    if ((rc = ensure_device_array(sc->d_group_means, sc->group_means_cap, n_groups)) != RT_OK) return rc;
+    if (n_rays) CU(cudaMemcpyAsync(sc->d_group_rays, rays, n_rays * sizeof(rt_ray), cudaMemcpyHostToDevice, sc->stream));
+    if ((rc = trace_groups(sc, sc->d_group_rays, n_rays, offsets, pixel_index, n_groups, max_depth, seed, sc->d_group_means)) != RT_OK)
+        return rc;
+    CU(cudaMemcpyAsync(means, sc->d_group_means, (uint64_t)n_groups * sizeof(rt_vec3), cudaMemcpyDeviceToHost, sc->stream));
+    const cudaError_t e = cudaStreamSynchronize(sc->stream);
+    resolve_spans(sc);
+    if (e != cudaSuccess) return fail(RT_ERR_CUDA, std::string("trace_pixel_samples_group: ") + cudaGetErrorString(e));
+    return RT_OK;
+}
+
+// the one-group case
 int rt_trace_pixel_samples(rt_scene* sc, const rt_ray* rays, uint32_t n_rays, uint32_t max_depth, uint64_t seed,
                            uint32_t pixel_index, rt_vec3* mean_out) {
     if (!sc || !rays || !mean_out) return fail(RT_ERR_INVALID, "null argument");
     if (n_rays == 0) return fail(RT_ERR_INVALID, "no rays");
-    if (max_depth + 2 > RT_MAX_LEVELS) return fail(RT_ERR_INVALID, "max_depth too large (limit 62)");
-    if (sc->rendering) return fail(RT_ERR_STATE, "a frame is in flight");
-    CU(cudaSetDevice(sc->device));
-    int rc = ensure_path_buffers(sc, std::max<uint64_t>(n_rays, 1024));
-    if (rc != RT_OK) return rc;
-    rt_ray* d_rays = nullptr;
-    Acc* d_acc = nullptr;
-    rt_vec3* d_mean = nullptr;
-    CU(cudaMalloc(&d_rays, n_rays * sizeof(rt_ray)));
-    cudaMalloc(&d_acc, sizeof(Acc));
-    cudaMalloc(&d_mean, sizeof(rt_vec3));
-    cudaMemcpyAsync(d_rays, rays, n_rays * sizeof(rt_ray), cudaMemcpyHostToDevice, sc->stream);
-    cudaMemsetAsync(sc->d_counts, 0, RT_CNT_WORDS * sizeof(uint32_t), sc->stream);
-    k_load_rays<<<(n_rays + 255) / 256, 256, 0, sc->stream>>>(d_rays, n_rays, sc->q[0], sc->d_counts, sc->hq.key, pixel_index);
-    sc->launches++;
-    // a 1-pixel-wide "image" whose only pixel is pixel_index: owned pixel 0 -> (x = pixel_index, y = 0)
-    ShardMap saved = sc->map;
-    ShardMap m;
-    m.width = 0xFFFFFFFFu; m.height = 1; m.tile_w = 0xFFFFFFFFu; m.tile_h = 1; m.tiles_x = 1; m.tiles_y = 1;
-    m.shard_count = 1; m.shard_index = 0; m.skew = 0;
-    sc->map = m;
-    // pixel_of(first_owned + 0) must give x = pixel_index: use first_owned = pixel_index
-    launch_bounces(sc, max_depth, pixel_index, n_rays, seed);
-    sc->map = saved;
-    k_resolve<<<1, 256, 0, sc->stream>>>(sc->d_radiance, 1, n_rays, 0, d_acc, d_mean, false);
-    sc->launches++;
-    cudaMemcpyAsync(mean_out, d_mean, sizeof(rt_vec3), cudaMemcpyDeviceToHost, sc->stream);
-    cudaError_t e = cudaStreamSynchronize(sc->stream);
-    resolve_spans(sc);
-    cudaFree(d_rays); cudaFree(d_acc); cudaFree(d_mean);
-    if (e != cudaSuccess) return fail(RT_ERR_CUDA, std::string("trace_pixel_samples: ") + cudaGetErrorString(e));
-    sc->paths += n_rays;
-    return RT_OK;
+    const uint64_t offsets[2] = {0, n_rays};
+    return rt_trace_pixel_samples_group(sc, rays, n_rays, offsets, &pixel_index, 1, max_depth, seed, mean_out);
 }
 
 // ---- instrumentation ---------------------------------------------------------------------------

@@ -24,8 +24,9 @@ struct HitQueue {
     uint32_t* fq_slot;  // the march queue after k_march_filter: the entries that still have a shape to march, compacted
     uint32_t* fq_mask;
     uint32_t* rq_slot;  // replay queue: degenerate rays (Sphere D == 0, NaN t) that must go through the literal loop
-    uint2* key;         // [path id] the path's RNG key (image pixel index, sample), written once by k_raygen /
-                        // k_load_rays: k_shade reads 8 B instead of redoing six integer divisions per segment
+    uint2* key;         // [path id] the path's RNG key (image pixel index, sample), written once by k_extend's raygen,
+                        // k_raygen or k_load_groups: k_shade / k_bounce read 8 B instead of redoing six integer divisions
+                        // per segment, and caller-supplied rays need no pixel geometry at all
 };
 
 // per-level counters of one batch (zeroed by one memset): live paths, march / replay queue lengths and

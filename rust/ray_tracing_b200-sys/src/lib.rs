@@ -103,6 +103,11 @@ extern "C" {
         n_pixels: *mut u64) -> c_int;
     pub fn rt_trace_pixel_samples(scene: *mut rt_scene, rays: *const rt_ray, n_rays: u32, max_depth: u32,
         seed: u64, pixel_index: u32, mean_out: *mut rt_vec3) -> c_int;
+    pub fn rt_trace_pixel_samples_group(scene: *mut rt_scene, rays: *const rt_ray, n_rays: u64, offsets: *const u64,
+        pixel_index: *const u32, n_groups: u32, max_depth: u32, seed: u64, means: *mut rt_vec3) -> c_int;
+    pub fn rt_trace_pixel_samples_group_device(scene: *mut rt_scene, d_rays: *const rt_ray, n_rays: u64,
+        offsets: *const u64, pixel_index: *const u32, n_groups: u32, max_depth: u32, seed: u64, d_means: *mut rt_vec3,
+        stream: *mut c_void) -> c_int;
     pub fn rt_get_stats(scene: *mut rt_scene, out: *mut rt_stats) -> c_int;
     pub fn rt_reset_stats(scene: *mut rt_scene) -> c_int;
     pub fn rt_set_counters(scene: *mut rt_scene, enabled: c_int) -> c_int;
