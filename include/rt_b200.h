@@ -272,6 +272,46 @@ int rt_render_stop(rt_scene* scene);
 int rt_render_set_accumulate(rt_scene* scene, int enabled);
 int rt_render_accumulated_samples(rt_scene* scene, uint32_t* samples);
 
+/* Adaptive sampling: per-pixel sample counts driven by a noise target.  Every pixel of an adaptive frame equals, bit for
+ * bit, what rt_render_start (or rt_trace_pixel_samples over the camera's primary rays) gives for that pixel at the
+ * sample count it ended with; only the choice of that count is new.
+ *   Luminance of a sample: y = (0.2126*r + 0.7152*g) + 0.0722*b of the path's float radiance widened to double, in that
+ *   order, without FMA.  Σy and Σy² are f64 sums in sample order, kept per pixel next to the rgb sums.
+ *   Schedule: pass 0 gives every pixel min_samples samples.  At each pass boundary, a pixel traced in the previous pass
+ *   holding n samples is tested; it continues when it is not converged and n < samples_number, with
+ *   m = min(n, samples_number - n) more samples numbered n .. n+m-1.  A pixel that stops is never tested again.  So
+ *   the counts lie in {min_samples * 2^j} and {samples_number}.
+ *   Stopping rule (in this operation order):
+ *       mean = Sy / n
+ *       var  = fmax(0, (Syy - Sy*mean) / (n-1))
+ *       se   = sqrt(var / n)
+ *       converged  iff  se <= fmax(rel_error * fabs(mean), abs_error)
+ *   Consequences: min_samples == samples_number (or a huge rel_error) gives the rt_render_start frame bit for bit, plus
+ *   its moments.  The result does not depend on the batch size, the lanes or the order in which pixels are listed:
+ *   every decision is a function of a pixel's own bit-exact sums.  Stopping on the samples themselves biases the frame
+ *   slightly, as any variance-driven sampler does (a pixel whose first samples missed a rare bright path stops early);
+ *   each pixel is still exactly the reference's trace_pixel_samples of its own camera rays. */
+typedef struct rt_adaptive_params {
+    uint32_t min_samples;   /* every pixel gets these; 2 <= min_samples <= samples_number                   */
+    double rel_error;       /* target standard error of the mean luminance, relative to the mean (>= 0)     */
+    double abs_error;       /* absolute floor of that target (>= 0); both finite                            */
+} rt_adaptive_params;
+
+/* Starts an adaptive frame of at most params->samples_number samples per pixel.  Non-blocking like rt_render_start (a
+ * frame in flight is stopped first): the whole frame is enqueued at once and runs without host synchronisation.
+ * rt_render_poll reports done = 0 and leaves the buffer alone until the last pass has resolved, then delivers the whole
+ * frame; rt_render_wait, rt_render_stop, rt_render_device_frame, rt_render_device_result and rt_tonemap_rgba8_device
+ * work on the result.  The frame never continues or seeds a progressive accumulation (rt_render_accumulated_samples
+ * reads 0 after it); rt_stats.paths grows by the sum of the counts once the frame is complete.
+ * RT_ERR_INVALID: a multi-device handle, shard_count > 1, or bad parameters.  RT_ERR_STATE: a scene with more than 32
+ * ray-marched shapes (the fused fallback renders it), as for rt_render_set_accumulate. */
+int rt_render_start_adaptive(rt_scene* scene, const rt_camera* camera, const rt_render_params* params,
+                             const rt_adaptive_params* adaptive);
+/* After a completed unsharded single-device frame (adaptive or not; waits for the frame in flight), per pixel x + y*width:
+ * counts[p] = the samples the pixel holds, moments[2p], moments[2p+1] = Σy, Σy² (adaptive frames only: RT_ERR_STATE
+ * otherwise).  Either output may be NULL. */
+int rt_render_pixel_stats(rt_scene* scene, uint32_t* counts, double* moments);
+
 /* Device-side result of the last started frame, for callers that gather shards over NCCL:
  * FOUR DOUBLES (r, g, b sums; samples) per owned pixel -- the f64 sums themselves, so that the assembled frame
  * equals the unsharded one bit for bit; they were floats before ABI 4, hence the names -- tile-packed in this

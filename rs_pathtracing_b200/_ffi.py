@@ -94,6 +94,14 @@ class RenderParams(C.Structure):
     ]
 
 
+class AdaptiveParams(C.Structure):
+    _fields_ = [
+        ("min_samples", C.c_uint32),
+        ("rel_error", C.c_double),
+        ("abs_error", C.c_double),
+    ]
+
+
 class Stats(C.Structure):
     _fields_ = [
         ("kernel_launches", C.c_uint64),
@@ -141,6 +149,9 @@ CORE_SYMBOLS = {
     "rt_render_stop": (C.c_int, [C.c_void_p]),
     "rt_render_set_accumulate": (C.c_int, [C.c_void_p, C.c_int]),
     "rt_render_accumulated_samples": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint32)]),
+    "rt_render_start_adaptive": (C.c_int, [C.c_void_p, C.POINTER(Camera), C.POINTER(RenderParams),
+                                           C.POINTER(AdaptiveParams)]),
+    "rt_render_pixel_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "rt_render_device_result": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]),
     "rt_shard_float4_count": (C.c_uint64, [C.POINTER(RenderParams), C.c_uint32]),
     "rt_assemble_frame": (C.c_int, [C.c_void_p, C.POINTER(RenderParams), C.POINTER(C.c_void_p), C.c_void_p,

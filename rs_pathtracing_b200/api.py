@@ -256,6 +256,7 @@ class GpuRenderer:
         over all of them by interleaved tiles; the frame is the single-device one, bit for bit"""
         self.scene = scene
         self.depth = depth
+        self.seed = seed
         self.devices = list(devices) if devices else None
         self.device = self.devices[0] if self.devices else device
         scene._device = self.device
@@ -297,6 +298,21 @@ class GpuRenderer:
         while not self.render_step(buf):
             pass
         return buf
+
+    def render_adaptive(self, camera: Camera, width: int, height: int, samples_number: int, min_samples: int,
+                        rel_error: float, abs_error: float = 0.0):
+        """An adaptive frame (rt_render_start_adaptive) on this renderer's device, depth and seed: returns
+        (frame[h, w, 3] float64, counts[h, w] uint32 samples per pixel, std_error[h, w] of each pixel's mean
+        luminance).  Single-device renderers only."""
+        if self.devices and len(self.devices) > 1:
+            raise ValueError("adaptive sampling renders on one device")
+        h = self.scene.device_scene(self.device)
+        params = render_params(width, height, samples_number, self.depth, self.seed)
+        render_start_adaptive(h, camera, params, min_samples, rel_error, abs_error)
+        frame = np.zeros((height, width, 3), np.float64)
+        render_wait(h, frame)
+        counts, moments = render_pixel_stats(h)
+        return frame, counts, standard_error(counts, moments)
 
 
 def tonemap_rgba8(scene: Scene, frame: np.ndarray, device: Optional[int] = None) -> np.ndarray:
@@ -353,8 +369,53 @@ def render_params(width: int, height: int, samples_number: int, max_depth: int, 
     return p
 
 
+_started = {}   # device handle -> (height, width, adaptive) of the last frame started through this module
+
+
+def _handle_key(dev_scene) -> int:
+    return dev_scene.value if isinstance(dev_scene, C.c_void_p) else int(dev_scene)
+
+
 def render_start(dev_scene, camera: Camera, params: RenderParams) -> None:
     _check(_ffi.core().rt_render_start(dev_scene, C.byref(camera), C.byref(params)))
+    _started[_handle_key(dev_scene)] = (params.image.height, params.image.width, False)
+
+
+def render_start_adaptive(dev_scene, camera: Camera, params: RenderParams, min_samples: int, rel_error: float,
+                          abs_error: float = 0.0) -> None:
+    """rt_render_start_adaptive: every pixel gets min_samples samples, then doubles its count while the standard error
+    of its mean luminance exceeds max(rel_error * |mean|, abs_error), up to params.samples_number.  Each pixel equals
+    the render_start frame's pixel at the count it ended with, bit for bit.  Poll / wait deliver the whole frame."""
+    ap = _ffi.AdaptiveParams(min_samples, rel_error, abs_error)
+    _check(_ffi.core().rt_render_start_adaptive(dev_scene, C.byref(camera), C.byref(params), C.byref(ap)))
+    _started[_handle_key(dev_scene)] = (params.image.height, params.image.width, True)
+
+
+def render_pixel_stats(dev_scene, shape=None):
+    """rt_render_pixel_stats of the last completed frame (waits for the frame in flight): counts[h, w] uint32 = samples
+    per pixel, moments[h, w, 2] float64 = (Σy, Σy²) of the samples' luminance, or None when the frame was not adaptive.
+    shape = (height, width) for a frame not started through render_start / render_start_adaptive."""
+    known = _started.get(_handle_key(dev_scene))
+    if shape is None:
+        if known is None:
+            raise ValueError("frame size unknown: pass shape=(height, width)")
+        shape = known[:2]
+    adaptive = known is not None and known[2]
+    h, w = shape
+    counts = np.empty((h, w), np.uint32)
+    moments = np.empty((h, w, 2), np.float64) if adaptive else None
+    _check(_ffi.core().rt_render_pixel_stats(dev_scene, counts.ctypes.data_as(C.c_void_p),
+                                             moments.ctypes.data_as(C.c_void_p) if adaptive else None))
+    return counts, moments
+
+
+def standard_error(counts: np.ndarray, moments: np.ndarray) -> np.ndarray:
+    """the standard error of each pixel's mean luminance, with the stopping rule's arithmetic (rt_b200.h)"""
+    n = counts.astype(np.float64)
+    sy, syy = moments[..., 0], moments[..., 1]
+    mean = sy / n
+    var = np.fmax(0.0, (syy - sy * mean) / (n - 1.0))
+    return np.sqrt(var / n)
 
 
 def render_poll(dev_scene, buffer: Optional[np.ndarray]) -> bool:

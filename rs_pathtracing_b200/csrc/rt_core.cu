@@ -8,6 +8,9 @@
 //   k_resolve           per-pixel mean (trace_pixel_samples) -> (f64 sums, samples) accumulator + f64 frame
 //   k_load_groups       caller-supplied rays of groups of any size -> level-0 queue + RNG keys (trace_pixel_samples_group)
 //   k_group_resolve     per-group mean of caller-supplied rays, continued across the batches of a large group
+//   k_adaptive_select   adaptive frames: stopping rule per pixel at a pass boundary -> list of the pixels that go on
+//   k_raygen_list       adaptive frames: level-0 loader of a refinement batch (listed pixels x the pass's samples)
+//   k_resolve_list      adaptive frames: continue a listed pixel's rgb and luminance sums over its new samples
 //   k_assemble          multi-GPU: gathered tile-packed shards -> frame
 //   k_tonemap           the bins' sqrt / clamp / *256 -> RGBA8
 // Compile with -fmad=false (see rt_math.cuh).
@@ -324,6 +327,24 @@ k_bounce(DevScene S, bool use_smem, PathQueue in, const uint32_t* __restrict__ c
 // busy and only QUEUES the rays whose bounding chord can still beat their best analytic hit; k_march
 // runs those rays densely packed; k_shade finalises the winner, scatters and compacts the survivors.
 
+// The primary ray of sample `sample` of pixel (x, y): MultisamplerRayCaster::next, src/camera/ray_caster.rs:100-118 --
+// the two draws of event 0 of the path's RNG, then the jittered viewport point and Ray::new.  The one place this
+// arithmetic lives: k_extend's raygen and k_raygen_list (adaptive refinement passes) both call it.
+__device__ __forceinline__ D3 camera_ray_dir(const RayCasterDev& rc, uint32_t x, uint32_t y, uint32_t pixel,
+                                            uint32_t sample, uint32_t k0, uint32_t k1) {
+    PathRng rng;
+    rng.k0 = k0; rng.k1 = k1;
+    rng.pixel = pixel;
+    rng.sample = sample;
+    rng.begin_event(0);
+    const double u = rng.next();   // ray_caster.rs:106-107
+    const double v = rng.next();
+    // :109-112
+    const D3 d = rc.left_top + (rc.pixel_resolution * ((double)x + u)) * rc.camera_right -
+                 (rc.pixel_resolution * ((double)y + v)) * rc.camera_up;
+    return normalize(d - rc.camera_position);  // Ray::new
+}
+
 #ifndef RT_EXTEND_MIN_BLOCKS
 #define RT_EXTEND_MIN_BLOCKS 3
 #endif
@@ -360,19 +381,11 @@ k_extend(DevScene S, bool use_smem, PathQueue in, const uint32_t* __restrict__ c
             const uint32_t pl = i / rg.spp, s = i - pl * rg.spp;
             uint32_t x, y;
             if (rg.map.pixel_of(rg.first_owned + pl, x, y)) {
-                PathRng rng;
-                rng.k0 = rg.k0; rng.k1 = rg.k1;
-                rng.pixel = x + y * rg.map.width;
-                rng.sample = rg.sample_base + s;  // (samples of earlier frames of a progressive accumulation come first)
-                rng.begin_event(0);
-                const double u = rng.next();   // ray_caster.rs:106-107
-                const double v = rng.next();
-                // :109-112
-                const D3 d = rg.rc.left_top + (rg.rc.pixel_resolution * ((double)x + u)) * rg.rc.camera_right -
-                             (rg.rc.pixel_resolution * ((double)y + v)) * rg.rc.camera_up;
+                const uint32_t pixel = x + y * rg.map.width;
+                const uint32_t sample = rg.sample_base + s;  // (samples of earlier frames of a progressive accumulation come first)
                 ro = rg.rc.camera_position;
-                rd = normalize(d - rg.rc.camera_position);  // Ray::new
-                hq.key[i] = make_uint2(rng.pixel, rng.sample);
+                rd = camera_ray_dir(rg.rc, x, y, pixel, sample, rg.k0, rg.k1);
+                hq.key[i] = make_uint2(pixel, sample);
                 in.ox[i] = ro.x; in.oy[i] = ro.y; in.oz[i] = ro.z;
                 in.dx[i] = rd.x; in.dy[i] = rd.y; in.dz[i] = rd.z;
                 in.bx[i] = 1.0; in.by[i] = 1.0; in.bz[i] = 1.0;
@@ -596,25 +609,144 @@ k_shade(DevScene S, PathQueue in, const uint32_t* __restrict__ count_in, HitQueu
 struct __align__(16) Acc {
     double r, g, b, n;
 };
+// Adaptive frames (rt_render_start_adaptive) also keep, per pixel, the f64 sums of the samples' luminance and of its
+// square, in sample order: y = (0.2126 r + 0.7152 g) + 0.0722 b of the float radiance widened to double (this file is
+// compiled with -fmad=false, so no product is fused into the sums).
+__device__ __forceinline__ double luminance(float4 v) {
+    return (0.2126 * (double)v.x + 0.7152 * (double)v.y) + 0.0722 * (double)v.z;
+}
+// MOMENTS: also Σy, Σy² into moments[] (pass 0 of an adaptive frame); the plain instantiation is the frame path's
+template <bool MOMENTS>
 __global__ void __launch_bounds__(256)
 k_resolve(const float4* __restrict__ radiance, uint32_t n_pixels, uint32_t spp, unsigned long long first_owned,
-          Acc* __restrict__ accum, rt_vec3* __restrict__ frame_owned, bool add) {
+          Acc* __restrict__ accum, rt_vec3* __restrict__ frame_owned, bool add, double2* __restrict__ moments) {
     uint32_t pl = blockIdx.x * blockDim.x + threadIdx.x;
     if (pl >= n_pixels) return;
     const float4* r = radiance + (size_t)pl * spp;
     double sx = 0.0, sy = 0.0, sz = 0.0, ln = (double)spp;
+    double my = 0.0, myy = 0.0;
     if (add) {  // progressive accumulation: continue the earlier frames' sums, sample by sample (k frames of n
                 // samples then hold the very sum one frame of k*n samples computes)
         const Acc prev = accum[first_owned + pl];
         sx = prev.r; sy = prev.g; sz = prev.b;
         ln += prev.n;
+        if (MOMENTS) {
+            const double2 pm = moments[first_owned + pl];
+            my = pm.x; myy = pm.y;
+        }
     }
     for (uint32_t s = 0; s < spp; s++) {
         float4 v = r[s];
         sx += (double)v.x; sy += (double)v.y; sz += (double)v.z;
+        if (MOMENTS) {
+            const double y = luminance(v);
+            my += y; myy += y * y;
+        }
     }
     accum[first_owned + pl] = Acc{sx, sy, sz, ln};
     frame_owned[first_owned + pl] = rt_vec3{sx / ln, sy / ln, sz / ln};
+    if (MOMENTS) moments[first_owned + pl] = make_double2(my, myy);
+}
+
+// ---- adaptive sampling (rt_render_start_adaptive) -------------------------------------------------------------------
+// The stopping rule, in the operation order the header documents (so that numpy can replay it bit for bit).
+__device__ __forceinline__ bool adaptive_converged(double n, double sum_y, double sum_yy, double rel_error, double abs_error) {
+    const double mean = sum_y / n;
+    const double var = fmax(0.0, (sum_yy - sum_y * mean) / (n - 1.0));
+    const double se = sqrt(var / n);
+    return se <= fmax(rel_error * fabs(mean), abs_error);
+}
+
+// One thread per owned pixel: the pixels that hold n_k samples (the ones traced in the previous pass) are tested; the
+// unconverged ones (while n_k < samples_number, which the host guarantees by not planning a pass past it) are appended
+// to list[] -- in no particular order: every later step of a pixel depends only on its own sums -- and counted in
+// *live.
+__global__ void __launch_bounds__(256)
+k_adaptive_select(const Acc* __restrict__ accum, const double2* __restrict__ moments, uint32_t n_pixels, double n_k,
+                  double rel_error, double abs_error, uint32_t* __restrict__ list, uint32_t* live) {
+    const uint32_t n_round = (n_pixels + 31u) & ~31u;
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < n_round; p += stride) {
+        bool go = false;
+        if (p < n_pixels && accum[p].n == n_k) {
+            const double2 m = moments[p];
+            go = !adaptive_converged(n_k, m.x, m.y, rel_error, abs_error);
+        }
+        const uint32_t slot = queue_append(go, live);
+        if (go) list[slot] = p;
+    }
+}
+
+// Level 0 of batch j of a refinement pass (modelled on k_load_groups): pixels list[base .. base + B) of the *live
+// listed ones, m samples each, numbered n_k .. n_k + m - 1.  Path i takes pixel list[base + i / m] and sample
+// n_k + i % m; the primary ray is the frame's own (camera_ray_dir).  *count_out = the batch's path count, 0 for a
+// batch past the end of the list (every kernel of the batch then exits at once).
+__global__ void __launch_bounds__(256)
+k_raygen_list(RayCasterDev rc, uint32_t width, const uint32_t* __restrict__ list, const uint32_t* __restrict__ live,
+              uint32_t base, uint32_t B, uint32_t m, uint32_t n_k, uint32_t k0, uint32_t k1, PathQueue q,
+              uint2* __restrict__ path_key, uint32_t* count_out) {
+    const uint32_t count = *live;
+    const uint32_t n = count > base ? min(count - base, B) * m : 0u;   // (B * m fits in 32 bits: planned so)
+    if (blockIdx.x == 0 && threadIdx.x == 0) *count_out = n;
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        const uint32_t pl = i / m, s = i - pl * m;
+        const uint32_t pixel = list[base + pl];
+        const uint32_t y = pixel / width, x = pixel - y * width;
+        const uint32_t sample = n_k + s;
+        const D3 rd = camera_ray_dir(rc, x, y, pixel, sample, k0, k1);
+        q.ox[i] = rc.camera_position.x; q.oy[i] = rc.camera_position.y; q.oz[i] = rc.camera_position.z;
+        q.dx[i] = rd.x; q.dy[i] = rd.y; q.dz[i] = rd.z;
+        q.bx[i] = 1.0; q.by[i] = 1.0; q.bz[i] = 1.0;
+        q.pid[i] = i;
+        path_key[i] = make_uint2(pixel, sample);
+    }
+}
+
+// One thread per listed pixel of the batch: continue its (Σrgb, n) and (Σy, Σy²) sample by sample over its m
+// contiguous radiance slots -- the very sums one frame of n + m samples computes -- and write the accumulator, the
+// moments and the frame.  The loads of 16 samples are issued together, as in k_group_resolve.
+__global__ void __launch_bounds__(256)
+k_resolve_list(const float4* __restrict__ radiance, const uint32_t* __restrict__ list, const uint32_t* __restrict__ live,
+               uint32_t base, uint32_t B, uint32_t m, Acc* __restrict__ accum, double2* __restrict__ moments,
+               rt_vec3* __restrict__ frame) {
+    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+    const uint32_t count = *live;
+    if (t >= B || count <= base || t >= count - base) return;
+    const uint32_t p = list[base + t];
+    const Acc prev = accum[p];
+    const double2 pm = moments[p];
+    double sx = prev.r, sy = prev.g, sz = prev.b, my = pm.x, myy = pm.y;
+    const float4* r = radiance + (size_t)t * m;
+    uint32_t s = 0;
+    for (; s + 16 <= m; s += 16) {
+        float4 v[16];
+#pragma unroll
+        for (int j = 0; j < 16; j++) v[j] = r[s + j];
+#pragma unroll
+        for (int j = 0; j < 16; j++) {
+            sx += (double)v[j].x; sy += (double)v[j].y; sz += (double)v[j].z;
+            const double y = luminance(v[j]);
+            my += y; myy += y * y;
+        }
+    }
+    for (; s < m; s++) {
+        const float4 v = r[s];
+        sx += (double)v.x; sy += (double)v.y; sz += (double)v.z;
+        const double y = luminance(v);
+        my += y; myy += y * y;
+    }
+    const double ln = prev.n + (double)m;
+    accum[p] = Acc{sx, sy, sz, ln};
+    moments[p] = make_double2(my, myy);
+    frame[p] = rt_vec3{sx / ln, sy / ln, sz / ln};
+}
+
+// rt_render_pixel_stats: the samples each pixel holds
+__global__ void __launch_bounds__(256)
+k_pixel_counts(const Acc* __restrict__ accum, uint32_t n_pixels, uint32_t* __restrict__ counts) {
+    const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p < n_pixels) counts[p] = (uint32_t)accum[p].n;
 }
 
 // K5b: per-group mean of caller rays (trace_pixel_samples, src/renderer/mod.rs:151-155, per group of :127-149), one
@@ -857,6 +989,18 @@ struct rt_scene {
     std::vector<uint64_t> h_group_off;
     std::vector<uint32_t> h_group_pix;
     cudaEvent_t ev_group_in = nullptr, ev_group_start = nullptr, ev_group_done = nullptr;
+    // adaptive sampling (rt_render_start_adaptive): whether the frame in flight / last completed is adaptive, its
+    // per-pixel (Σy, Σy²), the pixel list of the current refinement pass, the listed count of every pass, the samples
+    // every pass adds (pass 0: min_samples), and the event the lanes wait on after each k_adaptive_select
+    bool adaptive_frame = false;
+    double2* d_moments = nullptr;
+    uint32_t* d_plist = nullptr;
+    uint32_t* d_live = nullptr;
+    uint64_t moments_cap = 0, plist_cap = 0, live_cap = 0;
+    std::vector<uint32_t> adaptive_m;
+    cudaEvent_t ev_adaptive_fork = nullptr;
+    uint32_t* d_pix_counts = nullptr;   // rt_render_pixel_stats
+    uint64_t pix_counts_cap = 0;
 };
 
 template <class T>
@@ -973,7 +1117,8 @@ int rt_scene_create(const rt_scene_desc* d, int device, rt_scene** out) {
     cudaEventCreate(&sc->ev_frame_stop);
     if (cudaEventCreateWithFlags(&sc->ev_group_in, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&sc->ev_group_start, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&sc->ev_group_done, cudaEventDisableTiming) != cudaSuccess)
+        cudaEventCreateWithFlags(&sc->ev_group_done, cudaEventDisableTiming) != cudaSuccess ||
+        cudaEventCreateWithFlags(&sc->ev_adaptive_fork, cudaEventDisableTiming) != cudaSuccess)
         return bail(fail(RT_ERR_CUDA, "cudaEventCreate failed"));
 
     const uint32_t n = d->n_shapes;
@@ -1239,6 +1384,10 @@ void rt_scene_destroy(rt_scene* sc) {
     cudaFree(sc->d_group_pix);
     cudaFree(sc->d_group_means);
     cudaFree(sc->d_group_rays);
+    cudaFree(sc->d_moments);
+    cudaFree(sc->d_plist);
+    cudaFree(sc->d_live);
+    cudaFree(sc->d_pix_counts);
     if (sc->host_stage) cudaFreeHost(sc->host_stage);
     bind_lane(sc, 0);
     for (int l = 0; l < RT_MAX_LANES; l++)
@@ -1259,6 +1408,7 @@ void rt_scene_destroy(rt_scene* sc) {
     if (sc->ev_group_in) cudaEventDestroy(sc->ev_group_in);
     if (sc->ev_group_start) cudaEventDestroy(sc->ev_group_start);
     if (sc->ev_group_done) cudaEventDestroy(sc->ev_group_done);
+    if (sc->ev_adaptive_fork) cudaEventDestroy(sc->ev_adaptive_fork);
     if (sc->stream) cudaStreamDestroy(sc->stream);
     if (sc->copy_stream) cudaStreamDestroy(sc->copy_stream);
     delete sc;
@@ -1541,7 +1691,8 @@ static int ensure_path_buffers(rt_scene* sc, uint64_t need_paths) {
     return RT_OK;
 }
 
-static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_render_params* p);
+static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_render_params* p,
+                               const rt_adaptive_params* ap = nullptr);
 static int render_start_multi(rt_scene* sc, const rt_camera* cam, const rt_render_params* p);
 
 int rt_render_start(rt_scene* sc, const rt_camera* cam, const rt_render_params* p) {
@@ -1553,7 +1704,16 @@ int rt_render_start(rt_scene* sc, const rt_camera* cam, const rt_render_params* 
     return render_start_single(sc, cam, p);
 }
 
-static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_render_params* p) {
+// One refinement pass of an adaptive frame: the listed pixels hold n samples and get m more, B pixels per batch,
+// planned for the worst case of every owned pixel listed (nb batches; the ones past the list's end exit at once).
+struct RefinePass {
+    uint32_t n, m;
+    uint64_t B, nb;
+};
+
+// ap != NULL: an adaptive frame (rt_render_start_adaptive, validated there).  Pass 0 is the frame path with
+// min_samples samples (k_resolve<true> also writes the moments); the refinement passes follow in the same enqueue.
+static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const rt_adaptive_params* ap) {
     if (!sc || !cam || !p) return fail(RT_ERR_INVALID, "null argument");
     if (p->image.width == 0 || p->image.height == 0 || p->samples_number == 0)
         return fail(RT_ERR_INVALID, "empty image or zero samples");
@@ -1568,7 +1728,7 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
     // progressive accumulation: this frame adds its samples to the previous ones when it is the same frame
     // (image, sharding, depth, seed, camera) and nothing was abandoned; otherwise it starts afresh
     uint32_t sample_base = 0;
-    if (sc->accumulate && sc->accumulated_spp > 0 && sc->wavefront && memcmp(&sc->accum_cam, cam, sizeof *cam) == 0 &&
+    if (!ap && sc->accumulate && sc->accumulated_spp > 0 && sc->wavefront && memcmp(&sc->accum_cam, cam, sizeof *cam) == 0 &&
         sc->accum_rp.image.width == p->image.width && sc->accum_rp.image.height == p->image.height &&
         sc->accum_rp.max_depth == p->max_depth && sc->accum_rp.seed == p->seed &&
         (sc->accum_rp.shard_count ? sc->accum_rp.shard_count : 1) == shard_count &&
@@ -1577,13 +1737,29 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
         (uint64_t)sc->accumulated_spp + p->samples_number <= 0xFFFFFFFFull)
         sample_base = sc->accumulated_spp;
     sc->accumulated_spp = 0;  // until this frame is enqueued (an abandoned frame breaks the chain)
+    sc->adaptive_frame = false;
     sc->rp = *p;
     sc->rp.shard_count = shard_count;
     sc->map = make_shard_map(sc->rp, p->shard_index);
     sc->owned_pixels = owned_tiles(sc->map) * sc->map.tile_pixels();
 
-    const uint32_t spp = p->samples_number;
+    const uint32_t spp = ap ? ap->min_samples : p->samples_number;
     uint64_t cap_paths = env_size("RT_B200_BATCH_PATHS", (size_t)1 << 23);
+    // adaptive: the refinement passes n_k -> n_k + min(n_k, samples_number - n_k), B_k = max(1, cap / m_k) pixels per batch
+    std::vector<RefinePass> refine;
+    uint64_t refine_batches = 0, refine_paths = 0;
+    if (ap) {
+        const uint64_t cap = std::min<uint64_t>(std::max<uint64_t>(cap_paths, 1), 0xFFFFFFF0ull);
+        for (uint32_t n = ap->min_samples; n < p->samples_number;) {
+            const uint32_t m = std::min(n, p->samples_number - n);
+            const uint64_t B = std::min<uint64_t>(std::max<uint64_t>(1, cap / m), std::max<uint64_t>(sc->owned_pixels, 1));
+            const uint64_t nb = (sc->owned_pixels + B - 1) / B;
+            refine.push_back({n, m, B, nb});
+            refine_batches = std::max(refine_batches, nb);
+            refine_paths = std::max(refine_paths, B * m);
+            n += m;
+        }
+    }
     uint64_t px_per_batch = std::max<uint64_t>(1, cap_paths / spp);
     // batches alternate between lanes (streams); per-kernel timing wants the launches back to back
     int lanes_used = sc->ktiming ? 1 : sc->n_lanes;
@@ -1598,11 +1774,11 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
     px_per_batch = std::min<uint64_t>(px_per_batch, std::max<uint64_t>(sc->owned_pixels, 1));
     if (px_per_batch * spp > 0xFFFFFFF0ull) return fail(RT_ERR_INVALID, "samples_number too large for one batch");
     const uint64_t n_batches = (sc->owned_pixels + px_per_batch - 1) / px_per_batch;
-    lanes_used = (int)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)lanes_used, n_batches));
+    lanes_used = (int)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)lanes_used, std::max(n_batches, refine_batches)));
     int rc = RT_OK;
     for (int l = 0; l < lanes_used && rc == RT_OK; l++) {
         bind_lane(sc, l);
-        rc = ensure_path_buffers(sc, px_per_batch * spp);
+        rc = ensure_path_buffers(sc, std::max<uint64_t>(px_per_batch * spp, refine_paths));
     }
     bind_lane(sc, 0);
     if (rc != RT_OK) return rc;
@@ -1612,6 +1788,11 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
         CU(cudaMalloc(&sc->d_accum, std::max<uint64_t>(sc->owned_pixels, 1) * sizeof(Acc)));
         CU(cudaMalloc(&sc->d_frame, std::max<uint64_t>(sc->owned_pixels, 1) * sizeof(rt_vec3)));
         sc->frame_capacity = sc->owned_pixels;
+    }
+    if (ap) {
+        if ((rc = ensure_device_array(sc->d_moments, sc->moments_cap, sc->owned_pixels)) != RT_OK) return rc;
+        if ((rc = ensure_device_array(sc->d_plist, sc->plist_cap, sc->owned_pixels)) != RT_OK) return rc;
+        if ((rc = ensure_device_array(sc->d_live, sc->live_cap, std::max<uint64_t>(refine.size(), 1))) != RT_OK) return rc;
     }
     for (Batch& b : sc->batches) cudaEventDestroy(b.done);
     sc->batches.clear();
@@ -1624,6 +1805,7 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
     auto enqueue = [&]() -> int {
         CU(cudaEventRecord(sc->ev_frame_start, sc->stream));  // lane 0 = the main stream
         for (int l = 1; l < lanes_used; l++) CU(cudaStreamWaitEvent(sc->lanes[l].stream, sc->ev_frame_start, 0));
+        if (ap) CU(cudaMemsetAsync(sc->d_live, 0, std::max<size_t>(refine.size(), 1) * sizeof(uint32_t), sc->stream));
         uint64_t batch_no = 0;
         for (uint64_t first = 0; first < sc->owned_pixels; first += px_per_batch, batch_no++) {
             bind_lane(sc, (int)(batch_no % (uint64_t)lanes_used));
@@ -1643,8 +1825,14 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
             }
             {
                 KernelSpan span(sc, RT_KCLASS_RESOLVE);
-                k_resolve<<<(npx + 255) / 256, 256, 0, sc->stream>>>(sc->d_radiance, npx, spp, first, sc->d_accum, sc->d_frame, sample_base != 0);
+                if (ap)
+                    k_resolve<true><<<(npx + 255) / 256, 256, 0, sc->stream>>>(sc->d_radiance, npx, spp, first, sc->d_accum,
+                                                                             sc->d_frame, false, sc->d_moments);
+                else
+                    k_resolve<false><<<(npx + 255) / 256, 256, 0, sc->stream>>>(sc->d_radiance, npx, spp, first, sc->d_accum,
+                                                                              sc->d_frame, sample_base != 0, nullptr);
             }
+            if (ap) continue;   // an adaptive frame is delivered whole, after its last pass
             Batch b;
             b.first_owned = first;
             b.n_pixels = npx;
@@ -1653,10 +1841,56 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
             sc->batches.push_back(b);
             sc->paths += (uint64_t)npx * spp;
         }
+        // adaptive refinement passes: all lanes join the main stream, k_adaptive_select lists the pixels that go on,
+        // the lanes fork again and run the pass's batches.  Nothing waits on the host.
+        const uint32_t width = sc->map.width;
+        for (size_t k = 0; k < refine.size(); k++) {
+            const RefinePass& P = refine[k];
+            bind_lane(sc, 0);
+            for (int l = 1; l < lanes_used; l++) {
+                CU(cudaEventRecord(sc->lanes[l].done, sc->lanes[l].stream));
+                CU(cudaStreamWaitEvent(sc->stream, sc->lanes[l].done, 0));
+            }
+            {
+                KernelSpan span(sc, RT_KCLASS_RESOLVE);
+                const unsigned grid = (unsigned)std::min<uint64_t>((sc->owned_pixels + 255) / 256, (uint64_t)sc->n_sm * 8);
+                k_adaptive_select<<<std::max(grid, 1u), 256, 0, sc->stream>>>(sc->d_accum, sc->d_moments, (uint32_t)sc->owned_pixels,
+                                                                              (double)P.n, ap->rel_error, ap->abs_error,
+                                                                              sc->d_plist, sc->d_live + k);
+            }
+            CU(cudaEventRecord(sc->ev_adaptive_fork, sc->stream));
+            for (int l = 1; l < lanes_used; l++) CU(cudaStreamWaitEvent(sc->lanes[l].stream, sc->ev_adaptive_fork, 0));
+            const uint32_t B = (uint32_t)P.B;
+            const unsigned grid_gen = (unsigned)std::min<uint64_t>((P.B * P.m + 255) / 256, (uint64_t)sc->n_sm * 16);
+            for (uint64_t j = 0; j < P.nb; j++) {
+                bind_lane(sc, (int)(j % (uint64_t)lanes_used));
+                CU(cudaMemsetAsync(sc->d_counts, 0, RT_CNT_WORDS * sizeof(uint32_t), sc->stream));
+                {
+                    KernelSpan span(sc, RT_KCLASS_RAYGEN);
+                    k_raygen_list<<<grid_gen, 256, 0, sc->stream>>>(rcd, width, sc->d_plist, sc->d_live + k, (uint32_t)(j * P.B), B,
+                                                                    P.m, P.n, k0, k1, sc->q[0], sc->hq.key, sc->d_counts);
+                }
+                launch_bounces(sc, p->max_depth, p->seed);
+                {
+                    KernelSpan span(sc, RT_KCLASS_RESOLVE);
+                    k_resolve_list<<<(unsigned)((P.B + 255) / 256), 256, 0, sc->stream>>>(
+                        sc->d_radiance, sc->d_plist, sc->d_live + k, (uint32_t)(j * P.B), B, P.m, sc->d_accum, sc->d_moments,
+                        sc->d_frame);
+                }
+            }
+        }
         bind_lane(sc, 0);
         for (int l = 1; l < lanes_used; l++) {  // the main stream ends the frame after every lane
             CU(cudaEventRecord(sc->lanes[l].done, sc->lanes[l].stream));
             CU(cudaStreamWaitEvent(sc->stream, sc->lanes[l].done, 0));
+        }
+        if (ap) {   // one delivery unit: the whole frame, once the last pass has resolved
+            Batch b;
+            b.first_owned = 0;
+            b.n_pixels = (uint32_t)sc->owned_pixels;
+            CU(cudaEventCreateWithFlags(&b.done, cudaEventDisableTiming));
+            CU(cudaEventRecord(b.done, sc->stream));
+            sc->batches.push_back(b);
         }
         CU(cudaEventRecord(sc->ev_frame_stop, sc->stream));
         CU(cudaGetLastError());
@@ -1667,6 +1901,12 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
     if (rc != RT_OK) return rc;
     sc->rendering = true;
     sc->frame_complete = false;
+    if (ap) {   // rt_stats.paths grows when the frame completes (the listed counts are known on the device only)
+        sc->adaptive_frame = true;
+        sc->adaptive_m.assign(1, spp);
+        for (const RefinePass& P : refine) sc->adaptive_m.push_back(P.m);
+        return RT_OK;
+    }
     if (sc->accumulate && sc->wavefront) {  // (enqueued work always runs to completion: rt_render_stop drains it)
         sc->accumulated_spp = sample_base + spp;
         sc->accum_rp = *p;
@@ -1753,6 +1993,48 @@ int rt_render_set_accumulate(rt_scene* sc, int enabled) {
 int rt_render_accumulated_samples(rt_scene* sc, uint32_t* samples) {
     if (!sc || !samples) return fail(RT_ERR_INVALID, "null argument");
     *samples = sc->accumulated_spp;
+    return RT_OK;
+}
+
+int rt_render_start_adaptive(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const rt_adaptive_params* ap) {
+    if (!sc || !cam || !p || !ap) return fail(RT_ERR_INVALID, "null argument");
+    if (!sc->peers.empty()) return fail(RT_ERR_INVALID, "adaptive sampling: not available on a multi-device handle");
+    if (p->shard_count > 1) return fail(RT_ERR_INVALID, "adaptive sampling renders whole frames (shard_count 0 or 1)");
+    if (ap->min_samples < 2 || ap->min_samples > p->samples_number)
+        return fail(RT_ERR_INVALID, "adaptive sampling needs 2 <= min_samples <= samples_number");
+    if (!(std::isfinite(ap->rel_error) && ap->rel_error >= 0.0) || !(std::isfinite(ap->abs_error) && ap->abs_error >= 0.0))
+        return fail(RT_ERR_INVALID, "adaptive sampling: rel_error and abs_error must be finite and >= 0");
+    if (!sc->wavefront)
+        return fail(RT_ERR_STATE, "adaptive sampling needs the wavefront renderer (at most 32 ray-marched shapes)");
+    sc->multi_active = false;
+    return render_start_single(sc, cam, p, ap);
+}
+
+int rt_render_pixel_stats(rt_scene* sc, uint32_t* counts, double* moments) {
+    if (!sc) return fail(RT_ERR_INVALID, "null scene");
+    if (sc->multi_active) return fail(RT_ERR_STATE, "per-pixel statistics of a multi-device frame are not kept");
+    if (sc->rendering) {
+        CU(cudaSetDevice(sc->device));
+        CU(cudaStreamSynchronize(sc->stream));
+        int done = 0;
+        int rc = rt_render_poll(sc, nullptr, &done);
+        if (rc != RT_OK) return rc;
+    }
+    if (!sc->frame_complete) return fail(RT_ERR_STATE, "no completed frame");
+    if (sc->map.shard_count != 1) return fail(RT_ERR_STATE, "the last frame was one shard of a frame");
+    if (moments && !sc->adaptive_frame) return fail(RT_ERR_STATE, "moments are kept for adaptive frames only");
+    CU(cudaSetDevice(sc->device));
+    const uint64_t n = sc->owned_pixels;   // == width * height: owned order is x + y*width for an unsharded frame
+    if (counts && n) {
+        int rc = ensure_device_array(sc->d_pix_counts, sc->pix_counts_cap, n);
+        if (rc != RT_OK) return rc;
+        k_pixel_counts<<<(unsigned)((n + 255) / 256), 256, 0, sc->copy_stream>>>(sc->d_accum, (uint32_t)n, sc->d_pix_counts);
+        sc->launches++;
+        CU(cudaMemcpyAsync(counts, sc->d_pix_counts, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, sc->copy_stream));
+    }
+    if (moments && n) CU(cudaMemcpyAsync(moments, sc->d_moments, n * sizeof(double2), cudaMemcpyDeviceToHost, sc->copy_stream));
+    const cudaError_t e = cudaStreamSynchronize(sc->copy_stream);
+    if (e != cudaSuccess) return fail(RT_ERR_CUDA, std::string("pixel stats: ") + cudaGetErrorString(e));
     return RT_OK;
 }
 
@@ -1861,6 +2143,15 @@ int rt_render_poll(rt_scene* sc, rt_vec3* buffer, int* done) {
         cudaEventElapsedTime(&ms, sc->ev_frame_start, sc->ev_frame_stop);
         sc->last_frame_ms = ms;
         resolve_spans(sc);
+        if (sc->adaptive_frame) {   // paths = Σ counts: every pixel's pass-0 samples + the listed pixels' of every pass
+            std::vector<uint32_t> live(sc->adaptive_m.size() - 1);
+            if (!live.empty()) {
+                CU(cudaMemcpyAsync(live.data(), sc->d_live, live.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, sc->copy_stream));
+                CU(cudaStreamSynchronize(sc->copy_stream));
+            }
+            sc->paths += sc->owned_pixels * sc->adaptive_m[0];
+            for (size_t k = 0; k < live.size(); k++) sc->paths += (uint64_t)live[k] * sc->adaptive_m[k + 1];
+        }
         sc->rendering = false;
         sc->frame_complete = true;
         *done = 1;

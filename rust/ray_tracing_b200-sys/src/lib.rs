@@ -63,6 +63,8 @@ pub const RT_ISECT_VERIFY: c_int = 2;
 #[repr(C)] #[derive(Clone, Copy, Debug)] pub struct rt_render_params {
     pub image: rt_image_params, pub samples_number: u32, pub max_depth: u32, pub seed: u64,
     pub shard_count: u32, pub shard_index: u32, pub tile_width: u32, pub tile_height: u32 }
+#[repr(C)] #[derive(Clone, Copy, Debug)] pub struct rt_adaptive_params {
+    pub min_samples: u32, pub rel_error: f64, pub abs_error: f64 }
 #[repr(C)] #[derive(Clone, Copy, Default, Debug)] pub struct rt_stats {
     pub kernel_launches: u64, pub paths: u64, pub segments: u64, pub shape_tests: u64, pub cull_tests: u64,
     pub march_steps: u64, pub march_rays: u64, pub march_long_rays: u64, pub march_max_evals: u64,
@@ -93,6 +95,9 @@ extern "C" {
     pub fn rt_render_stop(scene: *mut rt_scene) -> c_int;
     pub fn rt_render_set_accumulate(scene: *mut rt_scene, enabled: c_int) -> c_int;
     pub fn rt_render_accumulated_samples(scene: *mut rt_scene, samples: *mut u32) -> c_int;
+    pub fn rt_render_start_adaptive(scene: *mut rt_scene, camera: *const rt_camera, params: *const rt_render_params,
+        adaptive: *const rt_adaptive_params) -> c_int;
+    pub fn rt_render_pixel_stats(scene: *mut rt_scene, counts: *mut u32, moments: *mut f64) -> c_int;
     pub fn rt_render_device_result(scene: *mut rt_scene, d_accum: *mut *const c_void, n_float4: *mut u64) -> c_int;
     pub fn rt_shard_float4_count(params: *const rt_render_params, shard_index: u32) -> u64;
     pub fn rt_assemble_frame(scene: *mut rt_scene, params: *const rt_render_params, d_shards: *const *const c_void,
