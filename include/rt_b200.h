@@ -231,7 +231,7 @@ int rt_intersect_batch_device(rt_scene* scene, const rt_ray* d_rays, uint64_t n,
 typedef struct rt_render_params {
     rt_image_params image;
     uint32_t samples_number;   /* start_rendering's samples_number                               */
-    uint32_t max_depth;        /* ThreadPoolRenderer::new's depth (ray_color's depth argument)   */
+    uint32_t max_depth;        /* ThreadPoolRenderer::new's depth (ray_color's depth argument); at most 62 */
     uint64_t seed;             /* counter-based RNG key                                          */
     /* image sharding (one process per GPU): this handle renders the tiles k with k % shard_count == shard_index.
      * 1 / 0 = whole image.  Tile NUMBERING (shard_count > 1): with tiles_x = ceil(width / tile_width), tile
@@ -242,7 +242,9 @@ typedef struct rt_render_params {
      * its tiles in increasing k, each tile row-major and padded to tile_width*tile_height at the image border.
      * rt_assemble_frame is the supported way to turn gathered accumulators back into a frame. */
     uint32_t shard_count, shard_index;
-    uint32_t tile_width, tile_height;   /* 0 = default (32 x 32)                                 */
+    uint32_t tile_width, tile_height;   /* 0 = default (32 x 32); tile_width * tile_height must be below 2^32
+                                           (RT_ERR_INVALID from rt_render_start / rt_assemble_frame, and
+                                           rt_shard_float4_count returns 0, otherwise)                        */
 } rt_render_params;
 
 /* Renderer::start_rendering: returns immediately, work proceeds on the library's stream. */

@@ -1,4 +1,6 @@
 // ORACLE — TEST INFRASTRUCTURE ONLY.  C entry points (ctypes) over oracle.cpp.
+#include <algorithm>
+#include <atomic>
 #include <chrono>
 #include <cstring>
 #include <thread>
@@ -196,24 +198,46 @@ void orc_trace_pixel_samples(void* sv, const rt_ray* rays, uint32_t n_rays, uint
     *mean_out = to(acc / (double)n_rays);
 }
 
-// Per-sample radiance of one pixel with the Philox schedule (raygen included): lets a test compare
-// individual GPU paths with the oracle.
+// Per-sample radiance of a list of pixels with the Philox schedule (raygen included), samples sample_base ..
+// sample_base + n_samples - 1 of each: lets a test compare individual GPU paths with the oracle.
+// colors_out[i * n_samples + s] = sample sample_base + s of pixel pixel_index[i] (= x + y * width).  Pixels are
+// spread over `threads` worker threads; every path is computed exactly as orc_render computes it.
+void orc_pixels_sample_colors(void* sv, const rt_camera* cam, uint32_t width, uint32_t height, uint64_t n_pixels,
+                              const uint32_t* pixel_index, uint32_t sample_base, uint32_t n_samples, uint32_t depth,
+                              uint64_t seed, uint32_t threads, rt_vec3* colors_out) {
+    const Scene& sc = *(Scene*)sv;
+    const RayCaster rc = raycaster_new(*cam, rt_image_params{width, height});
+    std::atomic<uint64_t> next{0};
+    auto work = [&]() {
+        PathRng rng;
+        rng.mode = RNG_PHILOX;
+        rng.key[0] = (uint32_t)seed;
+        rng.key[1] = (uint32_t)(seed >> 32);
+        for (uint64_t i = next++; i < n_pixels; i = next++) {
+            const uint32_t p = pixel_index[i], x = p % width, y = p / width;
+            rng.pixel = p;
+            for (uint32_t s = 0; s < n_samples; s++) {
+                rng.sample = sample_base + s;
+                rng.begin_event(0);
+                double u = rng.next(), v = rng.next();
+                Ray r = raycaster_get_ray(rc, (double)x + u, (double)y + v);
+                colors_out[i * n_samples + s] = to(ray_color(sc, false, r, depth, rng, 0, nullptr));
+            }
+        }
+    };
+    if (threads == 0) threads = 1;
+    if (threads > n_pixels) threads = (uint32_t)std::max<uint64_t>(n_pixels, 1);
+    std::vector<std::thread> th;
+    for (uint32_t k = 1; k < threads; k++) th.emplace_back(work);
+    work();
+    for (auto& t : th) t.join();
+}
+
+// The same for one pixel (x, y), samples 0 .. spp - 1, on the calling thread.
 void orc_pixel_sample_colors(void* sv, const rt_camera* cam, uint32_t width, uint32_t height, uint32_t x,
                              uint32_t y, uint32_t spp, uint32_t depth, uint64_t seed, rt_vec3* colors_out) {
-    const Scene& sc = *(Scene*)sv;
-    RayCaster rc = raycaster_new(*cam, rt_image_params{width, height});
-    PathRng rng;
-    rng.mode = RNG_PHILOX;
-    rng.key[0] = (uint32_t)seed;
-    rng.key[1] = (uint32_t)(seed >> 32);
-    rng.pixel = x + y * width;
-    for (uint32_t s = 0; s < spp; s++) {
-        rng.sample = s;
-        rng.begin_event(0);
-        double u = rng.next(), v = rng.next();
-        Ray r = raycaster_get_ray(rc, (double)x + u, (double)y + v);
-        colors_out[s] = to(ray_color(sc, false, r, depth, rng, 0, nullptr));
-    }
+    const uint32_t p = x + y * width;
+    orc_pixels_sample_colors(sv, cam, width, height, 1, &p, 0, spp, depth, seed, 1, colors_out);
 }
 
 uint32_t orc_hardware_threads(void) {

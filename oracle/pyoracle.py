@@ -83,6 +83,8 @@ def lib() -> C.CDLL:
                                           C.c_int, C.POINTER(Vec3)]
     L.orc_pixel_sample_colors.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32,
                                           C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint64, C.c_void_p]
+    L.orc_pixels_sample_colors.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint64, C.c_void_p,
+                                           C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint64, C.c_uint32, C.c_void_p]
     L.orc_hardware_threads.restype = C.c_uint32
     L.orc_shape_hits.argtypes = [C.c_void_p, C.c_void_p, C.c_double, C.c_void_p]
     L.orc_solve_quartic.argtypes = [C.c_double] * 5 + [d16, d16]
@@ -316,4 +318,17 @@ class OracleScene:
         out = np.empty((spp, 3))
         lib().orc_pixel_sample_colors(self._h, C.byref(cam), width, height, x, y, spp, depth, seed,
                                       out.ctypes.data_as(C.c_void_p))
+        return out
+
+    def frame_sample_colors(self, cam: Camera, width, height, spp, depth, seed=0, pixels=None, sample_base=0,
+                            threads=None):
+        """Per-sample FP64 radiance (Philox schedule) of samples sample_base .. sample_base + spp - 1 of the pixels
+        `pixels` (indices x + y*width; None = every pixel): float64[len(pixels), spp, 3]."""
+        if pixels is None:
+            pixels = np.arange(width * height)
+        pix = np.ascontiguousarray(pixels, dtype=np.uint32).reshape(-1)
+        out = np.empty((pix.size, spp, 3))
+        lib().orc_pixels_sample_colors(self._h, C.byref(cam), width, height, pix.size, pix.ctypes.data_as(C.c_void_p),
+                                       sample_base, spp, depth, seed, threads or hardware_threads(),
+                                       out.ctypes.data_as(C.c_void_p))
         return out

@@ -85,10 +85,12 @@ static ShardMap make_shard_map(const rt_render_params& p, uint32_t shard_index) 
         m.tile_w = p.tile_width ? p.tile_width : 32;
         m.tile_h = p.tile_height ? p.tile_height : 32;
     }
-    m.tiles_x = (m.width + m.tile_w - 1) / m.tile_w;
-    m.tiles_y = (m.height + m.tile_h - 1) / m.tile_h;
+    m.tiles_x = (uint32_t)(((uint64_t)m.width + m.tile_w - 1) / m.tile_w);
+    m.tiles_y = (uint32_t)(((uint64_t)m.height + m.tile_h - 1) / m.tile_h);
     return m;
 }
+// tile_pixels() and the owned-order index arithmetic are 32-bit: a tile must hold fewer than 2^32 pixels
+static bool tile_fits(const ShardMap& m) { return (uint64_t)m.tile_w * m.tile_h <= 0xFFFFFFFFull; }
 static uint64_t owned_tiles(const ShardMap& m) {
     uint64_t total = (uint64_t)m.tiles_x * m.tiles_y;
     if (m.shard_index >= total) return 0;
@@ -796,8 +798,10 @@ struct ShardPtrs {
 };
 __global__ void __launch_bounds__(256)
 k_assemble(ShardPtrs shards, ShardMap map0, rt_vec3* __restrict__ frame) {
-    uint32_t x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
-    if (x >= map0.width || y >= map0.height) return;
+    // one-dimensional grid over x + y*w: gridDim.y (at most 65535) would cap the image height
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (uint64_t)map0.width * map0.height) return;
+    const uint32_t y = (uint32_t)(i / map0.width), x = (uint32_t)(i - (uint64_t)y * map0.width);
     uint32_t tx = x / map0.tile_w, ty = y / map0.tile_h;
     uint32_t rot = ((ty % map0.tiles_x) * map0.skew) % map0.tiles_x;        // undo the row rotation of ShardMap
     uint32_t k = ty * map0.tiles_x + (tx + map0.tiles_x - rot) % map0.tiles_x;
@@ -1717,11 +1721,16 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
     if (!sc || !cam || !p) return fail(RT_ERR_INVALID, "null argument");
     if (p->image.width == 0 || p->image.height == 0 || p->samples_number == 0)
         return fail(RT_ERR_INVALID, "empty image or zero samples");
-    if (p->max_depth + 2 > RT_MAX_LEVELS) return fail(RT_ERR_INVALID, "max_depth too large (limit 62)");
+    if (p->max_depth > RT_MAX_LEVELS - 2) return fail(RT_ERR_INVALID, "max_depth too large (limit 62)");
     uint32_t shard_count = p->shard_count ? p->shard_count : 1;
     if (p->shard_index >= shard_count) return fail(RT_ERR_INVALID, "shard_index >= shard_count");
     if (shard_count > 16) return fail(RT_ERR_INVALID, "at most 16 shards");
     if ((uint64_t)p->image.width * p->image.height > 0xFFFFFFFFull) return fail(RT_ERR_INVALID, "image too large");
+    {
+        rt_render_params pp = *p;
+        pp.shard_count = shard_count;
+        if (!tile_fits(make_shard_map(pp, p->shard_index))) return fail(RT_ERR_INVALID, "tile_width * tile_height >= 2^32");
+    }
     CU(cudaSetDevice(sc->device));
     if (sc->rendering) rt_render_stop(sc);
 
@@ -1967,8 +1976,7 @@ static int render_start_multi(rt_scene* sc, const rt_camera* cam, const rt_rende
     ShardPtrs ptrs;
     for (uint32_t k = 0; k < 16; k++) ptrs.p[k] = k == 0 ? sc->d_accum : k < n_dev ? sc->d_peer_acc[k - 1] : nullptr;
     ShardMap m0 = make_shard_map(sp, 0);
-    dim3 grid((m0.width + 255) / 256, m0.height);
-    k_assemble<<<grid, 256, 0, sc->stream>>>(ptrs, m0, sc->d_full_frame);
+    k_assemble<<<(unsigned)((n_px + 255) / 256), 256, 0, sc->stream>>>(ptrs, m0, sc->d_full_frame);
     sc->launches++;
     CU(cudaEventRecord(sc->ev_multi_done, sc->stream));
     CU(cudaGetLastError());
@@ -2225,6 +2233,7 @@ int rt_render_device_result(rt_scene* sc, const void** d_accum, uint64_t* n_floa
 uint64_t rt_shard_float4_count(const rt_render_params* p, uint32_t shard_index) {
     if (!p || p->image.width == 0 || p->image.height == 0) return 0;
     ShardMap m = make_shard_map(*p, shard_index);
+    if (!tile_fits(m)) return 0;
     return owned_tiles(m) * m.tile_pixels();
 }
 
@@ -2232,15 +2241,17 @@ int rt_assemble_frame(rt_scene* sc, const rt_render_params* p, const void* const
     if (!sc || !p || !d_shards || !d_frame) return fail(RT_ERR_INVALID, "null argument");
     uint32_t shard_count = p->shard_count ? p->shard_count : 1;
     if (shard_count > 16) return fail(RT_ERR_INVALID, "at most 16 shards");
-    CU(cudaSetDevice(sc->device));
+    const uint64_t n_px = (uint64_t)p->image.width * p->image.height;
+    if (n_px == 0 || n_px > 0xFFFFFFFFull) return fail(RT_ERR_INVALID, "empty or too large image");
     rt_render_params pp = *p;
     pp.shard_count = shard_count;
     ShardMap m = make_shard_map(pp, 0);
+    if (!tile_fits(m)) return fail(RT_ERR_INVALID, "tile_width * tile_height >= 2^32");
+    CU(cudaSetDevice(sc->device));
     ShardPtrs sp;
     for (uint32_t s = 0; s < 16; s++) sp.p[s] = s < shard_count ? (const Acc*)d_shards[s] : nullptr;
     cudaStream_t st = stream ? (cudaStream_t)stream : sc->stream;
-    dim3 grid((m.width + 255) / 256, m.height);
-    k_assemble<<<grid, 256, 0, st>>>(sp, m, d_frame);
+    k_assemble<<<(unsigned)((n_px + 255) / 256), 256, 0, st>>>(sp, m, d_frame);
     sc->launches++;
     CU(cudaGetLastError());
     return RT_OK;

@@ -22,6 +22,7 @@ from rs_pathtracing_b200 import api
 from oracle import pyoracle as po
 
 from conftest import scene_path
+from test_gpu_frame_edges import check_pixels
 from test_gpu_intersect import TRIO, bench_rays, scene_rays
 
 pytestmark = pytest.mark.gpu
@@ -94,16 +95,10 @@ def test_cfg3_full_resolution_frame_is_schedule_independent(monkeypatch):
             api.render_wait(ds, buf)
         assert np.array_equal(buf, ref), shards
     # random pixels of the full-size frame against the oracle's samples of the same Philox streams
-    osc = po.OracleScene(sc.desc())
     rng = np.random.default_rng(5)
-    bad = 0
-    for x, y in zip(rng.integers(0, w, 96), rng.integers(0, h, 96)):
-        cols = osc.pixel_sample_colors(cam, w, h, int(x), int(y), spp, 8, seed=seed)
-        want = cols.astype(np.float32).astype(np.float64).sum(axis=0) / spp     # radiance is stored as float
-        scale = max(want.max(), 1.0) * spp
-        if (np.abs(ref[y, x] - want) / scale > 1e-7).any():
-            bad += 1
-    assert bad == 0, f"{bad} of 96 probed pixels differ from the oracle"
+    pix = rng.integers(0, w, 96) + rng.integers(0, h, 96) * w
+    cols = po.OracleScene(sc.desc()).frame_sample_colors(cam, w, h, spp, 8, seed, pixels=pix)
+    check_pixels(ref.reshape(-1, 3)[pix], cols, "cfg 3 probes")
 
 
 def test_cfg3_convergence_of_the_full_config():
@@ -170,13 +165,7 @@ def test_cfg4_cfg5_full_resolution_frames(monkeypatch, cfg, w, h, spp, shard_cou
             api.render_start(ds, cam, api.render_params(w, h, spp, depth, seed, shards, s, tile=32))
             api.render_wait(ds, buf)
         assert np.array_equal(buf, ref), shards
-    osc = po.OracleScene(sc.desc())
     rng = np.random.default_rng(11)
-    bad = []
-    for x, y in zip(rng.integers(0, w, 96), rng.integers(0, h, 96)):
-        cols = osc.pixel_sample_colors(cam, w, h, int(x), int(y), spp, depth, seed=seed)
-        want = cols.astype(np.float32).astype(np.float64).sum(axis=0) / spp     # radiance is stored as float
-        scale = max(want.max(), 1.0) * spp
-        if (np.abs(ref[y, x] - want) / scale > 1e-7).any():
-            bad.append((int(x), int(y)))
-    assert not bad, f"{len(bad)} of 96 probed pixels differ from the oracle: {bad}"
+    pix = rng.integers(0, w, 96) + rng.integers(0, h, 96) * w
+    cols = po.OracleScene(sc.desc()).frame_sample_colors(cam, w, h, spp, depth, seed, pixels=pix)
+    check_pixels(ref.reshape(-1, 3)[pix], cols, f"cfg {cfg} probes")

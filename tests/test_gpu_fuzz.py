@@ -10,6 +10,7 @@ import pytest
 import rs_pathtracing_b200 as rt
 from oracle import pyoracle as po
 
+from test_gpu_frame_edges import check_frame
 from test_gpu_intersect import SURFACES, _compare
 
 pytestmark = pytest.mark.gpu
@@ -101,7 +102,4 @@ def test_random_scene_parity(seed):
     assert st.verify_rays == 0 and st.verify_false_culls == 0, f"seed {seed}"
     w, h, spp, depth = 40, 30, 3, 6
     got = rt.GpuRenderer(sc, 12, depth, seed=seed).render(cam, w, h, spp)
-    ref, _ = osc.render(cam, w, h, spp, depth, seed=seed, rng="philox")
-    scale = np.maximum(ref.max(axis=2, keepdims=True), 1.0) * spp
-    bad = (np.abs(got - ref) / scale > 1e-7).any(axis=2)   # float32 rounding of the stored radiance; no pixel exempt
-    assert not bad.any(), f"seed {seed}: {bad.sum()} of {w * h} pixels differ, max {(np.abs(got - ref) / scale).max():.3e}"
+    check_frame(got, osc, cam, w, h, spp, depth, seed, f"random scene {seed}")   # no pixel exempt

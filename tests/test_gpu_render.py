@@ -2,11 +2,8 @@
 
 Two kinds of checks:
   * SAME paths: the oracle run with the shared Philox schedule follows exactly the GPU's paths, so
-    EVERY pixel agrees up to the float32 rounding of the stored per-path radiance: each of the spp samples of a
-    pixel is rounded once (2^-24 relative), so the pixel sum is off by at most 6e-8 x (sum of the samples); the
-    tolerance below is 1e-7 of max(mean, 1) x spp, and NO pixel may exceed it.  (Round 1 allowed 0.2 % of the
-    pixels to deviate; tools/pixel_allowance_probe.py found none on 553 k pixels of all seven scenes, max
-    relative error 1.4e-8 -- profiles/r2c_pixel_allowance_probe.jsonl -- so the allowance is gone.)
+    EVERY pixel agrees with the oracle's samples rounded to float and summed like the GPU sums them, within one
+    float ulp per path (check_pixels, tests/test_gpu_frame_edges.py); NO pixel may exceed it.
   * INDEPENDENT streams: against an oracle render with an unrelated RNG the frames must agree within
     the statistical tolerance of SURVEY §8(d): RMSE <= 1.25 * r0 + 1e-3 with r0 the oracle-vs-oracle
     noise floor, and mean luminance within 0.5 % (+ a noise allowance at the tiny test sizes).
@@ -23,6 +20,7 @@ from rs_pathtracing_b200 import api
 from oracle import pyoracle as po
 
 from conftest import scene_path
+from test_gpu_frame_edges import check_frame
 
 pytestmark = pytest.mark.gpu
 
@@ -30,9 +28,6 @@ pytestmark = pytest.mark.gpu
 def gpu_frame(sc, cam, w, h, spp, depth, seed):
     r = rt.GpuRenderer(sc, 12, depth, seed=seed)
     return r.render(cam, w, h, spp)
-
-
-SAME_PATH_TOL = 1e-7
 
 
 @pytest.mark.parametrize("name,w,h,spp,depth", [
@@ -47,12 +42,7 @@ def test_same_paths_as_oracle(name, w, h, spp, depth):
     sc = rt.Scene.from_file(scene_path(name), random_spheres_seed=1)
     cam = sc.camera()
     got = gpu_frame(sc, cam, w, h, spp, depth, seed=1234)
-    want, _ = po.OracleScene(sc.desc()).render(cam, w, h, spp, depth, seed=1234, rng="philox")
-    scale = np.maximum(want.max(axis=2, keepdims=True), 1.0) * spp   # a pixel is a mean of spp float-rounded samples
-    err = np.abs(got - want) / scale
-    bad = (err > SAME_PATH_TOL).any(axis=2)
-    assert not bad.any(), f"{bad.sum()} of {w*h} pixels differ (max err {err.max():.3e})"
-    assert np.isfinite(got).all()
+    check_frame(got, po.OracleScene(sc.desc()), cam, w, h, spp, depth, 1234, name)
 
 
 def test_same_paths_all_material_and_texture_branches():
@@ -67,10 +57,7 @@ def test_same_paths_all_material_and_texture_branches():
     cam = rt.camera_new(pos, -pos, (0, 1, 0), 1.0, c0.fov_rad)
     w, h, spp, depth = 96, 54, 4, 8
     got = gpu_frame(sc, cam, w, h, spp, depth, seed=99)
-    want, _ = po.OracleScene(sc.desc()).render(cam, w, h, spp, depth, seed=99, rng="philox")
-    scale = np.maximum(want.max(axis=2, keepdims=True), 1.0) * spp
-    err = np.abs(got - want) / scale
-    assert not (err > SAME_PATH_TOL).any(), err.max()
+    check_frame(got, po.OracleScene(sc.desc()), cam, w, h, spp, depth, 99, "cfg 4b")
 
 
 def luminance(img):
@@ -306,8 +293,17 @@ def test_work_counters_match_oracle():
     assert st.kernel_launches > 0
 
 
+def _load_named(name):
+    """a fixture scene, or "march32": 32 ray-marched shapes, the most the wavefront marcher takes (bit 31 of its mask)"""
+    if name == "march32":
+        import json
+        from test_gpu_frame_edges import marched_scene
+        return rt.Scene.from_json(json.dumps(marched_scene(32)), add_random_spheres=False)
+    return rt.Scene.from_file(scene_path(name), random_spheres_seed=1)
+
+
 @pytest.mark.parametrize("name", ["spheres.json", "cornell_box.json", "dupin.json", "detached_materials.json",
-                                  "light_source.json"])
+                                  "light_source.json", "march32"])
 def test_alternative_schedules_give_the_same_frame(monkeypatch, name):
     """the marching result does not depend on how the work is scheduled: the default is the one-ray-per-lane marcher
     k_march; the pooled marcher k_march3 (RT_B200_MARCH=3: a pool of ray records per SM, a queue per phase, dynamic
@@ -319,7 +315,7 @@ def test_alternative_schedules_give_the_same_frame(monkeypatch, name):
     The fused k_bounce draws random_in_unit_sphere with the sequential rejection loop and the default k_shade
     warp-cooperatively, so this also pins the cooperative sampler to the sequential one"""
     w, h, spp, depth, seed = 96, 72, 4, 8, 21
-    sc = rt.Scene.from_file(scene_path(name), random_spheres_seed=1)
+    sc = _load_named(name)
     ref = gpu_frame(sc, sc.camera(), w, h, spp, depth, seed)
     for var, val in (("RT_B200_MARCH", "3"), ("RT_B200_MARCH", "2"), ("RT_B200_FUSED_BOUNCE", "1"),
                      ("RT_B200_MARCH_TUNE", "2,30,3"),
@@ -327,7 +323,7 @@ def test_alternative_schedules_give_the_same_frame(monkeypatch, name):
                      ("RT_B200_DEFER_BOUND", "0"), ("RT_B200_MARCH_FILTER", "0"), ("RT_B200_SHADE_BINNED", "1"),
                      ("RT_B200_SHADE_BINNED", "0")):
         monkeypatch.setenv(var, val)
-        alt = rt.Scene.from_file(scene_path(name), random_spheres_seed=1)
+        alt = _load_named(name)
         got = gpu_frame(alt, alt.camera(), w, h, spp, depth, seed)
         monkeypatch.delenv(var)
         assert np.array_equal(got, ref), var
