@@ -233,6 +233,38 @@ void orc_pixels_sample_colors(void* sv, const rt_camera* cam, uint32_t width, ui
     for (auto& t : th) t.join();
 }
 
+// Per-ray radiance of caller-supplied rays in groups (trace_pixel_samples_group): group g is rays offsets[g] ..
+// offsets[g + 1] - 1, and ray r of it is traced with the RNG key (seed; pixel_index[g], r - offsets[g]), as
+// orc_trace_pixel_samples keys its rays.  The rays are used as given (not normalised).  Groups are spread over
+// `threads` worker threads; colors_out[r] = the FP64 colour of ray r.
+void orc_groups_sample_colors(void* sv, const rt_ray* rays, uint64_t n_rays, const uint64_t* offsets,
+                              const uint32_t* pixel_index, uint64_t n_groups, uint32_t depth, uint64_t seed,
+                              uint32_t threads, rt_vec3* colors_out) {
+    (void)n_rays;
+    const Scene& sc = *(Scene*)sv;
+    std::atomic<uint64_t> next{0};
+    auto work = [&]() {
+        PathRng rng;
+        rng.mode = RNG_PHILOX;
+        rng.key[0] = (uint32_t)seed;
+        rng.key[1] = (uint32_t)(seed >> 32);
+        for (uint64_t g = next++; g < n_groups; g = next++) {
+            rng.pixel = pixel_index[g];
+            for (uint64_t r = offsets[g]; r < offsets[g + 1]; r++) {
+                rng.sample = (uint32_t)(r - offsets[g]);
+                Ray ray{fr(rays[r].origin), fr(rays[r].direction)};
+                colors_out[r] = to(ray_color(sc, false, ray, depth, rng, 0, nullptr));
+            }
+        }
+    };
+    if (threads == 0) threads = 1;
+    if (threads > n_groups) threads = (uint32_t)std::max<uint64_t>(n_groups, 1);
+    std::vector<std::thread> th;
+    for (uint32_t k = 1; k < threads; k++) th.emplace_back(work);
+    work();
+    for (auto& t : th) t.join();
+}
+
 // The same for one pixel (x, y), samples 0 .. spp - 1, on the calling thread.
 void orc_pixel_sample_colors(void* sv, const rt_camera* cam, uint32_t width, uint32_t height, uint32_t x,
                              uint32_t y, uint32_t spp, uint32_t depth, uint64_t seed, rt_vec3* colors_out) {

@@ -85,6 +85,8 @@ def lib() -> C.CDLL:
                                           C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint64, C.c_void_p]
     L.orc_pixels_sample_colors.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint64, C.c_void_p,
                                            C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint64, C.c_uint32, C.c_void_p]
+    L.orc_groups_sample_colors.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint64,
+                                           C.c_uint32, C.c_uint64, C.c_uint32, C.c_void_p]
     L.orc_hardware_threads.restype = C.c_uint32
     L.orc_shape_hits.argtypes = [C.c_void_p, C.c_void_p, C.c_double, C.c_void_p]
     L.orc_solve_quartic.argtypes = [C.c_double] * 5 + [d16, d16]
@@ -313,6 +315,20 @@ class OracleScene:
         lib().orc_trace_pixel_samples(self._h, rays.ctypes.data_as(C.c_void_p), rays.shape[0], depth, seed, pixel_index,
                                       int(use_bvh), C.byref(mean))
         return np.array(mean.tuple())
+
+    def group_sample_colors(self, rays: np.ndarray, offsets, pixel_index, depth, seed=0, threads=None):
+        """Per-ray FP64 radiance of caller rays in groups (trace_pixel_samples_group): ray r of group g, rays
+        offsets[g] .. offsets[g+1]-1, is sample r - offsets[g] of pixel pixel_index[g].  float64[n_rays, 3]."""
+        rays = np.ascontiguousarray(rays, dtype=np.float64).reshape(-1, 6)
+        off = np.ascontiguousarray(offsets, dtype=np.uint64).reshape(-1)
+        pix = np.ascontiguousarray(pixel_index, dtype=np.uint32).reshape(-1)
+        if off.size != pix.size + 1 or off[0] != 0 or int(off[-1]) != rays.shape[0] or (np.diff(off.astype(np.int64)) < 0).any():
+            raise ValueError("offsets must rise from 0 to len(rays), one more than pixel_index")
+        out = np.empty((rays.shape[0], 3))
+        vp = lambda a: a.ctypes.data_as(C.c_void_p)
+        lib().orc_groups_sample_colors(self._h, vp(rays), rays.shape[0], vp(off), vp(pix), pix.size, depth, seed,
+                                       threads or hardware_threads(), vp(out))
+        return out
 
     def pixel_sample_colors(self, cam: Camera, width, height, x, y, spp, depth, seed=0):
         out = np.empty((spp, 3))

@@ -67,3 +67,43 @@ def test_oracle_sample_colours_reproduce_the_oracle_frame():
     assert np.array_equal(osc.frame_sample_colors(cam, w, h, spp, depth, seed, pixels=pix), cols[pix])
     for p in pix:
         assert np.array_equal(osc.pixel_sample_colors(cam, w, h, int(p % w), int(p // w), spp, depth, seed=seed), cols[p])
+
+
+def test_oracle_group_colours_reproduce_the_oracle_trace():
+    """the per-ray colours of caller rays in groups: each group's in-order f64 sum over its count is orc_trace_pixel_samples
+    bit for bit (an empty group: NaN), the camera's own primary rays give frame_sample_colors bit for bit, and the result
+    does not depend on the thread count"""
+    sc = rt.Scene.from_file(scene_path("light_source.json"), random_spheres_seed=1)
+    cam = sc.camera()
+    osc = po.OracleScene(sc.desc())
+    w, h, spp, depth, seed = 7, 5, 3, 6, (1 << 64) - 1
+    rays = np.empty((w * h * spp, 6))
+    for p in range(w * h):
+        for s in range(spp):
+            u, v = po.philox_stream(seed, p, s, 0, 2)
+            rays[p * spp + s] = po.get_ray(cam, w, h, p % w + u, p // w + v)
+    offsets = np.arange(0, w * h * spp + 1, spp, dtype=np.uint64)
+    cols = osc.group_sample_colors(rays, offsets, np.arange(w * h), depth, seed)
+    assert np.array_equal(cols.reshape(w * h, spp, 3), osc.frame_sample_colors(cam, w, h, spp, depth, seed))
+    # ragged groups with empty ones, repeated pixel indices and the key 0xFFFFFFFF; rays not of unit length
+    rng = np.random.default_rng(3)
+    sizes = [0, 1, 4, 0, 0, 9, 2, 0]
+    n = sum(sizes)
+    rays = np.concatenate([np.tile(cam.position.tuple(), (n, 1)), rng.normal(size=(n, 3)) * 2.0], axis=1)
+    offsets = np.concatenate([[0], np.cumsum(sizes)]).astype(np.uint64)
+    pix = np.array([5, 0xFFFFFFFF, 0, 5, 7, 0xFFFFFFFF, 12, 0], np.uint32)
+    cols = osc.group_sample_colors(rays, offsets, pix, depth, seed, threads=1)
+    assert np.isfinite(cols).all() and cols.max() > 0
+    for t in (2, 3, 16):
+        assert np.array_equal(osc.group_sample_colors(rays, offsets, pix, depth, seed, threads=t), cols), t
+    for g, n_g in enumerate(sizes):
+        acc = np.zeros(3)
+        for c in cols[int(offsets[g]):int(offsets[g + 1])]:
+            acc = acc + c
+        with np.errstate(invalid="ignore"):
+            mean = acc / n_g
+        if n_g == 0:
+            assert np.isnan(mean).all()
+            continue
+        want = osc.trace_pixel_samples(rays[int(offsets[g]):int(offsets[g + 1])], depth, seed=seed, pixel_index=int(pix[g]))
+        assert np.array_equal(mean, want), g

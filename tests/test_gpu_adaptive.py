@@ -89,6 +89,28 @@ def _luminance_sums(cols):
     return sy, syy
 
 
+def check_moments(got, cols):
+    """got: a pixel's (sum y, sum y^2) from the device; cols: the oracle's FP64 colours of its samples, in order.  Each path
+    may be one float ulp off per channel (check_pixels' rule), so with f_s the float-rounded colours and
+        dy_s = 0.2126 ulp32(r_s) + 0.7152 ulp32(g_s) + 0.0722 ulp32(b_s)
+    the device's sums must satisfy
+        |sum y - sum y_emu| <= sum dy_s + n ulp64(sum y_emu),
+        |sum y^2 - sum y^2_emu| <= sum (2 |y_s| dy_s + dy_s^2) + n ulp64(sum y^2_emu).
+    Returns True when both sums are bit-identical to the emulated ones."""
+    f32 = np.asarray(cols, dtype=np.float64).astype(np.float32)
+    want = _luminance_sums(cols)
+    sp = np.spacing(np.abs(f32)).astype(np.float64)
+    dy = 0.2126 * sp[:, 0] + 0.7152 * sp[:, 1] + 0.0722 * sp[:, 2]
+    f = f32.astype(np.float64)
+    y = (0.2126 * f[:, 0] + 0.7152 * f[:, 1]) + 0.0722 * f[:, 2]
+    n = len(f)
+    b1 = dy.sum() + n * np.spacing(abs(want[0]))
+    b2 = (2 * np.abs(y) * dy + dy * dy).sum() + n * np.spacing(abs(want[1]))
+    got = tuple(float(v) for v in got)
+    assert abs(got[0] - want[0]) <= b1 and abs(got[1] - want[1]) <= b2, (got, want, (b1, b2))
+    return got == want
+
+
 UNIFORM_CASES = [("spheres.json", ""), ("cornell_box.json", ""), ("detached_materials.json", "4b")]
 
 
@@ -110,18 +132,16 @@ def test_min_equal_to_samples_is_the_frame(name, variant):
     for x, y in zip(rng.integers(0, w, 24), rng.integers(0, h, 24)):
         x, y = int(x), int(y)
         cols = osc.pixel_sample_colors(cam, w, h, x, y, spp, DEPTH, seed=seed)
-        want = _luminance_sums(cols)
-        got = tuple(moments[y, x])
+        same = check_moments(moments[y, x], cols)
         c32 = cols.astype(np.float32).astype(np.float64)
         rgb = np.zeros(3)
         for c in c32:
             rgb = rgb + c
         if np.array_equal(rgb / spp, frame[y, x]):
             # the oracle reproduces this pixel's float radiance exactly: its moments must match bit for bit
-            assert got == want, (x, y, got, want)
-            exact += 1
-        else:   # an f64 difference the float rounding did not absorb: the same paths all the same
-            assert np.allclose(got, want, rtol=1e-6, atol=1e-9), (x, y, got, want)
+            assert same, (x, y, tuple(moments[y, x]), _luminance_sums(cols))
+        exact += same
+    print(f"moments: {24 - exact} of 24 pixels not bit-identical")
     assert exact >= 20, exact
 
 

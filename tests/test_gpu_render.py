@@ -105,12 +105,13 @@ def test_trace_pixel_samples_matches_oracle():
     cam = sc.camera()
     osc = po.OracleScene(sc.desc())
     rng = np.random.default_rng(0)
+    from test_gpu_caller_rays import check_groups
     for pix in (0, 17, 640 * 240 + 320):
         x, y = pix % 640, pix // 640
         rays = np.array([po.get_ray(cam, 640, 480, x + u, y + v) for u, v in rng.uniform(0, 1, (10, 2))])
         got = sc.trace_pixel_samples(rays, 10, seed=5, pixel_index=pix)
-        want = osc.trace_pixel_samples(rays, 10, seed=5, pixel_index=pix)
-        assert np.allclose(got, want, rtol=1e-5, atol=1e-6), (got, want)
+        cols = osc.group_sample_colors(rays, [0, 10], [pix], 10, seed=5)
+        check_groups(got, cols, [0, 10], f"trace_pixel_samples pixel {pix}")
 
 
 def test_renderer_trait_behaviour():
