@@ -122,8 +122,10 @@ enum {
 };
 typedef struct rt_texture {
     uint32_t kind;
-    uint32_t odd, even;   /* child texture indices; children always precede nothing in particular,
-                             but the graph must be acyclic and at most RT_TEX_MAX_DEPTH deep */
+    uint32_t odd, even;   /* child texture indices, in any order of the table.  Textures may share children, but
+                             the graph must be acyclic, and no path down from a texture may cross more than
+                             RT_TEX_MAX_DEPTH checker (CHECKER / UV_CHECKER) nodes before its leaf: 8 checkers
+                             above a leaf are accepted, 9 are RT_ERR_INVALID */
     uint32_t image;
     rt_vec3 color;
 } rt_texture;
@@ -174,7 +176,16 @@ int rt_device_count(void);
 
 /* Upload a flattened Scene to `device` (replaces Arc<RwLock<Scene>> handed to
  * ThreadPoolRenderer::new, src/renderer/step_by_step.rs:37).  The description is copied;
- * the caller may free it afterwards. */
+ * the caller may free it afterwards.
+ * The description is checked before any device is touched (so RT_ERR_INVALID comes before RT_ERR_NO_DEVICE;
+ * rt_scene_create_multi and rt_cull_tree_check apply the same check).  RT_ERR_INVALID when:
+ *   - a table with a non-zero count is NULL (shape arrays, materials, textures, images, noise);
+ *   - a kind is unknown, or a shape's material, a material's texture, a texture's child, image or noise index is
+ *     out of range;
+ *   - the texture graph has a cycle, or a path of more than RT_TEX_MAX_DEPTH checker nodes (see rt_texture);
+ *   - a Perlin permutation entry (perm_x / perm_y / perm_z) is 256 or more;
+ *   - an image has no pixels, no data, or more than SIZE_MAX / 4 texels (4 * width * height bytes must be
+ *     addressable). */
 int rt_scene_create(const rt_scene_desc* desc, int device, rt_scene** out);
 void rt_scene_destroy(rt_scene* scene);
 

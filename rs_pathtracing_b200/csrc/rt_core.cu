@@ -1053,7 +1053,8 @@ static int validate_desc(const rt_scene_desc* d) {
     if (!d) return fail(RT_ERR_INVALID, "null scene description");
     if (d->n_shapes && (!d->kind || !d->flags || !d->inverse || !d->direct || !d->params || !d->material))
         return fail(RT_ERR_INVALID, "scene description: null shape array");
-    if ((d->n_materials && !d->materials) || (d->n_textures && !d->textures) || (d->n_images && !d->images))
+    if ((d->n_materials && !d->materials) || (d->n_textures && !d->textures) || (d->n_images && !d->images) ||
+        (d->n_noise && !d->noise))
         return fail(RT_ERR_INVALID, "scene description: null table");
     for (uint32_t i = 0; i < d->n_shapes; i++) {
         if (d->kind[i] > RT_SHAPE_TORUS) return fail(RT_ERR_INVALID, "scene description: unknown shape kind");
@@ -1077,9 +1078,33 @@ static int validate_desc(const rt_scene_desc* d) {
             return fail(RT_ERR_INVALID, "scene description: child texture index out of range");
         if (t.kind == RT_TEX_IMAGE && t.image >= d->n_images) return fail(RT_ERR_INVALID, "scene description: image index out of range");
     }
-    for (uint32_t i = 0; i < d->n_images; i++)
+    {   // texture_value follows at most RT_TEX_MAX_DEPTH checker edges.  Let H(i) be the number of checker edges on the
+        // longest path down from texture i (infinite on a cycle).  h[i] never exceeds H(i), and after sweep r it is at
+        // least min(r, H(i)); so RT_TEX_MAX_DEPTH + 1 sweeps find every texture that is too deep or on a cycle, without
+        // recursion.
+        std::vector<uint8_t> h(d->n_textures, 0);
+        for (int r = 0; r <= RT_TEX_MAX_DEPTH; r++)
+            for (uint32_t i = 0; i < d->n_textures; i++) {
+                const rt_texture& t = d->textures[i];
+                if (t.kind == RT_TEX_CHECKER || t.kind == RT_TEX_UV_CHECKER)
+                    h[i] = (uint8_t)std::min(1 + std::max(h[t.odd], h[t.even]), RT_TEX_MAX_DEPTH + 1);
+            }
+        for (uint32_t i = 0; i < d->n_textures; i++)
+            if (h[i] > RT_TEX_MAX_DEPTH)
+                return fail(RT_ERR_INVALID, "scene description: texture graph cyclic or deeper than RT_TEX_MAX_DEPTH");
+    }
+    for (uint32_t i = 0; i < d->n_noise; i++) {
+        const rt_perlin& pn = d->noise[i];
+        for (int k = 0; k < 256; k++)
+            if (pn.perm_x[k] > 255 || pn.perm_y[k] > 255 || pn.perm_z[k] > 255)
+                return fail(RT_ERR_INVALID, "scene description: Perlin permutation entry out of range");
+    }
+    for (uint32_t i = 0; i < d->n_images; i++) {
         if (!d->images[i].rgba || !d->images[i].width || !d->images[i].height)
             return fail(RT_ERR_INVALID, "scene description: empty image");
+        if ((uint64_t)d->images[i].width * d->images[i].height > SIZE_MAX / 4)
+            return fail(RT_ERR_INVALID, "scene description: image too large to address");
+    }
     return RT_OK;
 }
 
