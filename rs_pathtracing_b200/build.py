@@ -20,7 +20,7 @@ CSRC = os.path.join(HERE, "csrc")
 CORE_SO = os.path.join(HERE, "librt_b200.so")
 HOST_SO = os.path.join(HERE, "librt_b200_host.so")
 
-CORE_SOURCES = [os.path.join(CSRC, f) for f in ("rt_core.cu", "rt_march_kernels.cu", "rt_march3.cu")]
+CORE_SOURCES = [os.path.join(CSRC, f) for f in ("rt_core.cu", "rt_march_kernels.cu")]
 OBJ_DIR = os.path.join(HERE, "build")
 CORE_HEADERS = [
     os.path.join(CSRC, "rt_queues.cuh"),
@@ -80,7 +80,7 @@ def build_core(force: bool = False) -> str:
     """one object per translation unit, compiled in parallel (no relocatable device code: every kernel is launched
     from its own unit), then linked into librt_b200.so"""
     deps = CORE_HEADERS + [os.path.abspath(__file__)]
-    extra = os.environ.get("RT_B200_NVCC_EXTRA", "").split()   # tuning experiments, e.g. -DRT_M3_R=64
+    extra = os.environ.get("RT_B200_NVCC_EXTRA", "").split()   # tuning experiments, e.g. -DRT_MARCH_MIN_BLOCKS=3
     os.makedirs(OBJ_DIR, exist_ok=True)
     objs, jobs = [], []
     for src in CORE_SOURCES:

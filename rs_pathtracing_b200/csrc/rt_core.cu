@@ -367,7 +367,7 @@ template <bool COUNT, bool RAYGEN>
 __global__ void __launch_bounds__(256, RT_EXTEND_MIN_BLOCKS)
 k_extend(DevScene S, bool use_smem, PathQueue in, const uint32_t* __restrict__ count_in, HitQueue hq,
          uint32_t* march_count, uint32_t* replay_count, DevCounters* g_counters, bool any_hit_suffices,
-         bool defer_bound, RaygenArgs rg) {
+         RaygenArgs rg) {
     Staged st = stage_scene(S, use_smem);
     DevCounters c = {};
     const uint32_t n = RAYGEN ? rg.n_paths : *count_in;
@@ -414,18 +414,10 @@ k_extend(DevScene S, bool use_smem, PathQueue in, const uint32_t* __restrict__ c
             // depth == 0 (renderer/mod.rs:26-27): a hit is black whatever it is, so a ray that already hit an
             // analytic shape needs no marching at the last level
             if (!degenerate && !(any_hit_suffices && winner >= 0)) {
-                for (int k = 0; k < S.n_march; k++) {
-                    if (!cull_pass(cr, S.march_cull[k])) continue;  // the line misses the marching bound
-                    if (defer_bound) {  // k_march_filter runs march_needed, with full warps
-                        mask |= 1u << k;
-                        continue;
-                    }
-                    const int si = S.march_index[k];
-                    D3 o, d;
-                    double start, end_c;
-                    if (march_needed(S, S.inv + 12 * si, S.params + RT_SHAPE_PARAMS * si, ro, rd, best, o, d, start, end_c))
-                        mask |= 1u << k;
-                }
+                // every shape whose marching bound the line touches; the bounding chord (march_needed) is left to
+                // k_march_filter, which runs it with full warps
+                for (int k = 0; k < S.n_march; k++)
+                    if (cull_pass(cr, S.march_cull[k])) mask |= 1u << k;
                 if (COUNT) c.cull_tests += S.n_march;
             }
             if (COUNT) c.segments++;
@@ -887,7 +879,6 @@ struct PathLane {
     HitQueue hq{};
     float4* d_radiance = nullptr;
     uint32_t* d_counts = nullptr;
-    void* d_march_state = nullptr;
     std::vector<void*> qallocs;
     uint64_t path_capacity = 0;
 };
@@ -932,16 +923,6 @@ struct rt_scene {
     uint32_t* d_counts = nullptr;  // RT_CNT_WORDS per batch (reset per batch), see RT_CNT_*
     int grid_extend = 0, grid_march = 0, grid_shade = 0;
     uint32_t kind_mask[6] = {0, 0, 0, 0, 0, 0};  // marched shapes (bits of the march-queue mask) per surface kind
-    void* d_march_state = nullptr;               // k_march2: its records (rt_march_kernels.cu)
-    int grid_march2 = 0, grid_march3 = 0;
-    size_t smem_march3 = 0;
-    bool defer_bound = true;                     // k_extend queues every ray whose line touches a marching bound's ball and leaves the bounding chord (march_needed: 8 % of its instructions at 7 of 32 lanes) to k_march_filter, which runs it with full warps (RT_B200_DEFER_BOUND=0: off; off without the filter)
-    bool march_filter = true;                    // k_march_filter before the marching kernels (RT_B200_MARCH_FILTER=0: off)
-    int march_version = 1;                       // 1: one ray per lane (k_march); RT_B200_MARCH=3: pool of rays per SM + per-phase queues
-                                                 // (k_march3, rt_march3.cu: correct but slower, see profiles/); =2: block-local wavefront (k_march2)
-    int3 march_tune = make_int3(8, 8, 8);        // k_march scheduling thresholds (RT_B200_MARCH_TUNE=a,b,c)
-    int3 march_tune0 = make_int3(32, 8, 8);      // ... at bounce level 0 (RT_B200_MARCH_TUNE0=a,b,c): neighbouring entries are samples of one pixel, so a warp refills only when all of its lanes are done and its 32 rays stay (nearly) in step: k_march -3 % on cornell_box, -4 % on dupin
-    int march_grid_scale = 100;                  // percent of the occupancy grid
     bool wavefront = true;         // extend/march/shade; false = fused k_bounce (more than 32 marched shapes)
     bool shade_binned = false;     // k_shade bins a block's slots by (material kind, texture kind) before shading them
     int n_shade_bins = 0;
@@ -953,7 +934,7 @@ struct rt_scene {
     uint32_t accumulated_spp = 0;
     rt_render_params accum_rp{};
     rt_camera accum_cam{};
-    // the fields q, hq, d_radiance, d_counts, d_march_state, qallocs, path_capacity and `stream` above are
+    // the fields q, hq, d_radiance, d_counts, qallocs, path_capacity and `stream` above are
     // the BOUND lane's (bind_lane swaps them); lanes[0].stream is the main stream
     PathLane lanes[RT_MAX_LANES];
     int n_lanes = 3, cur_lane = 0;
@@ -1283,27 +1264,7 @@ int rt_scene_create(const rt_scene_desc* d, int device, rt_scene** out) {
         return sc->n_sm * std::max(b, 1);
     };
     sc->grid_extend = occ_grid(k_extend<false, true>, 256, sc->smem_bytes);
-    if (const char* tv = getenv("RT_B200_MARCH_TUNE")) {
-        int a = 8, b = 8, c2 = 8, g = 0;
-        if (sscanf(tv, "%d,%d,%d,%d", &a, &b, &c2, &g) >= 3) sc->march_tune = make_int3(std::max(a, 1), std::max(b, 1), std::max(c2, 1));
-        if (g > 0) sc->march_grid_scale = g;
-    }
-    {
-        int per_sm[3] = {1, 1, 1};
-        rt_march_occupancy(per_sm, &sc->smem_march3);
-        sc->grid_march = std::max(sc->n_sm * per_sm[0] * sc->march_grid_scale / 100, 1);
-        sc->grid_march2 = sc->n_sm * per_sm[1];
-        sc->grid_march3 = std::max(sc->n_sm * per_sm[2] * sc->march_grid_scale / 100, 1);
-    }
-    if (const char* tv0 = getenv("RT_B200_MARCH_TUNE0")) {
-        int a = 0, b = 0, c2 = 0;
-        if (sscanf(tv0, "%d,%d,%d", &a, &b, &c2) == 3) sc->march_tune0 = make_int3(std::max(a, 1), std::max(b, 1), std::max(c2, 1));
-    }
-    if (const char* mv = getenv("RT_B200_MARCH")) sc->march_version = std::min(std::max(atoi(mv), 1), 3);
-    if (getenv("RT_B200_MARCH_V2")) sc->march_version = 2;
-    if (const char* mf = getenv("RT_B200_MARCH_FILTER")) sc->march_filter = atoi(mf) != 0;
-    if (!sc->march_filter && !getenv("RT_B200_DEFER_BOUND")) sc->defer_bound = false;   // (measured a net loss without the filter)
-    if (const char* db = getenv("RT_B200_DEFER_BOUND")) sc->defer_bound = atoi(db) != 0;
+    sc->grid_march = sc->n_sm * rt_march_occupancy();
     sc->grid_shade = occ_grid(k_shade<false, true>, 256, 0);
     sc->wavefront = sc->ds.n_march <= 32 && !getenv("RT_B200_FUSED_BOUNCE");
 
@@ -1368,11 +1329,11 @@ static void bind_lane(rt_scene* sc, int i) {
     if (i == sc->cur_lane) return;
     PathLane& a = sc->lanes[sc->cur_lane];
     a.stream = sc->stream; a.q[0] = sc->q[0]; a.q[1] = sc->q[1]; a.hq = sc->hq; a.d_radiance = sc->d_radiance;
-    a.d_counts = sc->d_counts; a.d_march_state = sc->d_march_state; a.qallocs.swap(sc->qallocs);
+    a.d_counts = sc->d_counts; a.qallocs.swap(sc->qallocs);
     a.path_capacity = sc->path_capacity;
     PathLane& b = sc->lanes[i];
     sc->stream = b.stream; sc->q[0] = b.q[0]; sc->q[1] = b.q[1]; sc->hq = b.hq; sc->d_radiance = b.d_radiance;
-    sc->d_counts = b.d_counts; sc->d_march_state = b.d_march_state; sc->qallocs.swap(b.qallocs);
+    sc->d_counts = b.d_counts; sc->qallocs.swap(b.qallocs);
     sc->path_capacity = b.path_capacity;
     sc->cur_lane = i;
 }
@@ -1382,7 +1343,6 @@ static void free_lane_buffers(rt_scene* sc) {  // of the bound lane
     sc->qallocs.clear();
     cudaFree(sc->d_radiance); sc->d_radiance = nullptr;
     cudaFree(sc->d_counts); sc->d_counts = nullptr;
-    cudaFree(sc->d_march_state); sc->d_march_state = nullptr;
     sc->path_capacity = 0;
 }
 
@@ -1600,6 +1560,12 @@ static int alloc_queue(rt_scene* sc, PathQueue& q, uint64_t cap) {
 }
 
 
+// k_march's scheduling thresholds (rt_march_kernels.cu: refill, attempt vote, literal burst)
+static const int3 march_tune = {8, 8, 8};
+// ... at bounce level 0: neighbouring entries are samples of one pixel, so a warp refills only when all of its lanes
+// are done and its 32 rays stay (nearly) in step: k_march -3 % on cornell_box, -4 % on dupin
+static const int3 march_tune0 = {32, 8, 8};
+
 // enqueue the bounce loop for paths already in q[0] (count in d_counts[0]); no host sync
 static void launch_bounces(rt_scene* sc, uint32_t max_depth, uint64_t seed, const RaygenArgs* raygen = nullptr) {
     uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
@@ -1629,8 +1595,7 @@ static void launch_bounces(rt_scene* sc, uint32_t max_depth, uint64_t seed, cons
             if (gen) rg = *raygen;
 #define RT_LAUNCH_EXTEND(C_, G_)                                                                                        \
     k_extend<C_, G_><<<sc->grid_extend, 256, sc->smem_bytes, sc->stream>>>(sc->ds, sc->use_smem, in, cnt_in, sc->hq, mcount, \
-                                                                           rcount, sc->d_counters, level == max_depth,     \
-                                                                           sc->defer_bound, rg)
+                                                                           rcount, sc->d_counters, level == max_depth, rg)
             if (sc->counters_on) {
                 if (gen) RT_LAUNCH_EXTEND(true, true); else RT_LAUNCH_EXTEND(true, false);
             } else {
@@ -1640,31 +1605,27 @@ static void launch_bounces(rt_scene* sc, uint32_t max_depth, uint64_t seed, cons
         }
         if (sc->ds.n_march > 0) {
             KernelSpan span(sc, RT_KCLASS_MARCH);
-            if (sc->march_filter) {   // the miss proof for every queued (ray, shape) pair, with full warps
+            uint32_t* fcount = sc->d_counts + RT_CNT_FILTERED + level;
+            {   // the bounding chord and the miss proof for every queued (ray, shape) pair, with full warps
                 MarchLaunch fl;
                 fl.ds = sc->ds; fl.in = in; fl.hq = sc->hq; fl.march_count = mcount; fl.counters = sc->d_counters;
                 fl.count = sc->counters_on; fl.stream = sc->stream; fl.grid_filter = sc->n_sm * 8;
-                fl.filtered_count = sc->d_counts + RT_CNT_FILTERED + level;
+                fl.filtered_count = fcount;
                 rt_launch_march_filter(fl);
                 sc->launches++;
             }
-            // the marching kernels read the compacted queue the filter wrote
+            // k_march reads the compacted queue the filter wrote
             HitQueue mhq = sc->hq;
-            const uint32_t* mq_count = mcount;
-            if (sc->march_filter) {
-                mhq.mq_slot = sc->hq.fq_slot;
-                mhq.mq_mask = sc->hq.fq_mask;
-                mq_count = sc->d_counts + RT_CNT_FILTERED + level;
-            }
+            mhq.mq_slot = sc->hq.fq_slot;
+            mhq.mq_mask = sc->hq.fq_mask;
             for (int kind = 0; kind < 6; kind++) {
                 if (!sc->kind_mask[kind]) continue;
                 uint32_t* head = sc->d_counts + RT_CNT_HEAD + kind * RT_MAX_LEVELS + level;
                 MarchLaunch ml;
                 ml.ds = sc->ds; ml.kind = kind; ml.kind_mask = sc->kind_mask[kind]; ml.in = in; ml.hq = mhq;
-                ml.march_count = mq_count; ml.head = head; ml.counters = sc->d_counters; ml.count = sc->counters_on;
-                ml.stream = sc->stream; ml.version = sc->march_version; ml.grid1 = sc->grid_march; ml.grid2 = sc->grid_march2;
-                ml.grid3 = sc->grid_march3; ml.smem3 = sc->smem_march3; ml.tune = level == 0 ? sc->march_tune0 : sc->march_tune; ml.march_state = sc->d_march_state;
-                ml.prefiltered = sc->march_filter; ml.grid_filter = 0;
+                ml.march_count = fcount; ml.head = head; ml.counters = sc->d_counters; ml.count = sc->counters_on;
+                ml.stream = sc->stream; ml.grid = sc->grid_march; ml.tune = level == 0 ? march_tune0 : march_tune;
+                ml.grid_filter = 0;
                 rt_launch_march(ml);
                 sc->launches++;
             }
@@ -1714,8 +1675,6 @@ static int ensure_path_buffers(rt_scene* sc, uint64_t need_paths) {
         CU(cudaMalloc(&p, need_paths * sizeof(uint2))); sc->qallocs.push_back(p); sc->hq.key = (uint2*)p;
     }
     if (!sc->d_counts) CU(cudaMalloc(&sc->d_counts, RT_CNT_WORDS * sizeof(uint32_t)));
-    if (!sc->d_march_state && sc->ds.n_march > 0 && sc->march_version == 2)
-        CU(cudaMalloc(&sc->d_march_state, rt_march2_state_bytes(sc->grid_march2)));
     sc->path_capacity = need_paths;
     return RT_OK;
 }

@@ -457,8 +457,7 @@ struct Marcher {
     unsigned long long n;  // surface evaluations (statistics, and the spin guard)
     // skip machinery
     double step0;
-    bool skip_ok, have_poly;
-    bool plan_miss_ok;   // attempt_plan may declare the ray a miss (off in the kernels that keep t in a record)
+    bool skip_ok;
     bool local_model;    // P is the model re-expanded around the level-0 crossing (refine_model)
     int cooldown, backoff;
     RayPoly<DEG> P;
@@ -478,18 +477,15 @@ struct Marcher {
         sd = step * d;  // `step * dir`, loop-invariant until the step changes
         cooldown = 0;
         backoff = 4;
-        have_poly = false;
         if (PROF) prof[0] = prof[1] = prof[2] = prof[3] = prof[4] = prof[5] = prof[6] = prof[7] = 0;
         // skipping pays when the chord holds many steps (NaN-proof comparisons)
         skip_ok = (G == G) && G < 1e300 && (F == F) && F < 1e300 && step > 0.0 && (end - start) > 64.0 * step &&
                   (end - start) < 1e300;
-        plan_miss_ok = true;
         local_model = false;
         if (skip_ok) {
             // the model along the ray, expanded around the first sample; covers every later sample of the ray
             expand_ray<KIND>(q, p, d, t, end, (end - t) + 4.0 * step0, G, F, P);
             n += 2;  // cost of the expansion in evaluation-equivalents (statistics only)
-            have_poly = true;
 #ifndef RT_MARCH_NO_MISS_PROOF
             // (3): no sample of this ray can see an event -> None.  The samples the loop TESTS are n = 1, 2, ... (the
             // first one only lends its sign to the comparison with the second), sample n sits at tau_n = t_n - t0 with
@@ -554,7 +550,7 @@ struct Marcher {
     // nothing changed except cooldown / skip_ok, so that phase() now answers RT_PHASE_LITERAL.
     // The attempt is split in three so that k_march can run the middle part -- the exact advance of the
     // four accumulators t, p.x, p.y, p.z, whose loops over binades are the most divergent code of the
-    // marcher -- cooperatively, one accumulator per lane (coop_advance in rt_core.cu):
+    // marcher -- cooperatively, one accumulator per lane (coop_advance in rt_march_kernels.cu):
     //   attempt_plan():  how many iterations m can provably be skipped (0: none; cooldown is set)
     //   [advance t, p by m steps exactly]
     //   attempt_land():  the reference's `r = next` at the landing sample + the model self-check
@@ -572,8 +568,7 @@ struct Marcher {
         bool more;            // stopped at the stage limit, not at the |g| = M boundary: attempt again after landing
     };
 #define RT_MARCH_MAX_STAGES 6
-    // plan_begin + plan_hop until it returns false + plan_end == attempt_plan (the hop loop is resumable so that
-    // a kernel can interleave it with other work).
+    // attempt_plan = plan_begin, then plan_hop until it returns false, then plan_end.
     //
     // The hops are planned in STAGES.  A stage bounds |g''| over its whole span, so from far away the bound
     // is loose and the hops stall (or the span, limited to twice the Newton distance, ends) well before the
@@ -629,12 +624,6 @@ struct Marcher {
         local_model = true;
     }
     __host__ __device__ __forceinline__ void plan_begin(Plan& pl) {
-        if (!have_poly) {   // (begin() expands when skip_ok; kept for marchers rebuilt from records)
-            double tau_hi = (end - t) + 4.0 * step0;
-            expand_ray<KIND>(q, p, d, t, end, tau_hi, G, F, P);
-            n += 2;
-            have_poly = true;
-        }
         double(&s)[DEG + 1] = pl.s;
         const double abs_step = fabs(step);
         const double dir = step > 0.0 ? 1.0 : -1.0;
@@ -676,7 +665,7 @@ struct Marcher {
 #ifndef RT_MARCH_NO_MISS_PROOF
         // (3) again, from wherever the ray is at level 0: let the hops run on to the end of the stretch the remaining
         // samples can fall on; if they get there the ray is a miss and nothing has to be advanced
-        if (plan_miss_ok && it == 0 && dir > 0.0) {
+        if (it == 0 && dir > 0.0) {
             const double L = miss_span(t);
             if (tau + L <= P.tau_hi && miss_drift_ok(L)) {
                 pl.span_limit = L;

@@ -1,9 +1,7 @@
-// rt_march_kernels.cu -- K3 of the wavefront renderer, first and second generation: exact-skip marching of the
-// queued (ray, marched shapes) entries with ONE RAY PER LANE (k_march: persistent lanes, phase voting, cooperative
-// exact advance) and the block-local wavefront experiment k_march2.  The default is k_march3 (rt_march3.cu: a pool
-// of rays per warp, every variable-length loop with dynamic pick-up); these two stay selectable
-// (RT_B200_MARCH=1 / 2) as bit-identity cross-checks (tests/test_gpu_render.py) and as the baseline the profiles
-// compare against.  Compile with -fmad=false (see rt_math.cuh).
+// rt_march_kernels.cu -- K3 of the wavefront renderer: the miss proof for every queued (ray, marched shape) pair
+// with full warps (k_march_filter), then exact-skip marching of what it leaves with ONE RAY PER LANE (k_march:
+// persistent lanes, phase voting, cooperative exact advance), one launch per surface kind.  Compile with
+// -fmad=false (see rt_math.cuh).
 #include <cuda_runtime.h>
 #include <cstdio>
 
@@ -85,7 +83,7 @@ __device__ __forceinline__ void coop_advance(unsigned jumping, long long mj, dou
 template <int KIND, bool COUNT>
 __global__ void __launch_bounds__(128, RT_MARCH_MIN_BLOCKS)
 k_march(DevScene S, uint32_t kind_mask, PathQueue in, HitQueue hq, const uint32_t* __restrict__ march_count,
-        uint32_t* head, DevCounters* g_counters, int3 tune, bool prefiltered) {
+        uint32_t* head, DevCounters* g_counters, int3 tune) {
     DevCounters c = {};
     const uint32_t n = *march_count;
     const unsigned FULL = 0xffffffffu;
@@ -132,10 +130,10 @@ k_march(DevScene S, uint32_t kind_mask, PathQueue in, HitQueue hq, const uint32_
         }
 #endif
         // ---- fill: lanes without a ray in flight fetch queue entries and start their shapes, again and again
-        //      (the `continue` below), until (nearly) every lane holds a ray that really has to be marched.  Most
-        //      entries never get that far -- the chord is clipped away by the best hit (march_needed), or begin()
-        //      proves the miss from the Bernstein hull -- so this is a filter that runs with many lanes at once, and
-        //      what it leaves in the lanes is the expensive minority.
+        //      (the `continue` below), until (nearly) every lane holds a ray that really has to be marched.  Entries
+        //      whose chord the best hit now clips away (march_needed: an earlier kind pass may have lowered it since
+        //      k_march_filter ran) never get that far, so what is left in the lanes is the expensive minority.  (No
+        //      hull proof in begin(): k_march_filter has tried it for every entry of this queue.)
         //      (Written as part of the one outer loop on purpose: the same logic as a nested `for (;;)` with two
         //      breaks hung k_march<Cushion> / k_march<Dupin> on the second frame of a scene -- deterministically per
         //      binary, gone with any instrumentation; profiles/README.md, r2n.  Keep the nesting shallow.) ---------
@@ -178,10 +176,10 @@ k_march(DevScene S, uint32_t kind_mask, PathQueue in, HitQueue hq, const uint32_
                     D3 o, d;
                     double start, end_c;
                     if (march_needed(S, S.inv + 12 * shape, q, ro, rd, best, o, d, start, end_c)) {
-                        m.begin(q, o, d, start, end_c, S.march_G[k], S.march_F[k], !prefiltered);
+                        m.begin(q, o, d, start, end_c, S.march_G[k], S.march_F[k], false);
                         marching = true;
                         if (COUNT) c.march_rays++;
-                        if (m.phase() == RT_PHASE_END) finish_shape();   // a proven miss (or an empty range)
+                        if (m.phase() == RT_PHASE_END) finish_shape();   // an empty range, or depth 0
                     }
                 }
                 // again, as long as the filter leaves lanes empty (the votes at the top decide)
@@ -228,340 +226,18 @@ k_march(DevScene S, uint32_t kind_mask, PathQueue in, HitQueue hq, const uint32_
     if (COUNT) flush_counters(c, g_counters);
 }
 
-// K3, experimental alternative (RT_B200_MARCH_V2=1): the same marching as a block-local wavefront.
-// Measured 27 % SLOWER than k_march on cornell_box (5.4 vs 4.3 ms per 4 Mi paths): the divergence that
-// matters is inside the phases (trip counts of advance_exact and of the hop loop), not between them.
-// k_march keeps one ray per lane; its lanes sit in different phases of their rays (start / exact-jump
-// attempt / literal steps / finish) and a warp executes the union of those instruction streams: ~10 of 32
-// lanes busy, 5.7x slower than a warp marching 32 copies of ONE ray (tools/march_coherence_probe.py).
-// k_march2 keeps the rays of a block in RECORDS instead (256 B each, in the block's slice of a global
-// buffer that stays L2-resident), RT_M2_SLOTS of them for RT_M2_THREADS threads, and runs the phases one
-// after the other over compacted lists of the records that want them, so that every warp executes one
-// phase with (nearly) all lanes busy.  The arithmetic per ray -- Marcher, rt_march.cuh -- is unchanged, so
-// the result is bit-identical to k_march and to the reference's loop.
-#define RT_M2_THREADS 256
-#define RT_M2_SLOTS 1024
-#define RT_M2_LITERAL_BURST 8
-struct __align__(16) MarchRec {
-    // [0] t [1] r [2] step [3..5] p [6..8] d [9] start [10] end [11] best so far
-    // [12..18] P.c [19] P.t0 [20..22] P.p0 [23] P.tau_hi [24] P.err0 [25] P.drift1
-    // [26] (it | cooldown << 8 | backoff << 16 | flags << 24, n)   [27] (path slot, queue entry)
-    // [28] (remaining shape mask, winner)   [29] (march-list index k or -1, shape index)
-    // [30] [31] work-profile counters (COUNT only)
-    double v[32];
-};
-enum { RT_M2_FREE = 0, RT_M2_TRANS = 1, RT_M2_ATTEMPT = 2, RT_M2_LITERAL = 3 };
-#define RT_M2_FLAG_SKIP_OK 1u
-#define RT_M2_FLAG_HAVE_POLY 2u
-
-__device__ __forceinline__ uint2 m2_get_u2(const MarchRec* rec, int i) {
-    return *reinterpret_cast<const uint2*>(&rec->v[i]);
-}
-__device__ __forceinline__ void m2_set_u2(MarchRec* rec, int i, uint32_t x, uint32_t y) {
-    *reinterpret_cast<uint2*>(&rec->v[i]) = make_uint2(x, y);
-}
-
-// the marcher's loop state (everything literal() and phase() touch)
-template <int KIND, bool COUNT>
-__device__ __forceinline__ void m2_load_core(const DevScene& S, const MarchRec* rec, Marcher<KIND, COUNT>& m, int& k) {
-    const double2* r2 = reinterpret_cast<const double2*>(rec->v);
-    const double2 a0 = r2[0], a1 = r2[1], a2 = r2[2], a3 = r2[3], a4 = r2[4], a5 = r2[5];
-    m.t = a0.x; m.r = a0.y; m.step = a1.x; m.p = mk(a1.y, a2.x, a2.y);
-    m.d = mk(a3.x, a3.y, a4.x); m.start = a4.y; m.end = a5.x;
-    const uint2 w = m2_get_u2(rec, 26), ks = m2_get_u2(rec, 29);
-    m.it = (int)(w.x & 0xffu);
-    m.cooldown = (int)((w.x >> 8) & 0xffu);
-    m.backoff = (int)((w.x >> 16) & 0xffu);
-    m.skip_ok = ((w.x >> 24) & RT_M2_FLAG_SKIP_OK) != 0;
-    m.have_poly = ((w.x >> 24) & RT_M2_FLAG_HAVE_POLY) != 0;
-    m.plan_miss_ok = true;   // (m2_store_core keeps the t = +inf a proven miss leaves behind)
-    m.local_model = false;   // (the record keeps the model of the chord's start: a refinement plan re-expands every time)
-    m.n = w.y;
-    k = (int)ks.x;
-    m.q = S.params + RT_SHAPE_PARAMS * (int)ks.y;
-    m.step0 = m.q[1];
-    m.depth = (int)m.q[2];
-    m.G = S.march_G[k];
-    m.F = S.march_F[k];
-    m.sd = m.step * m.d;
-    if (COUNT) {
-        const uint2 p0 = m2_get_u2(rec, 30), p1 = m2_get_u2(rec, 31);
-        m.prof[0] = p0.x; m.prof[1] = p0.y; m.prof[2] = p1.x; m.prof[3] = p1.y; m.prof[4] = m.prof[5] = m.prof[6] = m.prof[7] = 0;
-    }
-}
-template <int KIND, bool COUNT>
-__device__ __forceinline__ void m2_store_core(MarchRec* rec, const Marcher<KIND, COUNT>& m, bool with_ray) {
-    double2* r2 = reinterpret_cast<double2*>(rec->v);
-    r2[0] = make_double2(m.t, m.r);
-    r2[1] = make_double2(m.step, m.p.x);
-    r2[2] = make_double2(m.p.y, m.p.z);
-    if (with_ray) {
-        r2[3] = make_double2(m.d.x, m.d.y);
-        r2[4] = make_double2(m.d.z, m.start);
-        rec->v[10] = m.end;
-    }
-    const uint32_t flags = (m.skip_ok ? RT_M2_FLAG_SKIP_OK : 0u) | (m.have_poly ? RT_M2_FLAG_HAVE_POLY : 0u);
-    const uint32_t nn = m.n > 0xffffffffull ? 0xffffffffu : (uint32_t)m.n;
-    m2_set_u2(rec, 26, (uint32_t)m.it | ((uint32_t)m.cooldown << 8) | ((uint32_t)m.backoff << 16) | (flags << 24), nn);
-    if (COUNT) {
-        m2_set_u2(rec, 30, m.prof[0], m.prof[1]);
-        m2_set_u2(rec, 31, m.prof[2], m.prof[3]);
-    }
-}
-template <int KIND, bool COUNT>
-__device__ __forceinline__ void m2_load_poly(const MarchRec* rec, Marcher<KIND, COUNT>& m) {
-    constexpr int DEG = Marcher<KIND, COUNT>::DEG;
-    const double2* r2 = reinterpret_cast<const double2*>(rec->v);
-    double c[8];
-#pragma unroll
-    for (int i = 0; i < 4; i++) {
-        const double2 v = r2[6 + i];
-        c[2 * i] = v.x;
-        c[2 * i + 1] = v.y;
-    }
-#pragma unroll
-    for (int i = 0; i <= DEG; i++) m.P.c[i] = c[i];
-    m.P.t0 = c[7];
-    const double2 b0 = r2[10], b1 = r2[11], b2 = r2[12];
-    m.P.p0 = mk(b0.x, b0.y, b1.x);
-    m.P.tau_hi = b1.y; m.P.err0 = b2.x; m.P.drift1 = b2.y;
-}
-template <int KIND, bool COUNT>
-__device__ __forceinline__ void m2_store_poly(MarchRec* rec, const Marcher<KIND, COUNT>& m) {
-    constexpr int DEG = Marcher<KIND, COUNT>::DEG;
-    double c[8];
-#pragma unroll
-    for (int i = 0; i < 7; i++) c[i] = i <= DEG ? m.P.c[i] : 0.0;
-    c[7] = m.P.t0;
-    double2* r2 = reinterpret_cast<double2*>(rec->v);
-#pragma unroll
-    for (int i = 0; i < 4; i++) r2[6 + i] = make_double2(c[2 * i], c[2 * i + 1]);
-    r2[10] = make_double2(m.P.p0.x, m.P.p0.y);
-    r2[11] = make_double2(m.P.p0.z, m.P.tau_hi);
-    r2[12] = make_double2(m.P.err0, m.P.drift1);
-}
-__device__ __forceinline__ uint8_t m2_phase_of(int ph) {
-    return ph == RT_PHASE_ATTEMPT ? RT_M2_ATTEMPT : ph == RT_PHASE_LITERAL ? RT_M2_LITERAL : RT_M2_TRANS;
-}
-
-template <int KIND, bool COUNT>
-__global__ void __launch_bounds__(RT_M2_THREADS, 2)
-k_march2(DevScene S, uint32_t kind_mask, PathQueue in, HitQueue hq, const uint32_t* __restrict__ march_count,
-         uint32_t* head, MarchRec* state_all, DevCounters* g_counters) {
-    __shared__ uint8_t s_phase[RT_M2_SLOTS];
-    __shared__ uint16_t s_list[4][RT_M2_SLOTS];   // [RT_M2_FREE] = free slots
-    __shared__ uint32_t s_len[4];
-    __shared__ uint32_t s_base, s_take, s_next;
-    __shared__ int s_exhausted;
-    __shared__ unsigned char s_owner_all[RT_M2_THREADS];
-    unsigned char* const s_owner = s_owner_all + (threadIdx.x & ~31u);
-    DevCounters c = {};
-    MarchRec* state = state_all + (size_t)blockIdx.x * RT_M2_SLOTS;
-    const uint32_t n = *march_count;
-    const int tid = threadIdx.x;
-    // records this block works with: an even share of the queue, so that every SM gets work
-    uint32_t cap = (n + gridDim.x - 1) / gridDim.x;
-    cap = (cap + 31u) & ~31u;
-    cap = min((uint32_t)RT_M2_SLOTS, max((uint32_t)RT_M2_THREADS, cap));
-    for (uint32_t i = tid; i < cap; i += RT_M2_THREADS) s_phase[i] = RT_M2_FREE;
-    if (tid == 0) s_exhausted = n == 0;
-    __syncthreads();
-    for (;;) {
-        // ---- classify the records by the phase they want next -------------------------------------------
-        if (tid < 4) s_len[tid] = 0;
-        if (tid == 4) s_next = 0;
-        __syncthreads();
-        for (uint32_t i = tid; i < cap; i += RT_M2_THREADS) {
-            const int ph = s_phase[i];
-            s_list[ph][atomicAdd(&s_len[ph], 1u)] = (uint16_t)i;
-        }
-        __syncthreads();
-        const uint32_t n_free = s_len[RT_M2_FREE];
-        const uint32_t live = cap - n_free;
-        // ---- refill the free records from the march queue ------------------------------------------------
-        uint32_t take = 0;
-        if (!s_exhausted && n_free > 0 && (live == 0 || 4 * n_free >= cap)) {  // (block-uniform condition)
-            if (tid == 0) {
-                const uint32_t base = atomicAdd(head, n_free);
-                s_base = base;
-                s_take = base < n ? min(n_free, n - base) : 0u;
-                if (base + n_free >= n) s_exhausted = 1;
-            }
-            __syncthreads();
-            take = s_take;
-            for (uint32_t i = tid; i < take; i += RT_M2_THREADS) {
-                const uint32_t slot = s_list[RT_M2_FREE][i];
-                const uint32_t j = s_base + i;
-                const uint32_t pslot = hq.mq_slot[j];
-                MarchRec* rec = state + slot;
-                rec->v[11] = hq.t[pslot];
-                m2_set_u2(rec, 27, pslot, j);
-                m2_set_u2(rec, 28, hq.mq_mask[j] & kind_mask, (uint32_t)hq.index[pslot]);
-                m2_set_u2(rec, 29, 0xffffffffu, 0u);
-                s_phase[slot] = RT_M2_TRANS;
-                s_list[RT_M2_TRANS][atomicAdd(&s_len[RT_M2_TRANS], 1u)] = (uint16_t)slot;
-            }
-            __syncthreads();
-        }
-        if (live + take == 0 && s_exhausted) break;
-        // ---- one pass over the three lists, 32 records at a time; warps take chunks dynamically so that
-        //      different warps run different phases at the same time (attempts, the longest, first) ---------
-        const uint32_t n_att = s_len[RT_M2_ATTEMPT], n_lit = s_len[RT_M2_LITERAL], n_trans = s_len[RT_M2_TRANS];
-        const uint32_t c_att = (n_att + 31u) >> 5, c_lit = (n_lit + 31u) >> 5, c_trans = (n_trans + 31u) >> 5;
-        const uint32_t n_chunks = c_att + c_lit + c_trans;
-        for (;;) {
-            uint32_t chunk = 0;
-            if ((tid & 31) == 0) chunk = atomicAdd(&s_next, 1u);
-            chunk = __shfl_sync(0xffffffffu, chunk, 0);
-            if (chunk >= n_chunks) break;
-            if (chunk < c_att) {
-                // ---- exact-jump attempt (the whole warp takes part: coop_advance is warp-collective) --------
-                const uint32_t idx = chunk * 32u + (tid & 31);
-                const bool active = idx < n_att;
-                const uint32_t slot = active ? s_list[RT_M2_ATTEMPT][idx] : 0u;
-                MarchRec* rec = state + slot;
-                Marcher<KIND, COUNT> m;
-                typename Marcher<KIND, COUNT>::Plan pl;
-                long long mj = 0;
-                bool had_poly = true;
-                if (active) {
-                    int k;
-                    m2_load_core(S, rec, m, k);
-                    had_poly = m.have_poly;
-                    if (had_poly) m2_load_poly(rec, m);
-                    mj = m.attempt_plan(pl);
-                } else {
-                    m.t = m.step = 0.0;
-                    m.p = m.sd = mk(0.0, 0.0, 0.0);
-                }
-                const unsigned jumping = __ballot_sync(0xffffffffu, mj > 0);
-                if (jumping) {
-                    double nt = 0.0;
-                    D3 np = mk(0.0, 0.0, 0.0);
-                    coop_advance(jumping, mj, m.t, m.step, m.p, m.sd, nt, np, s_owner, []() {});
-                    if (mj > 0) m.attempt_land(pl, nt, np);
-                }
-                if (active) {
-                    m2_store_core(rec, m, false);
-                    if (!had_poly) m2_store_poly(rec, m);
-                    s_phase[slot] = m2_phase_of(m.phase());
-                }
-            } else if (chunk < c_att + c_lit) {
-                // ---- the reference's literal steps -----------------------------------------------------------
-                const uint32_t idx = (chunk - c_att) * 32u + (tid & 31);
-                if (idx < n_lit) {
-                    const uint32_t slot = s_list[RT_M2_LITERAL][idx];
-                    MarchRec* rec = state + slot;
-                    Marcher<KIND, COUNT> m;
-                    int k;
-                    m2_load_core(S, rec, m, k);
-#pragma unroll 1
-                    for (int rep = 0; rep < RT_M2_LITERAL_BURST; rep++) {
-                        m.literal();
-                        if (m.phase() != RT_PHASE_LITERAL) break;
-                    }
-                    m2_store_core(rec, m, false);
-                    s_phase[slot] = m2_phase_of(m.phase());
-                }
-            } else {
-                // ---- transition: finish a marched shape, start the next one, or retire the record -----------
-                const uint32_t idx = (chunk - c_att - c_lit) * 32u + (tid & 31);
-                if (idx < n_trans) {
-                    const uint32_t slot = s_list[RT_M2_TRANS][idx];
-                    MarchRec* rec = state + slot;
-                    const uint2 pe = m2_get_u2(rec, 27), mw = m2_get_u2(rec, 28), ks = m2_get_u2(rec, 29);
-                    const uint32_t pslot = pe.x, entry = pe.y;
-                    uint32_t mask = mw.x;
-                    int winner = (int)mw.y;
-                    double best = rec->v[11];
-                    bool retired = false;
-                    Marcher<KIND, COUNT> m;
-                    if (ks.x != 0xffffffffu) {  // a shape has just been marched to its end
-                        int k;
-                        m2_load_core(S, rec, m, k);
-                        const int shape = (int)ks.y;
-                        if (COUNT) {
-                            c.march_steps += m.n;
-                            for (int q = 0; q < 8; q++) c.march_prof[q] += m.prof[q];
-                            if (m.n > 2048) c.march_long_rays++;
-                            if (m.n > c.march_max_evals) c.march_max_evals = m.n;
-                        }
-                        if (m.finish() == RT_MARCH_DONE && !(m.t < 0.001)) {  // ray_marching.rs:55 with max_t = +inf
-                            const double t = m.t;
-                            if (t != t) {  // NaN candidate: replay now, and hide the entry from later kind passes
-                                replay_brute(S, in, hq, pslot);
-                                hq.mq_mask[entry] = 0;
-                                retired = true;
-                            } else if (t < best || (t == best && shape > winner)) {
-                                best = t;
-                                winner = shape;
-                            }
-                        }
-                    }
-                    bool started = false;
-                    while (!retired && mask != 0 && !started) {
-                        const int k = __ffs(mask) - 1;
-                        mask &= mask - 1;
-                        const int shape = S.march_index[k];
-                        const double* q = S.params + RT_SHAPE_PARAMS * shape;
-                        D3 ro = mk(in.ox[pslot], in.oy[pslot], in.oz[pslot]);
-                        D3 rd = mk(in.dx[pslot], in.dy[pslot], in.dz[pslot]);
-                        D3 o, d;
-                        double start, end_c;
-                        if (march_needed(S, S.inv + 12 * shape, q, ro, rd, best, o, d, start, end_c)) {
-                            m.begin(q, o, d, start, end_c, S.march_G[k], S.march_F[k]);
-                            if (COUNT) c.march_rays++;
-                            m2_store_core(rec, m, true);
-                            if (m.have_poly) m2_store_poly(rec, m);   // begin() expands the model when skip_ok
-                            m2_set_u2(rec, 29, (uint32_t)k, (uint32_t)shape);
-                            s_phase[slot] = m2_phase_of(m.phase());
-                            started = true;
-                        }
-                    }
-                    if (started) {
-                        rec->v[11] = best;
-                        m2_set_u2(rec, 28, mask, (uint32_t)winner);
-                    } else {
-                        if (!retired) {
-                            hq.t[pslot] = best;
-                            hq.index[pslot] = winner;
-                        }
-                        s_phase[slot] = RT_M2_FREE;
-                    }
-                }
-            }
-        }
-        __syncthreads();
-    }
-    if (COUNT) flush_counters(c, g_counters);
-}
-
-
-void rt_march_occupancy(int per_sm[3], size_t* smem3) {
+int rt_march_occupancy() {
     int b = 0;
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_march<RT_SURF_HEART, false>, 128, 0);
-    per_sm[0] = std::max(b, 1);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, k_march2<RT_SURF_HEART, false>, RT_M2_THREADS, 0);
-    per_sm[1] = std::max(b, 1);
-    per_sm[2] = rt_march3_occupancy(smem3);
+    return std::max(b, 1);
 }
-
-size_t rt_march2_state_bytes(int grid2) { return (size_t)grid2 * RT_M2_SLOTS * sizeof(MarchRec); }
 
 template <int K_>
 static void launch_kind(const MarchLaunch& ml) {
-    if (ml.version == 2) {
-        if (ml.count)
-            k_march2<K_, true><<<ml.grid2, RT_M2_THREADS, 0, ml.stream>>>(ml.ds, ml.kind_mask, ml.in, ml.hq, ml.march_count, ml.head,
-                                                                         (MarchRec*)ml.march_state, ml.counters);
-        else
-            k_march2<K_, false><<<ml.grid2, RT_M2_THREADS, 0, ml.stream>>>(ml.ds, ml.kind_mask, ml.in, ml.hq, ml.march_count, ml.head,
-                                                                          (MarchRec*)ml.march_state, ml.counters);
-    } else if (ml.count) {
-        k_march<K_, true><<<ml.grid1, 128, 0, ml.stream>>>(ml.ds, ml.kind_mask, ml.in, ml.hq, ml.march_count, ml.head, ml.counters, ml.tune, ml.prefiltered);
-    } else {
-        k_march<K_, false><<<ml.grid1, 128, 0, ml.stream>>>(ml.ds, ml.kind_mask, ml.in, ml.hq, ml.march_count, ml.head, ml.counters, ml.tune, ml.prefiltered);
-    }
+    if (ml.count)
+        k_march<K_, true><<<ml.grid, 128, 0, ml.stream>>>(ml.ds, ml.kind_mask, ml.in, ml.hq, ml.march_count, ml.head, ml.counters, ml.tune);
+    else
+        k_march<K_, false><<<ml.grid, 128, 0, ml.stream>>>(ml.ds, ml.kind_mask, ml.in, ml.hq, ml.march_count, ml.head, ml.counters, ml.tune);
 }
 
 // K3a: the miss proof of rt_march.cuh (3) for every queued (ray, marched shape) pair, one entry per thread, before the
@@ -641,10 +317,6 @@ void rt_launch_march_filter(const MarchLaunch& ml) {
 }
 
 void rt_launch_march(const MarchLaunch& ml) {
-    if (ml.version == 3) {
-        rt_launch_march3(ml);
-        return;
-    }
     switch (ml.kind) {
         case RT_SURF_HEART: launch_kind<RT_SURF_HEART>(ml); break;
         case RT_SURF_SINE: launch_kind<RT_SURF_SINE>(ml); break;

@@ -1,5 +1,5 @@
 // Path-state queues of the wavefront renderer and the helpers shared by its translation units
-// (rt_core.cu: raygen / extend / shade / resolve + the C ABI; rt_march3.cu: the pooled marching kernel).
+// (rt_core.cu: raygen / extend / shade / resolve + the C ABI; rt_march_kernels.cu: the marching kernels).
 #pragma once
 #include "rt_scene.cuh"
 
@@ -93,8 +93,8 @@ static __device__ __noinline__ void replay_brute(const DevScene& S, const PathQu
 }
 
 
-// ---- the marching kernels live in their own translation units (rt_march_kernels.cu: k_march, k_march2;
-//      rt_march3.cu: k_march3); rt_core.cu launches them through this interface -----------------------------
+// ---- the marching kernels live in their own translation unit (rt_march_kernels.cu: k_march_filter, k_march);
+//      rt_core.cu launches them through this interface -----------------------------------------------------------
 struct MarchLaunch {
     DevScene ds;
     int kind;                 // surface kind of this pass (one launch per kind present in the scene)
@@ -106,19 +106,11 @@ struct MarchLaunch {
     DevCounters* counters;
     bool count;
     cudaStream_t stream;
-    int version;              // 1 k_march, 2 k_march2, 3 k_march3
-    int grid1, grid2, grid3;
-    size_t smem3;
+    int grid;                 // k_march's CTAs
     int3 tune;
-    void* march_state;        // k_march2's records
-    bool prefiltered;         // k_march_filter has run on this queue: k_march need not try the hull proof again
     int grid_filter;
     uint32_t* filtered_count; // k_march_filter: length of the compacted queue it writes (hq.fq_slot / fq_mask)
 };
 void rt_launch_march(const MarchLaunch& ml);
 void rt_launch_march_filter(const MarchLaunch& ml);   // once per level, before the per-kind launches
-void rt_launch_march3(const MarchLaunch& ml);
-// CTAs per SM of k_march / k_march2 / k_march3 and k_march3's dynamic shared memory per CTA
-void rt_march_occupancy(int per_sm[3], size_t* smem3);
-int rt_march3_occupancy(size_t* smem3);
-size_t rt_march2_state_bytes(int grid2);
+int rt_march_occupancy();                             // CTAs per SM of k_march

@@ -13,8 +13,7 @@ fn main() {
                "-diag-suppress", "20014", "-shared", "-cudart", "static", "-o"])
         .arg(&lib)
         .arg(csrc.join("rt_core.cu"))              // C ABI, raygen / extend / shade / resolve / assemble / tonemap
-        .arg(csrc.join("rt_march_kernels.cu"))     // k_march, k_march2
-        .arg(csrc.join("rt_march3.cu"))            // k_march3
+        .arg(csrc.join("rt_march_kernels.cu"))     // k_march_filter, k_march
         .status()
         .expect("nvcc not found");
     assert!(status.success(), "nvcc failed");

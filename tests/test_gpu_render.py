@@ -306,23 +306,19 @@ def _load_named(name):
 @pytest.mark.parametrize("name", ["spheres.json", "cornell_box.json", "dupin.json", "detached_materials.json",
                                   "light_source.json", "march32"])
 def test_alternative_schedules_give_the_same_frame(monkeypatch, name):
-    """the marching result does not depend on how the work is scheduled: the default is the one-ray-per-lane marcher
-    k_march; the pooled marcher k_march3 (RT_B200_MARCH=3: a pool of ray records per SM, a queue per phase, dynamic
-    pick-up inside every variable-length loop), the block-local wavefront marcher k_march2 (RT_B200_MARCH=2), other
-    k_march voting thresholds and the fused k_bounce (RT_B200_FUSED_BOUNCE) reproduce the default frame bit for bit; so do the flat list without its
-    staged records (RT_B200_NO_FLAT_REC), marching-bound tests done by k_extend instead of k_march_filter
-    (RT_B200_DEFER_BOUND=0) and the marcher without the filter kernel in front of it (RT_B200_MARCH_FILTER=0: the miss
-    proof then runs inside k_march).
+    """the result does not depend on how the work is scheduled: the fused k_bounce (RT_B200_FUSED_BOUNCE), the
+    linear scan without the cull tree (RT_B200_NO_CULL_TREE), the literal marching loop (RT_B200_NO_MARCH_SKIP), the
+    flat list without its staged records (RT_B200_NO_FLAT_REC) and k_shade with and without its binned queue
+    (RT_B200_SHADE_BINNED) reproduce the default wavefront frame (k_extend, k_march_filter, k_march, k_shade) bit for
+    bit.
     The fused k_bounce draws random_in_unit_sphere with the sequential rejection loop and the default k_shade
     warp-cooperatively, so this also pins the cooperative sampler to the sequential one"""
     w, h, spp, depth, seed = 96, 72, 4, 8, 21
     sc = _load_named(name)
     ref = gpu_frame(sc, sc.camera(), w, h, spp, depth, seed)
-    for var, val in (("RT_B200_MARCH", "3"), ("RT_B200_MARCH", "2"), ("RT_B200_FUSED_BOUNCE", "1"),
-                     ("RT_B200_MARCH_TUNE", "2,30,3"),
+    for var, val in (("RT_B200_FUSED_BOUNCE", "1"),
                      ("RT_B200_NO_CULL_TREE", "1"), ("RT_B200_NO_MARCH_SKIP", "1"), ("RT_B200_NO_FLAT_REC", "1"),
-                     ("RT_B200_DEFER_BOUND", "0"), ("RT_B200_MARCH_FILTER", "0"), ("RT_B200_SHADE_BINNED", "1"),
-                     ("RT_B200_SHADE_BINNED", "0")):
+                     ("RT_B200_SHADE_BINNED", "1"), ("RT_B200_SHADE_BINNED", "0")):
         monkeypatch.setenv(var, val)
         alt = _load_named(name)
         got = gpu_frame(alt, alt.camera(), w, h, spp, depth, seed)
