@@ -325,6 +325,26 @@ int rt_render_start_adaptive(rt_scene* scene, const rt_camera* camera, const rt_
  * otherwise).  Either output may be NULL. */
 int rt_render_pixel_stats(rt_scene* scene, uint32_t* counts, double* moments);
 
+/* A frame whose pixel x + y*width gets counts[x + y*width] samples, numbered 0 .. counts[p]-1; every pixel equals, bit for
+ * bit, the rt_render_start pixel of the same camera, seed and depth at samples_number = counts[p] (and the adaptive
+ * frame's pixel wherever that frame stopped at counts[p]).  counts covers the WHOLE image on every shard.  A pixel with
+ * count 0 is 0/0 = NaN, like an empty group.  params->samples_number is the cap (>= 1): a count above it is
+ * RT_ERR_INVALID.  counts is read before the call returns.
+ *   - Non-blocking like rt_render_start; a frame in flight is stopped first.
+ *   - rt_render_poll delivers finished pixels progressively, as for rt_render_start; rt_render_wait, rt_render_stop,
+ *     rt_render_device_frame, rt_render_device_result, rt_tonemap_rgba8_device and rt_assemble_frame work unchanged.
+ *   - A multi-device handle with shard_count <= 1 shards the frame over its devices as rt_render_start does.  With
+ *     shard_count > 1 the call renders that shard's tiles on the first device; the tile-packed accumulator has the
+ *     layout of rt_render_device_result and rt_shard_float4_count (a count-0 pixel holds (0, 0, 0, 0)).
+ *   - Scenes with more than 32 ray-marched shapes (the fused fallback) are rendered too.
+ *   - The frame never continues or seeds a progressive accumulation (rt_render_accumulated_samples reads 0 after it).
+ *   - rt_render_pixel_stats returns the counts after an unsharded single-device frame (moments: RT_ERR_STATE).
+ *   - rt_stats.paths grows by the sum of the shard's counts.
+ * RT_ERR_INVALID, before any device work: a NULL argument, a count above samples_number, and every parameter
+ * rt_render_start rejects. */
+int rt_render_start_counts(rt_scene* scene, const rt_camera* camera, const rt_render_params* params,
+                           const uint32_t* counts);
+
 /* Device-side result of the last started frame, for callers that gather shards over NCCL:
  * FOUR DOUBLES (r, g, b sums; samples) per owned pixel -- the f64 sums themselves, so that the assembled frame
  * equals the unsharded one bit for bit; they were floats before ABI 4, hence the names -- tile-packed in this

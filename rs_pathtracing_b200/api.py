@@ -314,6 +314,26 @@ class GpuRenderer:
         counts, moments = render_pixel_stats(h)
         return frame, counts, standard_error(counts, moments)
 
+    def render_counts(self, camera: Camera, counts: np.ndarray, samples_number: Optional[int] = None) -> np.ndarray:
+        """A frame with the caller's sample count per pixel (rt_render_start_counts) on this renderer's devices, depth
+        and seed: counts is an (h, w) uint32 map, e.g. the counts render_adaptive returned.  Returns frame[h, w, 3]
+        float64; a pixel with count 0 is NaN.  samples_number is the cap the counts are checked against (default: the
+        largest count, 1 for an all-zero map)."""
+        if getattr(counts, "ndim", 0) != 2:
+            raise ValueError("counts: a (height, width) uint32 array")
+        height, width = counts.shape
+        counts = check_counts(counts, width, height)
+        if samples_number is None:
+            samples_number = max(int(counts.max(initial=0)), 1)
+        if self.devices and len(self.devices) > 1:
+            h = self.scene.device_scene_multi(self.devices)
+        else:
+            h = self.scene.device_scene(self.device)
+        render_start_counts(h, camera, render_params(width, height, samples_number, self.depth, self.seed), counts)
+        frame = np.zeros((height, width, 3), np.float64)
+        render_wait(h, frame)
+        return frame
+
 
 def tonemap_rgba8(scene: Scene, frame: np.ndarray, device: Optional[int] = None) -> np.ndarray:
     """src/bin/main_raylib.rs:239-247 on the device."""
@@ -389,6 +409,26 @@ def render_start_adaptive(dev_scene, camera: Camera, params: RenderParams, min_s
     ap = _ffi.AdaptiveParams(min_samples, rel_error, abs_error)
     _check(_ffi.core().rt_render_start_adaptive(dev_scene, C.byref(camera), C.byref(params), C.byref(ap)))
     _started[_handle_key(dev_scene)] = (params.image.height, params.image.width, True)
+
+
+def check_counts(counts, width: int, height: int) -> np.ndarray:
+    """a sample-count map for a width x height frame: a C-contiguous (height, width) uint32 array"""
+    if not isinstance(counts, np.ndarray) or counts.dtype != np.uint32:
+        raise ValueError(f"counts: a uint32 numpy array, got {getattr(counts, 'dtype', type(counts).__name__)}")
+    if counts.shape != (height, width):
+        raise ValueError(f"counts: shape (height, width) = {(height, width)} expected, got {counts.shape}")
+    return np.ascontiguousarray(counts)
+
+
+def render_start_counts(dev_scene, camera: Camera, params: RenderParams, counts: np.ndarray) -> None:
+    """rt_render_start_counts: pixel x + y*width gets counts[y, x] samples (0 .. counts-1), at most
+    params.samples_number; each pixel equals the render_start frame's pixel at that sample count, bit for bit, and a
+    pixel with count 0 is NaN.  counts covers the whole image, also for a shard.  Poll / wait deliver as for
+    render_start."""
+    counts = check_counts(counts, params.image.width, params.image.height)
+    _check(_ffi.core().rt_render_start_counts(dev_scene, C.byref(camera), C.byref(params),
+                                              counts.ctypes.data_as(C.c_void_p)))
+    _started[_handle_key(dev_scene)] = (params.image.height, params.image.width, False)
 
 
 def render_pixel_stats(dev_scene, shape=None):

@@ -11,6 +11,8 @@
 //   k_adaptive_select   adaptive frames: stopping rule per pixel at a pass boundary -> list of the pixels that go on
 //   k_raygen_list       adaptive frames: level-0 loader of a refinement batch (listed pixels x the pass's samples)
 //   k_resolve_list      adaptive frames: continue a listed pixel's rgb and luminance sums over its new samples
+//   k_load_counts       counts frames: level-0 loader, the caller's sample count per pixel -> queue + RNG keys
+//   k_counts_resolve    counts frames: a pixel's sums over its samples, continued across the pieces of a large pixel
 //   k_assemble          multi-GPU: gathered tile-packed shards -> frame
 //   k_tonemap           the bins' sqrt / clamp / *256 -> RGBA8
 // Compile with -fmad=false (see rt_math.cuh).
@@ -842,6 +844,76 @@ k_load_groups(const rt_ray* __restrict__ rays, uint32_t n, unsigned long long r0
     q.bx[i] = 1.0; q.by[i] = 1.0; q.bz[i] = 1.0;
     q.pid[i] = i;
     path_key[i] = make_uint2(pixel_index[lo], (uint32_t)(r - offsets[lo]));   // (groups have fewer than 2^32 rays)
+}
+
+// K6c: level 0 of a batch of a counts frame (rt_render_start_counts), modelled on k_load_groups: every owned pixel is a
+// group of counts[p] paths.  The batch is paths [r0, r0 + n) of the shard; `offsets` is the batch's slice of the owned
+// pixels' path offsets, starting at owned pixel q0 (n_pixels + 1 entries).  Path i finds its owned slot by binary search,
+// its sample is its number inside the pixel, and its primary ray is the frame's own (camera_ray_dir).  A padding slot of
+// a clipped border tile has no paths, so no path lands on one.
+__global__ void __launch_bounds__(256)
+k_load_counts(RayCasterDev rc, ShardMap map, uint32_t n, unsigned long long r0, unsigned long long q0,
+              const unsigned long long* __restrict__ offsets, uint32_t n_pixels, uint32_t k0, uint32_t k1, PathQueue q,
+              uint32_t* count_out, uint2* __restrict__ path_key) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i == 0) *count_out = n;
+    if (i >= n) return;
+    const unsigned long long r = r0 + i;
+    uint32_t lo = 0, hi = n_pixels;   // the last slot that starts at or before r (count-0 slots before it start there too)
+    while (hi - lo > 1) {
+        const uint32_t mid = lo + (hi - lo) / 2;
+        if (offsets[mid] <= r) lo = mid; else hi = mid;
+    }
+    uint32_t x, y;
+    map.pixel_of(q0 + lo, x, y);
+    const uint32_t pixel = x + y * map.width, sample = (uint32_t)(r - offsets[lo]);
+    const D3 rd = camera_ray_dir(rc, x, y, pixel, sample, k0, k1);
+    q.ox[i] = rc.camera_position.x; q.oy[i] = rc.camera_position.y; q.oz[i] = rc.camera_position.z;
+    q.dx[i] = rd.x; q.dy[i] = rd.y; q.dz[i] = rd.z;
+    q.bx[i] = 1.0; q.by[i] = 1.0; q.bz[i] = 1.0;
+    q.pid[i] = i;
+    path_key[i] = make_uint2(pixel, sample);
+}
+
+// K5c: one thread per owned pixel of a counts-frame batch (paths [r0, r1), pixel slice as in k_load_counts; accum and
+// frame point at the slice's first pixel).  k_group_resolve's arithmetic into the frame's accumulator: the f64 sums in
+// sample order from 0.0 -- continued from accum for the later pieces of a pixel cut over batches of one lane -- then
+// Acc{sums, n} and the mean, so that k_assemble and delivery need nothing new.  A count-0 pixel gets Acc{0, 0, 0, 0}
+// and 0 / 0 = NaN.
+__global__ void __launch_bounds__(256)
+k_counts_resolve(const float4* __restrict__ radiance, unsigned long long r0, unsigned long long r1,
+                 const unsigned long long* __restrict__ offsets, uint32_t n_pixels, Acc* __restrict__ accum,
+                 rt_vec3* __restrict__ frame) {
+    const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n_pixels) return;
+    const unsigned long long first = offsets[k], end = offsets[k + 1];
+    double sx = 0.0, sy = 0.0, sz = 0.0;
+    if (first < r0) {   // continued from the previous piece
+        const Acc prev = accum[k];
+        sx = prev.r; sy = prev.g; sz = prev.b;
+    }
+    const unsigned long long a = first > r0 ? first : r0, b = end < r1 ? end : r1;
+    unsigned long long r = a;
+    for (; r + 16 <= b; r += 16) {
+        float4 v[16];
+#pragma unroll
+        for (int j = 0; j < 16; j++) v[j] = radiance[r - r0 + j];
+#pragma unroll
+        for (int j = 0; j < 16; j++) {
+            sx += (double)v[j].x; sy += (double)v[j].y; sz += (double)v[j].z;
+        }
+    }
+    for (; r < b; r++) {
+        const float4 v = radiance[r - r0];
+        sx += (double)v.x; sy += (double)v.y; sz += (double)v.z;
+    }
+    if (end > r1) {
+        accum[k] = Acc{sx, sy, sz, 0.0};
+        return;
+    }
+    const double n = (double)(end - first);
+    accum[k] = Acc{sx, sy, sz, n};
+    frame[k] = rt_vec3{sx / n, sy / n, sz / n};
 }
 
 // FMA micro-benchmarks: 8 independent chains per thread, FMA counted as 2 flop
@@ -1681,7 +1753,8 @@ static int ensure_path_buffers(rt_scene* sc, uint64_t need_paths) {
 
 static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_render_params* p,
                                const rt_adaptive_params* ap = nullptr);
-static int render_start_multi(rt_scene* sc, const rt_camera* cam, const rt_render_params* p);
+static int render_start_multi(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const uint32_t* counts = nullptr);
+static int render_start_counts_single(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const uint32_t* counts);
 
 int rt_render_start(rt_scene* sc, const rt_camera* cam, const rt_render_params* p) {
     if (!sc || !cam || !p) return fail(RT_ERR_INVALID, "null argument");
@@ -1699,10 +1772,8 @@ struct RefinePass {
     uint64_t B, nb;
 };
 
-// ap != NULL: an adaptive frame (rt_render_start_adaptive, validated there).  Pass 0 is the frame path with
-// min_samples samples (k_resolve<true> also writes the moments); the refinement passes follow in the same enqueue.
-static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const rt_adaptive_params* ap) {
-    if (!sc || !cam || !p) return fail(RT_ERR_INVALID, "null argument");
+// the frame parameters rt_render_start accepts (checked before any device work)
+static int check_frame_params(const rt_render_params* p) {
     if (p->image.width == 0 || p->image.height == 0 || p->samples_number == 0)
         return fail(RT_ERR_INVALID, "empty image or zero samples");
     if (p->max_depth > RT_MAX_LEVELS - 2) return fail(RT_ERR_INVALID, "max_depth too large (limit 62)");
@@ -1710,11 +1781,30 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
     if (p->shard_index >= shard_count) return fail(RT_ERR_INVALID, "shard_index >= shard_count");
     if (shard_count > 16) return fail(RT_ERR_INVALID, "at most 16 shards");
     if ((uint64_t)p->image.width * p->image.height > 0xFFFFFFFFull) return fail(RT_ERR_INVALID, "image too large");
-    {
-        rt_render_params pp = *p;
-        pp.shard_count = shard_count;
-        if (!tile_fits(make_shard_map(pp, p->shard_index))) return fail(RT_ERR_INVALID, "tile_width * tile_height >= 2^32");
-    }
+    rt_render_params pp = *p;
+    pp.shard_count = shard_count;
+    if (!tile_fits(make_shard_map(pp, p->shard_index))) return fail(RT_ERR_INVALID, "tile_width * tile_height >= 2^32");
+    return RT_OK;
+}
+
+// the frame's accumulator and f64 frame, owned order (grown on demand)
+static int ensure_frame_buffers(rt_scene* sc) {
+    if (sc->frame_capacity >= sc->owned_pixels) return RT_OK;
+    cudaFree(sc->d_accum); cudaFree(sc->d_frame);
+    sc->d_accum = nullptr; sc->d_frame = nullptr; sc->frame_capacity = 0;
+    CU(cudaMalloc(&sc->d_accum, std::max<uint64_t>(sc->owned_pixels, 1) * sizeof(Acc)));
+    CU(cudaMalloc(&sc->d_frame, std::max<uint64_t>(sc->owned_pixels, 1) * sizeof(rt_vec3)));
+    sc->frame_capacity = sc->owned_pixels;
+    return RT_OK;
+}
+
+// ap != NULL: an adaptive frame (rt_render_start_adaptive, validated there).  Pass 0 is the frame path with
+// min_samples samples (k_resolve<true> also writes the moments); the refinement passes follow in the same enqueue.
+static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const rt_adaptive_params* ap) {
+    if (!sc || !cam || !p) return fail(RT_ERR_INVALID, "null argument");
+    int rc = check_frame_params(p);
+    if (rc != RT_OK) return rc;
+    const uint32_t shard_count = p->shard_count ? p->shard_count : 1;
     CU(cudaSetDevice(sc->device));
     if (sc->rendering) rt_render_stop(sc);
 
@@ -1768,20 +1858,13 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
     if (px_per_batch * spp > 0xFFFFFFF0ull) return fail(RT_ERR_INVALID, "samples_number too large for one batch");
     const uint64_t n_batches = (sc->owned_pixels + px_per_batch - 1) / px_per_batch;
     lanes_used = (int)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)lanes_used, std::max(n_batches, refine_batches)));
-    int rc = RT_OK;
     for (int l = 0; l < lanes_used && rc == RT_OK; l++) {
         bind_lane(sc, l);
         rc = ensure_path_buffers(sc, std::max<uint64_t>(px_per_batch * spp, refine_paths));
     }
     bind_lane(sc, 0);
     if (rc != RT_OK) return rc;
-    if (sc->frame_capacity < sc->owned_pixels) {
-        cudaFree(sc->d_accum); cudaFree(sc->d_frame);
-        sc->d_accum = nullptr; sc->d_frame = nullptr; sc->frame_capacity = 0;
-        CU(cudaMalloc(&sc->d_accum, std::max<uint64_t>(sc->owned_pixels, 1) * sizeof(Acc)));
-        CU(cudaMalloc(&sc->d_frame, std::max<uint64_t>(sc->owned_pixels, 1) * sizeof(rt_vec3)));
-        sc->frame_capacity = sc->owned_pixels;
-    }
+    if ((rc = ensure_frame_buffers(sc)) != RT_OK) return rc;
     if (ap) {
         if ((rc = ensure_device_array(sc->d_moments, sc->moments_cap, sc->owned_pixels)) != RT_OK) return rc;
         if ((rc = ensure_device_array(sc->d_plist, sc->plist_cap, sc->owned_pixels)) != RT_OK) return rc;
@@ -1912,8 +1995,9 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
 // ShardMap), all of them concurrently -- every call below only enqueues -- then each peer's accumulator travels to
 // the first device with ONE peer copy on the peer's own stream (so it is ordered behind that shard's last
 // k_resolve and the peer is free for its next frame as soon as the copy has left), and k_assemble builds the frame
-// behind the events of all copies.  Nothing here waits on the host.
-static int render_start_multi(rt_scene* sc, const rt_camera* cam, const rt_render_params* p) {
+// behind the events of all copies.  Nothing here waits on the host.  counts != NULL: a counts frame
+// (rt_render_start_counts, validated there), every shard reading the whole map.
+static int render_start_multi(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const uint32_t* counts) {
     if (p->image.width == 0 || p->image.height == 0 || p->samples_number == 0)
         return fail(RT_ERR_INVALID, "empty image or zero samples");
     const uint32_t n_dev = (uint32_t)sc->peers.size() + 1;
@@ -1946,14 +2030,14 @@ static int render_start_multi(rt_scene* sc, const rt_camera* cam, const rt_rende
     for (uint32_t k = 1; k < n_dev; k++) {
         rt_scene* peer = sc->peers[k - 1];
         sp.shard_index = k;
-        int rc = render_start_single(peer, cam, &sp);
+        int rc = counts ? render_start_counts_single(peer, cam, &sp, counts) : render_start_single(peer, cam, &sp);
         if (rc != RT_OK) return rc;
         const uint64_t cnt = rt_shard_float4_count(&sp, k);
         if (cnt) CU(cudaMemcpyPeerAsync(sc->d_peer_acc[k - 1], sc->device, peer->d_accum, peer->device, cnt * sizeof(Acc), peer->stream));
         CU(cudaEventRecord(sc->ev_peer[k - 1], peer->stream));
     }
     sp.shard_index = 0;
-    int rc = render_start_single(sc, cam, &sp);
+    int rc = counts ? render_start_counts_single(sc, cam, &sp, counts) : render_start_single(sc, cam, &sp);
     if (rc != RT_OK) return rc;
     CU(cudaSetDevice(sc->device));
     for (uint32_t k = 1; k < n_dev; k++) CU(cudaStreamWaitEvent(sc->stream, sc->ev_peer[k - 1], 0));
@@ -2314,20 +2398,22 @@ struct GroupBatch {
     int lane;
 };
 
-// Enqueue a validated call (n_groups > 0) on the library's streams; the main stream ends after every lane.  No host
-// synchronisation.  Whole groups are packed in order into batches of at most RT_B200_BATCH_PATHS paths that alternate
-// over the lanes like a frame's; a group larger than a batch is cut into batch-sized pieces that all run on ONE lane, so
-// its running sum (k_group_resolve) passes from piece to piece in stream order and no lane reads another's partial sum.
-static int trace_groups(rt_scene* sc, const rt_ray* d_rays, uint64_t n_rays, const uint64_t* offsets,
-                        const uint32_t* pixel_index, uint32_t n_groups, uint32_t max_depth, uint64_t seed, rt_vec3* d_means) {
+// Plan groups[0 .. n_groups) of paths (group g = paths [offsets[g], offsets[g+1]), n_groups > 0) and size the lanes'
+// path buffers: whole groups are packed in order into batches of at most RT_B200_BATCH_PATHS paths that alternate over
+// the lanes like a frame's; a group larger than a batch is cut into batch-sized pieces that all run on ONE lane, so its
+// running sum (k_group_resolve, k_counts_resolve) passes from piece to piece in stream order and no lane reads another's
+// partial sum.  Caller rays (trace_groups) and counts frames (render_start_counts_single) share it.
+static int plan_groups(rt_scene* sc, const uint64_t* offsets, uint32_t n_groups, std::vector<GroupBatch>& plan,
+                       int& lanes_used) {
+    const uint64_t n_rays = offsets[n_groups];
     uint64_t cap = std::min<uint64_t>(std::max<uint64_t>(env_size("RT_B200_BATCH_PATHS", (size_t)1 << 23), 1), 0xFFFFFFF0ull);
-    int lanes_used = sc->ktiming ? 1 : sc->n_lanes;   // the lane policy of render_start_single
+    lanes_used = sc->ktiming ? 1 : sc->n_lanes;   // the lane policy of render_start_single
     if (!sc->lanes_from_env && lanes_used > 2 && (n_rays + cap - 1) / cap < 6) lanes_used = 2;
     if (lanes_used > 1) {
         const uint64_t split = (n_rays + lanes_used - 1) / lanes_used;
         if (split >= ((uint64_t)1 << 20)) cap = std::min(cap, split);
     }
-    std::vector<GroupBatch> plan;
+    plan.clear();
     uint64_t lane_paths[RT_MAX_LANES] = {0, 0, 0};
     uint64_t unit = 0;
     for (uint32_t g = 0; g < n_groups; unit++) {
@@ -2351,6 +2437,16 @@ static int trace_groups(rt_scene* sc, const rt_ray* d_rays, uint64_t n_rays, con
         rc = ensure_path_buffers(sc, std::max<uint64_t>(lane_paths[l], 1024));
     }
     bind_lane(sc, 0);
+    return rc;
+}
+
+// Enqueue a validated call (n_groups > 0) on the library's streams (batches of plan_groups); the main stream ends after
+// every lane.  No host synchronisation.
+static int trace_groups(rt_scene* sc, const rt_ray* d_rays, uint64_t n_rays, const uint64_t* offsets,
+                        const uint32_t* pixel_index, uint32_t n_groups, uint32_t max_depth, uint64_t seed, rt_vec3* d_means) {
+    std::vector<GroupBatch> plan;
+    int lanes_used = 1;
+    int rc = plan_groups(sc, offsets, n_groups, plan, lanes_used);
     if (rc != RT_OK) return rc;
     if ((rc = ensure_device_array(sc->d_group_off, sc->group_off_cap, (uint64_t)n_groups + 1)) != RT_OK) return rc;
     if ((rc = ensure_device_array(sc->d_group_pix, sc->group_pix_cap, n_groups)) != RT_OK) return rc;
@@ -2445,6 +2541,112 @@ int rt_trace_pixel_samples(rt_scene* sc, const rt_ray* rays, uint32_t n_rays, ui
     if (n_rays == 0) return fail(RT_ERR_INVALID, "no rays");
     const uint64_t offsets[2] = {0, n_rays};
     return rt_trace_pixel_samples_group(sc, rays, n_rays, offsets, &pixel_index, 1, max_depth, seed, mean_out);
+}
+
+// ---- frames with the caller's sample count per pixel (rt_render_start_counts) ------------------------------------
+// Every owned pixel is a group of counts[p] paths, planned by plan_groups; a batch is a contiguous range of owned pixels,
+// recorded for delivery when its last pixel is complete (after the last piece of a pixel cut over batches).
+static int render_start_counts_single(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const uint32_t* counts) {
+    int rc = check_frame_params(p);
+    if (rc != RT_OK) return rc;
+    rt_render_params rp = *p;
+    rp.shard_count = p->shard_count ? p->shard_count : 1;
+    const ShardMap map = make_shard_map(rp, p->shard_index);
+    const uint64_t owned = owned_tiles(map) * map.tile_pixels();
+    if (owned > 0xFFFFFFFFull) return fail(RT_ERR_INVALID, "image too large: a shard owns 2^32 pixels or more");
+    CU(cudaSetDevice(sc->device));
+    if (sc->rendering) rt_render_stop(sc);
+    sc->accumulated_spp = 0;   // a counts frame neither continues nor seeds a progressive accumulation
+    sc->adaptive_frame = false;
+    sc->rp = rp;
+    sc->map = map;
+    sc->owned_pixels = owned;
+
+    // the owned pixels' path offsets, in owned order: whole tile rows of the image (owned order is x + y*width when
+    // unsharded); the padding slots of clipped border tiles get no paths
+    std::vector<uint64_t>& off = sc->h_group_off;   // (a group call never overlaps a frame: check_groups refuses then)
+    off.resize(owned + 1);
+    off[0] = 0;
+    const uint32_t tw = map.tile_w;
+    for (uint64_t q = 0; q < owned; q += tw) {
+        uint32_t x, y;
+        const bool real = map.pixel_of(q, x, y);
+        const uint32_t* c = real ? counts + (size_t)y * map.width + x : nullptr;
+        const uint64_t keep = real ? std::min<uint64_t>(tw, map.width - x) : 0;
+        for (uint64_t k = 0; k < tw; k++) off[q + k + 1] = off[q + k] + (k < keep ? c[k] : 0u);
+    }
+    std::vector<GroupBatch> plan;
+    int lanes_used = 1;
+    if ((rc = plan_groups(sc, off.data(), (uint32_t)owned, plan, lanes_used)) != RT_OK) return rc;
+    if ((rc = ensure_frame_buffers(sc)) != RT_OK) return rc;
+    if ((rc = ensure_device_array(sc->d_group_off, sc->group_off_cap, owned + 1)) != RT_OK) return rc;
+    for (Batch& b : sc->batches) cudaEventDestroy(b.done);
+    sc->batches.clear();
+    sc->delivered = 0;
+    sc->spans.clear();
+    sc->ev_used = 0;
+
+    const RayCasterDev rcd = make_raycaster(*cam, p->image);
+    const uint32_t k0 = (uint32_t)p->seed, k1 = (uint32_t)(p->seed >> 32);
+    auto enqueue = [&]() -> int {
+        // (pageable source: the offsets have been read when the call returns)
+        CU(cudaMemcpyAsync(sc->d_group_off, off.data(), (owned + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, sc->stream));
+        CU(cudaEventRecord(sc->ev_frame_start, sc->stream));  // lane 0 = the main stream
+        for (int l = 1; l < lanes_used; l++) CU(cudaStreamWaitEvent(sc->lanes[l].stream, sc->ev_frame_start, 0));
+        for (const GroupBatch& b : plan) {
+            bind_lane(sc, b.lane);
+            const uint32_t n = (uint32_t)(b.r1 - b.r0), ng = b.g1 - b.g0;
+            if (n > 0) {
+                CU(cudaMemsetAsync(sc->d_counts, 0, RT_CNT_WORDS * sizeof(uint32_t), sc->stream));
+                {
+                    KernelSpan span(sc, RT_KCLASS_RAYGEN);
+                    k_load_counts<<<(unsigned)(((uint64_t)n + 255) / 256), 256, 0, sc->stream>>>(
+                        rcd, sc->map, n, b.r0, b.g0, sc->d_group_off + b.g0, ng, k0, k1, sc->q[0], sc->d_counts, sc->hq.key);
+                }
+                launch_bounces(sc, p->max_depth, p->seed);
+            }
+            {
+                KernelSpan span(sc, RT_KCLASS_RESOLVE);
+                k_counts_resolve<<<(unsigned)(((uint64_t)ng + 255) / 256), 256, 0, sc->stream>>>(
+                    sc->d_radiance, b.r0, b.r1, sc->d_group_off + b.g0, ng, sc->d_accum + b.g0, sc->d_frame + b.g0);
+            }
+            if (b.r1 != off[b.g1]) continue;   // a piece of a pixel whose last piece is still to come
+            Batch rec;
+            rec.first_owned = b.g0;
+            rec.n_pixels = ng;
+            CU(cudaEventCreateWithFlags(&rec.done, cudaEventDisableTiming));
+            CU(cudaEventRecord(rec.done, sc->stream));
+            sc->batches.push_back(rec);
+        }
+        bind_lane(sc, 0);
+        for (int l = 1; l < lanes_used; l++) {  // the main stream ends the frame after every lane
+            CU(cudaEventRecord(sc->lanes[l].done, sc->lanes[l].stream));
+            CU(cudaStreamWaitEvent(sc->stream, sc->lanes[l].done, 0));
+        }
+        CU(cudaEventRecord(sc->ev_frame_stop, sc->stream));
+        CU(cudaGetLastError());
+        return RT_OK;
+    };
+    rc = enqueue();
+    bind_lane(sc, 0);
+    if (rc != RT_OK) return rc;
+    sc->rendering = true;
+    sc->frame_complete = false;
+    sc->paths += off[owned];
+    return RT_OK;
+}
+
+int rt_render_start_counts(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const uint32_t* counts) {
+    if (!sc || !cam || !p || !counts) return fail(RT_ERR_INVALID, "null argument");
+    int rc = check_frame_params(p);
+    if (rc != RT_OK) return rc;
+    const uint64_t n_px = (uint64_t)p->image.width * p->image.height;
+    uint32_t most = 0;
+    for (uint64_t i = 0; i < n_px; i++) most = std::max(most, counts[i]);
+    if (most > p->samples_number) return fail(RT_ERR_INVALID, "a count above samples_number");
+    if (!sc->peers.empty() && p->shard_count <= 1) return render_start_multi(sc, cam, p, counts);
+    sc->multi_active = false;
+    return render_start_counts_single(sc, cam, p, counts);
 }
 
 // ---- instrumentation ---------------------------------------------------------------------------

@@ -107,9 +107,11 @@ class DistributedRenderer:
     def _params(self, w, h, spp, shard):
         return api.render_params(w, h, spp, self.depth, self.seed, self.world, shard, tile=self.tile)
 
-    def render_device(self, camera: Camera, width: int, height: int, samples_number: int):
+    def render_device(self, camera: Camera, width: int, height: int, samples_number: int, counts=None):
         """Render this rank's tiles, gather, assemble on rank 0.  Returns the device frame tensor on
-        rank 0 (h x w x 3 float64), None elsewhere.  No host synchronisation besides NCCL's own."""
+        rank 0 (h x w x 3 float64), None elsewhere.  No host synchronisation besides NCCL's own.
+        counts: an (h, w) uint32 sample-count map (rt_render_start_counts; samples_number is then the cap), the WHOLE
+        map on every rank; the assembled frame is the unsharded counts frame, bit for bit."""
         torch, dist = self.torch, self.dist
         p = self._params(width, height, samples_number, self.rank)
         # The library renders on its own non-blocking streams, the exchange runs on torch's / NCCL's: the
@@ -117,7 +119,10 @@ class DistributedRenderer:
         # previous frame's send (rank 0: copy) reads, so that read must be over before the frame starts.
         if self._exchanged is not None:
             self._exchanged.synchronize()
-        api.render_start(self.dev_scene, camera, p)
+        if counts is None:
+            api.render_start(self.dev_scene, camera, p)
+        else:
+            api.render_start_counts(self.dev_scene, camera, p, counts)
         ptr, n = api.render_device_result(self.dev_scene)   # waits for this shard's kernels
         mine = torch.as_tensor(api.DevicePointer(ptr, (n, 4), "<f8", owner=self), device=f"cuda:{self.device}")
         counts = [api.shard_float4_count(p, s) for s in range(self.world)]
@@ -272,8 +277,8 @@ class DistributedRenderer:
             out.append(self._host2[i % 2].numpy().copy())
         return out
 
-    def render(self, camera: Camera, width: int, height: int, samples_number: int) -> Optional[np.ndarray]:
-        frame = self.render_device(camera, width, height, samples_number)
+    def render(self, camera: Camera, width: int, height: int, samples_number: int, counts=None) -> Optional[np.ndarray]:
+        frame = self.render_device(camera, width, height, samples_number, counts=counts)
         if frame is None:
             return None
         torch = self.torch

@@ -2,12 +2,16 @@
 
   python tools/render.py scenes/cornell_box.json out.png --size 1024 1024 --spp 256 [--depth 8] [--seed 1]
       [--adaptive REL [--min-samples N] [--abs-error A] [--heatmap counts.png]]
+      [--counts MAP.npy [--heatmap counts.png]]
 
 Scene::from_json -> GpuRenderer (Renderer trait: start_rendering / render_step until done) ->
 rt_tonemap_rgba8 (sqrt, clamp(0, 0.999) * 256, on the device) -> PNG.  With --adaptive, an adaptive frame
 (rt_render_start_adaptive): every pixel gets --min-samples samples and doubles its count, up to --spp, while the
 standard error of its mean luminance exceeds REL times the mean (or --abs-error); --heatmap writes the per-pixel
-sample counts as a grey PNG (black = min-samples, white = spp, log2 scale)."""
+sample counts as a grey PNG (black = min-samples, white = spp, log2 scale).  With --counts, a frame with the given
+sample count per pixel (rt_render_start_counts): MAP.npy is an (h, w) uint32 array, which sets the size; --heatmap
+then draws that map (black = 0 or 1 sample, white = its largest count, log2 scale) and the frame's count-0 pixels
+are black."""
 import argparse, os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -23,16 +27,28 @@ ap.add_argument("--seed", type=int, default=1)
 ap.add_argument("--adaptive", type=float, default=None, metavar="REL", help="relative standard-error target")
 ap.add_argument("--min-samples", type=int, default=8)
 ap.add_argument("--abs-error", type=float, default=0.0)
-ap.add_argument("--heatmap", default=None, help="PNG of the per-pixel sample counts (with --adaptive)")
+ap.add_argument("--counts", default=None, metavar="MAP.npy", help="(h, w) uint32 sample count per pixel")
+ap.add_argument("--heatmap", default=None, help="PNG of the per-pixel sample counts (with --adaptive or --counts)")
 a = ap.parse_args()
-if a.heatmap and a.adaptive is None:
-    ap.error("--heatmap needs --adaptive")
+if a.heatmap and a.adaptive is None and a.counts is None:
+    ap.error("--heatmap needs --adaptive or --counts")
+if a.adaptive is not None and a.counts is not None:
+    ap.error("--adaptive and --counts exclude each other")
 sc = rt.Scene.from_file(a.scene, random_spheres_seed=a.seed)
 cam = sc.camera()
 r = rt.GpuRenderer(sc, 12, a.depth, seed=a.seed)
 w, h = a.size
+if a.counts is not None:
+    given = np.load(a.counts)
+    if given.ndim != 2 or given.dtype != np.uint32:
+        ap.error(f"--counts: an (h, w) uint32 array expected, got {given.dtype} {given.shape}")
+    h, w = given.shape
 t0 = time.perf_counter()
-if a.adaptive is None:
+if a.counts is not None:
+    buf = r.render_counts(cam, given)
+    counts = given
+    paths = int(given.sum(dtype=np.uint64))
+elif a.adaptive is None:
     buf = np.zeros((h, w, 3))
     r.start_rendering(cam, rt.ImageParams(w, h), a.spp)
     while not r.render_step(buf):
@@ -42,12 +58,16 @@ else:
     buf, counts, _ = r.render_adaptive(cam, w, h, a.spp, min(a.min_samples, a.spp), a.adaptive, a.abs_error)
     paths = int(counts.sum())
 dt = time.perf_counter() - t0
-rt.save_png(a.out, rt.tonemap_rgba8(sc, buf))
+rt.save_png(a.out, rt.tonemap_rgba8(sc, buf))   # (a count-0 pixel is NaN, which the tone map makes black)
 print(f"{a.scene}: {w}x{h}, {paths / (w * h):.1f} spp on average, in {dt * 1e3:.1f} ms "
       f"({paths / dt / 1e6:.1f} Mpaths/s) -> {a.out}")
 if a.heatmap:
-    lo, hi = np.log2(min(a.min_samples, a.spp)), np.log2(a.spp)
-    level = (np.log2(counts.astype(np.float64)) - lo) / max(hi - lo, 1e-9)
+    if a.counts is not None:
+        lo, hi = 0.0, np.log2(max(int(counts.max()), 1))
+    else:
+        lo, hi = np.log2(min(a.min_samples, a.spp)), np.log2(a.spp)
+    with np.errstate(divide="ignore"):   # log2(0) = -inf: black
+        level = (np.log2(counts.astype(np.float64)) - lo) / max(hi - lo, 1e-9)
     grey = np.round(np.clip(level, 0.0, 1.0) * 255).astype(np.uint8)
     rgba = np.dstack([grey, grey, grey, np.full_like(grey, 255)])
     rt.save_png(a.heatmap, rgba)
