@@ -345,6 +345,25 @@ int rt_render_pixel_stats(rt_scene* scene, uint32_t* counts, double* moments);
 int rt_render_start_counts(rt_scene* scene, const rt_camera* camera, const rt_render_params* params,
                            const uint32_t* counts);
 
+/* A multi-view frame: n_views cameras of one scene in one frame.  params->image is the size w x h of ONE view; every view
+ * shares samples_number, max_depth, seed and tiling.  View v equals, bit for bit, the rt_render_start frame of
+ * cameras[v] with the same params: the RNG key of pixel (x, y) is x + y*w in every view, so the views share their random
+ * streams (start frames with different seeds for decorrelated views).  cameras is read before the call returns.
+ * The frame is the STACKED image of width w and height n_views*h, view v in rows v*h .. v*h+h-1:
+ *   - rt_render_poll / rt_render_wait write buffer[v*w*h + x + y*w], progressively as for rt_render_start;
+ *     rt_render_device_frame and rt_tonemap_rgba8_device cover n_views*w*h pixels.
+ *   - shard_count > 1 renders that shard's tiles of the stacked image (a tile may straddle two views): size and
+ *     assemble the shards with rt_shard_float4_count and rt_assemble_frame, passing params whose image.height is
+ *     n_views*h.  A multi-device handle with shard_count <= 1 shards the stacked image over its devices.
+ *   - Non-blocking like rt_render_start; a frame in flight is stopped first.  Scenes with more than 32 ray-marched
+ *     shapes (the fused fallback) are rendered too.
+ *   - The frame never continues or seeds a progressive accumulation (rt_render_accumulated_samples reads 0 after it).
+ *   - rt_render_pixel_stats returns RT_ERR_STATE after it (every count is samples_number).
+ *   - rt_stats.paths grows by samples_number per real pixel of the shard (tile padding is not counted).
+ * RT_ERR_INVALID, before any device work: a NULL argument, n_views == 0, n_views*h > UINT32_MAX, a stacked image of
+ * 2^32 pixels or more, and every parameter rt_render_start rejects. */
+int rt_render_start_views(rt_scene* scene, const rt_camera* cameras, uint32_t n_views, const rt_render_params* params);
+
 /* Device-side result of the last started frame, for callers that gather shards over NCCL:
  * FOUR DOUBLES (r, g, b sums; samples) per owned pixel -- the f64 sums themselves, so that the assembled frame
  * equals the unsharded one bit for bit; they were floats before ABI 4, hence the names -- tile-packed in this

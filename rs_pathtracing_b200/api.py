@@ -43,6 +43,19 @@ def camera_new(position, direction, up, focal_length: float, fov_rad: float) -> 
     return cam
 
 
+def orbit_cameras(camera: Camera, n: int) -> list:
+    """n cameras around the scene (a turntable): camera k is `camera` with its position, direction and up rotated about
+    the world y axis through the origin by 2*pi*k/n, made by Camera::new with the same focal length and fov"""
+    out = []
+    for k in range(n):
+        a = 2.0 * math.pi * k / n
+        c, s = math.cos(a), math.sin(a)
+        rot = lambda v: (c * v.x + s * v.z, v.y, c * v.z - s * v.x)
+        out.append(camera_new(rot(camera.position), rot(camera.direction), rot(camera.up), camera.focal_length,
+                              camera.fov_rad))
+    return out
+
+
 _pil_loader_ref = None
 
 
@@ -334,6 +347,20 @@ class GpuRenderer:
         render_wait(h, frame)
         return frame
 
+    def render_views(self, cameras, width: int, height: int, samples_number: int) -> np.ndarray:
+        """Several views of the scene in one frame (rt_render_start_views) on this renderer's devices, depth and seed:
+        returns frames[V, h, w, 3] float64, frames[v] equal to render(cameras[v], width, height, samples_number) bit for
+        bit."""
+        cameras = check_cameras(cameras)
+        if self.devices and len(self.devices) > 1:
+            h = self.scene.device_scene_multi(self.devices)
+        else:
+            h = self.scene.device_scene(self.device)
+        render_start_views(h, cameras, render_params(width, height, samples_number, self.depth, self.seed))
+        frames = np.zeros((len(cameras), height, width, 3), np.float64)
+        render_wait(h, frames)
+        return frames
+
 
 def tonemap_rgba8(scene: Scene, frame: np.ndarray, device: Optional[int] = None) -> np.ndarray:
     """src/bin/main_raylib.rs:239-247 on the device."""
@@ -429,6 +456,41 @@ def render_start_counts(dev_scene, camera: Camera, params: RenderParams, counts:
     _check(_ffi.core().rt_render_start_counts(dev_scene, C.byref(camera), C.byref(params),
                                               counts.ctypes.data_as(C.c_void_p)))
     _started[_handle_key(dev_scene)] = (params.image.height, params.image.width, False)
+
+
+def check_cameras(cameras) -> list:
+    """the cameras of a views frame: a non-empty sequence of Camera"""
+    if isinstance(cameras, Camera):
+        raise ValueError("cameras: a sequence of Camera, got a single Camera")
+    try:
+        cameras = list(cameras)
+    except TypeError:
+        raise ValueError(f"cameras: a sequence of Camera, got {type(cameras).__name__}") from None
+    if not cameras:
+        raise ValueError("cameras: at least one Camera")
+    for i, c in enumerate(cameras):
+        if not isinstance(c, Camera):
+            raise ValueError(f"cameras[{i}]: a Camera, got {type(c).__name__}")
+    return cameras
+
+
+def render_start_views(dev_scene, cameras, params: RenderParams) -> None:
+    """rt_render_start_views: one frame of len(cameras) views of params.image's size each.  The frame is the stacked
+    image (width, len(cameras) * height), view v in rows v*height .. v*height+height-1, so that poll / wait deliver
+    buffer[v, y, x] of a (V, h, w, 3) buffer; view v equals render_start of cameras[v] with params, bit for bit.  An
+    explicit shard (shard_count > 1) is a shard of the stacked image: size and assemble it with params whose
+    image.height is len(cameras) * height."""
+    cameras = check_cameras(cameras)
+    table = (Camera * len(cameras))(*cameras)
+    _check(_ffi.core().rt_render_start_views(dev_scene, table, len(cameras), C.byref(params)))
+    _started[_handle_key(dev_scene)] = (len(cameras) * params.image.height, params.image.width, False)
+
+
+def stacked_params(params: RenderParams, n_views: int) -> RenderParams:
+    """the params of the stacked image of a views frame (for shard_float4_count and assemble_frame)"""
+    p = RenderParams.from_buffer_copy(params)
+    p.image = ImageParams(params.image.width, n_views * params.image.height)
+    return p
 
 
 def render_pixel_stats(dev_scene, shape=None):

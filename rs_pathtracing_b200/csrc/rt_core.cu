@@ -3,6 +3,7 @@
 // Kernels
 //   k_intersect_batch   batched nearest hit (Scene::closest_hit with ShapeCollection semantics)
 //   k_raygen            MultisamplerRayCaster::next for a batch of pixels x samples
+//   k_raygen_views      views frames: k_raygen over the stacked image of several views, each with its own camera
 //   k_bounce            one segment of ray_color for every live path: nearest hit, scatter / emit /
 //                       sky, survivors compacted into the next queue (ballot + popc + one atomic per warp)
 //   k_resolve           per-pixel mean (trace_pixel_samples) -> (f64 sums, samples) accumulator + f64 frame
@@ -846,6 +847,46 @@ k_load_groups(const rt_ray* __restrict__ rays, uint32_t n, unsigned long long r0
     path_key[i] = make_uint2(pixel_index[lo], (uint32_t)(r - offsets[lo]));   // (groups have fewer than 2^32 rays)
 }
 
+// K1v: level 0 of a batch of a views frame (rt_render_start_views): k_raygen over the stacked image (n_views views of
+// view_h rows each, `map` is the stacked map), with the camera of each pixel's view.  Stacked row Y is row
+// y = Y - v*view_h of view v = Y / view_h, and its RNG key is x + y*width: the key of (x, y) in view v's own frame.
+__global__ void __launch_bounds__(256)
+k_raygen_views(const RayCasterDev* __restrict__ cams, uint32_t view_h, ShardMap map, unsigned long long first_owned,
+               uint32_t n_pixels, uint32_t spp, uint32_t k0, uint32_t k1, PathQueue q, uint32_t* count_out,
+               float4* __restrict__ radiance, uint2* __restrict__ path_key) {
+    const unsigned long long n = (unsigned long long)n_pixels * spp;
+    const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
+    // round the trip count up so that whole warps stay converged for the ballot in queue_append
+    const unsigned long long n_round = (n + 31ull) & ~31ull;
+    for (unsigned long long id = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; id < n_round; id += stride) {
+        bool alive = false;
+        uint32_t v = 0;
+        D3 dir = mk(0.0, 0.0, 0.0);
+        if (id < n) {
+            const uint32_t id32 = (uint32_t)id;   // (a batch holds fewer than 2^32 paths)
+            const uint32_t pl = id32 / spp, s = id32 - pl * spp;
+            uint32_t x, Y;
+            if (map.pixel_of(first_owned + pl, x, Y)) {
+                v = Y / view_h;
+                const uint32_t y = Y - v * view_h, pixel = x + y * map.width;
+                dir = camera_ray_dir(cams[v], x, y, pixel, s, k0, k1);
+                path_key[id] = make_uint2(pixel, s);
+                alive = true;
+            } else {
+                radiance[id] = make_float4(0.f, 0.f, 0.f, 0.f);
+            }
+        }
+        const uint32_t slot = queue_append(alive, count_out);
+        if (alive) {
+            const D3 o = cams[v].camera_position;
+            q.ox[slot] = o.x; q.oy[slot] = o.y; q.oz[slot] = o.z;
+            q.dx[slot] = dir.x; q.dy[slot] = dir.y; q.dz[slot] = dir.z;
+            q.bx[slot] = 1.0; q.by[slot] = 1.0; q.bz[slot] = 1.0;
+            q.pid[slot] = (uint32_t)id;
+        }
+    }
+}
+
 // K6c: level 0 of a batch of a counts frame (rt_render_start_counts), modelled on k_load_groups: every owned pixel is a
 // group of counts[p] paths.  The batch is paths [r0, r0 + n) of the shard; `offsets` is the batch's slice of the owned
 // pixels' path offsets, starting at owned pixel q0 (n_pixels + 1 entries).  Path i finds its owned slot by binary search,
@@ -1058,6 +1099,12 @@ struct rt_scene {
     cudaEvent_t ev_adaptive_fork = nullptr;
     uint32_t* d_pix_counts = nullptr;   // rt_render_pixel_stats
     uint64_t pix_counts_cap = 0;
+    // views frames (rt_render_start_views): whether the frame in flight / last completed is one, and its per-view
+    // ray casters (host copy, so that the upload has read them when the call returns; device table grown on demand)
+    bool views_frame = false;
+    std::vector<RayCasterDev> h_views;
+    RayCasterDev* d_views = nullptr;
+    uint64_t views_cap = 0;
 };
 
 template <class T>
@@ -1449,6 +1496,7 @@ void rt_scene_destroy(rt_scene* sc) {
     cudaFree(sc->d_plist);
     cudaFree(sc->d_live);
     cudaFree(sc->d_pix_counts);
+    cudaFree(sc->d_views);
     if (sc->host_stage) cudaFreeHost(sc->host_stage);
     bind_lane(sc, 0);
     for (int l = 0; l < RT_MAX_LANES; l++)
@@ -1752,8 +1800,9 @@ static int ensure_path_buffers(rt_scene* sc, uint64_t need_paths) {
 }
 
 static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_render_params* p,
-                               const rt_adaptive_params* ap = nullptr);
-static int render_start_multi(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const uint32_t* counts = nullptr);
+                               const rt_adaptive_params* ap = nullptr, uint32_t n_views = 0);
+static int render_start_multi(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const uint32_t* counts = nullptr,
+                              uint32_t n_views = 0);
 static int render_start_counts_single(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const uint32_t* counts);
 
 int rt_render_start(rt_scene* sc, const rt_camera* cam, const rt_render_params* p) {
@@ -1787,6 +1836,18 @@ static int check_frame_params(const rt_render_params* p) {
     return RT_OK;
 }
 
+// the real pixels a shard owns: its owned pixels less the padding of clipped border tiles
+static uint64_t real_pixels(const ShardMap& m) {
+    if (m.shard_count == 1) return (uint64_t)m.width * m.height;
+    uint64_t n = 0;
+    for (uint64_t j = 0, tiles = owned_tiles(m); j < tiles; j++) {
+        uint32_t x, y;
+        m.pixel_of(j * m.tile_pixels(), x, y);   // the tile's first pixel, always inside the image
+        n += (uint64_t)std::min(m.tile_w, m.width - x) * std::min(m.tile_h, m.height - y);
+    }
+    return n;
+}
+
 // the frame's accumulator and f64 frame, owned order (grown on demand)
 static int ensure_frame_buffers(rt_scene* sc) {
     if (sc->frame_capacity >= sc->owned_pixels) return RT_OK;
@@ -1800,7 +1861,10 @@ static int ensure_frame_buffers(rt_scene* sc) {
 
 // ap != NULL: an adaptive frame (rt_render_start_adaptive, validated there).  Pass 0 is the frame path with
 // min_samples samples (k_resolve<true> also writes the moments); the refinement passes follow in the same enqueue.
-static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const rt_adaptive_params* ap) {
+// n_views > 0: a views frame (rt_render_start_views, validated there): `cam` points to n_views cameras and p is the
+// stacked image; level 0 of every batch is k_raygen_views, then the bounce loop runs without raygen.
+static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const rt_adaptive_params* ap,
+                               uint32_t n_views) {
     if (!sc || !cam || !p) return fail(RT_ERR_INVALID, "null argument");
     int rc = check_frame_params(p);
     if (rc != RT_OK) return rc;
@@ -1811,7 +1875,7 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
     // progressive accumulation: this frame adds its samples to the previous ones when it is the same frame
     // (image, sharding, depth, seed, camera) and nothing was abandoned; otherwise it starts afresh
     uint32_t sample_base = 0;
-    if (!ap && sc->accumulate && sc->accumulated_spp > 0 && sc->wavefront && memcmp(&sc->accum_cam, cam, sizeof *cam) == 0 &&
+    if (!ap && !n_views && sc->accumulate && sc->accumulated_spp > 0 && sc->wavefront && memcmp(&sc->accum_cam, cam, sizeof *cam) == 0 &&
         sc->accum_rp.image.width == p->image.width && sc->accum_rp.image.height == p->image.height &&
         sc->accum_rp.max_depth == p->max_depth && sc->accum_rp.seed == p->seed &&
         (sc->accum_rp.shard_count ? sc->accum_rp.shard_count : 1) == shard_count &&
@@ -1821,6 +1885,7 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
         sample_base = sc->accumulated_spp;
     sc->accumulated_spp = 0;  // until this frame is enqueued (an abandoned frame breaks the chain)
     sc->adaptive_frame = false;
+    sc->views_frame = n_views > 0;
     sc->rp = *p;
     sc->rp.shard_count = shard_count;
     sc->map = make_shard_map(sc->rp, p->shard_index);
@@ -1870,6 +1935,14 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
         if ((rc = ensure_device_array(sc->d_plist, sc->plist_cap, sc->owned_pixels)) != RT_OK) return rc;
         if ((rc = ensure_device_array(sc->d_live, sc->live_cap, std::max<uint64_t>(refine.size(), 1))) != RT_OK) return rc;
     }
+    const uint32_t view_h = n_views ? p->image.height / n_views : 0;
+    if (n_views) {   // the ray caster of every view, made for the image of one view
+        rt_image_params vi = p->image;
+        vi.height = view_h;
+        sc->h_views.resize(n_views);
+        for (uint32_t v = 0; v < n_views; v++) sc->h_views[v] = make_raycaster(cam[v], vi);
+        if ((rc = ensure_device_array(sc->d_views, sc->views_cap, n_views)) != RT_OK) return rc;
+    }
     for (Batch& b : sc->batches) cudaEventDestroy(b.done);
     sc->batches.clear();
     sc->delivered = 0;
@@ -1879,6 +1952,8 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
     RayCasterDev rcd = make_raycaster(*cam, p->image);
     uint32_t k0 = (uint32_t)p->seed, k1 = (uint32_t)(p->seed >> 32);
     auto enqueue = [&]() -> int {
+        if (n_views)   // (pageable source: read when the call returns; the lanes wait for it through ev_frame_start)
+            CU(cudaMemcpyAsync(sc->d_views, sc->h_views.data(), n_views * sizeof(RayCasterDev), cudaMemcpyHostToDevice, sc->stream));
         CU(cudaEventRecord(sc->ev_frame_start, sc->stream));  // lane 0 = the main stream
         for (int l = 1; l < lanes_used; l++) CU(cudaStreamWaitEvent(sc->lanes[l].stream, sc->ev_frame_start, 0));
         if (ap) CU(cudaMemsetAsync(sc->d_live, 0, std::max<size_t>(refine.size(), 1) * sizeof(uint32_t), sc->stream));
@@ -1887,7 +1962,14 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
             bind_lane(sc, (int)(batch_no % (uint64_t)lanes_used));
             uint32_t npx = (uint32_t)std::min<uint64_t>(px_per_batch, sc->owned_pixels - first);
             CU(cudaMemsetAsync(sc->d_counts, 0, RT_CNT_WORDS * sizeof(uint32_t), sc->stream));
-            if (sc->wavefront) {   // primary rays are generated inside the level-0 k_extend
+            if (n_views) {
+                {
+                    KernelSpan span(sc, RT_KCLASS_RAYGEN);
+                    k_raygen_views<<<sc->grid, 256, 0, sc->stream>>>(sc->d_views, view_h, sc->map, first, npx, spp, k0, k1, sc->q[0],
+                                                                   sc->d_counts, sc->d_radiance, sc->hq.key);
+                }
+                launch_bounces(sc, p->max_depth, p->seed);
+            } else if (sc->wavefront) {   // primary rays are generated inside the level-0 k_extend
                 RaygenArgs rg;
                 rg.rc = rcd; rg.map = sc->map; rg.first_owned = first; rg.n_paths = npx * spp; rg.spp = spp;
                 rg.k0 = k0; rg.k1 = k1; rg.sample_base = sample_base; rg.radiance = sc->d_radiance; rg.count_out = sc->d_counts;
@@ -1915,7 +1997,7 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
             CU(cudaEventCreateWithFlags(&b.done, cudaEventDisableTiming));
             CU(cudaEventRecord(b.done, sc->stream));
             sc->batches.push_back(b);
-            sc->paths += (uint64_t)npx * spp;
+            if (!n_views) sc->paths += (uint64_t)npx * spp;
         }
         // adaptive refinement passes: all lanes join the main stream, k_adaptive_select lists the pixels that go on,
         // the lanes fork again and run the pass's batches.  Nothing waits on the host.
@@ -1977,6 +2059,10 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
     if (rc != RT_OK) return rc;
     sc->rendering = true;
     sc->frame_complete = false;
+    if (n_views) {   // real pixels only; the frame neither continues nor seeds an accumulation
+        sc->paths += real_pixels(sc->map) * spp;
+        return RT_OK;
+    }
     if (ap) {   // rt_stats.paths grows when the frame completes (the listed counts are known on the device only)
         sc->adaptive_frame = true;
         sc->adaptive_m.assign(1, spp);
@@ -1996,8 +2082,10 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
 // the first device with ONE peer copy on the peer's own stream (so it is ordered behind that shard's last
 // k_resolve and the peer is free for its next frame as soon as the copy has left), and k_assemble builds the frame
 // behind the events of all copies.  Nothing here waits on the host.  counts != NULL: a counts frame
-// (rt_render_start_counts, validated there), every shard reading the whole map.
-static int render_start_multi(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const uint32_t* counts) {
+// (rt_render_start_counts, validated there), every shard reading the whole map.  n_views > 0: a views frame
+// (rt_render_start_views, validated there; p is the stacked image), every shard uploading the whole camera table.
+static int render_start_multi(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const uint32_t* counts,
+                              uint32_t n_views) {
     if (p->image.width == 0 || p->image.height == 0 || p->samples_number == 0)
         return fail(RT_ERR_INVALID, "empty image or zero samples");
     const uint32_t n_dev = (uint32_t)sc->peers.size() + 1;
@@ -2030,14 +2118,14 @@ static int render_start_multi(rt_scene* sc, const rt_camera* cam, const rt_rende
     for (uint32_t k = 1; k < n_dev; k++) {
         rt_scene* peer = sc->peers[k - 1];
         sp.shard_index = k;
-        int rc = counts ? render_start_counts_single(peer, cam, &sp, counts) : render_start_single(peer, cam, &sp);
+        int rc = counts ? render_start_counts_single(peer, cam, &sp, counts) : render_start_single(peer, cam, &sp, nullptr, n_views);
         if (rc != RT_OK) return rc;
         const uint64_t cnt = rt_shard_float4_count(&sp, k);
         if (cnt) CU(cudaMemcpyPeerAsync(sc->d_peer_acc[k - 1], sc->device, peer->d_accum, peer->device, cnt * sizeof(Acc), peer->stream));
         CU(cudaEventRecord(sc->ev_peer[k - 1], peer->stream));
     }
     sp.shard_index = 0;
-    int rc = counts ? render_start_counts_single(sc, cam, &sp, counts) : render_start_single(sc, cam, &sp);
+    int rc = counts ? render_start_counts_single(sc, cam, &sp, counts) : render_start_single(sc, cam, &sp, nullptr, n_views);
     if (rc != RT_OK) return rc;
     CU(cudaSetDevice(sc->device));
     for (uint32_t k = 1; k < n_dev; k++) CU(cudaStreamWaitEvent(sc->stream, sc->ev_peer[k - 1], 0));
@@ -2089,6 +2177,7 @@ int rt_render_start_adaptive(rt_scene* sc, const rt_camera* cam, const rt_render
 int rt_render_pixel_stats(rt_scene* sc, uint32_t* counts, double* moments) {
     if (!sc) return fail(RT_ERR_INVALID, "null scene");
     if (sc->multi_active) return fail(RT_ERR_STATE, "per-pixel statistics of a multi-device frame are not kept");
+    if (sc->views_frame) return fail(RT_ERR_STATE, "per-pixel statistics of a views frame are not kept");
     if (sc->rendering) {
         CU(cudaSetDevice(sc->device));
         CU(cudaStreamSynchronize(sc->stream));
@@ -2558,6 +2647,7 @@ static int render_start_counts_single(rt_scene* sc, const rt_camera* cam, const 
     if (sc->rendering) rt_render_stop(sc);
     sc->accumulated_spp = 0;   // a counts frame neither continues nor seeds a progressive accumulation
     sc->adaptive_frame = false;
+    sc->views_frame = false;
     sc->rp = rp;
     sc->map = map;
     sc->owned_pixels = owned;
@@ -2647,6 +2737,22 @@ int rt_render_start_counts(rt_scene* sc, const rt_camera* cam, const rt_render_p
     if (!sc->peers.empty() && p->shard_count <= 1) return render_start_multi(sc, cam, p, counts);
     sc->multi_active = false;
     return render_start_counts_single(sc, cam, p, counts);
+}
+
+// ---- multi-view frames (rt_render_start_views) ------------------------------------------------------------------
+// The frame path over the stacked image of the views: owned order, batches, lanes, delivery, k_assemble and the peer
+// copies see one image of width w and height n_views*h; only level 0 (k_raygen_views) knows where the views meet.
+int rt_render_start_views(rt_scene* sc, const rt_camera* cams, uint32_t n_views, const rt_render_params* p) {
+    if (!sc || !cams || !p) return fail(RT_ERR_INVALID, "null argument");
+    if (n_views == 0) return fail(RT_ERR_INVALID, "no views");
+    if ((uint64_t)n_views * p->image.height > 0xFFFFFFFFull) return fail(RT_ERR_INVALID, "n_views * height >= 2^32");
+    rt_render_params sp = *p;
+    sp.image.height = n_views * p->image.height;
+    int rc = check_frame_params(&sp);
+    if (rc != RT_OK) return rc;
+    if (!sc->peers.empty() && p->shard_count <= 1) return render_start_multi(sc, cams, &sp, nullptr, n_views);
+    sc->multi_active = false;
+    return render_start_single(sc, cams, &sp, nullptr, n_views);
 }
 
 // ---- instrumentation ---------------------------------------------------------------------------

@@ -112,6 +112,24 @@ class DistributedRenderer:
         rank 0 (h x w x 3 float64), None elsewhere.  No host synchronisation besides NCCL's own.
         counts: an (h, w) uint32 sample-count map (rt_render_start_counts; samples_number is then the cap), the WHOLE
         map on every rank; the assembled frame is the unsharded counts frame, bit for bit."""
+        if counts is None:
+            start = lambda p: api.render_start(self.dev_scene, camera, p)
+        else:
+            start = lambda p: api.render_start_counts(self.dev_scene, camera, p, counts)
+        return self._render_shard(start, width, height, samples_number)
+
+    def render_views_device(self, cameras, width: int, height: int, samples_number: int):
+        """render_device for several views in one frame (rt_render_start_views): every rank renders its tiles of the
+        stacked image (width, V * height) and passes the same cameras.  Returns the device frames on rank 0
+        (V x h x w x 3 float64, view v equal to render_device(cameras[v], ...) bit for bit), None elsewhere."""
+        cameras = api.check_cameras(cameras)
+        view = self._params(width, height, samples_number, self.rank)
+        frame = self._render_shard(lambda p: api.render_start_views(self.dev_scene, cameras, view),
+                                   width, len(cameras) * height, samples_number)
+        return None if frame is None else frame.view(len(cameras), height, width, 3)
+
+    def _render_shard(self, start, width: int, height: int, samples_number: int):
+        """start(params) this rank's shard of a width x height frame, gather, assemble on rank 0"""
         torch, dist = self.torch, self.dist
         p = self._params(width, height, samples_number, self.rank)
         # The library renders on its own non-blocking streams, the exchange runs on torch's / NCCL's: the
@@ -119,10 +137,7 @@ class DistributedRenderer:
         # previous frame's send (rank 0: copy) reads, so that read must be over before the frame starts.
         if self._exchanged is not None:
             self._exchanged.synchronize()
-        if counts is None:
-            api.render_start(self.dev_scene, camera, p)
-        else:
-            api.render_start_counts(self.dev_scene, camera, p, counts)
+        start(p)
         ptr, n = api.render_device_result(self.dev_scene)   # waits for this shard's kernels
         mine = torch.as_tensor(api.DevicePointer(ptr, (n, 4), "<f8", owner=self), device=f"cuda:{self.device}")
         counts = [api.shard_float4_count(p, s) for s in range(self.world)]
@@ -278,7 +293,13 @@ class DistributedRenderer:
         return out
 
     def render(self, camera: Camera, width: int, height: int, samples_number: int, counts=None) -> Optional[np.ndarray]:
-        frame = self.render_device(camera, width, height, samples_number, counts=counts)
+        return self._to_host(self.render_device(camera, width, height, samples_number, counts=counts))
+
+    def render_views(self, cameras, width: int, height: int, samples_number: int) -> Optional[np.ndarray]:
+        """render_views_device with the frames copied to the host on rank 0: (V, h, w, 3) float64, None elsewhere"""
+        return self._to_host(self.render_views_device(cameras, width, height, samples_number))
+
+    def _to_host(self, frame):
         if frame is None:
             return None
         torch = self.torch

@@ -100,6 +100,8 @@ extern "C" {
     pub fn rt_render_pixel_stats(scene: *mut rt_scene, counts: *mut u32, moments: *mut f64) -> c_int;
     pub fn rt_render_start_counts(scene: *mut rt_scene, camera: *const rt_camera, params: *const rt_render_params,
         counts: *const u32) -> c_int;
+    pub fn rt_render_start_views(scene: *mut rt_scene, cameras: *const rt_camera, n_views: u32,
+        params: *const rt_render_params) -> c_int;
     pub fn rt_render_device_result(scene: *mut rt_scene, d_accum: *mut *const c_void, n_float4: *mut u64) -> c_int;
     pub fn rt_shard_float4_count(params: *const rt_render_params, shard_index: u32) -> u64;
     pub fn rt_assemble_frame(scene: *mut rt_scene, params: *const rt_render_params, d_shards: *const *const c_void,

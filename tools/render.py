@@ -3,6 +3,7 @@
   python tools/render.py scenes/cornell_box.json out.png --size 1024 1024 --spp 256 [--depth 8] [--seed 1]
       [--adaptive REL [--min-samples N] [--abs-error A] [--heatmap counts.png]]
       [--counts MAP.npy [--heatmap counts.png]]
+      [--orbit N]
 
 Scene::from_json -> GpuRenderer (Renderer trait: start_rendering / render_step until done) ->
 rt_tonemap_rgba8 (sqrt, clamp(0, 0.999) * 256, on the device) -> PNG.  With --adaptive, an adaptive frame
@@ -11,7 +12,9 @@ standard error of its mean luminance exceeds REL times the mean (or --abs-error)
 sample counts as a grey PNG (black = min-samples, white = spp, log2 scale).  With --counts, a frame with the given
 sample count per pixel (rt_render_start_counts): MAP.npy is an (h, w) uint32 array, which sets the size; --heatmap
 then draws that map (black = 0 or 1 sample, white = its largest count, log2 scale) and the frame's count-0 pixels
-are black."""
+are black.  With --orbit N, one frame of N views (rt_render_start_views): the scene camera's position and direction
+rotated about the world y axis through the origin by 360/N degrees at a time; view k goes to OUT_k.png (out_000.png,
+out_001.png, ... for out.png)."""
 import argparse, os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -29,7 +32,10 @@ ap.add_argument("--min-samples", type=int, default=8)
 ap.add_argument("--abs-error", type=float, default=0.0)
 ap.add_argument("--counts", default=None, metavar="MAP.npy", help="(h, w) uint32 sample count per pixel")
 ap.add_argument("--heatmap", default=None, help="PNG of the per-pixel sample counts (with --adaptive or --counts)")
+ap.add_argument("--orbit", type=int, default=None, metavar="N", help="N views around the scene, one PNG per view")
 a = ap.parse_args()
+if a.orbit is not None and (a.orbit < 1 or a.adaptive is not None or a.counts is not None):
+    ap.error("--orbit needs N >= 1 and excludes --adaptive and --counts")
 if a.heatmap and a.adaptive is None and a.counts is None:
     ap.error("--heatmap needs --adaptive or --counts")
 if a.adaptive is not None and a.counts is not None:
@@ -44,6 +50,16 @@ if a.counts is not None:
         ap.error(f"--counts: an (h, w) uint32 array expected, got {given.dtype} {given.shape}")
     h, w = given.shape
 t0 = time.perf_counter()
+if a.orbit is not None:
+    views = r.render_views(rt.api.orbit_cameras(cam, a.orbit), w, h, a.spp)
+    dt = time.perf_counter() - t0
+    stem, ext = os.path.splitext(a.out)
+    for k in range(a.orbit):
+        rt.save_png(f"{stem}_{k:03d}{ext or '.png'}", rt.tonemap_rgba8(sc, views[k]))
+    paths = a.orbit * w * h * a.spp
+    print(f"{a.scene}: {a.orbit} views of {w}x{h}x{a.spp} in {dt * 1e3:.1f} ms ({paths / dt / 1e6:.1f} Mpaths/s) "
+          f"-> {stem}_000{ext or '.png'} .. {stem}_{a.orbit - 1:03d}{ext or '.png'}")
+    sys.exit(0)
 if a.counts is not None:
     buf = r.render_counts(cam, given)
     counts = given
