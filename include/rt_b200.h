@@ -203,6 +203,42 @@ int rt_scene_create_multi(const rt_scene_desc* desc, int n_devices, const int* d
 /* number of devices behind the handle (1 for rt_scene_create) */
 int rt_scene_device_count(rt_scene* scene);
 
+/* ---- scene updates on a live handle (the reference renders whatever its Arc<RwLock<Scene>> holds when a frame starts,
+ *      src/renderer/step_by_step.rs:37) ----------------------------------------------------------------------------
+ * Contract of both entries: after the call, every entry point (rt_intersect_batch[_device] in every mode and with
+ * every output, rt_render_start and the adaptive, counts and views frames, rt_trace_pixel_samples[_group][_device])
+ * gives bit for bit what a handle freshly created from the edited description gives.  The handle keeps its streams,
+ * lanes, buffers, peer access and settings.
+ *   - RT_ERR_STATE while a frame is in flight (that frame goes on with the old scene).
+ *   - Any update ends a progressive accumulation (rt_render_accumulated_samples reads 0; the next frame starts afresh
+ *     even with the same camera and params); rt_render_set_accumulate's switch stays as it is.
+ *   - The last completed frame stays readable (rt_render_device_frame, rt_render_device_result, rt_render_pixel_stats,
+ *     rt_tonemap_rgba8_device); rt_stats is untouched.
+ *   - An update is ordered after all work the handle enqueued before it, rt_intersect_batch_device and
+ *     rt_trace_pixel_samples_group_device calls on caller streams included, and work enqueued after it sees the new
+ *     scene.  For that, rt_intersect_batch_device on a caller stream records an event there at the end of each call
+ *     (one per stream; past 32 streams they are joined on an internal stream, never waited for on the host) and waits
+ *     for the last update's event.
+ *   - rt_scene_update_transforms allocates what it needs before the host copy of the tree changes; if the device work
+ *     then fails (a CUDA error), further transforms updates return RT_ERR_STATE until rt_scene_update rebuilds.
+ * A multi-device handle updates every device. */
+
+/* Replace the handle's scene by `desc` (any table sizes) on every device of the handle.  Validates exactly as
+ * rt_scene_create, before any device work; on any failure the handle keeps rendering the old scene bit for bit.
+ * Rebuilds everything rt_scene_create derives (cull tree, shade bins, marching tables, the wavefront-or-fused choice
+ * at 32 ray-marched shapes).  May synchronise the handle's devices: not a per-frame path. */
+int rt_scene_update(rt_scene* scene, const rt_scene_desc* desc);
+
+/* Move shapes: shape_index[i] gets inverse rows inverse[12 i ..] and direct rows direct[12 i ..] (rows 0..2 of
+ * InversableTransform, as in rt_scene_desc).  Kinds, params, materials and everything else stay.  Any transform values
+ * are accepted.  n = 0 does nothing; RT_ERR_INVALID for a NULL array with n > 0, an index >= n_shapes or an index
+ * listed twice.  The per-frame path of an animation: the cull tree keeps its topology and is REFIT (the balls of the
+ * nodes above the moved shapes are recomputed, every node still encloses its members, so culling stays exact; only
+ * its tightness can suffer -- rt_scene_update rebuilds), and O(n) bytes go to the device.  The arrays are copied
+ * before the call returns; no host synchronisation. */
+int rt_scene_update_transforms(rt_scene* scene, uint32_t n, const uint32_t* shape_index, const double* inverse,
+                               const double* direct);
+
 /* ---- batched nearest hit (replaces Scene::closest_hit, src/world/mod.rs:42-44, with the
  *      ShapeCollection semantics of src/world/shapes/mod.rs:573-597) -------------------- */
 
@@ -509,6 +545,13 @@ int rt_bernstein_clear(const double* coefficients, int degree, double length, do
  * Needs no device. */
 int rt_cull_tree_check(const rt_scene_desc* desc, uint32_t* n_roots, uint32_t* n_groups, uint32_t* n_tree,
                        uint32_t* n_flat, double* worst);
+
+/* Host-only check of the refit behind rt_scene_update_transforms: builds the tree for `desc` like rt_cull_tree_check,
+ * moves shapes shape_index[0 .. n) to inverse rows inverse[12 i ..] with the same host refit, and reports *worst with
+ * rt_cull_tree_check's metric against every shape's true ball after the move (a node that is never rejected encloses
+ * anything; a shape without a finite ball under a node that can be rejected gives +inf).  Needs no device. */
+int rt_cull_refit_check(const rt_scene_desc* desc, uint32_t n, const uint32_t* shape_index, const double* inverse,
+                        double* worst);
 
 /* Host-only emulation of the cull decisions k_extend takes (same FP32 operations, each rounded once): for every
  * ray, reached[r * n_shapes + i] = 1 when shape i would be handed to its exact test -- flat-list entry passed,

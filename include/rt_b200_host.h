@@ -41,6 +41,15 @@ uint32_t rth_scene_shape_count(rth_scene* scene);
 const char* rth_scene_shape_name(rth_scene* scene, uint32_t index);
 const char* rth_scene_material_name(rth_scene* scene, uint32_t index);
 int rth_scene_assign_material(rth_scene* scene, uint32_t shape_index, const char* material_name);
+/* Move shapes: shape index[i] gets the transform whose row-major 4x4 direct and inverse matrices are direct16[16 i ..] and
+ * inverse16[16 i ..] (rth_transform_new's outputs).  Edits the description in place (rth_scene_desc pointers stay
+ * valid) and applies rt_scene_update_transforms to every device handle the scene has created (rth_scene_device,
+ * rth_scene_device_multi), so that the scene and its handles stay in step.  RT_ERR_INVALID for a NULL array with n > 0,
+ * an index out of range or listed twice, before anything changes.  The handles are updated one after the other: when
+ * one rejects the update (a frame in flight on it) the call fails, the handles before it were updated and the
+ * description was not. */
+int rth_scene_set_transforms(rth_scene* scene, uint32_t n, const uint32_t* index, const double* direct16,
+                             const double* inverse16);
 /* the device-resident rt_scene (uploaded on first use); owned by the rth_scene */
 int rth_scene_device(rth_scene* scene, int device, rt_scene** out);
 /* ONE rt_scene over several devices (rt_scene_create_multi), created on first use per device list */

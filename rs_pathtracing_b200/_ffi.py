@@ -138,6 +138,8 @@ CORE_SYMBOLS = {
     "rt_scene_destroy": (None, [C.c_void_p]),
     "rt_scene_create_multi": (C.c_int, [C.POINTER(SceneDesc), C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_void_p)]),
     "rt_scene_device_count": (C.c_int, [C.c_void_p]),
+    "rt_scene_update": (C.c_int, [C.c_void_p, C.POINTER(SceneDesc)]),
+    "rt_scene_update_transforms": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rt_intersect_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.c_double, C.c_int,
                                      C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rt_intersect_batch_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.c_double, C.c_int,
@@ -180,6 +182,7 @@ CORE_SYMBOLS = {
     "rt_cull_reached": (C.c_int, [C.POINTER(SceneDesc), C.c_void_p, C.c_uint64, C.c_void_p]),
     "rt_cull_tree_check": (C.c_int, [C.POINTER(SceneDesc), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32),
                                     C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_double)]),
+    "rt_cull_refit_check": (C.c_int, [C.POINTER(SceneDesc), C.c_uint32, C.c_void_p, C.c_void_p, C.POINTER(C.c_double)]),
     "rt_measure_peaks": (C.c_int, [C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
 }
 
@@ -197,6 +200,7 @@ HOST_SYMBOLS = {
     "rth_scene_shape_name": (C.c_char_p, [C.c_void_p, C.c_uint32]),
     "rth_scene_material_name": (C.c_char_p, [C.c_void_p, C.c_uint32]),
     "rth_scene_assign_material": (C.c_int, [C.c_void_p, C.c_uint32, C.c_char_p]),
+    "rth_scene_set_transforms": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rth_scene_device": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p)]),
     "rth_scene_device_multi": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_void_p)]),
     "rth_camera_new": (C.c_int, [Vec3, Vec3, Vec3, C.c_double, C.c_double, C.POINTER(Camera)]),

@@ -164,6 +164,31 @@ class Scene:
     def assign_material(self, shape_index: int, material_name: str) -> None:
         _check(_ffi.host().rth_scene_assign_material(self._h, shape_index, material_name.encode()), host=True)
 
+    def set_transforms(self, index, translate, rotate_deg, scale) -> None:
+        """Move shapes: shape index[i] gets InversableTransform::new(translate[i], rotate_deg[i], scale[i]) (k x 3 each).
+        The description and every device handle this scene has created change together (rth_scene_set_transforms);
+        a frame started afterwards on any of them renders the moved shapes."""
+        index = np.asarray(index).reshape(-1)
+        if index.dtype.kind not in "ui" or (index.size and (index.min() < 0 or index.max() > 0xFFFFFFFF)):
+            raise ValueError("set_transforms: shape indices must be integers in [0, 2^32)")
+        index = index.astype(np.uint32)
+        t, r, s = (np.asarray(a, np.float64).reshape(-1, 3) for a in (translate, rotate_deg, scale))
+        if not (len(t) == len(r) == len(s) == index.reshape(-1).shape[0]):
+            raise ValueError("set_transforms: index, translate, rotate_deg and scale need one entry per shape")
+        rows = [transform(t[k], r[k], s[k]) for k in range(len(t))]
+        inv = np.array([x[0] for x in rows]).reshape(-1, 12)
+        direct = np.array([x[1] for x in rows]).reshape(-1, 12)
+        self.set_transform_rows(index, inv, direct)
+
+    def set_transform_rows(self, index, inverse, direct) -> None:
+        """set_transforms with the description's rows 0..2 given directly: index (k,) uint32, inverse and direct (k, 12)
+        float64, as api.update_transforms takes them"""
+        index, inverse, direct = check_transforms(index, inverse, direct)
+        pad = lambda a: np.ascontiguousarray(np.concatenate([a, np.tile([0.0, 0.0, 0.0, 1.0], (len(a), 1))], axis=1))
+        inv16, dir16 = pad(inverse), pad(direct)
+        p = lambda a: a.ctypes.data_as(C.c_void_p)
+        _check(_ffi.host().rth_scene_set_transforms(self._h, len(index), p(index), p(dir16), p(inv16)), host=True)
+
     def device_scene(self, device: Optional[int] = None) -> C.c_void_p:
         """the rt_scene handle on `device` (one per device, created on first use, alive as long as this Scene).
         device=None: the device last asked for explicitly (a renderer's), 0 at first."""
@@ -436,6 +461,73 @@ def render_start_adaptive(dev_scene, camera: Camera, params: RenderParams, min_s
     ap = _ffi.AdaptiveParams(min_samples, rel_error, abs_error)
     _check(_ffi.core().rt_render_start_adaptive(dev_scene, C.byref(camera), C.byref(params), C.byref(ap)))
     _started[_handle_key(dev_scene)] = (params.image.height, params.image.width, True)
+
+
+def transform(translate, rotate_deg, scale):
+    """InversableTransform::new: (inverse, direct) rows 0..2 as two float64 arrays of 12, the rows rt_scene_desc holds"""
+    direct = np.zeros(16, np.float64)
+    inverse = np.zeros(16, np.float64)
+    _check(_ffi.host().rth_transform_new(vec3(translate), vec3(rotate_deg), vec3(scale),
+                                         direct.ctypes.data_as(C.POINTER(C.c_double)),
+                                         inverse.ctypes.data_as(C.POINTER(C.c_double))), host=True)
+    return inverse[:12].copy(), direct[:12].copy()
+
+
+def translated_rows(inverse, direct, shift):
+    """the description rows (k, 12) of shapes moved by world-space offsets shift (k, 3), rotation and scale kept:
+    T' = translate(shift) o T, so direct's translation column gains shift and inverse's loses M^-1 shift"""
+    inverse = np.array(inverse, np.float64).reshape(-1, 3, 4)
+    direct = np.array(direct, np.float64).reshape(-1, 3, 4)
+    shift = np.asarray(shift, np.float64).reshape(-1, 3)
+    inverse[:, :, 3] -= np.einsum("kij,kj->ki", inverse[:, :, :3], shift)
+    direct[:, :, 3] += shift
+    return inverse.reshape(-1, 12), direct.reshape(-1, 12)
+
+
+def random_walk(scene: "Scene", index, n_frames: int, step: float, seed: int = 0):
+    """n_frames positions of the shapes `index` of `scene` on a seeded random walk in the x-z plane (N(0, step) per
+    axis and frame): a list of (index, inverse, direct), the arguments of update_transforms, one per frame"""
+    index = np.asarray(index, np.uint32)
+    d = scene.desc()
+    inv = np.ctypeslib.as_array(d.inverse, shape=(d.n_shapes, 12))[index].copy()
+    direct = np.ctypeslib.as_array(d.direct, shape=(d.n_shapes, 12))[index].copy()
+    rng = np.random.default_rng(seed)
+    frames = []
+    for _ in range(n_frames):
+        shift = rng.normal(0.0, step, (len(index), 3)) * (1.0, 0.0, 1.0)
+        inv, direct = translated_rows(inv, direct, shift)
+        frames.append((index, inv, direct))
+    return frames
+
+
+def scene_update(dev_scene, desc: _ffi.SceneDesc) -> None:
+    """rt_scene_update: the handle renders `desc` from now on (validated like rt_scene_create; on failure it keeps its
+    scene)"""
+    _check(_ffi.core().rt_scene_update(dev_scene, C.byref(desc)))
+
+
+def check_transforms(index, inverse, direct):
+    """the arguments of update_transforms as contiguous arrays: index (k,) uint32, inverse and direct (k, 12) float64"""
+    index = np.asarray(index)
+    inverse = np.asarray(inverse)
+    direct = np.asarray(direct)
+    if index.ndim != 1 or index.dtype != np.uint32:
+        raise ValueError(f"index must be a (k,) uint32 array, got {index.shape} {index.dtype}")
+    k = index.shape[0]
+    for name, a in (("inverse", inverse), ("direct", direct)):
+        if a.shape != (k, 12) or a.dtype != np.float64:
+            raise ValueError(f"{name} must be a ({k}, 12) float64 array, got {a.shape} {a.dtype}")
+    return (np.ascontiguousarray(index), np.ascontiguousarray(inverse), np.ascontiguousarray(direct))
+
+
+def update_transforms(dev_scene, index, inverse, direct) -> None:
+    """rt_scene_update_transforms: shapes index[i] get inverse rows inverse[i] and direct rows direct[i] (rows 0..2 of
+    InversableTransform); the cull tree is refit in place, nothing waits for the device.  This moves the shapes of this
+    handle only: for a handle of a Scene (Scene.device_scene) use Scene.set_transforms, which keeps the Scene's
+    description and all its handles in step."""
+    index, inverse, direct = check_transforms(index, inverse, direct)
+    p = lambda a: a.ctypes.data_as(C.c_void_p)
+    _check(_ffi.core().rt_scene_update_transforms(dev_scene, index.shape[0], p(index), p(inverse), p(direct)))
 
 
 def check_counts(counts, width: int, height: int) -> np.ndarray:

@@ -77,6 +77,11 @@ int rth_scene_assign_material(rth_scene* s, uint32_t shape_index, const char* na
     if (!s || !name) { g_err = "null argument"; return RT_ERR_INVALID; }
     return guarded([&] { s->scene->assign_material(shape_index, name); });
 }
+int rth_scene_set_transforms(rth_scene* s, uint32_t n, const uint32_t* index, const double* direct16,
+                             const double* inverse16) {
+    if (!s) { g_err = "null argument"; return RT_ERR_INVALID; }
+    return guarded([&] { s->scene->set_transforms(n, index, direct16, inverse16); });
+}
 int rth_scene_device(rth_scene* s, int device, rt_scene** out) {
     if (!s || !out) { g_err = "null argument"; return RT_ERR_INVALID; }
     return guarded([&] { *out = s->scene->device_scene(device); });

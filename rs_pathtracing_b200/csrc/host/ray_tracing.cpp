@@ -3,6 +3,7 @@
 // (compile with -ffp-contract=off); all tracing is delegated to the CUDA core via the C ABI.
 #include "ray_tracing.hpp"
 
+#include <algorithm>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -559,6 +560,33 @@ void Scene::assign_material(uint32_t shape_index, const std::string& material_na
             return;
         }
     throw std::runtime_error("material `" + material_name + "` not found");
+}
+
+void Scene::set_transforms(uint32_t n, const uint32_t* index, const double* direct16, const double* inverse16) {
+    if (n == 0) return;
+    if (!index || !direct16 || !inverse16) throw std::runtime_error("set_transforms: null array");
+    std::vector<uint32_t> sorted(index, index + n);
+    std::sort(sorted.begin(), sorted.end());
+    if (sorted.back() >= shape_count()) throw std::runtime_error("set_transforms: bad shape index");
+    if (std::adjacent_find(sorted.begin(), sorted.end()) != sorted.end())
+        throw std::runtime_error("set_transforms: a shape index is listed twice");
+    std::vector<double> inv((size_t)12 * n), dir((size_t)12 * n);   // rows 0..2, the rows the description holds
+    for (uint32_t k = 0; k < n; k++)
+        for (int j = 0; j < 12; j++) {
+            inv[(size_t)12 * k + j] = inverse16[(size_t)16 * k + j];
+            dir[(size_t)12 * k + j] = direct16[(size_t)16 * k + j];
+        }
+    std::vector<rt_scene*> handles;
+    for (auto& kv : dev_) handles.push_back(kv.second);
+    for (auto& kv : multi_) handles.push_back(kv.second);
+    for (rt_scene* h : handles)
+        if (rt_scene_update_transforms(h, n, index, inv.data(), dir.data()) != RT_OK)
+            throw std::runtime_error(std::string("rt_scene_update_transforms: ") + rt_last_error());
+    for (uint32_t k = 0; k < n; k++)
+        for (int j = 0; j < 12; j++) {
+            flat_.inverse[(size_t)12 * index[k] + j] = inv[(size_t)12 * k + j];
+            flat_.direct[(size_t)12 * index[k] + j] = dir[(size_t)12 * k + j];
+        }
 }
 
 // One rt_scene per device, created on first use and kept until the Scene dies: a handle given out for one device

@@ -152,6 +152,13 @@ public:
     // where every material / texture branch is live).  Must be called before the first device use.
     void assign_material(uint32_t shape_index, const std::string& material_name);
 
+    // Move shapes: shape index[i] gets the InversableTransform whose rows 0..3 are direct16[16 i ..] and inverse16[16 i ..]
+    // (row-major 4x4, as rth_transform_new gives them).  The description is edited and every device handle this scene
+    // has created gets rt_scene_update_transforms, so that the scene and its handles stay in step.  Throws on a bad or
+    // repeated index before anything changes; a handle that rejects the update (a frame in flight) throws after the
+    // handles before it were updated.
+    void set_transforms(uint32_t n, const uint32_t* index, const double* direct16, const double* inverse16);
+
     // Scene::closest_hit (:42-44) for a batch of rays — runs on the GPU.
     std::vector<RayHit> closest_hit(const std::vector<Ray>& rays, double min_t, double max_t,
                                     int mode = RT_ISECT_BRUTE, int device = 0);

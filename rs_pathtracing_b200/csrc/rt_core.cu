@@ -16,6 +16,7 @@
 //   k_counts_resolve    counts frames: a pixel's sums over its samples, continued across the pieces of a large pixel
 //   k_assemble          multi-GPU: gathered tile-packed shards -> frame
 //   k_tonemap           the bins' sqrt / clamp / *256 -> RGBA8
+//   k_scene_scatter     rt_scene_update_transforms: (slot, value) records of a refit into the scene's tables, in place
 // Compile with -fmad=false (see rt_math.cuh).
 #include <cuda_runtime.h>
 
@@ -957,6 +958,30 @@ k_counts_resolve(const float4* __restrict__ radiance, unsigned long long r0, uns
     frame[k] = rt_vec3{sx / n, sy / n, sz / n};
 }
 
+// rt_scene_update_transforms: one record = 16 bytes for one 16-byte slot of one table (a cull-table entry, or two
+// doubles of an inverse / direct row or of a flat record's inverse rows).  The host refit lists every slot once.
+enum { RT_SCATTER_CTAB = 0, RT_SCATTER_CUPPER, RT_SCATTER_CULL, RT_SCATTER_MARCH_CULL, RT_SCATTER_FREC, RT_SCATTER_INV,
+       RT_SCATTER_DIR, RT_SCATTER_TABLES };
+struct ScatterRec {
+    uint32_t table, pad;
+    uint64_t slot;
+    uint4 value;
+};
+struct ScatterDst {
+    uint4* p[RT_SCATTER_TABLES];
+};
+__global__ void __launch_bounds__(256)
+k_scene_scatter(ScatterDst dst, const ScatterRec* __restrict__ rec, uint32_t n) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const ScatterRec r = rec[i];
+    uint4* p = dst.p[0];   // a select chain: indexing the parameter array would copy it to the stack
+#pragma unroll
+    for (int k = 1; k < RT_SCATTER_TABLES; k++)
+        if (r.table == (uint32_t)k) p = dst.p[k];
+    p[r.slot] = r.value;
+}
+
 // FMA micro-benchmarks: 8 independent chains per thread, FMA counted as 2 flop
 template <typename T>
 __global__ void __launch_bounds__(256) k_fma_peak(T* out, int iters, T a, T b) {
@@ -995,6 +1020,156 @@ struct PathLane {
     std::vector<void*> qallocs;
     uint64_t path_capacity = 0;
 };
+
+// ---- what a scene description derives on a device (rt_scene_create, rt_scene_update) ------------------------------
+
+static float4 march_cull_entry(const double* inverse12, const double* q) {   // q: the shape's params row
+    double radius[3] = {q[7], q[7], q[7]};
+    if ((int)q[0] == RT_SURF_HEART) { radius[0] = 1.45; radius[1] = 1.45 / 2.05; radius[2] = 1.45; }  // march_bound
+    return cull_entry_march_bound(inverse12, radius);
+}
+
+// The host side of the cull tree a handle's tables were built from, kept for rt_scene_update_transforms: the tree with
+// its FP64 balls, the shapes' kinds, params and current inverse rows, and where each shape sits in the tables.
+struct SceneRefit {
+    CullTree ct;
+    std::vector<uint8_t> kind;
+    std::vector<double> params, inv;
+    std::vector<int> slot;      // [n_shapes] the shape's position in ct.ids (leaf or flat slot), -1: not in the analytic loop
+    std::vector<int> march_k;   // [n_shapes] the shape's position in the march list, -1: not ray-marched
+    bool no_cull = false, frec_on = false;
+};
+
+static SceneRefit make_refit(const rt_scene_desc* d, bool no_cull, bool no_tree, bool no_frec) {
+    SceneRefit s;
+    const int n = (int)d->n_shapes;
+    s.no_cull = no_cull;
+    s.ct = cull_build(d->inverse, d->kind, n, no_cull, no_tree || no_cull, d->params);
+    s.frec_on = s.ct.n_flat_real > 0 && s.ct.n_flat_real <= RT_FLAT_REC_MAX && !no_frec;
+    if (n > 0) {
+        s.kind.assign(d->kind, d->kind + n);
+        s.params.assign(d->params, d->params + (size_t)RT_SHAPE_PARAMS * n);
+        s.inv.assign(d->inverse, d->inverse + (size_t)12 * n);
+    }
+    s.slot.assign(n, -1);
+    for (size_t j = 0; j < s.ct.ids.size(); j++)
+        if (s.ct.ids[j] >= 0) s.slot[s.ct.ids[j]] = (int)j;
+    s.march_k.assign(n, -1);
+    for (int i = 0, k = 0; i < n; i++)
+        if (d->kind[i] == RT_SHAPE_MARCH) s.march_k[i] = k++;
+    return s;
+}
+
+// The refit of rt_scene_update_transforms.  Shapes idx[0 .. n) get inverse rows inverse[12 k ..] (and direct rows
+// direct[12 k ..], which only go to the device); their leaf entries, flat records and march-cull entries are recomputed
+// with the functions cull_build uses, then the balls of every group, root and upper node above a moved shape.
+// The one invariant it keeps is ENCLOSURE: every node ball encloses the balls of its members, the only property of the
+// tree the rejection proof in rt_cull.cuh uses.  So the refit tree culls exactly as safely as a rebuilt one; groups,
+// roots, table sizes, flat-list membership and ids stay, and a moved shape only costs tightness.  A member whose ball
+// is not finite (kappa > 30, singular, overflow) keeps its leaf entry's A = +inf inside its group and makes every node
+// above it never rejected.  `out` (may be null) receives one (table, 16-byte slot, value) record per slot written.
+static_assert(RT_FLAT_REC * sizeof(double) % 16 == 0, "flat records must be whole 16-byte slots for k_scene_scatter");
+// records a refit of n shapes writes at most: per shape 6 inverse, 6 direct, 6 flat-record slots, its own entry and its
+// table (or march-cull) entry, plus one group, one root and one node per upper level above it
+static uint64_t refit_record_bound(uint32_t n) { return (uint64_t)n * (20 + 2 + RT_CULL_UPPER_MAX); }
+
+static void refit(SceneRefit& s, uint32_t n, const uint32_t* idx, const double* inverse, const double* direct,
+                  std::vector<ScatterRec>* out) {
+    CullTree& ct = s.ct;
+    auto put = [&](uint32_t table, uint64_t slot, const void* v) {
+        if (!out) return;
+        ScatterRec r{table, 0, slot, {}};
+        memcpy(&r.value, v, sizeof r.value);
+        out->push_back(r);
+    };
+    auto put_row = [&](uint32_t table, uint64_t slot0, const double* row) {   // 12 doubles = 6 slots
+        for (int j = 0; j < 6; j++) put(table, slot0 + j, row + 2 * j);
+    };
+    auto enclose = [](const std::vector<CullBall>& m) {
+        for (const CullBall& b : m)
+            if (!(std::isfinite(b.r) && std::isfinite(b.c[0]) && std::isfinite(b.c[1]) && std::isfinite(b.c[2])))
+                return CullBall{{0.0, 0.0, 0.0}, INFINITY};
+        return cull_enclose(m);
+    };
+    auto node = [&](uint32_t table, uint64_t slot, float4* entry, const CullBall& b) {
+        *entry = cull_node_entry(b);   // A = +inf for an infinite ball: never rejected
+        put(table, slot, entry);
+    };
+    const size_t leaves0 = (size_t)ct.n_roots + ct.n_groups;   // table index of ids slot 0
+    std::vector<int> dirty;
+    for (uint32_t k = 0; k < n; k++) {
+        const uint32_t i = idx[k];
+        const double* m = inverse + (size_t)12 * k;
+        memcpy(&s.inv[(size_t)12 * i], m, 12 * sizeof(double));
+        put_row(RT_SCATTER_INV, (uint64_t)6 * i, m);
+        if (direct) put_row(RT_SCATTER_DIR, (uint64_t)6 * i, direct + (size_t)12 * k);
+        const double* q = &s.params[(size_t)RT_SHAPE_PARAMS * i];
+        if (s.kind[i] == RT_SHAPE_MARCH) {
+            float4 e = march_cull_entry(m, q);
+            if (s.no_cull) e.w = INFINITY;
+            put(RT_SCATTER_MARCH_CULL, (uint64_t)s.march_k[i], &e);
+            continue;
+        }
+        CullBall b;
+        const float4 e = cull_leaf(m, s.kind[i], q, s.no_cull, &b);
+        if (!(std::isfinite(e.w) && std::isfinite(b.r))) b = CullBall{{0.0, 0.0, 0.0}, INFINITY};
+        ct.leaf[i] = e;
+        ct.leaf_ball[i] = b;
+        put(RT_SCATTER_CULL, i, &e);
+        const int j = s.slot[i];
+        ct.table[leaves0 + j] = e;
+        put(RT_SCATTER_CTAB, leaves0 + j, &e);
+        if (ct.group_of[i] >= 0) {
+            dirty.push_back(ct.group_of[i]);
+        } else if (s.frec_on) {
+            const size_t f = (size_t)j - (size_t)RT_CULL_GROUP * ct.n_groups;   // flat record f: inverse rows first
+            put_row(RT_SCATTER_FREC, (uint64_t)(RT_FLAT_REC * sizeof(double) / 16) * f, m);
+        }
+    }
+    auto settle = [](std::vector<int>& v) {
+        std::sort(v.begin(), v.end());
+        v.erase(std::unique(v.begin(), v.end()), v.end());
+    };
+    settle(dirty);
+    std::vector<int> up;
+    for (int g : dirty) {
+        std::vector<CullBall> m;
+        for (int k = 0; k < RT_CULL_GROUP; k++) {
+            const int id = ct.ids[(size_t)RT_CULL_GROUP * g + k];
+            if (id >= 0) m.push_back(ct.leaf_ball[id]);
+        }
+        ct.group_ball[g] = enclose(m);
+        ct.group_radius[g] = ct.group_ball[g].r;
+        node(RT_SCATTER_CTAB, (uint64_t)ct.n_roots + g, &ct.table[(size_t)ct.n_roots + g], ct.group_ball[g]);
+        up.push_back(g / RT_CULL_ROOT_FANOUT);
+    }
+    settle(up);
+    dirty.swap(up);
+    up.clear();
+    for (int r : dirty) {
+        std::vector<CullBall> m(ct.group_ball.begin() + (size_t)r * RT_CULL_ROOT_FANOUT,
+                                ct.group_ball.begin() + std::min(ct.group_ball.size(), (size_t)(r + 1) * RT_CULL_ROOT_FANOUT));
+        ct.root_ball[r] = enclose(m);
+        node(RT_SCATTER_CTAB, (uint64_t)r, &ct.table[r], ct.root_ball[r]);
+        up.push_back(r / 32);
+    }
+    for (int l = 1; l <= ct.n_upper; l++) {
+        settle(up);
+        dirty.swap(up);
+        up.clear();
+        const CullBall* below = l == 1 ? ct.root_ball.data() : ct.upper_ball.data() + ct.upper_off[l - 1];
+        const int n_below = l == 1 ? ct.n_roots : ct.upper_count[l - 1];
+        for (int i : dirty) {
+            std::vector<CullBall> m;
+            for (int k = 32 * i; k < std::min(32 * i + 32, n_below); k++)
+                if (below[k].r >= 0.0) m.push_back(below[k]);
+            const size_t at = (size_t)ct.upper_off[l] + i;
+            ct.upper_ball[at] = enclose(m);
+            node(RT_SCATTER_CUPPER, at, &ct.upper[at], ct.upper_ball[at]);
+            up.push_back(i / 32);
+        }
+    }
+}
 
 struct rt_scene {
     int device = 0;
@@ -1105,18 +1280,19 @@ struct rt_scene {
     std::vector<RayCasterDev> h_views;
     RayCasterDev* d_views = nullptr;
     uint64_t views_cap = 0;
+    // scene updates (rt_scene_update[_transforms]): the host side of the cull tree the tables were built from (a
+    // multi-device handle refits its first device's and applies the records on every device), the pinned staging and
+    // the device copy of a refit's records, the event after which the staging may be rewritten, the event of the last
+    // update, and per caller stream of rt_intersect_batch_device the event recorded at the end of its last call there
+    SceneRefit refit;
+    ScatterRec* h_scatter = nullptr;
+    ScatterRec* d_scatter = nullptr;
+    uint64_t h_scatter_cap = 0, d_scatter_cap = 0;
+    cudaEvent_t ev_scatter_read = nullptr, ev_update = nullptr;
+    std::vector<std::pair<cudaStream_t, cudaEvent_t>> caller_done;
+    cudaStream_t fold_stream = nullptr;   // joins the caller events when more than 32 streams have been seen
+    bool refit_broken = false;   // a transforms update reached the host tree but not every device (rt_scene_update clears it)
 };
-
-template <class T>
-static int upload(rt_scene* sc, const T* src, size_t count, const T** out) {
-    void* d = nullptr;
-    size_t bytes = std::max<size_t>(count * sizeof(T), 16);
-    CU(cudaMalloc(&d, bytes));
-    sc->allocs.push_back(d);
-    if (count) CU(cudaMemcpy(d, src, count * sizeof(T), cudaMemcpyHostToDevice));
-    *out = (const T*)d;
-    return RT_OK;
-}
 
 template <class T>
 static int ensure_device_array(T*& p, uint64_t& cap, uint64_t n) {   // persistent buffer, grown on demand
@@ -1133,6 +1309,189 @@ static size_t env_size(const char* name, size_t dflt) {
     const char* v = getenv(name);
     if (!v || !*v) return dflt;
     return (size_t)strtoull(v, nullptr, 10);
+}
+
+// Everything rt_scene_create derives from a description on one device: the tables (owned by `allocs`), the launch
+// policy read from them, and the host side of the cull tree.
+struct SceneTables {
+    DevScene ds{};
+    std::vector<void*> allocs;
+    bool use_smem = false;
+    size_t smem_bytes = 0;
+    int grid = 0, grid_extend = 0, grid_march = 0, grid_shade = 0;
+    uint32_t kind_mask[6] = {0, 0, 0, 0, 0, 0};
+    bool wavefront = true, shade_binned = false;
+    int n_shade_bins = 0;
+    SceneRefit refit;
+};
+
+template <class T>
+static int upload(std::vector<void*>& allocs, const T* src, size_t count, const T** out) {
+    void* d = nullptr;
+    size_t bytes = std::max<size_t>(count * sizeof(T), 16);
+    CU(cudaMalloc(&d, bytes));
+    allocs.push_back(d);
+    if (count) CU(cudaMemcpy(d, src, count * sizeof(T), cudaMemcpyHostToDevice));
+    *out = (const T*)d;
+    return RT_OK;
+}
+
+// Builds the tables of a validated description on the current device (a device of n_sm SMs and smem_optin bytes of
+// opt-in shared memory per block).  On failure t.allocs holds what was allocated.
+static int build_tables(const rt_scene_desc* d, int n_sm, size_t smem_optin, SceneTables& t) {
+    int rc = RT_OK;
+    const bool no_cull = getenv("RT_B200_NO_CULL") != nullptr;
+    const uint32_t n = d->n_shapes;
+    t.ds.n_shapes = (int)n;
+    if ((rc = upload(t.allocs, d->inverse, (size_t)n * 12, &t.ds.inv)) != RT_OK) return rc;
+    if ((rc = upload(t.allocs, d->direct, (size_t)n * 12, &t.ds.dir)) != RT_OK) return rc;
+    if ((rc = upload(t.allocs, d->params, (size_t)n * RT_SHAPE_PARAMS, &t.ds.params)) != RT_OK) return rc;
+    if ((rc = upload(t.allocs, d->kind, (size_t)n, &t.ds.kind)) != RT_OK) return rc;
+    if ((rc = upload(t.allocs, d->flags, (size_t)n, &t.ds.flags)) != RT_OK) return rc;
+    if ((rc = upload(t.allocs, d->material, (size_t)n, &t.ds.material)) != RT_OK) return rc;
+    if ((rc = upload(t.allocs, d->materials, (size_t)d->n_materials, &t.ds.materials)) != RT_OK) return rc;
+    if ((rc = upload(t.allocs, d->textures, (size_t)d->n_textures, &t.ds.textures)) != RT_OK) return rc;
+    {   // shade keys: one bin per (material kind, root texture kind) pair present in the scene (k_shade, BINNED)
+        std::vector<uint8_t> mat_bin(d->n_materials, 0);
+        std::vector<int> seen;   // pair codes in order of first appearance
+        for (uint32_t i = 0; i < d->n_materials; i++) {
+            const rt_material& m = d->materials[i];
+            const bool has_tex = m.kind == RT_MAT_LAMBERTIAN || m.kind == RT_MAT_METAL || m.kind == RT_MAT_DIFFUSE_LIGHT;
+            int code = (int)m.kind * 16 + (has_tex ? (int)d->textures[m.texture].kind : 15);
+            if (m.kind == RT_MAT_METAL && m.scalar == 0.0) code += 8;   // (a mirror draws no unit-ball sample)
+            size_t b = std::find(seen.begin(), seen.end(), code) - seen.begin();
+            if (b == seen.size()) seen.push_back(code);
+            mat_bin[i] = (uint8_t)std::min<size_t>(b, RT_SHADE_MAX_BINS - 1);
+        }
+        if ((rc = upload(t.allocs, mat_bin.data(), mat_bin.size(), &t.ds.mat_bin)) != RT_OK) return rc;
+        // Binning pays when a warp in arrival order would see many keys: measured on the all-materials variant of
+        // detached_materials.json (8 keys; k_shade at bounce levels 1 / 2: 15 / 13 -> 28 / 28 of 32 lanes, 332 / 142 ->
+        // 188 / 83 us, frame + 8 %) against cornell_box.json (4 keys, nearly every hit Lambertian: - 0.6 %).  So: on
+        // by default when the shapes of the scene reference at least 5 different keys; RT_B200_SHADE_BINNED=0 / 1 overrides.
+        std::vector<char> used(seen.size(), 0);
+        for (uint32_t i = 0; i < n; i++) used[std::min<size_t>(mat_bin[d->material[i]], used.size() - 1)] = 1;
+        t.n_shade_bins = (int)std::count(used.begin(), used.end(), 1);
+        const char* sb = getenv("RT_B200_SHADE_BINNED");
+        t.shade_binned = sb ? atoi(sb) != 0 : t.n_shade_bins >= 5;
+    }
+    std::vector<DevImage> imgs(d->n_images);
+    for (uint32_t i = 0; i < d->n_images; i++) {
+        imgs[i].width = d->images[i].width;
+        imgs[i].height = d->images[i].height;
+        if ((rc = upload(t.allocs, d->images[i].rgba, (size_t)4 * imgs[i].width * imgs[i].height, &imgs[i].rgba)) != RT_OK) return rc;
+    }
+    if ((rc = upload(t.allocs, imgs.data(), imgs.size(), &t.ds.images)) != RT_OK) return rc;
+    if ((rc = upload(t.allocs, d->noise, (size_t)d->n_noise, &t.ds.noise)) != RT_OK) return rc;
+    std::vector<int> march;
+    for (uint32_t i = 0; i < n; i++)
+        if (d->kind[i] == RT_SHAPE_MARCH) march.push_back((int)i);
+    t.ds.n_march = (int)march.size();
+    if ((rc = upload(t.allocs, march.data(), march.size(), &t.ds.march_index)) != RT_OK) return rc;
+    // exact-skip marching: gradient bound of each marched surface over its region (rt_march.cuh)
+    std::vector<double> march_G(march.size());
+    for (size_t k = 0; k < march.size(); k++) {
+        double H;
+        bounds::region_bounds(d->params + (size_t)march[k] * RT_SHAPE_PARAMS, &march_G[k], &H);
+        if (getenv("RT_B200_NO_MARCH_SKIP")) march_G[k] = INFINITY;
+    }
+    if ((rc = upload(t.allocs, march_G.data(), march_G.size(), &t.ds.march_G)) != RT_OK) return rc;
+    std::vector<double> march_F(march.size());
+    for (size_t k = 0; k < march.size(); k++) {
+        const double* q = d->params + (size_t)march[k] * RT_SHAPE_PARAMS;
+        march_F[k] = bounds::region_magnitude(q);
+        if (k < 32) t.kind_mask[(int)q[0]] |= 1u << k;
+    }
+    if ((rc = upload(t.allocs, march_F.data(), march_F.size(), &t.ds.march_F)) != RT_OK) return rc;
+    std::vector<float4> march_cull(march.size());
+    for (size_t k = 0; k < march.size(); k++) {
+        const double* q = d->params + (size_t)march[k] * RT_SHAPE_PARAMS;
+        march_cull[k] = march_cull_entry(d->inverse + (size_t)12 * march[k], q);
+        if (no_cull) march_cull[k].w = INFINITY;
+    }
+    if ((rc = upload(t.allocs, march_cull.data(), march_cull.size(), &t.ds.march_cull)) != RT_OK) return rc;
+
+    // conservative cull tree (rt_cull.cuh)
+    {
+        t.refit = make_refit(d, no_cull, getenv("RT_B200_NO_CULL_TREE") != nullptr, getenv("RT_B200_NO_FLAT_REC") != nullptr);
+        const CullTree& ct = t.refit.ct;
+        t.ds.n_roots = ct.n_roots;
+        t.ds.n_upper = ct.n_upper;
+        for (int l = 0; l <= RT_CULL_UPPER_MAX; l++) t.ds.upper_off[l] = ct.upper_off[l];
+        if ((rc = upload(t.allocs, ct.upper.data(), ct.upper.size(), &t.ds.cupper)) != RT_OK) return rc;
+        t.ds.n_groups = ct.n_groups;
+        t.ds.n_flat = ct.n_flat;
+        t.ds.n_flat_real = ct.n_flat_real;
+        if ((rc = upload(t.allocs, ct.table.data(), ct.table.size(), &t.ds.ctab)) != RT_OK) return rc;
+        if ((rc = upload(t.allocs, ct.ids.data(), ct.ids.size(), &t.ds.cids)) != RT_OK) return rc;
+        if ((rc = upload(t.allocs, ct.leaf.data(), ct.leaf.size(), &t.ds.cull)) != RT_OK) return rc;
+        if ((rc = upload(t.allocs, ct.group_of.data(), ct.group_of.size(), &t.ds.cull_group)) != RT_OK) return rc;
+        // the flat list's shapes as self-contained records (rt_scene.cuh, FlatRec): inverse rows, Rectangle
+        // bounds, index and kind side by side, so that the exact test of flat entry j starts from one address
+        // known in advance instead of the chain cids[j] -> kind[id] -> inv[12 id] of dependent loads
+        t.ds.n_frec = 0;
+        t.ds.frec = nullptr;
+        if (t.refit.frec_on) {
+            std::vector<double> frec((size_t)RT_FLAT_REC * ct.n_flat_real, 0.0);
+            for (int k = 0; k < ct.n_flat_real; k++) {
+                const int id = ct.ids[(size_t)RT_CULL_GROUP * ct.n_groups + k];
+                double* r = frec.data() + (size_t)RT_FLAT_REC * k;
+                for (int j = 0; j < 12; j++) r[j] = d->inverse[(size_t)12 * id + j];
+                for (int j = 0; j < 4; j++) r[12 + j] = d->params[(size_t)RT_SHAPE_PARAMS * id + j];
+                const int tag[2] = {id, (int)d->kind[id]};
+                memcpy(r + 16, tag, sizeof tag);
+            }
+            if ((rc = upload(t.allocs, frec.data(), frec.size(), &t.ds.frec)) != RT_OK) return rc;
+            t.ds.n_frec = ct.n_flat_real;
+        }
+    }
+    // shared-memory staging: 16 B per table entry + the flat list's records
+    t.smem_bytes = (size_t)t.ds.ctab_entries() * sizeof(float4) + (size_t)t.ds.n_frec * RT_FLAT_REC * sizeof(double);
+    t.use_smem = n > 0 && t.smem_bytes > 0 && t.smem_bytes <= smem_optin;
+    if (!t.use_smem) t.smem_bytes = 0;
+    if (t.smem_bytes > 48 * 1024) {
+        cudaFuncSetAttribute(k_intersect_batch<false, RT_ISECT_BRUTE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
+        cudaFuncSetAttribute(k_intersect_batch<true, RT_ISECT_BRUTE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
+        cudaFuncSetAttribute(k_intersect_batch<false, RT_ISECT_FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
+        cudaFuncSetAttribute(k_intersect_batch<true, RT_ISECT_FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
+        cudaFuncSetAttribute(k_intersect_batch<false, RT_ISECT_VERIFY>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
+        cudaFuncSetAttribute(k_bounce<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
+        cudaFuncSetAttribute(k_bounce<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
+        cudaFuncSetAttribute(k_extend<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
+        cudaFuncSetAttribute(k_extend<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
+        cudaFuncSetAttribute(k_extend<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
+        cudaFuncSetAttribute(k_extend<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
+    }
+    // persistent grid: a whole number of CTAs per SM
+    int per_sm = 0;
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_bounce<false>, 256, t.smem_bytes);
+    if (per_sm < 1) per_sm = 1;
+    t.grid = n_sm * per_sm;
+    auto occ_grid = [&](auto kernel, int threads, size_t smem) {
+        int b = 0;
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, kernel, threads, smem);
+        return n_sm * std::max(b, 1);
+    };
+    t.grid_extend = occ_grid(k_extend<false, true>, 256, t.smem_bytes);
+    t.grid_march = n_sm * rt_march_occupancy();
+    t.grid_shade = occ_grid(k_shade<false, true>, 256, 0);
+    t.wavefront = t.ds.n_march <= 32 && !getenv("RT_B200_FUSED_BOUNCE");
+    return RT_OK;
+}
+
+static void install_tables(rt_scene* sc, SceneTables& t) {   // t receives the tables the handle had
+    std::swap(sc->ds, t.ds);
+    std::swap(sc->allocs, t.allocs);
+    sc->use_smem = t.use_smem;
+    sc->smem_bytes = t.smem_bytes;
+    sc->grid = t.grid;
+    sc->grid_extend = t.grid_extend;
+    sc->grid_march = t.grid_march;
+    sc->grid_shade = t.grid_shade;
+    memcpy(sc->kind_mask, t.kind_mask, sizeof t.kind_mask);
+    sc->wavefront = t.wavefront;
+    sc->shade_binned = t.shade_binned;
+    sc->n_shade_bins = t.n_shade_bins;
+    std::swap(sc->refit, t.refit);
 }
 
 extern "C" {
@@ -1250,142 +1609,12 @@ int rt_scene_create(const rt_scene_desc* d, int device, rt_scene** out) {
         cudaEventCreateWithFlags(&sc->ev_adaptive_fork, cudaEventDisableTiming) != cudaSuccess)
         return bail(fail(RT_ERR_CUDA, "cudaEventCreate failed"));
 
-    const uint32_t n = d->n_shapes;
-    sc->ds.n_shapes = (int)n;
-    if ((rc = upload(sc, d->inverse, (size_t)n * 12, &sc->ds.inv)) != RT_OK) return bail(rc);
-    if ((rc = upload(sc, d->direct, (size_t)n * 12, &sc->ds.dir)) != RT_OK) return bail(rc);
-    if ((rc = upload(sc, d->params, (size_t)n * RT_SHAPE_PARAMS, &sc->ds.params)) != RT_OK) return bail(rc);
-    if ((rc = upload(sc, d->kind, (size_t)n, &sc->ds.kind)) != RT_OK) return bail(rc);
-    if ((rc = upload(sc, d->flags, (size_t)n, &sc->ds.flags)) != RT_OK) return bail(rc);
-    if ((rc = upload(sc, d->material, (size_t)n, &sc->ds.material)) != RT_OK) return bail(rc);
-    if ((rc = upload(sc, d->materials, (size_t)d->n_materials, &sc->ds.materials)) != RT_OK) return bail(rc);
-    if ((rc = upload(sc, d->textures, (size_t)d->n_textures, &sc->ds.textures)) != RT_OK) return bail(rc);
-    {   // shade keys: one bin per (material kind, root texture kind) pair present in the scene (k_shade, BINNED)
-        std::vector<uint8_t> mat_bin(d->n_materials, 0);
-        std::vector<int> seen;   // pair codes in order of first appearance
-        for (uint32_t i = 0; i < d->n_materials; i++) {
-            const rt_material& m = d->materials[i];
-            const bool has_tex = m.kind == RT_MAT_LAMBERTIAN || m.kind == RT_MAT_METAL || m.kind == RT_MAT_DIFFUSE_LIGHT;
-            int code = (int)m.kind * 16 + (has_tex ? (int)d->textures[m.texture].kind : 15);
-            if (m.kind == RT_MAT_METAL && m.scalar == 0.0) code += 8;   // (a mirror draws no unit-ball sample)
-            size_t b = std::find(seen.begin(), seen.end(), code) - seen.begin();
-            if (b == seen.size()) seen.push_back(code);
-            mat_bin[i] = (uint8_t)std::min<size_t>(b, RT_SHADE_MAX_BINS - 1);
-        }
-        if ((rc = upload(sc, mat_bin.data(), mat_bin.size(), &sc->ds.mat_bin)) != RT_OK) return bail(rc);
-        // Binning pays when a warp in arrival order would see many keys: measured on the all-materials variant of
-        // detached_materials.json (8 keys; k_shade at bounce levels 1 / 2: 15 / 13 -> 28 / 28 of 32 lanes, 332 / 142 ->
-        // 188 / 83 us, frame + 8 %) against cornell_box.json (4 keys, nearly every hit Lambertian: - 0.6 %).  So: on
-        // by default when the shapes of the scene reference at least 5 different keys; RT_B200_SHADE_BINNED=0 / 1 overrides.
-        std::vector<char> used(seen.size(), 0);
-        for (uint32_t i = 0; i < n; i++) used[std::min<size_t>(mat_bin[d->material[i]], used.size() - 1)] = 1;
-        sc->n_shade_bins = (int)std::count(used.begin(), used.end(), 1);
-        const char* sb = getenv("RT_B200_SHADE_BINNED");
-        sc->shade_binned = sb ? atoi(sb) != 0 : sc->n_shade_bins >= 5;
+    SceneTables t;
+    if ((rc = build_tables(d, sc->n_sm, sc->smem_optin, t)) != RT_OK) {
+        for (void* p : t.allocs) cudaFree(p);
+        return bail(rc);
     }
-    std::vector<DevImage> imgs(d->n_images);
-    for (uint32_t i = 0; i < d->n_images; i++) {
-        imgs[i].width = d->images[i].width;
-        imgs[i].height = d->images[i].height;
-        if ((rc = upload(sc, d->images[i].rgba, (size_t)4 * imgs[i].width * imgs[i].height, &imgs[i].rgba)) != RT_OK) return bail(rc);
-    }
-    if ((rc = upload(sc, imgs.data(), imgs.size(), &sc->ds.images)) != RT_OK) return bail(rc);
-    if ((rc = upload(sc, d->noise, (size_t)d->n_noise, &sc->ds.noise)) != RT_OK) return bail(rc);
-    std::vector<int> march;
-    for (uint32_t i = 0; i < n; i++)
-        if (d->kind[i] == RT_SHAPE_MARCH) march.push_back((int)i);
-    sc->ds.n_march = (int)march.size();
-    if ((rc = upload(sc, march.data(), march.size(), &sc->ds.march_index)) != RT_OK) return bail(rc);
-    // exact-skip marching: gradient bound of each marched surface over its region (rt_march.cuh)
-    std::vector<double> march_G(march.size());
-    for (size_t k = 0; k < march.size(); k++) {
-        double H;
-        bounds::region_bounds(d->params + (size_t)march[k] * RT_SHAPE_PARAMS, &march_G[k], &H);
-        if (getenv("RT_B200_NO_MARCH_SKIP")) march_G[k] = INFINITY;
-    }
-    if ((rc = upload(sc, march_G.data(), march_G.size(), &sc->ds.march_G)) != RT_OK) return bail(rc);
-    std::vector<double> march_F(march.size());
-    for (size_t k = 0; k < march.size(); k++) {
-        const double* q = d->params + (size_t)march[k] * RT_SHAPE_PARAMS;
-        march_F[k] = bounds::region_magnitude(q);
-        if (k < 32) sc->kind_mask[(int)q[0]] |= 1u << k;
-    }
-    if ((rc = upload(sc, march_F.data(), march_F.size(), &sc->ds.march_F)) != RT_OK) return bail(rc);
-    std::vector<float4> march_cull(march.size());
-    for (size_t k = 0; k < march.size(); k++) {
-        const double* q = d->params + (size_t)march[k] * RT_SHAPE_PARAMS;
-        double radius[3] = {q[7], q[7], q[7]};
-        if ((int)q[0] == RT_SURF_HEART) { radius[0] = 1.45; radius[1] = 1.45 / 2.05; radius[2] = 1.45; }  // march_bound
-        march_cull[k] = cull_entry_march_bound(d->inverse + (size_t)12 * march[k], radius);
-        if (getenv("RT_B200_NO_CULL")) march_cull[k].w = INFINITY;
-    }
-    if ((rc = upload(sc, march_cull.data(), march_cull.size(), &sc->ds.march_cull)) != RT_OK) return bail(rc);
-
-    // conservative cull tree (rt_cull.cuh)
-    {
-        CullTree ct = cull_build(d->inverse, d->kind, (int)n, getenv("RT_B200_NO_CULL") != nullptr,
-                                 getenv("RT_B200_NO_CULL_TREE") != nullptr || getenv("RT_B200_NO_CULL") != nullptr, d->params);
-        sc->ds.n_roots = ct.n_roots;
-        sc->ds.n_upper = ct.n_upper;
-        for (int l = 0; l <= RT_CULL_UPPER_MAX; l++) sc->ds.upper_off[l] = ct.upper_off[l];
-        if ((rc = upload(sc, ct.upper.data(), ct.upper.size(), &sc->ds.cupper)) != RT_OK) return bail(rc);
-        sc->ds.n_groups = ct.n_groups;
-        sc->ds.n_flat = ct.n_flat;
-        sc->ds.n_flat_real = ct.n_flat_real;
-        if ((rc = upload(sc, ct.table.data(), ct.table.size(), &sc->ds.ctab)) != RT_OK) return bail(rc);
-        if ((rc = upload(sc, ct.ids.data(), ct.ids.size(), &sc->ds.cids)) != RT_OK) return bail(rc);
-        if ((rc = upload(sc, ct.leaf.data(), ct.leaf.size(), &sc->ds.cull)) != RT_OK) return bail(rc);
-        if ((rc = upload(sc, ct.group_of.data(), ct.group_of.size(), &sc->ds.cull_group)) != RT_OK) return bail(rc);
-        // the flat list's shapes as self-contained records (rt_scene.cuh, FlatRec): inverse rows, Rectangle
-        // bounds, index and kind side by side, so that the exact test of flat entry j starts from one address
-        // known in advance instead of the chain cids[j] -> kind[id] -> inv[12 id] of dependent loads
-        sc->ds.n_frec = 0;
-        sc->ds.frec = nullptr;
-        if (ct.n_flat_real > 0 && ct.n_flat_real <= RT_FLAT_REC_MAX && !getenv("RT_B200_NO_FLAT_REC")) {
-            std::vector<double> frec((size_t)RT_FLAT_REC * ct.n_flat_real, 0.0);
-            for (int k = 0; k < ct.n_flat_real; k++) {
-                const int id = ct.ids[(size_t)RT_CULL_GROUP * ct.n_groups + k];
-                double* r = frec.data() + (size_t)RT_FLAT_REC * k;
-                for (int j = 0; j < 12; j++) r[j] = d->inverse[(size_t)12 * id + j];
-                for (int j = 0; j < 4; j++) r[12 + j] = d->params[(size_t)RT_SHAPE_PARAMS * id + j];
-                const int tag[2] = {id, (int)d->kind[id]};
-                memcpy(r + 16, tag, sizeof tag);
-            }
-            if ((rc = upload(sc, frec.data(), frec.size(), &sc->ds.frec)) != RT_OK) return bail(rc);
-            sc->ds.n_frec = ct.n_flat_real;
-        }
-    }
-    // shared-memory staging: 16 B per table entry + the flat list's records
-    sc->smem_bytes = (size_t)sc->ds.ctab_entries() * sizeof(float4) + (size_t)sc->ds.n_frec * RT_FLAT_REC * sizeof(double);
-    sc->use_smem = n > 0 && sc->smem_bytes > 0 && sc->smem_bytes <= sc->smem_optin;
-    if (!sc->use_smem) sc->smem_bytes = 0;
-    if (sc->smem_bytes > 48 * 1024) {
-        cudaFuncSetAttribute(k_intersect_batch<false, RT_ISECT_BRUTE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sc->smem_bytes);
-        cudaFuncSetAttribute(k_intersect_batch<true, RT_ISECT_BRUTE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sc->smem_bytes);
-        cudaFuncSetAttribute(k_intersect_batch<false, RT_ISECT_FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sc->smem_bytes);
-        cudaFuncSetAttribute(k_intersect_batch<true, RT_ISECT_FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sc->smem_bytes);
-        cudaFuncSetAttribute(k_intersect_batch<false, RT_ISECT_VERIFY>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sc->smem_bytes);
-        cudaFuncSetAttribute(k_bounce<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sc->smem_bytes);
-        cudaFuncSetAttribute(k_bounce<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sc->smem_bytes);
-        cudaFuncSetAttribute(k_extend<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sc->smem_bytes);
-        cudaFuncSetAttribute(k_extend<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sc->smem_bytes);
-        cudaFuncSetAttribute(k_extend<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sc->smem_bytes);
-        cudaFuncSetAttribute(k_extend<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sc->smem_bytes);
-    }
-    // persistent grid: a whole number of CTAs per SM
-    int per_sm = 0;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_bounce<false>, 256, sc->smem_bytes);
-    if (per_sm < 1) per_sm = 1;
-    sc->grid = sc->n_sm * per_sm;
-    auto occ_grid = [&](auto kernel, int threads, size_t smem) {
-        int b = 0;
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, kernel, threads, smem);
-        return sc->n_sm * std::max(b, 1);
-    };
-    sc->grid_extend = occ_grid(k_extend<false, true>, 256, sc->smem_bytes);
-    sc->grid_march = sc->n_sm * rt_march_occupancy();
-    sc->grid_shade = occ_grid(k_shade<false, true>, 256, 0);
-    sc->wavefront = sc->ds.n_march <= 32 && !getenv("RT_B200_FUSED_BOUNCE");
+    install_tables(sc, t);
 
     if (cudaMalloc(&sc->d_counters, sizeof(DevCounters)) != cudaSuccess) return bail(fail(RT_ERR_NOMEM, "cudaMalloc failed"));
     cudaMemset(sc->d_counters, 0, sizeof(DevCounters));
@@ -1443,6 +1672,135 @@ int rt_scene_create_multi(const rt_scene_desc* d, int n_devices, const int* devi
 
 int rt_scene_device_count(rt_scene* sc) { return sc ? (int)sc->peers.size() + 1 : 0; }
 
+// ---- scene updates -----------------------------------------------------------------------------------------------
+static int check_shape_indices(uint32_t n_shapes, uint32_t n, const uint32_t* idx) {
+    std::vector<uint32_t> v(idx, idx + n);
+    std::sort(v.begin(), v.end());
+    if (v.back() >= n_shapes) return fail(RT_ERR_INVALID, "shape index out of range");
+    if (std::adjacent_find(v.begin(), v.end()) != v.end()) return fail(RT_ERR_INVALID, "a shape index is listed twice");
+    return RT_OK;
+}
+
+static int check_idle(rt_scene* sc) {
+    if (sc->rendering) return fail(RT_ERR_STATE, "a frame is in flight");
+    for (rt_scene* peer : sc->peers)
+        if (peer->rendering) return fail(RT_ERR_STATE, "a frame is in flight");
+    return RT_OK;
+}
+
+int rt_scene_update(rt_scene* sc, const rt_scene_desc* d) {
+    int rc = validate_desc(d);   // first, like rt_scene_create: a bad description is named whatever the handle
+    if (rc != RT_OK) return rc;
+    if (!sc) return fail(RT_ERR_INVALID, "null scene");
+    if ((rc = check_idle(sc)) != RT_OK) return rc;
+    std::vector<rt_scene*> hs(1, sc);
+    hs.insert(hs.end(), sc->peers.begin(), sc->peers.end());
+    std::vector<SceneTables> ts(hs.size());
+    auto drop = [&]() {   // the new tables when the update fails, the old ones when it succeeds
+        for (size_t k = 0; k < hs.size(); k++) {
+            cudaSetDevice(hs[k]->device);
+            for (void* p : ts[k].allocs) cudaFree(p);
+            ts[k].allocs.clear();
+        }
+        cudaSetDevice(sc->device);
+    };
+    // build everything first: on any failure the handle keeps its scene
+    for (size_t k = 0; k < hs.size() && rc == RT_OK; k++) {
+        if (cudaSetDevice(hs[k]->device) != cudaSuccess) rc = fail(RT_ERR_CUDA, "cudaSetDevice failed");
+        else rc = build_tables(d, hs[k]->n_sm, hs[k]->smem_optin, ts[k]);
+    }
+    // the old tables are read by all work enqueued so far, on the handle's streams and on callers' streams
+    for (size_t k = 0; k < hs.size() && rc == RT_OK; k++) {
+        cudaSetDevice(hs[k]->device);
+        const cudaError_t e = cudaDeviceSynchronize();
+        if (e != cudaSuccess) rc = fail(RT_ERR_CUDA, std::string("scene update: ") + cudaGetErrorString(e));
+    }
+    if (rc != RT_OK) {
+        drop();
+        return rc;
+    }
+    for (size_t k = 0; k < hs.size(); k++) {
+        install_tables(hs[k], ts[k]);
+        hs[k]->accumulated_spp = 0;
+    }
+    sc->refit_broken = false;
+    drop();
+    for (auto& c : sc->caller_done) cudaEventDestroy(c.second);   // complete: the devices were synchronised
+    sc->caller_done.clear();
+    return RT_OK;
+}
+
+// the staging and device buffers for up to `bound` records, and the events of the updates: everything of an update that
+// can fail for want of memory, done before the host tree changes
+static int reserve_scatter(rt_scene* sc, uint64_t bound) {
+    CU(cudaSetDevice(sc->device));
+    if (!sc->ev_update) {
+        CU(cudaEventCreateWithFlags(&sc->ev_update, cudaEventDisableTiming));
+        CU(cudaEventCreateWithFlags(&sc->ev_scatter_read, cudaEventDisableTiming));
+    }
+    CU(cudaEventSynchronize(sc->ev_scatter_read));   // the previous update's copy has read the staging
+    if (sc->h_scatter_cap < bound) {
+        if (sc->h_scatter) cudaFreeHost(sc->h_scatter);
+        sc->h_scatter = nullptr;
+        sc->h_scatter_cap = 0;
+        if (cudaMallocHost(&sc->h_scatter, bound * sizeof(ScatterRec)) != cudaSuccess) {
+            cudaGetLastError();
+            sc->h_scatter = nullptr;
+            return fail(RT_ERR_NOMEM, "cudaMallocHost failed");
+        }
+        sc->h_scatter_cap = bound;
+    }
+    return ensure_device_array(sc->d_scatter, sc->d_scatter_cap, bound);
+}
+
+// enqueue a refit's records (reserve_scatter was called for at least as many) on the handle's main stream, after the
+// caller-stream work that read the tables
+static int apply_scatter(rt_scene* sc, const std::vector<ScatterRec>& recs) {
+    CU(cudaSetDevice(sc->device));
+    for (auto& c : sc->caller_done) CU(cudaStreamWaitEvent(sc->stream, c.second, 0));
+    const uint64_t n = recs.size();
+    memcpy(sc->h_scatter, recs.data(), n * sizeof(ScatterRec));
+    CU(cudaMemcpyAsync(sc->d_scatter, sc->h_scatter, n * sizeof(ScatterRec), cudaMemcpyHostToDevice, sc->stream));
+    CU(cudaEventRecord(sc->ev_scatter_read, sc->stream));
+    const DevScene& S = sc->ds;
+    const ScatterDst dst{{(uint4*)S.ctab, (uint4*)S.cupper, (uint4*)S.cull, (uint4*)S.march_cull, (uint4*)S.frec,
+                          (uint4*)S.inv, (uint4*)S.dir}};
+    k_scene_scatter<<<(unsigned)((n + 255) / 256), 256, 0, sc->stream>>>(dst, sc->d_scatter, (uint32_t)n);
+    sc->launches++;
+    CU(cudaGetLastError());
+    CU(cudaEventRecord(sc->ev_update, sc->stream));
+    sc->accumulated_spp = 0;
+    return RT_OK;
+}
+
+int rt_scene_update_transforms(rt_scene* sc, uint32_t n, const uint32_t* idx, const double* inverse, const double* direct) {
+    if (!sc) return fail(RT_ERR_INVALID, "null scene");
+    if (n == 0) return RT_OK;
+    if (!idx || !inverse || !direct) return fail(RT_ERR_INVALID, "null array");
+    int rc = check_shape_indices((uint32_t)sc->ds.n_shapes, n, idx);
+    if (rc != RT_OK) return rc;
+    if ((rc = check_idle(sc)) != RT_OK) return rc;
+    if (sc->refit_broken)
+        return fail(RT_ERR_STATE, "an earlier transforms update failed on the device; rt_scene_update rebuilds the scene");
+    std::vector<rt_scene*> hs(sc->peers.begin(), sc->peers.end());
+    hs.push_back(sc);
+    const uint64_t bound = refit_record_bound(n);
+    if (bound > 0xFFFFFFFFull) return fail(RT_ERR_INVALID, "too many shapes in one update");
+    for (rt_scene* h : hs)
+        if ((rc = reserve_scatter(h, bound)) != RT_OK) return rc;   // nothing has changed yet
+    std::vector<ScatterRec> recs;
+    recs.reserve(bound);
+    refit(sc->refit, n, idx, inverse, direct, &recs);
+    // from here on the host tree has moved: a device that misses the records would keep nodes the next refit does not
+    // rewrite, so a failure (a CUDA error, nothing else is left to fail) blocks further refits until a rebuild
+    for (rt_scene* h : hs)
+        if ((rc = apply_scatter(h, recs)) != RT_OK) {
+            sc->refit_broken = true;
+            return rc;
+        }
+    return RT_OK;
+}
+
 // make lane i the one the launch code sees (sc->stream, sc->q, ...)
 static void bind_lane(rt_scene* sc, int i) {
     if (i == sc->cur_lane) return;
@@ -1498,6 +1856,7 @@ void rt_scene_destroy(rt_scene* sc) {
     cudaFree(sc->d_pix_counts);
     cudaFree(sc->d_views);
     if (sc->host_stage) cudaFreeHost(sc->host_stage);
+    cudaFree(sc->d_scatter);
     bind_lane(sc, 0);
     for (int l = 0; l < RT_MAX_LANES; l++)
         if (sc->lanes[l].stream) cudaStreamSynchronize(l == 0 ? sc->stream : sc->lanes[l].stream);
@@ -1518,6 +1877,11 @@ void rt_scene_destroy(rt_scene* sc) {
     if (sc->ev_group_start) cudaEventDestroy(sc->ev_group_start);
     if (sc->ev_group_done) cudaEventDestroy(sc->ev_group_done);
     if (sc->ev_adaptive_fork) cudaEventDestroy(sc->ev_adaptive_fork);
+    if (sc->h_scatter) cudaFreeHost(sc->h_scatter);
+    if (sc->ev_scatter_read) cudaEventDestroy(sc->ev_scatter_read);
+    if (sc->ev_update) cudaEventDestroy(sc->ev_update);
+    for (auto& c : sc->caller_done) cudaEventDestroy(c.second);
+    if (sc->fold_stream) cudaStreamDestroy(sc->fold_stream);
     if (sc->stream) cudaStreamDestroy(sc->stream);
     if (sc->copy_stream) cudaStreamDestroy(sc->copy_stream);
     delete sc;
@@ -1533,6 +1897,8 @@ int rt_intersect_batch_device(rt_scene* sc, const rt_ray* d_rays, uint64_t n, do
     if (!d_rays) return fail(RT_ERR_INVALID, "null rays");
     CU(cudaSetDevice(sc->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : sc->stream;
+    const bool caller = st != sc->stream;
+    if (caller && sc->ev_update) CU(cudaStreamWaitEvent(st, sc->ev_update, 0));   // after the last scene update
     uint64_t want = (n + 255) / 256;
     int grid = (int)std::min<uint64_t>(want, (uint64_t)sc->grid);
 #define RT_LAUNCH_ISECT(C_, M_)                                                                                  \
@@ -1548,6 +1914,24 @@ int rt_intersect_batch_device(rt_scene* sc, const rt_ray* d_rays, uint64_t n, do
 #undef RT_LAUNCH_ISECT
     sc->launches++;
     CU(cudaGetLastError());
+    if (caller) {   // a scene update waits for this call's reads of the tables
+        auto it = std::find_if(sc->caller_done.begin(), sc->caller_done.end(), [&](const auto& c) { return c.first == st; });
+        if (it == sc->caller_done.end()) {
+            if (sc->caller_done.size() >= 32) {   // many distinct streams: fold their events into one, without a host wait
+                if (!sc->fold_stream) CU(cudaStreamCreateWithFlags(&sc->fold_stream, cudaStreamNonBlocking));
+                for (auto& c : sc->caller_done) CU(cudaStreamWaitEvent(sc->fold_stream, c.second, 0));
+                for (size_t k = 1; k < sc->caller_done.size(); k++) cudaEventDestroy(sc->caller_done[k].second);
+                sc->caller_done.resize(1);
+                sc->caller_done[0].first = sc->fold_stream;
+                CU(cudaEventRecord(sc->caller_done[0].second, sc->fold_stream));
+            }
+            cudaEvent_t e = nullptr;
+            CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+            sc->caller_done.push_back({st, e});
+            it = sc->caller_done.end() - 1;
+        }
+        CU(cudaEventRecord(it->second, st));
+    }
     return RT_OK;
 }
 
@@ -2942,6 +3326,71 @@ int rt_cull_tree_check(const rt_scene_desc* d, uint32_t* n_roots, uint32_t* n_gr
     }
     *n_tree = in_tree;
     *worst = in_tree ? w : 0.0;
+    return RT_OK;
+}
+
+int rt_cull_refit_check(const rt_scene_desc* d, uint32_t n, const uint32_t* idx, const double* inverse, double* worst) {
+    int rc = validate_desc(d);
+    if (rc != RT_OK) return rc;
+    if (!worst || (n && (!idx || !inverse))) return fail(RT_ERR_INVALID, "null argument");
+    if (n && (rc = check_shape_indices(d->n_shapes, n, idx)) != RT_OK) return rc;
+    SceneRefit s = make_refit(d, false, false, false);
+    refit(s, n, idx, inverse, nullptr, nullptr);
+    const CullTree& ct = s.ct;
+    // the metric of rt_cull_tree_check, against every shape's true ball from its current inverse rows; a node entry
+    // with A = +inf is never rejected and encloses anything, a member without a finite ball needs such a node
+    auto node_radius = [](float4 e) {
+        const double cn = sqrt((double)e.x * e.x + (double)e.y * e.y + (double)e.z * e.z);
+        const double x = sqrt((double)e.w / 1.0101);
+        return (x - sqrt(3.0 * RT_CULL_B) * cn) / (sqrt(1.1) + sqrt(3.0 * RT_CULL_B));
+    };
+    double w = -INFINITY;
+    bool any = false;
+    auto reach = [&](float4 e, const double c[3], double r) {
+        if (e.w == INFINITY) return;
+        if (!(std::isfinite(r) && std::isfinite(c[0]) && std::isfinite(c[1]) && std::isfinite(c[2]))) {
+            w = INFINITY;
+            return;
+        }
+        const double nr = node_radius(e);
+        const double dx = c[0] - e.x, dy = c[1] - e.y, dz = c[2] - e.z;
+        w = fmax(w, (sqrt(dx * dx + dy * dy + dz * dz) + r - nr) / nr);
+    };
+    for (int i = 0; i < (int)d->n_shapes; i++) {
+        const int g = ct.group_of[i];
+        if (g < 0) continue;
+        any = true;
+        const double* m = &s.inv[(size_t)12 * i];
+        const double* q = &s.params[(size_t)RT_SHAPE_PARAMS * i];
+        double r;
+        cull_entry(m, s.kind[i], &r, fabs(q[0]) + fabs(q[1]));
+        // the ball's centre -M^-1 t in FP64 (Cramer's rule)
+        const double a[3][3] = {{m[0], m[1], m[2]}, {m[4], m[5], m[6]}, {m[8], m[9], m[10]}};
+        const double b[3] = {-m[3], -m[7], -m[11]};
+        auto det3 = [](const double x[3][3]) {
+            return x[0][0] * (x[1][1] * x[2][2] - x[1][2] * x[2][1]) - x[0][1] * (x[1][0] * x[2][2] - x[1][2] * x[2][0]) +
+                   x[0][2] * (x[1][0] * x[2][1] - x[1][1] * x[2][0]);
+        };
+        const double det = det3(a);
+        double c[3];
+        for (int k = 0; k < 3; k++) {
+            double x[3][3];
+            for (int rr = 0; rr < 3; rr++)
+                for (int cc = 0; cc < 3; cc++) x[rr][cc] = cc == k ? b[rr] : a[rr][cc];
+            c[k] = det3(x) / det;
+        }
+        const float4 grp = ct.table[(size_t)ct.n_roots + g], root = ct.table[g / RT_CULL_ROOT_FANOUT];
+        reach(grp, c, r);
+        reach(root, c, r);
+        reach(root, ct.group_ball[g].c, ct.group_ball[g].r);
+    }
+    for (int l = 1; l <= ct.n_upper; l++) {
+        const CullBall* below = l == 1 ? ct.root_ball.data() : ct.upper_ball.data() + ct.upper_off[l - 1];
+        const int n_below = l == 1 ? ct.n_roots : ct.upper_count[l - 1];
+        for (int k = 0; k < n_below; k++)
+            if (below[k].r >= 0.0) reach(ct.upper[ct.upper_off[l] + k / 32], below[k].c, below[k].r);
+    }
+    *worst = any ? w : 0.0;
     return RT_OK;
 }
 

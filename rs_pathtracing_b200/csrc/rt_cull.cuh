@@ -161,7 +161,26 @@ struct CullTree {
     std::vector<float4> upper;
     std::vector<CullBall> upper_ball;  // the FP64 balls the entries were made from (rt_cull_tree_check)
     std::vector<CullBall> root_ball;
+    // the FP64 balls the leaf and group entries were made from, kept for the refit (rt_scene_update_transforms)
+    std::vector<CullBall> leaf_ball;   // [n_shapes]
+    std::vector<CullBall> group_ball;  // [groups built]
 };
+
+// One analytic shape's leaf entry and the FP64 ball the nodes above it must enclose: the entry's FP32-rounded centre
+// with the radius padded by that rounding.  `inverse12`: its inverse rows; `params8`: its params row (may be null:
+// a Torus is then never culled).  A non-finite radius means never culled (the entry has A = +inf).
+inline float4 cull_leaf(const double* inverse12, int kind, const double* params8, bool no_cull, CullBall* ball) {
+    double r;
+    const double ext = (kind == RT_SHAPE_TORUS && params8) ? fabs(params8[0]) + fabs(params8[1]) : 0.0;
+    float4 e = cull_entry(inverse12, kind, &r, ext);
+    if (no_cull) e.w = INFINITY;
+    *ball = CullBall{{(double)e.x, (double)e.y, (double)e.z}, r};
+    if (isfinite(r)) {
+        double cn = fabs(ball->c[0]) + fabs(ball->c[1]) + fabs(ball->c[2]);
+        ball->r = r + cn * 1.2e-7;
+    }
+    return e;
+}
 
 // ball around member balls, FP32-representable centre
 inline CullBall cull_enclose(const std::vector<CullBall>& m) {
@@ -207,19 +226,11 @@ inline CullTree cull_build(const double* inverse, const uint8_t* kind, int n, bo
     std::vector<double> radii;
     for (int i = 0; i < n; i++) {
         if (kind[i] == RT_SHAPE_MARCH) continue;
-        double r;
-        const double ext = (kind[i] == RT_SHAPE_TORUS && params)
-                               ? fabs(params[(size_t)RT_SHAPE_PARAMS * i]) + fabs(params[(size_t)RT_SHAPE_PARAMS * i + 1]) : 0.0;
-        t.leaf[i] = cull_entry(inverse + (size_t)12 * i, kind[i], &r, ext);
-        if (no_cull) t.leaf[i].w = INFINITY;
-        ball[i] = CullBall{{(double)t.leaf[i].x, (double)t.leaf[i].y, (double)t.leaf[i].z}, r};
         // the leaf entry's centre is the FP32-rounded one; the enclosing balls must contain the true ball:
-        // pad the radius by the rounding of the centre
-        if (isfinite(r)) {
-            double cn = fabs(ball[i].c[0]) + fabs(ball[i].c[1]) + fabs(ball[i].c[2]);
-            ball[i].r = r + cn * 1.2e-7;
-            radii.push_back(ball[i].r);
-        }
+        // cull_leaf pads the radius by the rounding of the centre
+        t.leaf[i] = cull_leaf(inverse + (size_t)12 * i, kind[i], params ? params + (size_t)RT_SHAPE_PARAMS * i : nullptr,
+                              no_cull, &ball[i]);
+        if (isfinite(ball[i].r)) radii.push_back(ball[i].r);
     }
     double typical = 0.0;
     if (!radii.empty()) {
@@ -288,6 +299,8 @@ inline CullTree cull_build(const double* inverse, const uint8_t* kind, int n, bo
         grp[g] = cull_node_entry(gball[g]);
         t.group_radius.push_back(gball[g].r);
     }
+    t.leaf_ball = ball;
+    t.group_ball = gball;
     t.root_ball.assign(t.n_roots, CullBall{{0.0, 0.0, 0.0}, -1.0});
     for (int r = 0; r < t.n_roots; r++) {
         std::vector<CullBall> m;

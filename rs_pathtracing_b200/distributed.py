@@ -180,8 +180,21 @@ class DistributedRenderer:
                            stream=int(torch.cuda.current_stream().cuda_stream) or CUDA_STREAM_LEGACY)
         return self._frame
 
+    def update_transforms(self, index, inverse, direct):
+        """Move shapes (api.update_transforms' arguments) in the scene and in both handles of this renderer: the Scene's
+        description and every handle it created (Scene.set_transform_rows), and the second handle of the pipelined
+        sequences.  Frames started afterwards render the moved shapes."""
+        index, inverse, direct = api.check_transforms(index, inverse, direct)
+        self.scene.set_transform_rows(index, inverse, direct)
+        if self._dev_scene_b is not None:
+            api.update_transforms(self._dev_scene_b, index, inverse, direct)
+
     def render_jobs_device(self, jobs, on_frame=None, on_rendered=None):
-        """A SEQUENCE of frames, pipelined: jobs = [(camera, width, height, samples_number), ...].  While frame n's
+        """A SEQUENCE of frames, pipelined: jobs = [(camera, width, height, samples_number), ...].  A job may carry a
+        fifth element (index, inverse, direct), the arguments of update_transforms: the shapes move from that frame on.
+        The edit is applied to the handle that renders the job just before the job starts, and to the other handle
+        before its next job, so a moving-object sequence keeps two frames in flight; once the sequence is done the
+        scene and both handles hold the last position of every moved shape.  While frame n's
         accumulators travel to rank 0 and are assembled there, every rank already renders frame n+1 (two frames are in
         flight on two handles of the same device): the serial tail of render_device (host wait -> NCCL send/recv ->
         k_assemble, about 1 ms whatever the frame) and the drain of a frame's last batches disappear from every step
@@ -205,11 +218,23 @@ class DistributedRenderer:
         # accumulator) when frame n completes, so the drain of a frame's last batches -- the thin deep bounce levels
         # overlap with nothing -- and the host's turn-around between two frames are filled with the next frame's work.
         handles = [self.dev_scene, self._second_handle()] if len(jobs) > 1 else [self.dev_scene]
+        edits = [api.check_transforms(*job[4]) if len(job) > 4 and job[4] is not None else None for job in jobs]
+        applied = [0] * len(handles)   # jobs whose edits each handle has received (edits are absolute rows, so in order)
+
+        def start(j):
+            hnd = j % len(handles)
+            for e in edits[applied[hnd]:j + 1]:
+                if e is not None:
+                    api.update_transforms(handles[hnd], *e)
+            applied[hnd] = j + 1
+            cam, w, h, spp = jobs[j][:4]
+            api.render_start(handles[hnd], cam, self._params(w, h, spp, self.rank))
+
         frame = None
         for i in range(min(len(handles), len(jobs))):
-            cam, w, h, spp = jobs[i]
-            api.render_start(handles[i], cam, self._params(w, h, spp, self.rank))
-        for i, (cam, w, h, spp) in enumerate(jobs):
+            start(i)
+        for i, job in enumerate(jobs):
+            cam, w, h, spp = job[:4]
             hnd = handles[i % len(handles)]
             ptr, n = api.render_device_result(hnd)   # host: this shard's kernels are done
             if on_rendered is not None:
@@ -229,8 +254,7 @@ class DistributedRenderer:
             self._stage_ready[k].synchronize()                  # host: this handle's accumulator may be overwritten now
             nxt = i + len(handles)
             if nxt < len(jobs):
-                ncam, nw, nh, nspp = jobs[nxt]
-                api.render_start(hnd, ncam, self._params(nw, nh, nspp, self.rank))
+                start(nxt)
             torch.cuda.current_stream().wait_event(self._stage_ready[k])
             frame = self._exchange_assemble(self._stage[k], w, h, spp)
             if self._stage_free[k] is None:
@@ -238,6 +262,19 @@ class DistributedRenderer:
             self._stage_free[k].record()
             if frame is not None and on_frame is not None:
                 on_frame(i, frame)
+        # the last position of every moved shape, into the scene's description (and its handles) and the other handle
+        last = {}
+        for e in edits:
+            if e is not None:
+                for k, s in enumerate(e[0]):
+                    last[int(s)] = (e[1][k], e[2][k])
+        if last:
+            index = np.array(sorted(last), np.uint32)
+            inverse = np.array([last[s][0] for s in index])
+            direct = np.array([last[s][1] for s in index])
+            self.scene.set_transform_rows(index, inverse, direct)
+            for hnd in handles[1:]:
+                api.update_transforms(hnd, index, inverse, direct)
         return frame
 
     def _second_handle(self):

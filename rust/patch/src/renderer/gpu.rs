@@ -16,7 +16,48 @@ use crate::{
 fn v(a: &Vector3d) -> sys::rt_vec3 { sys::rt_vec3 { x: a.x, y: a.y, z: a.z } }
 fn check(rc: i32) { if rc != sys::RT_OK { panic!("rt_b200: {}", sys::last_error()) } }  // the reference unwraps too
 
-pub struct GpuRenderer { scene: *mut sys::rt_scene, depth: u32, seed: u64, progressive: bool }
+/// The reference renders whatever its `Arc<RwLock<Scene>>` holds when a frame starts (step_by_step.rs:37): the renderer
+/// keeps the lock and, at every start_rendering, compares the flattened scene with what the device holds.
+pub struct GpuRenderer {
+    scene: *mut sys::rt_scene, depth: u32, seed: u64, progressive: bool,
+    world: Arc<RwLock<Scene>>,
+    uploaded: Vec<u8>,   // the bytes of the description the device holds (every table, images included)
+}
+
+/// every byte a description points at, in a fixed order: two descriptions give the same bytes iff they describe the
+/// same scene
+fn desc_bytes(d: &sys::rt_scene_desc) -> Vec<u8> {
+    fn raw<T>(p: *const T, n: usize, out: &mut Vec<u8>) {
+        if n > 0 && !p.is_null() {
+            out.extend_from_slice(unsafe { std::slice::from_raw_parts(p as *const u8, n * std::mem::size_of::<T>()) });
+        }
+    }
+    let n = d.n_shapes as usize;
+    let mut out = Vec::new();
+    out.extend_from_slice(&d.n_shapes.to_le_bytes());
+    raw(d.kind, n, &mut out);
+    raw(d.flags, n, &mut out);
+    raw(d.inverse, 12 * n, &mut out);
+    raw(d.direct, 12 * n, &mut out);
+    raw(d.params, sys::RT_SHAPE_PARAMS as usize * n, &mut out);
+    raw(d.material, n, &mut out);
+    for (count, bytes) in [(d.n_materials, std::mem::size_of::<sys::rt_material>()),
+                           (d.n_textures, std::mem::size_of::<sys::rt_texture>()),
+                           (d.n_noise, std::mem::size_of::<sys::rt_perlin>())] {
+        out.extend_from_slice(&count.to_le_bytes());
+        out.extend_from_slice(&(bytes as u64).to_le_bytes());
+    }
+    raw(d.materials, d.n_materials as usize, &mut out);
+    raw(d.textures, d.n_textures as usize, &mut out);
+    raw(d.noise, d.n_noise as usize, &mut out);
+    for i in 0..d.n_images as usize {
+        let im = unsafe { &*d.images.add(i) };
+        out.extend_from_slice(&im.width.to_le_bytes());
+        out.extend_from_slice(&im.height.to_le_bytes());
+        raw(im.rgba, 4 * im.width as usize * im.height as usize, &mut out);
+    }
+    out
+}
 
 impl GpuRenderer {
     /// same constructor convention as ThreadPoolRenderer::new (step_by_step.rs:37); `thread_number` is ignored
@@ -26,14 +67,31 @@ impl GpuRenderer {
     /// the same renderer over several GPUs of the box: ONE handle (rt_scene_create_multi), frames sharded by
     /// interleaved tiles over all of them, the assembled frame identical to the single-GPU one
     pub fn with_devices(scene: Arc<RwLock<Scene>>, _thread_number: u32, depth: u32, devices: &[i32]) -> Self {
-        let s = scene.read().unwrap();
+        let (h, uploaded) = {
+            let s = scene.read().unwrap();
+            let f: &FlatScene = s.flat();
+            let mut images = Vec::new();
+            let desc = f.desc(&mut images);
+            let mut h = std::ptr::null_mut();
+            // (the library copies the description)
+            check(unsafe { sys::rt_scene_create_multi(&desc, devices.len() as i32, devices.as_ptr(), &mut h) });
+            (h, desc_bytes(&desc))
+        };
+        GpuRenderer { scene: h, depth, seed: 0, progressive: false, world: scene, uploaded }
+    }
+    /// Re-reads the RwLock'd scene and, when it differs from what the device holds, replaces the handle's scene in
+    /// place (rt_scene_update: the handle keeps its streams, buffers and devices; the frame equals a fresh handle's).
+    /// start_rendering calls it, so an edit made between two frames renders in the next one, as in the reference.
+    pub fn sync_scene(&mut self) {
+        let s = self.world.read().unwrap();
         let f: &FlatScene = s.flat();
         let mut images = Vec::new();
         let desc = f.desc(&mut images);
-        let mut h = std::ptr::null_mut();
-        // (the library copies the description)
-        check(unsafe { sys::rt_scene_create_multi(&desc, devices.len() as i32, devices.as_ptr(), &mut h) });
-        GpuRenderer { scene: h, depth, seed: 0, progressive: false }
+        let bytes = desc_bytes(&desc);
+        if bytes != self.uploaded {
+            check(unsafe { sys::rt_scene_update(self.scene, &desc) });
+            self.uploaded = bytes;
+        }
     }
     /// Progressive accumulation (rt_render_set_accumulate): while on, start_rendering calls with an unchanged
     /// camera ADD their samples to the frame instead of starting over -- what RendererState::render
@@ -46,6 +104,8 @@ impl GpuRenderer {
 
 impl Renderer for GpuRenderer {
     fn start_rendering(&mut self, camera: Arc<RwLock<Camera>>, img: &ImageParams, samples_number: u32) {
+        self.stop_rendering();   // (rt_render_start stops a frame in flight too; the update must not meet one)
+        self.sync_scene();
         let c = camera.read().unwrap();
         let cam = sys::rt_camera {
             position: v(c.position()), direction: v(c.direction()), up: v(c.up()), right: v(c.rigth()),

@@ -83,6 +83,9 @@ extern "C" {
     pub fn rt_scene_create_multi(desc: *const rt_scene_desc, n_devices: c_int, device_ids: *const c_int,
         out: *mut *mut rt_scene) -> c_int;
     pub fn rt_scene_device_count(scene: *mut rt_scene) -> c_int;
+    pub fn rt_scene_update(scene: *mut rt_scene, desc: *const rt_scene_desc) -> c_int;
+    pub fn rt_scene_update_transforms(scene: *mut rt_scene, n: u32, shape_index: *const u32, inverse: *const f64,
+        direct: *const f64) -> c_int;
     pub fn rt_intersect_batch(scene: *mut rt_scene, rays: *const rt_ray, n: u64, t_min: f64, t_max: f64,
         mode: c_int, shape_index: *mut i32, t: *mut f64, normal: *mut rt_vec3, point: *mut rt_vec3,
         uv: *mut f64, front_face: *mut u8) -> c_int;
@@ -130,6 +133,8 @@ extern "C" {
     pub fn rt_cull_reached(desc: *const rt_scene_desc, rays: *const rt_ray, n_rays: u64, reached: *mut u8) -> c_int;
     pub fn rt_cull_tree_check(desc: *const rt_scene_desc, n_roots: *mut u32, n_groups: *mut u32, n_tree: *mut u32,
         n_flat: *mut u32, worst: *mut f64) -> c_int;
+    pub fn rt_cull_refit_check(desc: *const rt_scene_desc, n: u32, shape_index: *const u32, inverse: *const f64,
+        worst: *mut f64) -> c_int;
     pub fn rt_measure_peaks(device: c_int, fp64_tflops: *mut f64, fp32_tflops: *mut f64) -> c_int;
 }
 

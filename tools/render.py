@@ -3,7 +3,7 @@
   python tools/render.py scenes/cornell_box.json out.png --size 1024 1024 --spp 256 [--depth 8] [--seed 1]
       [--adaptive REL [--min-samples N] [--abs-error A] [--heatmap counts.png]]
       [--counts MAP.npy [--heatmap counts.png]]
-      [--orbit N]
+      [--orbit N] [--animate N [--step S]]
 
 Scene::from_json -> GpuRenderer (Renderer trait: start_rendering / render_step until done) ->
 rt_tonemap_rgba8 (sqrt, clamp(0, 0.999) * 256, on the device) -> PNG.  With --adaptive, an adaptive frame
@@ -14,7 +14,10 @@ sample count per pixel (rt_render_start_counts): MAP.npy is an (h, w) uint32 arr
 then draws that map (black = 0 or 1 sample, white = its largest count, log2 scale) and the frame's count-0 pixels
 are black.  With --orbit N, one frame of N views (rt_render_start_views): the scene camera's position and direction
 rotated about the world y axis through the origin by 360/N degrees at a time; view k goes to OUT_k.png (out_000.png,
-out_001.png, ... for out.png)."""
+out_001.png, ... for out.png).  With --animate N, N frames in which the scene's random spheres move on a seeded
+random walk in the x-z plane (--step per axis and frame), each frame on the same renderer after
+Scene.set_transforms-style edits of the scene (rt_scene_update_transforms: the cull tree is refit in place); frame k
+goes to OUT_k.png."""
 import argparse, os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -33,9 +36,13 @@ ap.add_argument("--abs-error", type=float, default=0.0)
 ap.add_argument("--counts", default=None, metavar="MAP.npy", help="(h, w) uint32 sample count per pixel")
 ap.add_argument("--heatmap", default=None, help="PNG of the per-pixel sample counts (with --adaptive or --counts)")
 ap.add_argument("--orbit", type=int, default=None, metavar="N", help="N views around the scene, one PNG per view")
+ap.add_argument("--animate", type=int, default=None, metavar="N", help="N frames of the random spheres on a random walk")
+ap.add_argument("--step", type=float, default=0.05, help="--animate: random-walk step per axis and frame")
 a = ap.parse_args()
 if a.orbit is not None and (a.orbit < 1 or a.adaptive is not None or a.counts is not None):
     ap.error("--orbit needs N >= 1 and excludes --adaptive and --counts")
+if a.animate is not None and (a.animate < 1 or a.orbit is not None or a.adaptive is not None or a.counts is not None):
+    ap.error("--animate needs N >= 1 and excludes --orbit, --adaptive and --counts")
 if a.heatmap and a.adaptive is None and a.counts is None:
     ap.error("--heatmap needs --adaptive or --counts")
 if a.adaptive is not None and a.counts is not None:
@@ -59,6 +66,17 @@ if a.orbit is not None:
     paths = a.orbit * w * h * a.spp
     print(f"{a.scene}: {a.orbit} views of {w}x{h}x{a.spp} in {dt * 1e3:.1f} ms ({paths / dt / 1e6:.1f} Mpaths/s) "
           f"-> {stem}_000{ext or '.png'} .. {stem}_{a.orbit - 1:03d}{ext or '.png'}")
+    sys.exit(0)
+if a.animate is not None:
+    n_file = rt.Scene.from_file(a.scene, add_random_spheres=False).shape_count
+    walk = rt.api.random_walk(sc, np.arange(n_file, sc.shape_count), a.animate, a.step, seed=a.seed)
+    stem, ext = os.path.splitext(a.out)
+    for k, (index, inverse, direct) in enumerate(walk):
+        sc.set_transform_rows(index, inverse, direct)   # the scene and the renderer's handle move together
+        rt.save_png(f"{stem}_{k:03d}{ext or '.png'}", rt.tonemap_rgba8(sc, r.render(cam, w, h, a.spp)))
+    dt = time.perf_counter() - t0
+    print(f"{a.scene}: {a.animate} frames of {w}x{h}x{a.spp}, {sc.shape_count - n_file} spheres moving, in "
+          f"{dt * 1e3:.1f} ms -> {stem}_000{ext or '.png'} .. {stem}_{a.animate - 1:03d}{ext or '.png'}")
     sys.exit(0)
 if a.counts is not None:
     buf = r.render_counts(cam, given)
