@@ -206,7 +206,7 @@ int rt_scene_device_count(rt_scene* scene);
 /* ---- scene updates on a live handle (the reference renders whatever its Arc<RwLock<Scene>> holds when a frame starts,
  *      src/renderer/step_by_step.rs:37) ----------------------------------------------------------------------------
  * Contract of both entries: after the call, every entry point (rt_intersect_batch[_device] in every mode and with
- * every output, rt_render_start and the adaptive, counts and views frames, rt_trace_pixel_samples[_group][_device])
+ * every output, rt_occluded_batch[_device], rt_render_start and the adaptive, counts and views frames, rt_trace_pixel_samples[_group][_device])
  * gives bit for bit what a handle freshly created from the edited description gives.  The handle keeps its streams,
  * lanes, buffers, peer access and settings.
  *   - RT_ERR_STATE while a frame is in flight (that frame goes on with the old scene).
@@ -214,9 +214,10 @@ int rt_scene_device_count(rt_scene* scene);
  *     even with the same camera and params); rt_render_set_accumulate's switch stays as it is.
  *   - The last completed frame stays readable (rt_render_device_frame, rt_render_device_result, rt_render_pixel_stats,
  *     rt_tonemap_rgba8_device); rt_stats is untouched.
- *   - An update is ordered after all work the handle enqueued before it, rt_intersect_batch_device and
- *     rt_trace_pixel_samples_group_device calls on caller streams included, and work enqueued after it sees the new
- *     scene.  For that, rt_intersect_batch_device on a caller stream records an event there at the end of each call
+ *   - An update is ordered after all work the handle enqueued before it, rt_intersect_batch_device,
+ *     rt_occluded_batch_device and rt_trace_pixel_samples_group_device calls on caller streams included, and work
+ *     enqueued after it sees the new scene.  For that, rt_intersect_batch_device and rt_occluded_batch_device on a
+ *     caller stream record an event there at the end of each call
  *     (one per stream; past 32 streams they are joined on an internal stream, never waited for on the host) and waits
  *     for the last update's event.
  *   - rt_scene_update_transforms allocates what it needs before the host copy of the tree changes; if the device work
@@ -272,6 +273,26 @@ int rt_intersect_batch_device(rt_scene* scene, const rt_ray* d_rays, uint64_t n,
                               double t_max, int mode, int32_t* d_shape_index, double* d_t,
                               rt_vec3* d_normal, rt_vec3* d_point, double* d_uv,
                               uint8_t* d_front_face, void* stream);
+
+/* ---- batched any-hit (occlusion: shadow rays, ambient occlusion, line of sight) ------------------------------------
+ * Any-hit: occluded[i] = 1 iff rt_intersect_batch (RT_ISECT_BRUTE) of ray i over [t_min, tmax_i] returns a hit
+ * (shape_index != -1), else 0, bit for bit in every mode; tmax_i = t_max_per_ray[i], or t_max when that array is NULL.
+ * The literal loop's max_t only shrinks at an acceptance, so it returns a hit iff at least one shape accepts the ray at
+ * (t_min, tmax_i) -- a Sphere D == 0 hit and a NaN t included -- in whatever order the shapes are tested.  So the
+ * query stops at the first shape that accepts the ray.  mode: RT_ISECT_BRUTE (literal loop in index order, early
+ * exit), RT_ISECT_FAST (cull tree + early exit), RT_ISECT_VERIFY (FAST and the literal nearest hit on every ray;
+ * disagreements and falsely culled pairs into rt_stats.verify_rays / verify_false_culls).  n = 0 does nothing.
+ * RT_ERR_INVALID for a NULL scene, an unknown mode (checked in that order, before n = 0), or NULL rays / occluded with
+ * n > 0.  The host form copies through the handle's stream and synchronises it.  With counters on, a query counts as
+ * one rt_stats.segments, and shape_tests / cull_tests / march_* count the tests actually run; last_intersect_ms is not
+ * touched.  A multi-device handle answers on device_ids[0]. */
+int rt_occluded_batch(rt_scene* scene, const rt_ray* rays, uint64_t n, double t_min, double t_max,
+                      const double* t_max_per_ray, int mode, uint8_t* occluded);
+/* Same, with every pointer a DEVICE pointer on the scene's device and no copies; runs on `stream` like
+ * rt_intersect_batch_device (NULL = the library's own stream, cudaStreamLegacy = 0x1 the legacy default stream), does
+ * not synchronise, and is ordered against scene updates like it. */
+int rt_occluded_batch_device(rt_scene* scene, const rt_ray* d_rays, uint64_t n, double t_min, double t_max,
+                             const double* d_t_max_per_ray, int mode, uint8_t* d_occluded, void* stream);
 
 /* ---- frame rendering (replaces the Renderer trait, src/renderer/mod.rs:47-56) -------- */
 

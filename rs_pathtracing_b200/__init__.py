@@ -9,10 +9,10 @@ from . import _ffi
 from ._ffi import (Camera, ImageParams, Ray, RenderParams, Stats, Vec3, NativeLibraryMissing,
                    RT_ISECT_BRUTE, RT_ISECT_FAST, RT_ISECT_VERIFY)
 from .api import (GpuRenderer, RtError, Scene, camera_new, device_count, make_rays, measure_peaks,
-                  save_png, tonemap_rgba8)
+                  save_png, shadow_rays, tonemap_rgba8)
 
 __all__ = [
     "Camera", "ImageParams", "Ray", "RenderParams", "Stats", "Vec3", "NativeLibraryMissing",
     "RT_ISECT_BRUTE", "RT_ISECT_FAST", "RT_ISECT_VERIFY", "GpuRenderer", "RtError", "Scene", "camera_new",
-    "device_count", "make_rays", "measure_peaks", "save_png", "tonemap_rgba8",
+    "device_count", "make_rays", "measure_peaks", "save_png", "shadow_rays", "tonemap_rgba8",
 ]

@@ -145,6 +145,10 @@ CORE_SYMBOLS = {
     "rt_intersect_batch_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.c_double, C.c_int,
                                             C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                             C.c_void_p, C.c_void_p]),
+    "rt_occluded_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.c_double, C.c_void_p, C.c_int,
+                                    C.c_void_p]),
+    "rt_occluded_batch_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.c_double, C.c_void_p,
+                                           C.c_int, C.c_void_p, C.c_void_p]),
     "rt_render_start": (C.c_int, [C.c_void_p, C.POINTER(Camera), C.POINTER(RenderParams)]),
     "rt_render_poll": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(C.c_int)]),
     "rt_render_wait": (C.c_int, [C.c_void_p, C.c_void_p]),

@@ -97,6 +97,34 @@ def make_rays(origins: np.ndarray, directions: np.ndarray, normalize: bool = Tru
     return np.ascontiguousarray(np.concatenate([o, d], axis=1))
 
 
+def shadow_rays(points: np.ndarray, targets: np.ndarray):
+    """rays from points (n, 3) toward targets (n, 3) and the distance of each target: (rays (n, 6), dist (n,)).  The
+    direction is Ray::new's unit vector (make_rays) and dist = sqrt((x*x + y*y) + z*z) of targets - points, the same
+    length it divides by.  For a shadow ray, pass a t_max a little below dist (e.g. (1 - 1e-9) * dist) to Scene.occluded
+    so that the light's own surface at the target does not count."""
+    p = np.ascontiguousarray(points, dtype=np.float64).reshape(-1, 3)
+    q = np.ascontiguousarray(targets, dtype=np.float64).reshape(-1, 3)
+    if p.shape != q.shape:
+        raise ValueError(f"points and targets need the same number of rows, got {p.shape[0]} and {q.shape[0]}")
+    d = q - p
+    dist = np.sqrt(d[:, 0] * d[:, 0] + d[:, 1] * d[:, 1] + d[:, 2] * d[:, 2])
+    return make_rays(p, d), dist
+
+
+def check_t_max(t_max, n: int):
+    """occluded's bound: a float (one bound for every ray) or n per-ray bounds as a contiguous (n,) float64 array (numpy,
+    or a CUDA torch tensor for occluded_device); returns (scalar, array or None)"""
+    if isinstance(t_max, (int, float, np.floating, np.integer)):
+        return float(t_max), None
+    shape, dtype = tuple(getattr(t_max, "shape", ())), str(getattr(t_max, "dtype", type(t_max).__name__))
+    if shape != (n,) or dtype not in ("float64", "torch.float64"):
+        raise ValueError(f"t_max must be a float or a ({n},) float64 array, got shape {shape} dtype {dtype}")
+    contiguous = t_max.is_contiguous() if hasattr(t_max, "is_contiguous") else t_max.flags["C_CONTIGUOUS"]
+    if not contiguous:
+        raise ValueError("t_max must be contiguous")
+    return math.inf, t_max
+
+
 class Scene:
     """world::Scene (src/world/mod.rs:20-49)."""
 
@@ -225,6 +253,20 @@ class Scene:
                                               p(out["t"]), p(out["normal"]), p(out["point"]), p(out["uv"]),
                                               p(out["front"])))
         return {k: v for k, v in out.items() if v is not None}
+
+    def occluded(self, rays: np.ndarray, min_t: float = 0.001, max_t=math.inf, mode: int = _ffi.RT_ISECT_FAST,
+                 device: Optional[int] = None) -> np.ndarray:
+        """any-hit (rt_occluded_batch): is something between min_t and max_t along each ray?  Exactly
+        closest_hit(rays, min_t, max_t, RT_ISECT_BRUTE)["index"] != -1, stopping at the first shape that accepts the
+        ray.  max_t: a float, or a contiguous (n,) float64 array of per-ray bounds.  Returns an (n,) bool array."""
+        rays = np.ascontiguousarray(rays, dtype=np.float64).reshape(-1, 6)
+        n = rays.shape[0]
+        t_max, per_ray = check_t_max(max_t, n)
+        out = np.empty(n, np.uint8)
+        p = lambda a: a.ctypes.data_as(C.c_void_p) if a is not None else None
+        _check(_ffi.core().rt_occluded_batch(self.device_scene(device), p(rays), n, min_t, t_max, p(per_ray), mode,
+                                             p(out)))
+        return out.view(np.bool_)
 
     def trace_pixel_samples(self, rays: np.ndarray, depth: int, seed: int = 0, pixel_index: int = 0,
                             device: Optional[int] = None):
@@ -528,6 +570,31 @@ def update_transforms(dev_scene, index, inverse, direct) -> None:
     index, inverse, direct = check_transforms(index, inverse, direct)
     p = lambda a: a.ctypes.data_as(C.c_void_p)
     _check(_ffi.core().rt_scene_update_transforms(dev_scene, index.shape[0], p(index), p(inverse), p(direct)))
+
+
+def occluded_device(dev_scene, rays, out, t_max=math.inf, t_min: float = 0.001, mode: int = _ffi.RT_ISECT_FAST):
+    """rt_occluded_batch_device on torch CUDA tensors of the handle's device, queued on torch's current stream without a
+    host synchronisation: rays (n, 6) float64, out (n,) uint8 or bool (1 = occluded), t_max a float or an (n,) float64
+    tensor, all contiguous.  Returns out."""
+    import torch
+    if not (rays.is_cuda and rays.dtype == torch.float64 and rays.dim() == 2 and rays.shape[1] == 6
+            and rays.is_contiguous()):
+        raise ValueError("rays: a contiguous float64 CUDA tensor of shape (n, 6)")
+    n = rays.shape[0]
+    if not (out.is_cuda and out.dtype in (torch.uint8, torch.bool) and tuple(out.shape) == (n,) and out.is_contiguous()):
+        raise ValueError(f"out: a contiguous uint8 or bool CUDA tensor of shape ({n},)")
+    t_scalar, per_ray = check_t_max(t_max, n)
+    if per_ray is not None and not per_ray.is_cuda:
+        raise ValueError("t_max: per-ray bounds must be a CUDA tensor")
+    for name, tns in (("out", out), ("t_max", per_ray)):
+        if tns is not None and tns.device != rays.device:
+            raise ValueError(f"{name} is on {tns.device}, rays are on {rays.device}")
+    # torch's default stream is the legacy default stream (handle 0), which the ABI names cudaStreamLegacy = 0x1
+    stream = torch.cuda.current_stream(rays.device).cuda_stream or 1
+    _check(_ffi.core().rt_occluded_batch_device(dev_scene, rays.data_ptr(), n, t_min, t_scalar,
+                                                per_ray.data_ptr() if per_ray is not None else None, mode,
+                                                out.data_ptr(), stream))
+    return out
 
 
 def check_counts(counts, width: int, height: int) -> np.ndarray:

@@ -215,6 +215,40 @@ k_intersect_batch(DevScene S, bool use_smem, const rt_ray* __restrict__ rays, un
     if (COUNT || MODE == RT_ISECT_VERIFY) flush_counters(c, g_counters);
 }
 
+// rt_occluded_batch: occluded[i] = some shape accepts ray i at (t_min, tmax_i) (rt_scene.cuh, any_hit_brute /
+// any_hit_fast).  VERIFY answers with FAST and checks it against the literal nearest hit.
+template <bool COUNT, int MODE>
+__global__ void __launch_bounds__(256)
+k_occluded_batch(DevScene S, bool use_smem, const rt_ray* __restrict__ rays, unsigned long long n, double t_min,
+                 double t_max, const double* __restrict__ t_max_per_ray, uint8_t* __restrict__ occluded,
+                 DevCounters* g_counters) {
+    Staged st = stage_scene(S, use_smem);
+    DevCounters c = {};
+    const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
+    for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        rt_ray r = rays[i];
+        D3 ro = mk(r.origin.x, r.origin.y, r.origin.z), rd = mk(r.direction.x, r.direction.y, r.direction.z);
+        const double tmax = t_max_per_ray ? t_max_per_ray[i] : t_max;
+        bool hit;
+        if (MODE == RT_ISECT_BRUTE) {
+            hit = any_hit_brute<COUNT>(S, ro, rd, t_min, tmax, c);
+        } else if (MODE == RT_ISECT_FAST) {
+            hit = any_hit_fast<COUNT>(S, st, ro, rd, t_min, tmax, c);
+        } else {
+            DevCounters cc = {};
+            hit = any_hit_fast<false>(S, st, ro, rd, t_min, tmax, cc);
+            double bt;
+            int bi;
+            nearest_hit_brute<false>(S, ro, rd, t_min, tmax, bt, bi, cc);
+            if (hit != (bi >= 0)) c.verify_rays++;
+            c.verify_false_culls += count_false_culls(S, ro, rd, t_min);
+        }
+        if (COUNT) c.segments++;
+        occluded[i] = hit ? 1 : 0;
+    }
+    if (COUNT || MODE == RT_ISECT_VERIFY) flush_counters(c, g_counters);
+}
+
 // ------------------------------------------------------------------------------------------------
 // wavefront path tracer
 // ------------------------------------------------------------------------------------------------
@@ -1454,6 +1488,11 @@ static int build_tables(const rt_scene_desc* d, int n_sm, size_t smem_optin, Sce
         cudaFuncSetAttribute(k_intersect_batch<false, RT_ISECT_FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
         cudaFuncSetAttribute(k_intersect_batch<true, RT_ISECT_FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
         cudaFuncSetAttribute(k_intersect_batch<false, RT_ISECT_VERIFY>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
+        cudaFuncSetAttribute(k_occluded_batch<false, RT_ISECT_BRUTE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
+        cudaFuncSetAttribute(k_occluded_batch<true, RT_ISECT_BRUTE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
+        cudaFuncSetAttribute(k_occluded_batch<false, RT_ISECT_FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
+        cudaFuncSetAttribute(k_occluded_batch<true, RT_ISECT_FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
+        cudaFuncSetAttribute(k_occluded_batch<false, RT_ISECT_VERIFY>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
         cudaFuncSetAttribute(k_bounce<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
         cudaFuncSetAttribute(k_bounce<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
         cudaFuncSetAttribute(k_extend<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
@@ -1887,7 +1926,35 @@ void rt_scene_destroy(rt_scene* sc) {
     delete sc;
 }
 
-// ---- batched nearest hit -----------------------------------------------------------------------
+// ---- batched nearest hit ----------------------------------------------------------------------
+// A _device query on a caller stream st (st != sc->stream) is ordered against scene updates: it waits for the last
+// update's event before its launch, and afterwards records the stream's caller_done event, for which the next update
+// waits (a scene update waits for this call's reads of the tables).
+static int caller_wait_update(rt_scene* sc, cudaStream_t st) {
+    if (st != sc->stream && sc->ev_update) CU(cudaStreamWaitEvent(st, sc->ev_update, 0));   // after the last scene update
+    return RT_OK;
+}
+static int caller_record_done(rt_scene* sc, cudaStream_t st) {
+    if (st == sc->stream) return RT_OK;
+    auto it = std::find_if(sc->caller_done.begin(), sc->caller_done.end(), [&](const auto& c) { return c.first == st; });
+    if (it == sc->caller_done.end()) {
+        if (sc->caller_done.size() >= 32) {   // many distinct streams: fold their events into one, without a host wait
+            if (!sc->fold_stream) CU(cudaStreamCreateWithFlags(&sc->fold_stream, cudaStreamNonBlocking));
+            for (auto& c : sc->caller_done) CU(cudaStreamWaitEvent(sc->fold_stream, c.second, 0));
+            for (size_t k = 1; k < sc->caller_done.size(); k++) cudaEventDestroy(sc->caller_done[k].second);
+            sc->caller_done.resize(1);
+            sc->caller_done[0].first = sc->fold_stream;
+            CU(cudaEventRecord(sc->caller_done[0].second, sc->fold_stream));
+        }
+        cudaEvent_t e = nullptr;
+        CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+        sc->caller_done.push_back({st, e});
+        it = sc->caller_done.end() - 1;
+    }
+    CU(cudaEventRecord(it->second, st));
+    return RT_OK;
+}
+
 int rt_intersect_batch_device(rt_scene* sc, const rt_ray* d_rays, uint64_t n, double t_min, double t_max, int mode,
                               int32_t* d_idx, double* d_t, rt_vec3* d_normal, rt_vec3* d_point, double* d_uv,
                               uint8_t* d_ff, void* stream) {
@@ -1897,8 +1964,8 @@ int rt_intersect_batch_device(rt_scene* sc, const rt_ray* d_rays, uint64_t n, do
     if (!d_rays) return fail(RT_ERR_INVALID, "null rays");
     CU(cudaSetDevice(sc->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : sc->stream;
-    const bool caller = st != sc->stream;
-    if (caller && sc->ev_update) CU(cudaStreamWaitEvent(st, sc->ev_update, 0));   // after the last scene update
+    int rc = caller_wait_update(sc, st);
+    if (rc != RT_OK) return rc;
     uint64_t want = (n + 255) / 256;
     int grid = (int)std::min<uint64_t>(want, (uint64_t)sc->grid);
 #define RT_LAUNCH_ISECT(C_, M_)                                                                                  \
@@ -1914,25 +1981,7 @@ int rt_intersect_batch_device(rt_scene* sc, const rt_ray* d_rays, uint64_t n, do
 #undef RT_LAUNCH_ISECT
     sc->launches++;
     CU(cudaGetLastError());
-    if (caller) {   // a scene update waits for this call's reads of the tables
-        auto it = std::find_if(sc->caller_done.begin(), sc->caller_done.end(), [&](const auto& c) { return c.first == st; });
-        if (it == sc->caller_done.end()) {
-            if (sc->caller_done.size() >= 32) {   // many distinct streams: fold their events into one, without a host wait
-                if (!sc->fold_stream) CU(cudaStreamCreateWithFlags(&sc->fold_stream, cudaStreamNonBlocking));
-                for (auto& c : sc->caller_done) CU(cudaStreamWaitEvent(sc->fold_stream, c.second, 0));
-                for (size_t k = 1; k < sc->caller_done.size(); k++) cudaEventDestroy(sc->caller_done[k].second);
-                sc->caller_done.resize(1);
-                sc->caller_done[0].first = sc->fold_stream;
-                CU(cudaEventRecord(sc->caller_done[0].second, sc->fold_stream));
-            }
-            cudaEvent_t e = nullptr;
-            CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-            sc->caller_done.push_back({st, e});
-            it = sc->caller_done.end() - 1;
-        }
-        CU(cudaEventRecord(it->second, st));
-    }
-    return RT_OK;
+    return caller_record_done(sc, st);
 }
 
 int rt_intersect_batch(rt_scene* sc, const rt_ray* rays, uint64_t n, double t_min, double t_max, int mode,
@@ -1983,6 +2032,72 @@ int rt_intersect_batch(rt_scene* sc, const rt_ray* rays, uint64_t n, double t_mi
     float ms = 0.f;
     cudaEventElapsedTime(&ms, sc->ev_a, sc->ev_b);
     sc->last_intersect_ms = ms;
+    cleanup();
+#undef CUX
+    return RT_OK;
+}
+
+// ---- batched any-hit (occlusion) ---------------------------------------------------------------
+int rt_occluded_batch_device(rt_scene* sc, const rt_ray* d_rays, uint64_t n, double t_min, double t_max,
+                             const double* d_t_max_per_ray, int mode, uint8_t* d_occluded, void* stream) {
+    if (!sc) return fail(RT_ERR_INVALID, "null scene");
+    if (mode != RT_ISECT_BRUTE && mode != RT_ISECT_FAST && mode != RT_ISECT_VERIFY) return fail(RT_ERR_INVALID, "unknown intersect mode");
+    if (n == 0) return RT_OK;
+    if (!d_rays) return fail(RT_ERR_INVALID, "null rays");
+    if (!d_occluded) return fail(RT_ERR_INVALID, "null occluded");
+    CU(cudaSetDevice(sc->device));
+    cudaStream_t st = stream ? (cudaStream_t)stream : sc->stream;
+    int rc = caller_wait_update(sc, st);
+    if (rc != RT_OK) return rc;
+    const int grid = (int)std::min<uint64_t>((n + 255) / 256, (uint64_t)sc->grid);
+#define RT_LAUNCH_OCC(C_, M_)                                                                                      \
+    k_occluded_batch<C_, M_><<<grid, 256, sc->smem_bytes, st>>>(sc->ds, sc->use_smem, d_rays, n, t_min, t_max,       \
+                                                                d_t_max_per_ray, d_occluded, sc->d_counters)
+    if (mode == RT_ISECT_VERIFY) {
+        RT_LAUNCH_OCC(false, RT_ISECT_VERIFY);
+    } else if (sc->counters_on) {
+        if (mode == RT_ISECT_FAST) RT_LAUNCH_OCC(true, RT_ISECT_FAST); else RT_LAUNCH_OCC(true, RT_ISECT_BRUTE);
+    } else {
+        if (mode == RT_ISECT_FAST) RT_LAUNCH_OCC(false, RT_ISECT_FAST); else RT_LAUNCH_OCC(false, RT_ISECT_BRUTE);
+    }
+#undef RT_LAUNCH_OCC
+    sc->launches++;
+    CU(cudaGetLastError());
+    return caller_record_done(sc, st);
+}
+
+int rt_occluded_batch(rt_scene* sc, const rt_ray* rays, uint64_t n, double t_min, double t_max,
+                      const double* t_max_per_ray, int mode, uint8_t* occluded) {
+    if (!sc) return fail(RT_ERR_INVALID, "null scene");
+    if (mode != RT_ISECT_BRUTE && mode != RT_ISECT_FAST && mode != RT_ISECT_VERIFY) return fail(RT_ERR_INVALID, "unknown intersect mode");
+    if (n == 0) return RT_OK;
+    if (!rays) return fail(RT_ERR_INVALID, "null rays");
+    if (!occluded) return fail(RT_ERR_INVALID, "null occluded");
+    CU(cudaSetDevice(sc->device));
+    rt_ray* d_rays = nullptr;
+    double* d_tmax = nullptr;
+    uint8_t* d_occ = nullptr;
+    auto cleanup = [&]() { cudaFree(d_rays); cudaFree(d_tmax); cudaFree(d_occ); };
+#define CUX(call)                                                                             \
+    do {                                                                                      \
+        cudaError_t e_ = (call);                                                              \
+        if (e_ != cudaSuccess) {                                                              \
+            cleanup();                                                                        \
+            return fail(RT_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_));     \
+        }                                                                                     \
+    } while (0)
+    CUX(cudaMalloc(&d_rays, n * sizeof(rt_ray)));
+    CUX(cudaMalloc(&d_occ, n));
+    if (t_max_per_ray) CUX(cudaMalloc(&d_tmax, n * sizeof(double)));
+    CUX(cudaMemcpyAsync(d_rays, rays, n * sizeof(rt_ray), cudaMemcpyHostToDevice, sc->stream));
+    if (t_max_per_ray) CUX(cudaMemcpyAsync(d_tmax, t_max_per_ray, n * sizeof(double), cudaMemcpyHostToDevice, sc->stream));
+    int rc = rt_occluded_batch_device(sc, d_rays, n, t_min, t_max, d_tmax, mode, d_occ, sc->stream);
+    if (rc != RT_OK) {
+        cleanup();
+        return rc;
+    }
+    CUX(cudaMemcpyAsync(occluded, d_occ, n, cudaMemcpyDeviceToHost, sc->stream));
+    CUX(cudaStreamSynchronize(sc->stream));
     cleanup();
 #undef CUX
     return RT_OK;

@@ -275,7 +275,9 @@ __device__ __forceinline__ void analytic_test(const DevScene& S, int i, D3 ro, D
 
 // step 1.  Returns true when the ray is degenerate.  FP32 culling first (rt_cull.cuh): the flat list,
 // then roots -> groups -> leaves of the tree; each lane runs the exact test on its own survivors.
-template <bool COUNT, bool SMEM>
+// ANY (any_hit_fast): return at the first exact test that accepts the ray, winner >= 0.  Until then best == max_t, so
+// every test runs at the caller's bound.
+template <bool COUNT, bool SMEM, bool ANY = false>
 __device__ __forceinline__ bool analytic_nearest_impl(const DevScene& S, const CullRay& cr, D3 ro, D3 rd, double min_t,
                                                       double max_t, double& best, int& winner, DevCounters& c) {
     best = max_t;
@@ -299,6 +301,10 @@ __device__ __forceinline__ bool analytic_nearest_impl(const DevScene& S, const C
             const int2 tag = *reinterpret_cast<const int2*>(r + 16);
             if (SMEM) analytic_test_at<COUNT, false>(tag.x, tag.y, reinterpret_cast<const double2*>(r), r + 12, ro, rd, min_t, best, winner, degenerate, c);
             else analytic_test_at<COUNT, true>(tag.x, tag.y, reinterpret_cast<const double2*>(r), r + 12, ro, rd, min_t, best, winner, degenerate, c);
+            if (ANY && winner >= 0) {
+                if (COUNT) c.cull_tests += j + 1;
+                return degenerate;
+            }
         }
     } else
     for (int f0 = 0; f0 < S.n_flat; f0 += 32) {
@@ -313,6 +319,10 @@ __device__ __forceinline__ bool analytic_nearest_impl(const DevScene& S, const C
             // (a NaN ray passes every pre-test, the padding entries' too: their id is -1)
             const int id = __ldg(flat_ids + f0 + j);
             if (id >= 0) analytic_test<COUNT>(S, id, ro, rd, min_t, best, winner, degenerate, c);
+            if (ANY && winner >= 0) {
+                if (COUNT) c.cull_tests += min(f0 + nf, S.n_flat_real);
+                return degenerate;
+            }
         }
     }
     if (COUNT) c.cull_tests += S.n_flat_real;
@@ -354,16 +364,17 @@ __device__ __forceinline__ bool analytic_nearest_impl(const DevScene& S, const C
                 mask &= mask - 1;
                 const int id = __ldg(S.cids + RT_CULL_GROUP * g + j);
                 if (id >= 0) analytic_test<COUNT>(S, id, ro, rd, min_t, best, winner, degenerate, c);
+                if (ANY && winner >= 0) return degenerate;
             }
         }
     }
     return degenerate;
 }
-template <bool COUNT>
+template <bool COUNT, bool ANY = false>
 __device__ __forceinline__ bool analytic_nearest(const DevScene& S, const Staged& st, const CullRay& cr, D3 ro, D3 rd,
                                                  double min_t, double max_t, double& best, int& winner, DevCounters& c) {
-    if (st.smem) return analytic_nearest_impl<COUNT, true>(S, cr, ro, rd, min_t, max_t, best, winner, c);
-    return analytic_nearest_impl<COUNT, false>(S, cr, ro, rd, min_t, max_t, best, winner, c);
+    if (st.smem) return analytic_nearest_impl<COUNT, true, ANY>(S, cr, ro, rd, min_t, max_t, best, winner, c);
+    return analytic_nearest_impl<COUNT, false, ANY>(S, cr, ro, rd, min_t, max_t, best, winner, c);
 }
 
 // does marched shape number k (position in S.march_index) have to be marched for this ray, given the
@@ -433,6 +444,43 @@ __device__ __forceinline__ void nearest_hit_fast(const DevScene& S, const Staged
     if (COUNT) c.segments++;
     best_t = best;
     best_i = winner;
+}
+
+// Any-hit (rt_occluded_batch): does some shape accept the ray at (min_t, max_t)?  The literal loop's max_t only
+// shrinks at an acceptance, so its first acceptance is tested at max_t, and it returns a hit iff some shape accepts at
+// max_t -- a Sphere D == 0 hit and a NaN t included.  So the answer is nearest_hit_brute's `index != -1`, in any
+// order of the shapes, and the walk stops at the first acceptance.
+template <bool COUNT>
+__device__ __forceinline__ bool any_hit_brute(const DevScene& S, D3 ro, D3 rd, double min_t, double max_t,
+                                              DevCounters& c) {
+    for (int i = 0; i < S.n_shapes; i++) {
+        double t;
+        if (shape_candidate<COUNT>(S, i, S.kind[i], S.inv + 12 * i, ro, rd, min_t, max_t, t, c)) return true;
+    }
+    return false;
+}
+
+// The same answer through the cull tree: the analytic shapes first, then the marched ones (exact skipping, chords
+// that start past max_t skipped), each stopping at the first acceptance.  A degenerate ray (a Sphere D == 0 branch or
+// a NaN t the analytic pass did not accept, a Torus ball touched, a NaN marched t) finishes through the literal loop.
+// A NaN bound does too: march_needed drops every chord against it, the literal loop does not.  The marcher runs without
+// the Bernstein miss proof, like k_intersect_batch's: on a B200 the proof made dupin's shadow rays 10 % slower (424.6 ->
+// 383.9 Mrays/s) and the bench trio's config 2 rays 7 % faster (2381 -> 2540), so the simpler form stays.
+template <bool COUNT>
+__device__ __forceinline__ bool any_hit_fast(const DevScene& S, const Staged& st, D3 ro, D3 rd, double min_t,
+                                             double max_t, DevCounters& c) {
+    if (max_t != max_t || min_t != min_t) return any_hit_brute<COUNT>(S, ro, rd, min_t, max_t, c);
+    double best;
+    int winner;
+    const CullRay cr = make_cull_ray(ro.x, ro.y, ro.z, rd.x, rd.y, rd.z);
+    bool degenerate = analytic_nearest<COUNT, true>(S, st, cr, ro, rd, min_t, max_t, best, winner, c);
+    if (winner >= 0) return true;
+    for (int k = 0; k < S.n_march && !degenerate; k++) {
+        degenerate = march_shape_update<COUNT>(S, cr, S.inv, k, ro, rd, min_t, max_t, best, winner, c);
+        if (winner >= 0) return true;
+    }
+    if (degenerate) return any_hit_brute<COUNT>(S, ro, rd, min_t, max_t, c);
+    return false;
 }
 
 // ------------------------------------------------------------------------------------------------

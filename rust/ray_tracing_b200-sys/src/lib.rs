@@ -92,6 +92,10 @@ extern "C" {
     pub fn rt_intersect_batch_device(scene: *mut rt_scene, d_rays: *const rt_ray, n: u64, t_min: f64, t_max: f64,
         mode: c_int, d_shape_index: *mut i32, d_t: *mut f64, d_normal: *mut rt_vec3, d_point: *mut rt_vec3,
         d_uv: *mut f64, d_front_face: *mut u8, stream: *mut c_void) -> c_int;
+    pub fn rt_occluded_batch(scene: *mut rt_scene, rays: *const rt_ray, n: u64, t_min: f64, t_max: f64,
+        t_max_per_ray: *const f64, mode: c_int, occluded: *mut u8) -> c_int;
+    pub fn rt_occluded_batch_device(scene: *mut rt_scene, d_rays: *const rt_ray, n: u64, t_min: f64, t_max: f64,
+        d_t_max_per_ray: *const f64, mode: c_int, d_occluded: *mut u8, stream: *mut c_void) -> c_int;
     pub fn rt_render_start(scene: *mut rt_scene, camera: *const rt_camera, params: *const rt_render_params) -> c_int;
     pub fn rt_render_poll(scene: *mut rt_scene, buffer: *mut rt_vec3, done: *mut c_int) -> c_int;
     pub fn rt_render_wait(scene: *mut rt_scene, buffer: *mut rt_vec3) -> c_int;
