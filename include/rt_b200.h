@@ -206,7 +206,8 @@ int rt_scene_device_count(rt_scene* scene);
 /* ---- scene updates on a live handle (the reference renders whatever its Arc<RwLock<Scene>> holds when a frame starts,
  *      src/renderer/step_by_step.rs:37) ----------------------------------------------------------------------------
  * Contract of both entries: after the call, every entry point (rt_intersect_batch[_device] in every mode and with
- * every output, rt_occluded_batch[_device], rt_render_start and the adaptive, counts and views frames, rt_trace_pixel_samples[_group][_device])
+ * every output, rt_occluded_batch[_device], rt_scatter_batch[_device], rt_render_start and the adaptive, counts and views
+ * frames, rt_trace_pixel_samples[_group][_device])
  * gives bit for bit what a handle freshly created from the edited description gives.  The handle keeps its streams,
  * lanes, buffers, peer access and settings.
  *   - RT_ERR_STATE while a frame is in flight (that frame goes on with the old scene).
@@ -215,9 +216,10 @@ int rt_scene_device_count(rt_scene* scene);
  *   - The last completed frame stays readable (rt_render_device_frame, rt_render_device_result, rt_render_pixel_stats,
  *     rt_tonemap_rgba8_device); rt_stats is untouched.
  *   - An update is ordered after all work the handle enqueued before it, rt_intersect_batch_device,
- *     rt_occluded_batch_device and rt_trace_pixel_samples_group_device calls on caller streams included, and work
- *     enqueued after it sees the new scene.  For that, rt_intersect_batch_device and rt_occluded_batch_device on a
- *     caller stream record an event there at the end of each call
+ *     rt_occluded_batch_device, rt_scatter_batch_device and rt_trace_pixel_samples_group_device calls on caller
+ *     streams included, and work enqueued after it sees the new scene.  For that, rt_intersect_batch_device,
+ *     rt_occluded_batch_device and rt_scatter_batch_device on a caller stream record an event there at the end of each
+ *     call
  *     (one per stream; past 32 streams they are joined on an internal stream, never waited for on the host) and waits
  *     for the last update's event.
  *   - rt_scene_update_transforms allocates what it needs before the host copy of the tree changes; if the device work
@@ -293,6 +295,41 @@ int rt_occluded_batch(rt_scene* scene, const rt_ray* rays, uint64_t n, double t_
  * not synchronise, and is ordered against scene updates like it. */
 int rt_occluded_batch_device(rt_scene* scene, const rt_ray* d_rays, uint64_t n, double t_min, double t_max,
                              const double* d_t_max_per_ray, int mode, uint8_t* d_occluded, void* stream);
+
+/* ---- batched scatter (one segment of ray_color, src/renderer/mod.rs:23-45, for caller rays) ------------------------
+ * What the surface does with each ray: the nearest hit, then Material::scatter / Material::emitted or
+ * Scene::background, with the path RNG of the frame.  Iterating it from a pixel's camera rays and multiplying the
+ * throughput forward (beta = beta * color at a scatter, L = beta * color at a miss or an emission, L = 0 at a hit on
+ * the last level, L rounded to float) gives rt_trace_pixel_samples_group and the rt_render_start frame bit for bit.
+ *   - Nearest hit: rt_intersect_batch's in `mode` (RT_ISECT_VERIFY counts into rt_stats as it does there);
+ *     shape_index[i] and t[i] are bit for bit what that call returns.
+ *   - Miss: outcome[i] = RT_BOUNCE_MISS, color[i] = Scene::background(direction) (world/mod.rs:199-202).
+ *   - Hit: the hit is finalised as the frame finalises it, and Material::scatter runs with the Philox stream keyed by
+ *     (seed; keys[2i], keys[2i+1]) at event level + 1: the stream the frame uses at the level-th hit of sample
+ *     keys[2i+1] of pixel keys[2i].  A material that scatters gives outcome RT_BOUNCE_SCATTER, color = the attenuation
+ *     and scattered[i] = (RayHit.point, the unit new direction); otherwise outcome RT_BOUNCE_EMIT and color =
+ *     Material::emitted (zero for EmptyMaterial).
+ *   - Outputs that do not apply to a ray are zero (t and scattered of a miss, scattered of an emission).
+ *   - The depth == 0 rule (mod.rs:26-27) is the caller's: on the last level of a path a hit is black.
+ *   - level <= 62 (the deepest level a frame reaches); n = 0 does nothing.  RT_ERR_INVALID for a NULL scene, an
+ *     unknown mode, a level above 62 (checked in that order, before n = 0), or NULL rays / keys with n > 0.
+ *   - The host form copies through the handle's stream and synchronises it; every output may be NULL.  With counters
+ *     on, the work counters are rt_intersect_batch's for the same rays; last_intersect_ms is not touched.  The call
+ *     may be made while a frame is in flight and leaves that frame, its accumulator and rt_stats.paths alone.  A
+ *     multi-device handle answers on device_ids[0]. */
+enum { RT_BOUNCE_MISS = 0, RT_BOUNCE_SCATTER = 1, RT_BOUNCE_EMIT = 2 };
+int rt_scatter_batch(rt_scene* scene, const rt_ray* rays, const uint32_t* keys, uint64_t n, uint32_t level,
+                     uint64_t seed, double t_min, double t_max, int mode, int32_t* shape_index, double* t,
+                     uint8_t* outcome, rt_vec3* color, rt_ray* scattered);
+/* Same, with every pointer a DEVICE pointer on the scene's device and no copies; runs on `stream` like
+ * rt_intersect_batch_device (NULL = the library's own stream, cudaStreamLegacy = 0x1 the legacy default stream), does
+ * not synchronise, and is ordered against scene updates like it.  d_shape_index and d_t are required (RT_ERR_INVALID
+ * when NULL with n > 0, after the checks above): the nearest hit is written there first and shaded by a second
+ * kernel.  The other outputs may be NULL. */
+int rt_scatter_batch_device(rt_scene* scene, const rt_ray* d_rays, const uint32_t* d_keys, uint64_t n,
+                            uint32_t level, uint64_t seed, double t_min, double t_max, int mode,
+                            int32_t* d_shape_index, double* d_t, uint8_t* d_outcome, rt_vec3* d_color,
+                            rt_ray* d_scattered, void* stream);
 
 /* ---- frame rendering (replaces the Renderer trait, src/renderer/mod.rs:47-56) -------- */
 

@@ -13,6 +13,7 @@ HOST_SO = os.path.join(HERE, "librt_b200_host.so")
 RT_OK = 0
 RT_ERR_INVALID, RT_ERR_NO_DEVICE, RT_ERR_CUDA, RT_ERR_STATE, RT_ERR_NOMEM = -1, -2, -3, -4, -5
 RT_ISECT_BRUTE, RT_ISECT_FAST, RT_ISECT_VERIFY = 0, 1, 2
+RT_BOUNCE_MISS, RT_BOUNCE_SCATTER, RT_BOUNCE_EMIT = 0, 1, 2
 RT_SHAPE_SPHERE, RT_SHAPE_CUBE, RT_SHAPE_RECTANGLE, RT_SHAPE_MARCH, RT_SHAPE_TORUS = 0, 1, 2, 3, 4
 RT_SURF_HEART, RT_SURF_SINE, RT_SURF_STAR, RT_SURF_DUPIN, RT_SURF_HUNTS, RT_SURF_CUSHION = range(6)
 RT_MAT_LAMBERTIAN, RT_MAT_METAL, RT_MAT_DIELECTRIC, RT_MAT_DIFFUSE_LIGHT, RT_MAT_EMPTY = range(5)
@@ -149,6 +150,11 @@ CORE_SYMBOLS = {
                                     C.c_void_p]),
     "rt_occluded_batch_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.c_double, C.c_void_p,
                                            C.c_int, C.c_void_p, C.c_void_p]),
+    "rt_scatter_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint64, C.c_double,
+                                   C.c_double, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "rt_scatter_batch_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint64,
+                                          C.c_double, C.c_double, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                          C.c_void_p, C.c_void_p, C.c_void_p]),
     "rt_render_start": (C.c_int, [C.c_void_p, C.POINTER(Camera), C.POINTER(RenderParams)]),
     "rt_render_poll": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(C.c_int)]),
     "rt_render_wait": (C.c_int, [C.c_void_p, C.c_void_p]),

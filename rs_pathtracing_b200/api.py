@@ -125,6 +125,34 @@ def check_t_max(t_max, n: int):
     return math.inf, t_max
 
 
+SCATTER_OUTPUTS = ("index", "t", "outcome", "color", "scattered")   # rt_scatter_batch's output order
+
+
+def check_scatter_inputs(rays, keys) -> None:
+    """Scene.scatter's inputs: rays a contiguous (n, 6) float64 array and keys a contiguous (n, 2) uint32 array (pixel,
+    sample), both numpy or both CUDA torch tensors on one device"""
+    is_torch = type(rays).__module__.split(".")[0] == "torch"
+    if is_torch != (type(keys).__module__.split(".")[0] == "torch"):
+        raise ValueError("rays and keys: both numpy arrays or both torch tensors")
+    if is_torch:
+        if not (rays.is_cuda and keys.is_cuda):
+            raise ValueError("rays and keys: CUDA tensors")
+        if keys.device != rays.device:
+            raise ValueError(f"keys are on {keys.device}, rays are on {rays.device}")
+        contiguous = rays.is_contiguous() and keys.is_contiguous()
+    elif not (isinstance(rays, np.ndarray) and isinstance(keys, np.ndarray)):
+        raise ValueError("rays and keys: numpy arrays or CUDA torch tensors")
+    else:
+        contiguous = rays.flags["C_CONTIGUOUS"] and keys.flags["C_CONTIGUOUS"]
+    rdt, kdt = str(rays.dtype).replace("torch.", ""), str(keys.dtype).replace("torch.", "")
+    if len(rays.shape) != 2 or rays.shape[1] != 6 or rdt != "float64":
+        raise ValueError(f"rays: an (n, 6) float64 array, got shape {tuple(rays.shape)} dtype {rdt}")
+    if tuple(keys.shape) != (rays.shape[0], 2) or kdt != "uint32":
+        raise ValueError(f"keys: an ({rays.shape[0]}, 2) uint32 array, got shape {tuple(keys.shape)} dtype {kdt}")
+    if not contiguous:
+        raise ValueError("rays and keys must be contiguous")
+
+
 class Scene:
     """world::Scene (src/world/mod.rs:20-49)."""
 
@@ -267,6 +295,38 @@ class Scene:
         _check(_ffi.core().rt_occluded_batch(self.device_scene(device), p(rays), n, min_t, t_max, p(per_ray), mode,
                                              p(out)))
         return out.view(np.bool_)
+
+    def scatter(self, rays, keys, level: int, seed: int = 0, min_t: float = 0.001, max_t: float = math.inf,
+                mode: int = _ffi.RT_ISECT_FAST, device: Optional[int] = None) -> dict:
+        """one segment of ray_color for each ray (rt_scatter_batch): the nearest hit, then what its material does with
+        the ray, with the frame's RNG stream of sample keys[i, 1] of pixel keys[i, 0] at its level-th hit.  Returns
+        {"index": (n,) int32, "t": (n,) float64, "outcome": (n,) uint8 (RT_BOUNCE_MISS / _SCATTER / _EMIT), "color":
+        (n, 3) float64 (sky, attenuation or emission), "scattered": (n, 6) float64 (origin, unit direction)}.
+        rays (n, 6) float64 and keys (n, 2) uint32, both contiguous: numpy arrays -> numpy results after the host round
+        trip; or CUDA torch tensors on the scene's device -> torch tensors there, queued on torch's current stream
+        without a host synchronisation (rt_scatter_batch_device)."""
+        check_scatter_inputs(rays, keys)
+        n = rays.shape[0]
+        if type(rays).__module__.split(".")[0] == "torch":
+            import torch
+            h = self.device_scene(device)
+            if rays.device.index != self._device:
+                raise ValueError(f"rays are on {rays.device}, the scene's device is cuda:{self._device}")
+            new = lambda shape, dt: torch.empty(shape, dtype=dt, device=rays.device)
+            out = {"index": new((n,), torch.int32), "t": new((n,), torch.float64), "outcome": new((n,), torch.uint8),
+                   "color": new((n, 3), torch.float64), "scattered": new((n, 6), torch.float64)}
+            # torch's default stream is the legacy default stream (handle 0), which the ABI names cudaStreamLegacy = 0x1
+            stream = torch.cuda.current_stream(rays.device).cuda_stream or 1
+            _check(_ffi.core().rt_scatter_batch_device(h, rays.data_ptr(), keys.data_ptr(), n, level, seed, min_t,
+                                                       max_t, mode, *(out[k].data_ptr() for k in SCATTER_OUTPUTS),
+                                                       stream))
+            return out
+        out = {"index": np.empty(n, np.int32), "t": np.empty(n), "outcome": np.empty(n, np.uint8),
+               "color": np.empty((n, 3)), "scattered": np.empty((n, 6))}
+        p = lambda a: a.ctypes.data_as(C.c_void_p)
+        _check(_ffi.core().rt_scatter_batch(self.device_scene(device), p(rays), p(keys), n, level, seed, min_t, max_t,
+                                            mode, *(p(out[k]) for k in SCATTER_OUTPUTS)))
+        return out
 
     def trace_pixel_samples(self, rays: np.ndarray, depth: int, seed: int = 0, pixel_index: int = 0,
                             device: Optional[int] = None):
@@ -595,6 +655,123 @@ def occluded_device(dev_scene, rays, out, t_max=math.inf, t_min: float = 0.001, 
                                                 per_ray.data_ptr() if per_ray is not None else None, mode,
                                                 out.data_ptr(), stream))
     return out
+
+
+MAX_LEVEL = 62   # the deepest level a frame reaches (rt_render_params.max_depth <= 62)
+
+
+def trace_paths(scene: Scene, rays, keys, depth: int, seed: int = 0, record: bool = False):
+    """ray_color (src/renderer/mod.rs:23-45) as a bounce loop over Scene.scatter, in the frame's own arithmetic: the
+    throughput starts at (1, 1, 1) and is multiplied forward (beta = beta * color at a scatter), a path ends with
+    L = beta * color at a miss or an emission and with L = 0 at a hit on level `depth`, and only the paths still alive
+    go to the next level's call.  Ray i is sample keys[i, 1] of pixel keys[i, 0]; fed a frame's primary rays, the
+    result averaged by group_means is that frame bit for bit.  rays / keys as Scene.scatter takes them (numpy, or CUDA
+    torch tensors: then every level runs on torch's current stream).
+    Returns the (n, 3) float32 radiance; with record=True also a list with one dict per level of the paths alive there:
+    "ray" (which input ray), "shape", "outcome", "origin", "color" and "beta" (the throughput the path arrives with)."""
+    if not 0 <= depth <= MAX_LEVEL:
+        raise ValueError(f"depth must be in [0, {MAX_LEVEL}], got {depth}")
+    check_scatter_inputs(rays, keys)
+    n = rays.shape[0]
+    if type(rays).__module__.split(".")[0] == "torch":
+        import torch
+        full = lambda v: torch.full((n, 3), v, dtype=torch.float64, device=rays.device)
+        live = torch.arange(n, device=rays.device)
+        where = lambda m: torch.nonzero(m).reshape(-1)
+        # (uint32 tensors cannot be gathered on every torch build: the keys are moved as int32)
+        ikeys = keys.view(torch.int32)
+        take_keys = lambda idx: ikeys[idx].view(torch.uint32)
+        to_f32 = lambda a: a.to(torch.float32)
+    else:
+        full = lambda v: np.full((n, 3), v)
+        live = np.arange(n)
+        where = np.flatnonzero
+        take_keys = lambda idx: keys[idx]
+        to_f32 = lambda a: a.astype(np.float32)
+    beta, L = full(1.0), full(0.0)
+    levels = []
+    cur = rays
+    for level in range(depth + 1):
+        if len(live) == 0:
+            break
+        out = scene.scatter(cur, keys if level == 0 else take_keys(live), level, seed)
+        oc, col, b = out["outcome"], out["color"], beta[live]
+        if record:
+            levels.append({"ray": live, "shape": out["index"], "outcome": oc, "origin": cur[:, :3], "color": col,
+                           "beta": b})
+        # a miss ends the path with the sky, an emission with its light; on the last level a hit is black (mod.rs:26-27)
+        end = where(oc == _ffi.RT_BOUNCE_MISS) if level == depth else where(oc != _ffi.RT_BOUNCE_SCATTER)
+        L[live[end]] = b[end] * col[end]
+        if level == depth:
+            break
+        go = where(oc == _ffi.RT_BOUNCE_SCATTER)
+        live = live[go]
+        beta[live] = b[go] * col[go]
+        cur = out["scattered"][go]
+    return (to_f32(L), levels) if record else to_f32(L)
+
+
+def _philox_uniforms(seed: int, pixel, sample, event: int):
+    """the first two doubles of the path RNG's stream (seed; pixel, sample, event): Philox4x32-10 of the counter
+    (pixel, sample, event, 0) under the key (seed low, seed high) -- the device's PathRng.next(), twice"""
+    m32 = np.uint64(0xFFFFFFFF)
+    c0, c1 = pixel.astype(np.uint64), sample.astype(np.uint64)
+    c2, c3 = np.full_like(c0, event), np.zeros_like(c0)
+    k0, k1 = seed & 0xFFFFFFFF, seed >> 32
+    for _ in range(10):
+        p0, p1 = np.uint64(0xD2511F53) * c0, np.uint64(0xCD9E8D57) * c2
+        c0, c1, c2, c3 = (p1 >> np.uint64(32)) ^ c1 ^ np.uint64(k0), p1 & m32, (p0 >> np.uint64(32)) ^ c3 ^ np.uint64(k1), p0 & m32
+        k0, k1 = (k0 + 0x9E3779B9) & 0xFFFFFFFF, (k1 + 0xBB67AE85) & 0xFFFFFFFF
+    a = (c1 << np.uint64(32)) | c0
+    b = (c3 << np.uint64(32)) | c2
+    s53 = 1.0 / 9007199254740992.0
+    return (a >> np.uint64(11)).astype(np.float64) * s53, (b >> np.uint64(11)).astype(np.float64) * s53
+
+
+def primary_rays(camera: Camera, width: int, height: int, pixels, spp: int, seed: int = 0):
+    """the frame's own primary rays of `pixels` (indices x + y*width), samples 0 .. spp-1 of each, sample-minor, with
+    their keys (pixel, sample): MultisamplerRayCaster::next (src/camera/ray_caster.rs:100-118) with the two draws of
+    event 0 of each path's RNG, in the frame's arithmetic.  Returns (rays (n, 6) float64, keys (n, 2) uint32), what
+    trace_paths takes to reproduce those pixels of a render_start frame of this camera, size and seed."""
+    pix = np.repeat(np.asarray(pixels, np.uint32).reshape(-1), spp)
+    smp = np.tile(np.arange(spp, dtype=np.uint32), pix.size // max(spp, 1))
+    u, v = _philox_uniforms(seed, pix, smp, 0)
+    # MultisamplerRayCaster::new (ray_caster.rs:30-48), as the library computes it on the host
+    pos, dirn = camera.position.tuple(), camera.direction.tuple()
+    right, up = camera.right.tuple(), camera.up.tuple()
+    center = [pos[k] + dirn[k] * camera.focal_length for k in range(3)]
+    vw = math.tan(camera.fov_rad / 2.0) * camera.focal_length * 2.0
+    vh = vw / (width / height)
+    hw, hh = vw / 2.0, vh / 2.0
+    left_top = [(center[k] - hw * right[k]) + hh * up[k] for k in range(3)]
+    res = vw / width
+    x = (pix % width).astype(np.float64) + u
+    y = (pix // width).astype(np.float64) + v
+    d = np.stack([(left_top[k] + (res * x) * right[k]) - (res * y) * up[k] - pos[k] for k in range(3)], 1)
+    ln = np.sqrt((d[:, 0] * d[:, 0] + d[:, 1] * d[:, 1]) + d[:, 2] * d[:, 2])
+    rays = np.empty((pix.size, 6))
+    rays[:, :3] = pos
+    rays[:, 3:] = d / ln[:, None]
+    return rays, np.ascontiguousarray(np.stack([pix, smp], 1))
+
+
+def group_means(radiance, offsets) -> np.ndarray:
+    """the per-group mean of per-ray radiance as trace_pixel_samples_group and the frame take it: group g = rays
+    offsets[g] .. offsets[g+1]-1, f64 sums of the float radiance in ray order from 0.0, one division by the group's
+    count (an empty group is NaN).  radiance (n, 3) float32 (numpy or torch); returns (G, 3) float64 numpy."""
+    if type(radiance).__module__.split(".")[0] == "torch":
+        radiance = radiance.cpu().numpy()
+    f = np.asarray(radiance, dtype=np.float32).reshape(-1, 3).astype(np.float64)
+    off = np.asarray(offsets, dtype=np.int64).reshape(-1)
+    if off.size == 0 or off[0] != 0 or off[-1] != f.shape[0] or (np.diff(off) < 0).any():
+        raise ValueError("offsets must rise from 0 to len(radiance)")
+    count = np.diff(off)
+    s = np.zeros((count.size, 3))
+    for k in range(int(count.max(initial=0))):   # step k adds ray k of every group that has one: the in-order sums
+        m = count > k
+        s[m] = s[m] + f[off[:-1][m] + k]
+    with np.errstate(invalid="ignore"):
+        return s / count[:, None]
 
 
 def check_counts(counts, width: int, height: int) -> np.ndarray:

@@ -6,6 +6,7 @@
 //   k_raygen_views      views frames: k_raygen over the stacked image of several views, each with its own camera
 //   k_bounce            one segment of ray_color for every live path: nearest hit, scatter / emit /
 //                       sky, survivors compacted into the next queue (ballot + popc + one atomic per warp)
+//   k_scatter_shade     rt_scatter_batch: the shading half of that segment for caller rays after k_intersect_batch
 //   k_resolve           per-pixel mean (trace_pixel_samples) -> (f64 sums, samples) accumulator + f64 frame
 //   k_load_groups       caller-supplied rays of groups of any size -> level-0 queue + RNG keys (trace_pixel_samples_group)
 //   k_group_resolve     per-group mean of caller-supplied rays, continued across the batches of a large group
@@ -631,6 +632,65 @@ k_shade(DevScene S, PathQueue in, const uint32_t* __restrict__ count_in, HitQueu
             shade_slot(S, in, hq, out, count_out, level, max_depth, k0, k1, radiance, s_id, i, valid);
         }
         __syncthreads();
+    }
+}
+
+// rt_scatter_batch: shade_slot's segment for caller rays whose nearest hit k_intersect_batch already wrote -- sky at a
+// miss, else finalize_hit and scatter_or_emit with the path RNG of (seed; keys[2i], keys[2i+1]) at event level + 1.  No
+// depth rule, no throughput, no queue: the caller multiplies and decides.  The trip count is rounded up to whole warps
+// so that every lane of a warp reaches coop_random_in_unit_sphere (level is uniform over the call, so is its event).
+__global__ void __launch_bounds__(256)
+k_scatter_shade(DevScene S, const rt_ray* __restrict__ rays, const uint32_t* __restrict__ keys, unsigned long long n,
+                uint32_t level, uint32_t k0, uint32_t k1, const int32_t* __restrict__ shape_index,
+                const double* __restrict__ t_in, uint8_t* __restrict__ outcome, rt_vec3* __restrict__ color,
+                rt_ray* __restrict__ scattered) {
+    __shared__ uint4 s_ball_id[256];
+    uint4* const s_id = s_ball_id + (threadIdx.x & ~31u);
+    const unsigned long long n_round = (n + 31ull) & ~31ull;
+    const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
+    for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < n_round; i += stride) {
+        const bool valid = i < n;
+        bool shading = false, need_ball = false;
+        uint8_t oc = RT_BOUNCE_MISS;
+        D3 rd = mk(0, 0, 0), col = mk(0.0, 0.0, 0.0), so = mk(0.0, 0.0, 0.0), sd = mk(0.0, 0.0, 0.0);
+        HitRec h;
+        PathRng rng;
+        rng.k0 = k0; rng.k1 = k1;
+        rng.pixel = 0; rng.sample = 0;
+        rng.begin_event(level + 1);
+        if (valid) {
+            const rt_ray r = rays[i];
+            rd = mk(r.direction.x, r.direction.y, r.direction.z);
+            const int bi = shape_index[i];
+            if (bi < 0) {
+                col = sky(rd);  // renderer/mod.rs:41-43
+            } else {
+                const D3 ro = mk(r.origin.x, r.origin.y, r.origin.z);
+                const rt_material mat = S.materials[S.material[bi]];
+                finalize_hit(S, bi, t_in[i], ro, rd, h, material_reads_uv(S, mat));
+                rng.pixel = keys[2 * i];
+                rng.sample = keys[2 * i + 1];
+                shading = true;
+                need_ball = material_needs_ball(mat);
+            }
+        }
+        const D3 ball = coop_random_in_unit_sphere(need_ball, rng.pixel, rng.sample, level + 1, k0, k1, s_id);
+        if (shading) {
+            D3 ndir, atten;
+            if (scatter_or_emit(S, h, rd, rng, ndir, atten, &ball)) {  // :29-32
+                oc = RT_BOUNCE_SCATTER;
+                so = h.point;
+                sd = ndir;
+            } else {
+                oc = RT_BOUNCE_EMIT;  // :34-36
+            }
+            col = atten;
+        }
+        if (valid) {
+            if (outcome) outcome[i] = oc;
+            if (color) color[i] = rt_vec3{col.x, col.y, col.z};
+            if (scattered) scattered[i] = rt_ray{rt_vec3{so.x, so.y, so.z}, rt_vec3{sd.x, sd.y, sd.z}};
+        }
     }
 }
 
@@ -2097,6 +2157,90 @@ int rt_occluded_batch(rt_scene* sc, const rt_ray* rays, uint64_t n, double t_min
         return rc;
     }
     CUX(cudaMemcpyAsync(occluded, d_occ, n, cudaMemcpyDeviceToHost, sc->stream));
+    CUX(cudaStreamSynchronize(sc->stream));
+    cleanup();
+#undef CUX
+    return RT_OK;
+}
+
+// ---- batched scatter (one segment of ray_color) -----------------------------------------------------------------------
+// Two launches on the call's stream: k_intersect_batch writes index and t, k_scatter_shade shades.  Shading inside the
+// nearest-hit kernel would add to its spills (FAST sits at 255 registers), and the split leaves that kernel as it is.
+static int scatter_args(rt_scene* sc, uint32_t level, int mode) {
+    if (!sc) return fail(RT_ERR_INVALID, "null scene");
+    if (mode != RT_ISECT_BRUTE && mode != RT_ISECT_FAST && mode != RT_ISECT_VERIFY) return fail(RT_ERR_INVALID, "unknown intersect mode");
+    if (level > RT_MAX_LEVELS - 2) return fail(RT_ERR_INVALID, "level too large (limit 62)");
+    return RT_OK;
+}
+
+int rt_scatter_batch_device(rt_scene* sc, const rt_ray* d_rays, const uint32_t* d_keys, uint64_t n, uint32_t level,
+                            uint64_t seed, double t_min, double t_max, int mode, int32_t* d_idx, double* d_t,
+                            uint8_t* d_outcome, rt_vec3* d_color, rt_ray* d_scattered, void* stream) {
+    int rc = scatter_args(sc, level, mode);
+    if (rc != RT_OK) return rc;
+    if (n == 0) return RT_OK;
+    if (!d_rays) return fail(RT_ERR_INVALID, "null rays");
+    if (!d_keys) return fail(RT_ERR_INVALID, "null keys");
+    if (!d_idx || !d_t) return fail(RT_ERR_INVALID, "the device form needs d_shape_index and d_t");
+    // (rt_intersect_batch_device orders the first launch against scene updates; the second follows it on the stream)
+    rc = rt_intersect_batch_device(sc, d_rays, n, t_min, t_max, mode, d_idx, d_t, nullptr, nullptr, nullptr, nullptr,
+                                   stream);
+    if (rc != RT_OK) return rc;
+    cudaStream_t st = stream ? (cudaStream_t)stream : sc->stream;
+    const int grid = (int)std::min<uint64_t>((n + 255) / 256, (uint64_t)sc->grid);
+    k_scatter_shade<<<grid, 256, 0, st>>>(sc->ds, d_rays, d_keys, n, level, (uint32_t)seed, (uint32_t)(seed >> 32),
+                                          d_idx, d_t, d_outcome, d_color, d_scattered);
+    sc->launches++;
+    CU(cudaGetLastError());
+    return caller_record_done(sc, st);
+}
+
+int rt_scatter_batch(rt_scene* sc, const rt_ray* rays, const uint32_t* keys, uint64_t n, uint32_t level, uint64_t seed,
+                     double t_min, double t_max, int mode, int32_t* idx, double* t, uint8_t* outcome, rt_vec3* color,
+                     rt_ray* scattered) {
+    int rc = scatter_args(sc, level, mode);
+    if (rc != RT_OK) return rc;
+    if (n == 0) return RT_OK;
+    if (!rays) return fail(RT_ERR_INVALID, "null rays");
+    if (!keys) return fail(RT_ERR_INVALID, "null keys");
+    CU(cudaSetDevice(sc->device));
+    rt_ray *d_rays = nullptr, *d_sc = nullptr;
+    uint32_t* d_keys = nullptr;
+    int32_t* d_idx = nullptr;
+    double* d_t = nullptr;
+    uint8_t* d_oc = nullptr;
+    rt_vec3* d_col = nullptr;
+    auto cleanup = [&]() {
+        cudaFree(d_rays); cudaFree(d_keys); cudaFree(d_idx); cudaFree(d_t); cudaFree(d_oc); cudaFree(d_col); cudaFree(d_sc);
+    };
+#define CUX(call)                                                                             \
+    do {                                                                                      \
+        cudaError_t e_ = (call);                                                              \
+        if (e_ != cudaSuccess) {                                                              \
+            cleanup();                                                                        \
+            return fail(RT_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_));     \
+        }                                                                                     \
+    } while (0)
+    CUX(cudaMalloc(&d_rays, n * sizeof(rt_ray)));
+    CUX(cudaMalloc(&d_keys, 2 * n * sizeof(uint32_t)));
+    CUX(cudaMalloc(&d_idx, n * sizeof(int32_t)));
+    CUX(cudaMalloc(&d_t, n * sizeof(double)));
+    if (outcome) CUX(cudaMalloc(&d_oc, n));
+    if (color) CUX(cudaMalloc(&d_col, n * sizeof(rt_vec3)));
+    if (scattered) CUX(cudaMalloc(&d_sc, n * sizeof(rt_ray)));
+    CUX(cudaMemcpyAsync(d_rays, rays, n * sizeof(rt_ray), cudaMemcpyHostToDevice, sc->stream));
+    CUX(cudaMemcpyAsync(d_keys, keys, 2 * n * sizeof(uint32_t), cudaMemcpyHostToDevice, sc->stream));
+    rc = rt_scatter_batch_device(sc, d_rays, d_keys, n, level, seed, t_min, t_max, mode, d_idx, d_t, d_oc, d_col, d_sc,
+                                 sc->stream);
+    if (rc != RT_OK) {
+        cleanup();
+        return rc;
+    }
+    if (idx) CUX(cudaMemcpyAsync(idx, d_idx, n * sizeof(int32_t), cudaMemcpyDeviceToHost, sc->stream));
+    if (t) CUX(cudaMemcpyAsync(t, d_t, n * sizeof(double), cudaMemcpyDeviceToHost, sc->stream));
+    if (outcome) CUX(cudaMemcpyAsync(outcome, d_oc, n, cudaMemcpyDeviceToHost, sc->stream));
+    if (color) CUX(cudaMemcpyAsync(color, d_col, n * sizeof(rt_vec3), cudaMemcpyDeviceToHost, sc->stream));
+    if (scattered) CUX(cudaMemcpyAsync(scattered, d_sc, n * sizeof(rt_ray), cudaMemcpyDeviceToHost, sc->stream));
     CUX(cudaStreamSynchronize(sc->stream));
     cleanup();
 #undef CUX

@@ -40,6 +40,9 @@ pub const RT_TEX_NOISE: u32 = 4;
 pub const RT_ISECT_BRUTE: c_int = 0;
 pub const RT_ISECT_FAST: c_int = 1;
 pub const RT_ISECT_VERIFY: c_int = 2;
+pub const RT_BOUNCE_MISS: u8 = 0;
+pub const RT_BOUNCE_SCATTER: u8 = 1;
+pub const RT_BOUNCE_EMIT: u8 = 2;
 
 #[repr(C)] #[derive(Clone, Copy, Default, Debug)] pub struct rt_vec3 { pub x: f64, pub y: f64, pub z: f64 }
 #[repr(C)] #[derive(Clone, Copy, Debug)] pub struct rt_ray { pub origin: rt_vec3, pub direction: rt_vec3 }
@@ -96,6 +99,12 @@ extern "C" {
         t_max_per_ray: *const f64, mode: c_int, occluded: *mut u8) -> c_int;
     pub fn rt_occluded_batch_device(scene: *mut rt_scene, d_rays: *const rt_ray, n: u64, t_min: f64, t_max: f64,
         d_t_max_per_ray: *const f64, mode: c_int, d_occluded: *mut u8, stream: *mut c_void) -> c_int;
+    pub fn rt_scatter_batch(scene: *mut rt_scene, rays: *const rt_ray, keys: *const u32, n: u64, level: u32, seed: u64,
+        t_min: f64, t_max: f64, mode: c_int, shape_index: *mut i32, t: *mut f64, outcome: *mut u8,
+        color: *mut rt_vec3, scattered: *mut rt_ray) -> c_int;
+    pub fn rt_scatter_batch_device(scene: *mut rt_scene, d_rays: *const rt_ray, d_keys: *const u32, n: u64,
+        level: u32, seed: u64, t_min: f64, t_max: f64, mode: c_int, d_shape_index: *mut i32, d_t: *mut f64,
+        d_outcome: *mut u8, d_color: *mut rt_vec3, d_scattered: *mut rt_ray, stream: *mut c_void) -> c_int;
     pub fn rt_render_start(scene: *mut rt_scene, camera: *const rt_camera, params: *const rt_render_params) -> c_int;
     pub fn rt_render_poll(scene: *mut rt_scene, buffer: *mut rt_vec3, done: *mut c_int) -> c_int;
     pub fn rt_render_wait(scene: *mut rt_scene, buffer: *mut rt_vec3) -> c_int;

@@ -3,7 +3,7 @@
   python tools/render.py scenes/cornell_box.json out.png --size 1024 1024 --spp 256 [--depth 8] [--seed 1]
       [--adaptive REL [--min-samples N] [--abs-error A] [--heatmap counts.png]]
       [--counts MAP.npy [--heatmap counts.png]]
-      [--orbit N] [--animate N [--step S]]
+      [--orbit N] [--animate N [--step S]] [--inspect X Y]
 
 Scene::from_json -> GpuRenderer (Renderer trait: start_rendering / render_step until done) ->
 rt_tonemap_rgba8 (sqrt, clamp(0, 0.999) * 256, on the device) -> PNG.  With --adaptive, an adaptive frame
@@ -17,7 +17,10 @@ rotated about the world y axis through the origin by 360/N degrees at a time; vi
 out_001.png, ... for out.png).  With --animate N, N frames in which the scene's random spheres move on a seeded
 random walk in the x-z plane (--step per axis and frame), each frame on the same renderer after
 Scene.set_transforms-style edits of the scene (rt_scene_update_transforms: the cull tree is refit in place); frame k
-goes to OUT_k.png."""
+goes to OUT_k.png.  With --inspect X Y, after the frame: every sample's path of pixel (X, Y), traced again level by
+level with Scene.scatter (api.trace_paths on the frame's own primary rays, api.primary_rays): at each level the shape
+and material hit, the outcome and the throughput, then the sample's radiance; the mean of the samples must be the
+frame's pixel bit for bit."""
 import argparse, os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -38,7 +41,14 @@ ap.add_argument("--heatmap", default=None, help="PNG of the per-pixel sample cou
 ap.add_argument("--orbit", type=int, default=None, metavar="N", help="N views around the scene, one PNG per view")
 ap.add_argument("--animate", type=int, default=None, metavar="N", help="N frames of the random spheres on a random walk")
 ap.add_argument("--step", type=float, default=0.05, help="--animate: random-walk step per axis and frame")
+ap.add_argument("--inspect", type=int, nargs=2, default=None, metavar=("X", "Y"),
+                help="print each sample's path of pixel (X, Y) and check their mean against the frame")
 a = ap.parse_args()
+if a.inspect is not None and (a.orbit is not None or a.animate is not None or a.adaptive is not None
+                              or a.counts is not None):
+    ap.error("--inspect excludes --orbit, --animate, --adaptive and --counts")
+if a.inspect is not None and not (0 <= a.inspect[0] < a.size[0] and 0 <= a.inspect[1] < a.size[1]):
+    ap.error(f"--inspect: pixel {tuple(a.inspect)} outside the {a.size[0]}x{a.size[1]} image")
 if a.orbit is not None and (a.orbit < 1 or a.adaptive is not None or a.counts is not None):
     ap.error("--orbit needs N >= 1 and excludes --adaptive and --counts")
 if a.animate is not None and (a.animate < 1 or a.orbit is not None or a.adaptive is not None or a.counts is not None):
@@ -106,3 +116,34 @@ if a.heatmap:
     rgba = np.dstack([grey, grey, grey, np.full_like(grey, 255)])
     rt.save_png(a.heatmap, rgba)
     print(f"sample counts: {dict(zip(*[v.tolist() for v in np.unique(counts, return_counts=True)]))} -> {a.heatmap}")
+if a.inspect is not None:
+    x, y = a.inspect
+    rays, keys = rt.api.primary_rays(cam, w, h, [x + y * w], a.spp, a.seed)
+    radiance, levels = rt.trace_paths(sc, rays, keys, a.depth, a.seed, record=True)
+    d = sc.desc()
+    kinds = ("Lambertian", "Metal", "Dielectric", "DiffuseLight", "EmptyMaterial")
+    outcome = {rt.RT_BOUNCE_MISS: "miss (sky)", rt.RT_BOUNCE_SCATTER: "scatter", rt.RT_BOUNCE_EMIT: "emit"}
+    for s in range(a.spp):
+        print(f"pixel ({x}, {y}) sample {s}:")
+        for level, v in enumerate(levels):
+            at = np.flatnonzero(v["ray"] == s)
+            if at.size == 0:
+                break
+            k = int(at[0])
+            i, oc = int(v["shape"][k]), int(v["outcome"][k])
+            col, beta = v["color"][k], v["beta"][k]
+            what = "-" if i < 0 else f"{sc.shape_name(i)} ({kinds[d.materials[d.material[i]].kind]})"
+            if oc != rt.RT_BOUNCE_MISS and level == a.depth:
+                tag = "hit on the last level: black"
+            else:
+                tag = outcome[oc]
+            after = beta * col if oc == rt.RT_BOUNCE_SCATTER and level < a.depth else beta
+            print(f"  level {level:2d}: {what:40s} {tag:28s} colour {np.round(col, 4).tolist()}  "
+                  f"throughput {np.round(after, 4).tolist()}")
+        print(f"  radiance {radiance[s].tolist()}")
+    mean = rt.group_means(radiance, [0, a.spp])[0]
+    got = buf[y, x]
+    print(f"pixel ({x}, {y}): mean of the {a.spp} paths {mean.tolist()}, frame {got.tolist()} -> "
+          f"{'bit for bit' if np.array_equal(mean, got) else 'DIFFERENT'}")
+    if not np.array_equal(mean, got):
+        sys.exit(1)
