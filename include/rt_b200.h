@@ -458,6 +458,46 @@ int rt_render_start_counts(rt_scene* scene, const rt_camera* camera, const rt_re
  * 2^32 pixels or more, and every parameter rt_render_start rejects. */
 int rt_render_start_views(rt_scene* scene, const rt_camera* cameras, uint32_t n_views, const rt_render_params* params);
 
+/* Bounce layers: the rt_render_start frame, with each pixel's radiance also split by the level that ended its paths.
+ *   - Level of a path: the level of the segment that ended it, the camera ray being level 0.  A path ends at a miss (the
+ *     sky), at a material that does not scatter (an emission, or black), or with a hit on level max_depth (radiance 0).
+ *     It is the last level at which the path appears in a record of the path's segments.
+ *   - Layer b of pixel p is S_b / n: S_b is the f64 sum, in sample order from +0.0, of the float radiance (widened to
+ *     double) of the pixel's samples whose level k has min(k, n_layers - 1) == b; n is the pixel's sample count.  The
+ *     last layer collects every level at or beyond n_layers - 1; layers above max_depth are zero.
+ *   - Consequences: with n_layers == 1, layer 0 is the frame bit for bit.  A pixel whose samples all end on one level has
+ *     that layer equal to the frame pixel bit for bit and +0.0 in the others.  In general the layers add up to the frame
+ *     up to the reassociation of f64 sums only.  The sum of layers 0..d is the frame of depth d in value, not bit for
+ *     bit: the frame of depth d cuts at level d, black, the paths this frame continues.
+ *   - The frame itself is the rt_render_start frame bit for bit: rt_render_poll / wait / stop with progressive delivery,
+ *     rt_render_device_frame, rt_render_device_result, rt_assemble_frame and the tone map work unchanged, and
+ *     rt_stats.paths grows as for rt_render_start.  Multi-device handles shard it as rt_render_start does; shard_count > 1
+ *     renders one shard.  Scenes with more than 32 ray-marched shapes (the fused fallback) are rendered too.
+ *   - The frame never continues or seeds a progressive accumulation (rt_render_accumulated_samples reads 0 after it);
+ *     rt_render_pixel_stats behaves as after rt_render_start.
+ * RT_ERR_INVALID before any device work, checked in this order: a NULL scene, camera or params; n_layers outside
+ * [1, 63] (levels run 0 .. 62); every parameter rt_render_start rejects; a layer buffer of n_layers * (the shard's
+ * owned pixels, tile padding included) 24-byte slots whose size overflows 64 bits.  A rejected call leaves the last
+ * frame as it was. */
+int rt_render_start_layers(rt_scene* scene, const rt_camera* camera, const rt_render_params* params, uint32_t n_layers);
+/* After a completed layers frame, unsharded, on a single-device or multi-device handle (waits for the frame in flight):
+ * n_layers x w x h rt_vec3, layer-major: layer b of pixel (x, y) at [b * w * h + x + y * w].  host (may be NULL)
+ * receives a copy; *d_layers (may be NULL) = the library's device copy on device_ids[0], valid until the next frame
+ * starts; *n (may be NULL) = n_layers * w * h.  RT_ERR_STATE after any other frame or a shard of one. */
+int rt_render_layers(rt_scene* scene, rt_vec3* host, const rt_vec3** d_layers, uint64_t* n);
+/* This shard's f64 layer SUMS S_b after a completed layers frame (waits for it): layer-major, each layer the shard's
+ * rt_shard_float4_count slots of 3 doubles in the tile-packed owned order of rt_render_device_result.  *n_slots =
+ * n_layers times that count.  Valid until the next frame starts.  RT_ERR_STATE on a multi-device handle (use
+ * rt_render_layers) and after any other frame. */
+int rt_render_device_layers(rt_scene* scene, const rt_vec3** d_sums, uint64_t* n_slots);
+/* rt_assemble_frame for the layers: d_accs[s] = shard s's accumulator (rt_render_device_result), d_layer_sums[s] = its
+ * layer sums (rt_render_device_layers), all DEVICE pointers on the scene's device; d_out = n_layers x w x h rt_vec3 in
+ * the layout of rt_render_layers, each sum divided by the n of the gathered accumulator.  Runs on `stream` like
+ * rt_assemble_frame (NULL = the library's own stream, cudaStreamLegacy = 0x1 the legacy default stream) and does not
+ * synchronise.  RT_ERR_INVALID for a NULL argument, n_layers outside [1, 63], and what rt_assemble_frame rejects. */
+int rt_assemble_layers(rt_scene* scene, const rt_render_params* params, uint32_t n_layers, const void* const* d_accs,
+                       const void* const* d_layer_sums, rt_vec3* d_out, void* stream);
+
 /* Device-side result of the last started frame, for callers that gather shards over NCCL:
  * FOUR DOUBLES (r, g, b sums; samples) per owned pixel -- the f64 sums themselves, so that the assembled frame
  * equals the unsharded one bit for bit; they were floats before ABI 4, hence the names -- tile-packed in this

@@ -166,6 +166,11 @@ CORE_SYMBOLS = {
     "rt_render_pixel_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "rt_render_start_counts": (C.c_int, [C.c_void_p, C.POINTER(Camera), C.POINTER(RenderParams), C.c_void_p]),
     "rt_render_start_views": (C.c_int, [C.c_void_p, C.POINTER(Camera), C.c_uint32, C.POINTER(RenderParams)]),
+    "rt_render_start_layers": (C.c_int, [C.c_void_p, C.POINTER(Camera), C.POINTER(RenderParams), C.c_uint32]),
+    "rt_render_layers": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]),
+    "rt_render_device_layers": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]),
+    "rt_assemble_layers": (C.c_int, [C.c_void_p, C.POINTER(RenderParams), C.c_uint32, C.POINTER(C.c_void_p),
+                                     C.POINTER(C.c_void_p), C.c_void_p, C.c_void_p]),
     "rt_render_device_result": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]),
     "rt_shard_float4_count": (C.c_uint64, [C.POINTER(RenderParams), C.c_uint32]),
     "rt_assemble_frame": (C.c_int, [C.c_void_p, C.POINTER(RenderParams), C.POINTER(C.c_void_p), C.c_void_p,

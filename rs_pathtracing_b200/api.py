@@ -488,6 +488,20 @@ class GpuRenderer:
         render_wait(h, frames)
         return frames
 
+    def render_layers(self, camera: Camera, width: int, height: int, samples_number: int, n_layers: int):
+        """A frame with its bounce layers (rt_render_start_layers) on this renderer's devices, depth and seed: returns
+        (frame[h, w, 3], layers[n_layers, h, w, 3]) float64.  frame is render(camera, ...) bit for bit; layer b holds the
+        radiance of the paths that ended on level b (the last layer: on level n_layers - 1 or deeper), divided by the
+        pixel's sample count, so the layers add up to the frame."""
+        if self.devices and len(self.devices) > 1:
+            h = self.scene.device_scene_multi(self.devices)
+        else:
+            h = self.scene.device_scene(self.device)
+        render_start_layers(h, camera, render_params(width, height, samples_number, self.depth, self.seed), n_layers)
+        frame = np.zeros((height, width, 3), np.float64)
+        render_wait(h, frame)
+        return frame, render_layers(h)
+
 
 def tonemap_rgba8(scene: Scene, frame: np.ndarray, device: Optional[int] = None) -> np.ndarray:
     """src/bin/main_raylib.rs:239-247 on the device."""
@@ -827,6 +841,108 @@ def stacked_params(params: RenderParams, n_views: int) -> RenderParams:
     p = RenderParams.from_buffer_copy(params)
     p.image = ImageParams(params.image.width, n_views * params.image.height)
     return p
+
+
+MAX_LAYERS = MAX_LEVEL + 1   # a layers frame keeps at most one layer per level
+
+
+def check_n_layers(n_layers) -> int:
+    if isinstance(n_layers, bool) or not isinstance(n_layers, (int, np.integer)):
+        raise ValueError(f"n_layers: an int, got {type(n_layers).__name__}")
+    if not 1 <= n_layers <= MAX_LAYERS:
+        raise ValueError(f"n_layers must be in [1, {MAX_LAYERS}], got {n_layers}")
+    return int(n_layers)
+
+
+def render_start_layers(dev_scene, camera: Camera, params: RenderParams, n_layers: int) -> None:
+    """rt_render_start_layers: the render_start frame (poll / wait deliver it as for render_start), and with it layer b
+    of every pixel = the f64 sum, in sample order, of the radiance of its samples whose path ended on level
+    min(level, n_layers - 1) == b, over the pixel's sample count (render_layers)"""
+    n_layers = check_n_layers(n_layers)
+    _check(_ffi.core().rt_render_start_layers(dev_scene, C.byref(camera), C.byref(params), n_layers))
+    _started[_handle_key(dev_scene)] = (params.image.height, params.image.width, False)
+
+
+def render_layers(dev_scene, device: bool = False, shape=None):
+    """rt_render_layers after a completed unsharded layers frame (waits for the frame in flight): layers[L, h, w, 3]
+    float64, layer b of pixel (x, y) at [b, y, x].  device=True returns (device pointer, n) of the library's copy on
+    the handle's first device instead (n = L * h * w rt_vec3, valid until the next frame starts).  shape = (height,
+    width) for a frame not started through render_start_layers."""
+    ptr, n = C.c_void_p(), C.c_uint64()
+    _check(_ffi.core().rt_render_layers(dev_scene, None, C.byref(ptr), C.byref(n)))
+    if device:
+        return ptr.value, n.value
+    if shape is None:
+        known = _started.get(_handle_key(dev_scene))
+        if known is None:
+            raise ValueError("frame size unknown: pass shape=(height, width)")
+        shape = known[:2]
+    h, w = shape
+    if h * w == 0 or n.value % (h * w):
+        raise ValueError(f"shape {shape} does not divide the {n.value} pixels of the layers")
+    out = np.empty((n.value // (h * w), h, w, 3), np.float64)
+    _check(_ffi.core().rt_render_layers(dev_scene, out.ctypes.data_as(C.c_void_p), None, None))
+    return out
+
+
+def render_device_layers(dev_scene):
+    """(device pointer, n) of the shard's layer sums: n = L * shard_float4_count slots of 3 doubles, layer-major, each
+    layer in the tile-packed order of render_device_result"""
+    ptr, n = C.c_void_p(), C.c_uint64()
+    _check(_ffi.core().rt_render_device_layers(dev_scene, C.byref(ptr), C.byref(n)))
+    return ptr.value, n.value
+
+
+def assemble_layers(dev_scene, params: RenderParams, n_layers: int, acc_ptrs, sum_ptrs, d_out_ptr: int,
+                    stream: int = 0) -> None:
+    """rt_assemble_layers: the gathered accumulators and layer sums of every shard -> L x h x w x 3 layers at
+    d_out_ptr, on `stream` (0: the library's stream)"""
+    if len(acc_ptrs) != len(sum_ptrs):
+        raise ValueError("one accumulator and one layer-sum buffer per shard")
+    accs = (C.c_void_p * len(acc_ptrs))(*acc_ptrs)
+    sums = (C.c_void_p * len(sum_ptrs))(*sum_ptrs)
+    _check(_ffi.core().rt_assemble_layers(dev_scene, C.byref(params), n_layers, accs, sums, C.c_void_p(d_out_ptr),
+                                          C.c_void_p(stream) if stream else None))
+
+
+def path_levels(record, n: int) -> np.ndarray:
+    """the level that ended each of the n paths of trace_paths(..., record=True): the last level whose record lists the
+    path (record[k]["ray"]).  Returns (n,) int32; -1 for a path no level lists (none, when every path is recorded)."""
+    levels = np.full(n, -1, np.int32)
+    for k, rec in enumerate(record):
+        ray = rec["ray"]
+        if type(ray).__module__.split(".")[0] == "torch":
+            ray = ray.cpu().numpy()
+        levels[np.asarray(ray, np.int64)] = k
+    return levels
+
+
+def layer_means(radiance, levels, offsets, n_layers: int) -> np.ndarray:
+    """the layers of groups of paths as the layers frame takes them: layer b of group g = the f64 sum of the float
+    radiance of its rays (offsets[g] .. offsets[g+1]-1) whose level has min(level, n_layers - 1) == b, in ray order
+    from +0.0, over the group's ray count (an empty group is NaN).  radiance (n, 3) float32 (numpy or torch), levels
+    (n,) integers in [0, 62]; returns (n_layers, G, 3) float64."""
+    n_layers = check_n_layers(n_layers)
+    if type(radiance).__module__.split(".")[0] == "torch":
+        radiance = radiance.cpu().numpy()
+    f = np.asarray(radiance, dtype=np.float32).reshape(-1, 3).astype(np.float64)
+    lv = np.asarray(levels).reshape(-1)
+    if lv.shape[0] != f.shape[0] or not np.issubdtype(lv.dtype, np.integer):
+        raise ValueError("levels: one integer level per ray")
+    if lv.size and (lv.min() < 0 or lv.max() > MAX_LEVEL):
+        raise ValueError(f"levels must be in [0, {MAX_LEVEL}]")
+    off = np.asarray(offsets, dtype=np.int64).reshape(-1)
+    if off.size == 0 or off[0] != 0 or off[-1] != f.shape[0] or (np.diff(off) < 0).any():
+        raise ValueError("offsets must rise from 0 to len(radiance)")
+    count = np.diff(off)
+    b = np.minimum(lv, n_layers - 1)
+    s = np.zeros((n_layers, count.size, 3))
+    for k in range(int(count.max(initial=0))):   # step k adds ray k of every group that has one, to its layer
+        g = np.flatnonzero(count > k)
+        r = off[:-1][g] + k
+        s[b[r], g] = s[b[r], g] + f[r]
+    with np.errstate(invalid="ignore"):
+        return s / count[None, :, None]
 
 
 def render_pixel_stats(dev_scene, shape=None):

@@ -15,7 +15,9 @@
 //   k_resolve_list      adaptive frames: continue a listed pixel's rgb and luminance sums over its new samples
 //   k_load_counts       counts frames: level-0 loader, the caller's sample count per pixel -> queue + RNG keys
 //   k_counts_resolve    counts frames: a pixel's sums over its samples, continued across the pieces of a large pixel
+//   k_resolve_layers    layers frames: k_resolve, plus each pixel's f64 sums per ending bounce level
 //   k_assemble          multi-GPU: gathered tile-packed shards -> frame
+//   k_assemble_layers   layers frames: (gathered) layer sums / the accumulator's n -> layer-major layers
 //   k_tonemap           the bins' sqrt / clamp / *256 -> RGBA8
 //   k_scene_scatter     rt_scene_update_transforms: (slot, value) records of a refit into the scene's tables, in place
 // Compile with -fmad=false (see rt_math.cuh).
@@ -349,7 +351,7 @@ k_bounce(DevScene S, bool use_smem, PathQueue in, const uint32_t* __restrict__ c
                     L = hadamard(beta, atten);  // :34-36
                 }
             }
-            if (!alive) radiance[pid] = make_float4((float)L.x, (float)L.y, (float)L.z, 1.0f);
+            if (!alive) radiance[pid] = make_float4((float)L.x, (float)L.y, (float)L.z, (float)(level + 1));   // (.w: ending level + 1)
         }
         uint32_t slot = queue_append(alive, count_out);
         if (alive) {
@@ -538,7 +540,8 @@ __device__ __forceinline__ void shade_slot(const DevScene& S, const PathQueue& i
             L = hadamard(beta, atten);  // :34-36
         }
     }
-    if (valid && !alive) radiance[pid] = make_float4((float)L.x, (float)L.y, (float)L.z, 1.0f);
+    // .w = the level that ended the path + 1 (0 only in a padding slot k_raygen wrote): k_resolve_layers bins by it
+    if (valid && !alive) radiance[pid] = make_float4((float)L.x, (float)L.y, (float)L.z, (float)(level + 1));
     uint32_t slot = queue_append(alive, count_out);
     if (alive) {
         out.ox[slot] = no.x; out.oy[slot] = no.y; out.oz[slot] = no.z;
@@ -740,6 +743,51 @@ k_resolve(const float4* __restrict__ radiance, uint32_t n_pixels, uint32_t spp, 
     if (MOMENTS) moments[first_owned + pl] = make_double2(my, myy);
 }
 
+// K5l: layers frames (rt_render_start_layers).  k_resolve<false>'s accumulator and frame, and the pixel's radiance split
+// by the level that ended each path (radiance.w = level + 1): sums[b * layer_stride + q] = the f64 sum, in sample order
+// from +0.0, of the samples whose level k has min(k, n_layers - 1) == b; a layer no sample reaches is +0.0.  Per-layer
+// sums in registers would spill at 63 layers, so the pixel's own slots in global memory are read-modified-written, and
+// the sum of the layer the last sample went to stays in registers while the following samples go there too.  Each
+// layer's sum is still one chain of additions in sample order.  A padding slot (.w = 0) goes to layer 0 (its radiance is
+// zero and nobody reads a padding pixel's sums).
+__global__ void __launch_bounds__(256)
+k_resolve_layers(const float4* __restrict__ radiance, uint32_t n_pixels, uint32_t spp, unsigned long long first_owned,
+                 Acc* __restrict__ accum, rt_vec3* __restrict__ frame_owned, rt_vec3* __restrict__ sums,
+                 unsigned long long layer_stride, uint32_t n_layers) {
+    const uint32_t pl = blockIdx.x * blockDim.x + threadIdx.x;
+    if (pl >= n_pixels) return;
+    const float4* r = radiance + (size_t)pl * spp;
+    rt_vec3* S = sums + first_owned + pl;
+    double sx = 0.0, sy = 0.0, sz = 0.0;
+    double cx = 0.0, cy = 0.0, cz = 0.0;   // the running sum of layer `cur`
+    unsigned long long touched = 0;        // layers with a sum in S (or in registers)
+    uint32_t cur = 0xFFFFFFFFu;
+    for (uint32_t s = 0; s < spp; s++) {
+        const float4 v = r[s];
+        sx += (double)v.x; sy += (double)v.y; sz += (double)v.z;
+        const uint32_t w = (uint32_t)v.w;
+        const uint32_t b = min(w ? w - 1u : 0u, n_layers - 1u);
+        if (b != cur) {
+            if (cur != 0xFFFFFFFFu) S[cur * layer_stride] = rt_vec3{cx, cy, cz};
+            cur = b;
+            if ((touched >> b) & 1ull) {
+                const rt_vec3 prev = S[b * layer_stride];
+                cx = prev.x; cy = prev.y; cz = prev.z;
+            } else {
+                cx = 0.0; cy = 0.0; cz = 0.0;
+                touched |= 1ull << b;
+            }
+        }
+        cx += (double)v.x; cy += (double)v.y; cz += (double)v.z;
+    }
+    if (cur != 0xFFFFFFFFu) S[cur * layer_stride] = rt_vec3{cx, cy, cz};
+    for (uint32_t b = 0; b < n_layers; b++)
+        if (!((touched >> b) & 1ull)) S[b * layer_stride] = rt_vec3{0.0, 0.0, 0.0};
+    const double ln = (double)spp;
+    accum[first_owned + pl] = Acc{sx, sy, sz, ln};
+    frame_owned[first_owned + pl] = rt_vec3{sx / ln, sy / ln, sz / ln};
+}
+
 // ---- adaptive sampling (rt_render_start_adaptive) -------------------------------------------------------------------
 // The stopping rule, in the operation order the header documents (so that numpy can replay it bit for bit).
 __device__ __forceinline__ bool adaptive_converged(double n, double sum_y, double sum_yy, double rel_error, double abs_error) {
@@ -899,6 +947,33 @@ k_assemble(ShardPtrs shards, ShardMap map0, rt_vec3* __restrict__ frame) {
     size_t q = (size_t)j * map0.tile_pixels() + (size_t)(y % map0.tile_h) * map0.tile_w + (x % map0.tile_w);
     const Acc v = shards.p[s][q];
     frame[(size_t)y * map0.width + x] = rt_vec3{v.r / v.n, v.g / v.n, v.b / v.n};
+}
+
+// K7l: the layers of a layers frame (rt_render_start_layers): shard s's layer sums are layer-major with stride[s] slots
+// per layer (its owned pixels, tile-packed as its accumulator); out[b * w * h + x + y * w] = sum / the gathered Acc's n.
+// k_assemble's tile arithmetic; an unsharded frame is the one-shard case (one tile row per image row).
+struct LayerPtrs {
+    const rt_vec3* p[16];
+    unsigned long long stride[16];
+};
+__global__ void __launch_bounds__(256)
+k_assemble_layers(ShardPtrs shards, LayerPtrs layers, ShardMap map0, uint32_t n_layers, rt_vec3* __restrict__ out) {
+    const uint64_t n_px = (uint64_t)map0.width * map0.height;
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_px) return;
+    const uint32_t y = (uint32_t)(i / map0.width), x = (uint32_t)(i - (uint64_t)y * map0.width);
+    uint32_t tx = x / map0.tile_w, ty = y / map0.tile_h;
+    uint32_t rot = ((ty % map0.tiles_x) * map0.skew) % map0.tiles_x;
+    uint32_t k = ty * map0.tiles_x + (tx + map0.tiles_x - rot) % map0.tiles_x;
+    uint32_t s = k % map0.shard_count, j = k / map0.shard_count;
+    size_t q = (size_t)j * map0.tile_pixels() + (size_t)(y % map0.tile_h) * map0.tile_w + (x % map0.tile_w);
+    const double n = shards.p[s][q].n;
+    const rt_vec3* src = layers.p[s] + q;
+    const unsigned long long stride = layers.stride[s];
+    for (uint32_t b = 0; b < n_layers; b++) {
+        const rt_vec3 v = src[b * stride];
+        out[b * n_px + i] = rt_vec3{v.x / n, v.y / n, v.z / n};
+    }
 }
 
 // src/bin/main_raylib.rs:239-247
@@ -1374,6 +1449,15 @@ struct rt_scene {
     std::vector<RayCasterDev> h_views;
     RayCasterDev* d_views = nullptr;
     uint64_t views_cap = 0;
+    // layers frames (rt_render_start_layers): the layer count of the frame in flight / last completed (0: not one), its
+    // layer sums (layer-major, owned_pixels slots per layer), the layers themselves (x + y*w per layer, the whole image
+    // of an unsharded or multi-device frame, on this device), and a multi-device handle's staging for the peers' sums
+    uint32_t n_layers = 0;
+    rt_vec3* d_layer_sums = nullptr;
+    rt_vec3* d_layers = nullptr;
+    uint64_t layer_sums_cap = 0, layers_cap = 0;
+    std::vector<rt_vec3*> d_peer_layers;
+    std::vector<uint64_t> peer_layers_cap;
     // scene updates (rt_scene_update[_transforms]): the host side of the cull tree the tables were built from (a
     // multi-device handle refits its first device's and applies the records on every device), the pinned staging and
     // the device copy of a refit's records, the event after which the staging may be rewritten, the event of the last
@@ -1954,6 +2038,9 @@ void rt_scene_destroy(rt_scene* sc) {
     cudaFree(sc->d_live);
     cudaFree(sc->d_pix_counts);
     cudaFree(sc->d_views);
+    cudaFree(sc->d_layer_sums);
+    cudaFree(sc->d_layers);
+    for (rt_vec3* a : sc->d_peer_layers) cudaFree(a);
     if (sc->host_stage) cudaFreeHost(sc->host_stage);
     cudaFree(sc->d_scatter);
     bind_lane(sc, 0);
@@ -2443,9 +2530,9 @@ static int ensure_path_buffers(rt_scene* sc, uint64_t need_paths) {
 }
 
 static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_render_params* p,
-                               const rt_adaptive_params* ap = nullptr, uint32_t n_views = 0);
+                               const rt_adaptive_params* ap = nullptr, uint32_t n_views = 0, uint32_t n_layers = 0);
 static int render_start_multi(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const uint32_t* counts = nullptr,
-                              uint32_t n_views = 0);
+                              uint32_t n_views = 0, uint32_t n_layers = 0);
 static int render_start_counts_single(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const uint32_t* counts);
 
 int rt_render_start(rt_scene* sc, const rt_camera* cam, const rt_render_params* p) {
@@ -2507,7 +2594,7 @@ static int ensure_frame_buffers(rt_scene* sc) {
 // n_views > 0: a views frame (rt_render_start_views, validated there): `cam` points to n_views cameras and p is the
 // stacked image; level 0 of every batch is k_raygen_views, then the bounce loop runs without raygen.
 static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const rt_adaptive_params* ap,
-                               uint32_t n_views) {
+                               uint32_t n_views, uint32_t n_layers) {
     if (!sc || !cam || !p) return fail(RT_ERR_INVALID, "null argument");
     int rc = check_frame_params(p);
     if (rc != RT_OK) return rc;
@@ -2518,7 +2605,7 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
     // progressive accumulation: this frame adds its samples to the previous ones when it is the same frame
     // (image, sharding, depth, seed, camera) and nothing was abandoned; otherwise it starts afresh
     uint32_t sample_base = 0;
-    if (!ap && !n_views && sc->accumulate && sc->accumulated_spp > 0 && sc->wavefront && memcmp(&sc->accum_cam, cam, sizeof *cam) == 0 &&
+    if (!ap && !n_views && !n_layers && sc->accumulate && sc->accumulated_spp > 0 && sc->wavefront && memcmp(&sc->accum_cam, cam, sizeof *cam) == 0 &&
         sc->accum_rp.image.width == p->image.width && sc->accum_rp.image.height == p->image.height &&
         sc->accum_rp.max_depth == p->max_depth && sc->accum_rp.seed == p->seed &&
         (sc->accum_rp.shard_count ? sc->accum_rp.shard_count : 1) == shard_count &&
@@ -2529,6 +2616,7 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
     sc->accumulated_spp = 0;  // until this frame is enqueued (an abandoned frame breaks the chain)
     sc->adaptive_frame = false;
     sc->views_frame = n_views > 0;
+    sc->n_layers = n_layers;
     sc->rp = *p;
     sc->rp.shard_count = shard_count;
     sc->map = make_shard_map(sc->rp, p->shard_index);
@@ -2573,6 +2661,11 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
     bind_lane(sc, 0);
     if (rc != RT_OK) return rc;
     if ((rc = ensure_frame_buffers(sc)) != RT_OK) return rc;
+    if (n_layers) {   // the layer sums; an unsharded frame also keeps its layers
+        if ((rc = ensure_device_array(sc->d_layer_sums, sc->layer_sums_cap, n_layers * sc->owned_pixels)) != RT_OK) return rc;
+        if (shard_count == 1 && (rc = ensure_device_array(sc->d_layers, sc->layers_cap, n_layers * sc->owned_pixels)) != RT_OK)
+            return rc;
+    }
     if (ap) {
         if ((rc = ensure_device_array(sc->d_moments, sc->moments_cap, sc->owned_pixels)) != RT_OK) return rc;
         if ((rc = ensure_device_array(sc->d_plist, sc->plist_cap, sc->owned_pixels)) != RT_OK) return rc;
@@ -2626,7 +2719,11 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
             }
             {
                 KernelSpan span(sc, RT_KCLASS_RESOLVE);
-                if (ap)
+                if (n_layers)
+                    k_resolve_layers<<<(npx + 255) / 256, 256, 0, sc->stream>>>(sc->d_radiance, npx, spp, first, sc->d_accum,
+                                                                              sc->d_frame, sc->d_layer_sums, sc->owned_pixels,
+                                                                              n_layers);
+                else if (ap)
                     k_resolve<true><<<(npx + 255) / 256, 256, 0, sc->stream>>>(sc->d_radiance, npx, spp, first, sc->d_accum,
                                                                              sc->d_frame, false, sc->d_moments);
                 else
@@ -2685,6 +2782,16 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
             CU(cudaEventRecord(sc->lanes[l].done, sc->lanes[l].stream));
             CU(cudaStreamWaitEvent(sc->stream, sc->lanes[l].done, 0));
         }
+        if (n_layers && shard_count == 1) {   // the layers of an unsharded frame (owned order is x + y*width)
+            KernelSpan span(sc, RT_KCLASS_RESOLVE);
+            ShardPtrs accs{};
+            LayerPtrs lp{};
+            accs.p[0] = sc->d_accum;
+            lp.p[0] = sc->d_layer_sums;
+            lp.stride[0] = sc->owned_pixels;
+            k_assemble_layers<<<(unsigned)((sc->owned_pixels + 255) / 256), 256, 0, sc->stream>>>(accs, lp, sc->map, n_layers,
+                                                                                                  sc->d_layers);
+        }
         if (ap) {   // one delivery unit: the whole frame, once the last pass has resolved
             Batch b;
             b.first_owned = 0;
@@ -2712,6 +2819,7 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
         for (const RefinePass& P : refine) sc->adaptive_m.push_back(P.m);
         return RT_OK;
     }
+    if (n_layers) return RT_OK;   // the frame neither continues nor seeds an accumulation
     if (sc->accumulate && sc->wavefront) {  // (enqueued work always runs to completion: rt_render_stop drains it)
         sc->accumulated_spp = sample_base + spp;
         sc->accum_rp = *p;
@@ -2728,7 +2836,7 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
 // (rt_render_start_counts, validated there), every shard reading the whole map.  n_views > 0: a views frame
 // (rt_render_start_views, validated there; p is the stacked image), every shard uploading the whole camera table.
 static int render_start_multi(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const uint32_t* counts,
-                              uint32_t n_views) {
+                              uint32_t n_views, uint32_t n_layers) {
     if (p->image.width == 0 || p->image.height == 0 || p->samples_number == 0)
         return fail(RT_ERR_INVALID, "empty image or zero samples");
     const uint32_t n_dev = (uint32_t)sc->peers.size() + 1;
@@ -2757,18 +2865,32 @@ static int render_start_multi(rt_scene* sc, const rt_camera* cam, const rt_rende
             sc->peer_acc_cap[k - 1] = need;
         }
     }
+    if (n_layers) {   // the peers' layer sums (n_layers slots per owned pixel) and the layers, on this device
+        sc->d_peer_layers.resize(n_dev - 1, nullptr);
+        sc->peer_layers_cap.resize(n_dev - 1, 0);
+        for (uint32_t k = 1; k < n_dev; k++) {
+            int rc = ensure_device_array(sc->d_peer_layers[k - 1], sc->peer_layers_cap[k - 1], n_layers * rt_shard_float4_count(&sp, k));
+            if (rc != RT_OK) return rc;
+        }
+        int rc = ensure_device_array(sc->d_layers, sc->layers_cap, n_layers * n_px);
+        if (rc != RT_OK) return rc;
+    }
     // enqueue every shard (the peers first: the first device also assembles)
     for (uint32_t k = 1; k < n_dev; k++) {
         rt_scene* peer = sc->peers[k - 1];
         sp.shard_index = k;
-        int rc = counts ? render_start_counts_single(peer, cam, &sp, counts) : render_start_single(peer, cam, &sp, nullptr, n_views);
+        int rc = counts ? render_start_counts_single(peer, cam, &sp, counts)
+                        : render_start_single(peer, cam, &sp, nullptr, n_views, n_layers);
         if (rc != RT_OK) return rc;
         const uint64_t cnt = rt_shard_float4_count(&sp, k);
         if (cnt) CU(cudaMemcpyPeerAsync(sc->d_peer_acc[k - 1], sc->device, peer->d_accum, peer->device, cnt * sizeof(Acc), peer->stream));
+        if (cnt && n_layers)
+            CU(cudaMemcpyPeerAsync(sc->d_peer_layers[k - 1], sc->device, peer->d_layer_sums, peer->device,
+                                   n_layers * cnt * sizeof(rt_vec3), peer->stream));
         CU(cudaEventRecord(sc->ev_peer[k - 1], peer->stream));
     }
     sp.shard_index = 0;
-    int rc = counts ? render_start_counts_single(sc, cam, &sp, counts) : render_start_single(sc, cam, &sp, nullptr, n_views);
+    int rc = counts ? render_start_counts_single(sc, cam, &sp, counts) : render_start_single(sc, cam, &sp, nullptr, n_views, n_layers);
     if (rc != RT_OK) return rc;
     CU(cudaSetDevice(sc->device));
     for (uint32_t k = 1; k < n_dev; k++) CU(cudaStreamWaitEvent(sc->stream, sc->ev_peer[k - 1], 0));
@@ -2777,6 +2899,15 @@ static int render_start_multi(rt_scene* sc, const rt_camera* cam, const rt_rende
     ShardMap m0 = make_shard_map(sp, 0);
     k_assemble<<<(unsigned)((n_px + 255) / 256), 256, 0, sc->stream>>>(ptrs, m0, sc->d_full_frame);
     sc->launches++;
+    if (n_layers) {
+        LayerPtrs lp{};
+        for (uint32_t k = 0; k < n_dev; k++) {
+            lp.p[k] = k == 0 ? sc->d_layer_sums : sc->d_peer_layers[k - 1];
+            lp.stride[k] = rt_shard_float4_count(&sp, k);
+        }
+        k_assemble_layers<<<(unsigned)((n_px + 255) / 256), 256, 0, sc->stream>>>(ptrs, lp, m0, n_layers, sc->d_layers);
+        sc->launches++;
+    }
     CU(cudaEventRecord(sc->ev_multi_done, sc->stream));
     CU(cudaGetLastError());
     sc->multi_active = true;
@@ -3291,6 +3422,7 @@ static int render_start_counts_single(rt_scene* sc, const rt_camera* cam, const 
     sc->accumulated_spp = 0;   // a counts frame neither continues nor seeds a progressive accumulation
     sc->adaptive_frame = false;
     sc->views_frame = false;
+    sc->n_layers = 0;
     sc->rp = rp;
     sc->map = map;
     sc->owned_pixels = owned;
@@ -3396,6 +3528,100 @@ int rt_render_start_views(rt_scene* sc, const rt_camera* cams, uint32_t n_views,
     if (!sc->peers.empty() && p->shard_count <= 1) return render_start_multi(sc, cams, &sp, nullptr, n_views);
     sc->multi_active = false;
     return render_start_single(sc, cams, &sp, nullptr, n_views);
+}
+
+// ---- bounce layers (rt_render_start_layers) -----------------------------------------------------------------------
+// The rt_render_start frame with k_resolve_layers in place of k_resolve: every path's radiance slot carries the level
+// that ended it, and the resolve bins each pixel's samples by it.  Pixels are never split over batches in a uniform
+// frame, so each pixel's sums are written by one thread of one batch.
+static const uint32_t RT_MAX_LAYERS = RT_MAX_LEVELS - 1;   // levels 0 .. 62
+
+int rt_render_start_layers(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, uint32_t n_layers) {
+    if (!sc || !cam || !p) return fail(RT_ERR_INVALID, "null argument");
+    if (n_layers < 1 || n_layers > RT_MAX_LAYERS) return fail(RT_ERR_INVALID, "n_layers must be in [1, 63]");
+    int rc = check_frame_params(p);
+    if (rc != RT_OK) return rc;
+    // the shard's owned pixels include the padding of its border tiles, which a thin image with tall tiles makes huge
+    rt_render_params pp = *p;
+    pp.shard_count = p->shard_count ? p->shard_count : 1;
+    const ShardMap m = make_shard_map(pp, p->shard_index);
+    const uint64_t owned = owned_tiles(m) * m.tile_pixels();
+    if (owned > UINT64_MAX / sizeof(rt_vec3) / n_layers) return fail(RT_ERR_INVALID, "n_layers * owned pixels overflows");
+    if (!sc->peers.empty() && p->shard_count <= 1) return render_start_multi(sc, cam, p, nullptr, 0, n_layers);
+    sc->multi_active = false;
+    return render_start_single(sc, cam, p, nullptr, 0, n_layers);
+}
+
+int rt_render_layers(rt_scene* sc, rt_vec3* host, const rt_vec3** d_layers, uint64_t* n) {
+    if (!sc) return fail(RT_ERR_INVALID, "null scene");
+    if (sc->rendering) {
+        int rc = rt_render_wait(sc, nullptr);
+        if (rc != RT_OK) return rc;
+    }
+    if (!sc->frame_complete) return fail(RT_ERR_STATE, "no completed frame");
+    if (!sc->n_layers) return fail(RT_ERR_STATE, "the last frame was not a layers frame (rt_render_start_layers)");
+    uint64_t n_px;
+    if (sc->multi_active) {
+        n_px = (uint64_t)sc->multi_rp.image.width * sc->multi_rp.image.height;
+    } else {
+        if (sc->map.shard_count != 1)
+            return fail(RT_ERR_STATE, "the last frame was one shard of a frame: use rt_render_device_layers + rt_assemble_layers");
+        n_px = (uint64_t)sc->map.width * sc->map.height;
+    }
+    const uint64_t count = (uint64_t)sc->n_layers * n_px;
+    CU(cudaSetDevice(sc->device));
+    if (host) {
+        CU(cudaMemcpyAsync(host, sc->d_layers, count * sizeof(rt_vec3), cudaMemcpyDeviceToHost, sc->copy_stream));
+        const cudaError_t e = cudaStreamSynchronize(sc->copy_stream);
+        if (e != cudaSuccess) return fail(RT_ERR_CUDA, std::string("layers: ") + cudaGetErrorString(e));
+    }
+    if (d_layers) *d_layers = sc->d_layers;
+    if (n) *n = count;
+    return RT_OK;
+}
+
+int rt_render_device_layers(rt_scene* sc, const rt_vec3** d_sums, uint64_t* n_slots) {
+    if (!sc || !d_sums || !n_slots) return fail(RT_ERR_INVALID, "null argument");
+    if (sc->multi_active) return fail(RT_ERR_STATE, "a multi-device handle delivers the assembled layers: rt_render_layers");
+    if (sc->rendering) {
+        CU(cudaSetDevice(sc->device));
+        CU(cudaStreamSynchronize(sc->stream));
+        int done = 0;
+        int rc = rt_render_poll(sc, nullptr, &done);
+        if (rc != RT_OK) return rc;
+    }
+    if (!sc->frame_complete) return fail(RT_ERR_STATE, "no completed frame");
+    if (!sc->n_layers) return fail(RT_ERR_STATE, "the last frame was not a layers frame (rt_render_start_layers)");
+    *d_sums = sc->d_layer_sums;
+    *n_slots = (uint64_t)sc->n_layers * sc->owned_pixels;
+    return RT_OK;
+}
+
+int rt_assemble_layers(rt_scene* sc, const rt_render_params* p, uint32_t n_layers, const void* const* d_accs,
+                       const void* const* d_layer_sums, rt_vec3* d_out, void* stream) {
+    if (!sc || !p || !d_accs || !d_layer_sums || !d_out) return fail(RT_ERR_INVALID, "null argument");
+    if (n_layers < 1 || n_layers > RT_MAX_LAYERS) return fail(RT_ERR_INVALID, "n_layers must be in [1, 63]");
+    uint32_t shard_count = p->shard_count ? p->shard_count : 1;
+    if (shard_count > 16) return fail(RT_ERR_INVALID, "at most 16 shards");
+    const uint64_t n_px = (uint64_t)p->image.width * p->image.height;
+    if (n_px == 0 || n_px > 0xFFFFFFFFull) return fail(RT_ERR_INVALID, "empty or too large image");
+    rt_render_params pp = *p;
+    pp.shard_count = shard_count;
+    ShardMap m = make_shard_map(pp, 0);
+    if (!tile_fits(m)) return fail(RT_ERR_INVALID, "tile_width * tile_height >= 2^32");
+    CU(cudaSetDevice(sc->device));
+    ShardPtrs accs{};
+    LayerPtrs lp{};
+    for (uint32_t s = 0; s < shard_count; s++) {
+        accs.p[s] = (const Acc*)d_accs[s];
+        lp.p[s] = (const rt_vec3*)d_layer_sums[s];
+        lp.stride[s] = rt_shard_float4_count(&pp, s);
+    }
+    cudaStream_t st = stream ? (cudaStream_t)stream : sc->stream;
+    k_assemble_layers<<<(unsigned)((n_px + 255) / 256), 256, 0, st>>>(accs, lp, m, n_layers, d_out);
+    sc->launches++;
+    CU(cudaGetLastError());
+    return RT_OK;
 }
 
 // ---- instrumentation ---------------------------------------------------------------------------

@@ -54,7 +54,7 @@ def exchange_to_rank0(dist, mine, counts, rank: int, world: int, bufs=None):
     ops = []
     if rank == 0:
         if bufs is None or [b.shape[0] for b in bufs] != list(counts):
-            bufs = [torch.empty((c, 4), dtype=torch.float64, device=mine.device) for c in counts]
+            bufs = [torch.empty((c,) + tuple(mine.shape[1:]), dtype=torch.float64, device=mine.device) for c in counts]
         bufs[0].copy_(mine)
         for s in range(1, world):
             ops.append(dist.P2POp(dist.irecv, bufs[s], s))
@@ -103,6 +103,7 @@ class DistributedRenderer:
         self._copy_stream = None
         self._host2 = [None, None]
         self._dev_scene_b = None           # a second rt_scene on the same device: two frames of a sequence in flight
+        self._layer_bufs = None            # rank 0: the gathered layer sums of layers frames
 
     def _params(self, w, h, spp, shard):
         return api.render_params(w, h, spp, self.depth, self.seed, self.world, shard, tile=self.tile)
@@ -128,8 +129,17 @@ class DistributedRenderer:
                                    width, len(cameras) * height, samples_number)
         return None if frame is None else frame.view(len(cameras), height, width, 3)
 
-    def _render_shard(self, start, width: int, height: int, samples_number: int):
-        """start(params) this rank's shard of a width x height frame, gather, assemble on rank 0"""
+    def render_layers_device(self, camera: Camera, width: int, height: int, samples_number: int, n_layers: int):
+        """render_device of a layers frame (rt_render_start_layers): every rank renders its tiles, and its layer sums
+        travel to rank 0 in one more exchange.  Returns (frame h x w x 3, layers n_layers x h x w x 3) float64 device
+        tensors on rank 0, each equal to the unsharded layers frame's bit for bit, None elsewhere."""
+        n_layers = api.check_n_layers(n_layers)
+        return self._render_shard(lambda p: api.render_start_layers(self.dev_scene, camera, p, n_layers),
+                                  width, height, samples_number, n_layers)
+
+    def _render_shard(self, start, width: int, height: int, samples_number: int, n_layers: int = 0):
+        """start(params) this rank's shard of a width x height frame, gather, assemble on rank 0 (n_layers > 0: a
+        layers frame, whose layers are gathered and assembled too: (frame, layers) on rank 0)"""
         torch, dist = self.torch, self.dist
         p = self._params(width, height, samples_number, self.rank)
         # The library renders on its own non-blocking streams, the exchange runs on torch's / NCCL's: the
@@ -143,6 +153,12 @@ class DistributedRenderer:
         counts = [api.shard_float4_count(p, s) for s in range(self.world)]
         # one exchange per frame: every rank's tile-packed accumulator to rank 0 over NVLink
         shards = exchange_to_rank0(dist, mine, counts, self.rank, self.world, self._gather_bufs)
+        layer_shards = None
+        if n_layers:   # the second exchange: every rank's layer sums, n_layers slots of 3 doubles per owned pixel
+            lptr, ln = api.render_device_layers(self.dev_scene)
+            mine_l = torch.as_tensor(api.DevicePointer(lptr, (ln, 3), "<f8", owner=self), device=f"cuda:{self.device}")
+            layer_shards = exchange_to_rank0(dist, mine_l, [n_layers * c for c in counts], self.rank, self.world,
+                                             self._layer_bufs)
         if self._exchanged is None:
             self._exchanged = torch.cuda.Event()
         self._exchanged.record()   # (the current stream waits for the NCCL work: req.wait() in exchange_to_rank0)
@@ -150,6 +166,8 @@ class DistributedRenderer:
             return None
         if self.world > 1:
             self._gather_bufs = shards
+            if n_layers:
+                self._layer_bufs = layer_shards
         if self._frame is None or tuple(self._frame.shape) != (height, width, 3):
             self._frame = torch.empty((height, width, 3), dtype=torch.float64, device=mine.device)
         # (2) k_assemble must run after the receives, i.e. on torch's current stream, and the host copy of
@@ -159,8 +177,14 @@ class DistributedRenderer:
         api.assemble_frame(self.dev_scene, self._params(width, height, samples_number, 0),
                            [int(s.data_ptr()) for s in shards], int(self._frame.data_ptr()),
                            stream=int(torch.cuda.current_stream().cuda_stream) or CUDA_STREAM_LEGACY)
+        if n_layers:
+            layers = torch.empty((n_layers, height, width, 3), dtype=torch.float64, device=mine.device)
+            api.assemble_layers(self.dev_scene, self._params(width, height, samples_number, 0), n_layers,
+                                [int(s.data_ptr()) for s in shards], [int(s.data_ptr()) for s in layer_shards],
+                                int(layers.data_ptr()),
+                                stream=int(torch.cuda.current_stream().cuda_stream) or CUDA_STREAM_LEGACY)
         self._exchanged.record()   # rank 0's own accumulator is read by k_assemble when it is the only shard
-        return self._frame
+        return (self._frame, layers) if n_layers else self._frame
 
     # ---- pipelined sequences: frame n's exchange and assembly overlap frame n+1's render ---------------------------
     def _exchange_assemble(self, mine, width, height, samples_number):
@@ -335,6 +359,15 @@ class DistributedRenderer:
     def render_views(self, cameras, width: int, height: int, samples_number: int) -> Optional[np.ndarray]:
         """render_views_device with the frames copied to the host on rank 0: (V, h, w, 3) float64, None elsewhere"""
         return self._to_host(self.render_views_device(cameras, width, height, samples_number))
+
+    def render_layers(self, camera: Camera, width: int, height: int, samples_number: int, n_layers: int):
+        """render_layers_device with both copied to the host on rank 0: (frame (h, w, 3), layers (L, h, w, 3)) float64
+        numpy arrays of their own, None elsewhere"""
+        out = self.render_layers_device(camera, width, height, samples_number, n_layers)
+        if out is None:
+            return None
+        frame, layers = out
+        return frame.cpu().numpy(), layers.cpu().numpy()
 
     def _to_host(self, frame):
         if frame is None:

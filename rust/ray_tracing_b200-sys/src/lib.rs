@@ -118,6 +118,13 @@ extern "C" {
         counts: *const u32) -> c_int;
     pub fn rt_render_start_views(scene: *mut rt_scene, cameras: *const rt_camera, n_views: u32,
         params: *const rt_render_params) -> c_int;
+    pub fn rt_render_start_layers(scene: *mut rt_scene, camera: *const rt_camera, params: *const rt_render_params,
+        n_layers: u32) -> c_int;
+    pub fn rt_render_layers(scene: *mut rt_scene, host: *mut rt_vec3, d_layers: *mut *const rt_vec3, n: *mut u64) -> c_int;
+    pub fn rt_render_device_layers(scene: *mut rt_scene, d_sums: *mut *const rt_vec3, n_slots: *mut u64) -> c_int;
+    pub fn rt_assemble_layers(scene: *mut rt_scene, params: *const rt_render_params, n_layers: u32,
+        d_accs: *const *const c_void, d_layer_sums: *const *const c_void, d_out: *mut rt_vec3,
+        stream: *mut c_void) -> c_int;
     pub fn rt_render_device_result(scene: *mut rt_scene, d_accum: *mut *const c_void, n_float4: *mut u64) -> c_int;
     pub fn rt_shard_float4_count(params: *const rt_render_params, shard_index: u32) -> u64;
     pub fn rt_assemble_frame(scene: *mut rt_scene, params: *const rt_render_params, d_shards: *const *const c_void,

@@ -3,7 +3,12 @@
   python tools/render.py scenes/cornell_box.json out.png --size 1024 1024 --spp 256 [--depth 8] [--seed 1]
       [--adaptive REL [--min-samples N] [--abs-error A] [--heatmap counts.png]]
       [--counts MAP.npy [--heatmap counts.png]]
-      [--orbit N] [--animate N [--step S]] [--inspect X Y]
+      [--orbit N] [--animate N [--step S]] [--inspect X Y] [--layers N]
+
+With --layers N, the frame and its N bounce layers (rt_render_start_layers): layer b holds the light of the paths that
+ended on bounce level b (the last layer: on level N-1 or deeper); layer b goes to OUT_Lb.png (out_L00.png, ... for
+out.png), tone-mapped like the frame, and each layer's share of the frame's mean luminance is printed -- what depth is
+enough for the scene.
 
 Scene::from_json -> GpuRenderer (Renderer trait: start_rendering / render_step until done) ->
 rt_tonemap_rgba8 (sqrt, clamp(0, 0.999) * 256, on the device) -> PNG.  With --adaptive, an adaptive frame
@@ -41,6 +46,7 @@ ap.add_argument("--heatmap", default=None, help="PNG of the per-pixel sample cou
 ap.add_argument("--orbit", type=int, default=None, metavar="N", help="N views around the scene, one PNG per view")
 ap.add_argument("--animate", type=int, default=None, metavar="N", help="N frames of the random spheres on a random walk")
 ap.add_argument("--step", type=float, default=0.05, help="--animate: random-walk step per axis and frame")
+ap.add_argument("--layers", type=int, default=None, metavar="N", help="N bounce layers, one PNG per layer")
 ap.add_argument("--inspect", type=int, nargs=2, default=None, metavar=("X", "Y"),
                 help="print each sample's path of pixel (X, Y) and check their mean against the frame")
 a = ap.parse_args()
@@ -53,6 +59,9 @@ if a.orbit is not None and (a.orbit < 1 or a.adaptive is not None or a.counts is
     ap.error("--orbit needs N >= 1 and excludes --adaptive and --counts")
 if a.animate is not None and (a.animate < 1 or a.orbit is not None or a.adaptive is not None or a.counts is not None):
     ap.error("--animate needs N >= 1 and excludes --orbit, --adaptive and --counts")
+if a.layers is not None and (not 1 <= a.layers <= 63 or a.orbit is not None or a.animate is not None
+                             or a.adaptive is not None or a.counts is not None or a.inspect is not None):
+    ap.error("--layers needs 1 <= N <= 63 and excludes --orbit, --animate, --adaptive, --counts and --inspect")
 if a.heatmap and a.adaptive is None and a.counts is None:
     ap.error("--heatmap needs --adaptive or --counts")
 if a.adaptive is not None and a.counts is not None:
@@ -67,6 +76,20 @@ if a.counts is not None:
         ap.error(f"--counts: an (h, w) uint32 array expected, got {given.dtype} {given.shape}")
     h, w = given.shape
 t0 = time.perf_counter()
+if a.layers is not None:
+    frame, layers = r.render_layers(cam, w, h, a.spp, a.layers)
+    dt = time.perf_counter() - t0
+    stem, ext = os.path.splitext(a.out)
+    rt.save_png(a.out, rt.tonemap_rgba8(sc, frame))
+    y = lambda f: float(np.mean((0.2126 * f[..., 0] + 0.7152 * f[..., 1]) + 0.0722 * f[..., 2]))
+    total = y(frame)
+    print(f"{a.scene}: {w}x{h}x{a.spp}, depth {a.depth}, {a.layers} layers in {dt * 1e3:.1f} ms -> {a.out}")
+    for b in range(a.layers):
+        rt.save_png(f"{stem}_L{b:02d}{ext or '.png'}", rt.tonemap_rgba8(sc, layers[b]))
+        share = y(layers[b]) / total if total else 0.0
+        last = "+" if b == a.layers - 1 and a.layers <= a.depth else " "
+        print(f"  level {b:2d}{last} {100.0 * share:8.4f} % of the mean luminance  -> {stem}_L{b:02d}{ext or '.png'}")
+    sys.exit(0)
 if a.orbit is not None:
     views = r.render_views(rt.api.orbit_cameras(cam, a.orbit), w, h, a.spp)
     dt = time.perf_counter() - t0
