@@ -498,6 +498,59 @@ int rt_render_device_layers(rt_scene* scene, const rt_vec3** d_sums, uint64_t* n
 int rt_assemble_layers(rt_scene* scene, const rt_render_params* params, uint32_t n_layers, const void* const* d_accs,
                        const void* const* d_layer_sums, rt_vec3* d_out, void* stream);
 
+/* First-hit feature buffers: the rt_render_start frame, with per-pixel features of the first hit of each sample's
+ * camera ray -- the auxiliary inputs of a denoiser (albedo, normal), a hit probe (shape), depth and coverage.
+ *   - Sample s of pixel p has the frame's own camera ray r_s.  H_s = rt_intersect_batch(r_s, 0.001, +inf) (any mode),
+ *     C_s = the color of rt_scatter_batch(r_s, keys (p, s), level 0, seed): the material's attenuation at the hit
+ *     (Lambertian / Metal texture value, Dielectric (1, 1, 1)), Material::emitted for DiffuseLight / Empty, and
+ *     Scene::background(dir) at a miss.  C_s draws no random number, so the features depend on the seed only through
+ *     the camera jitter.
+ *   - With n = samples_number and every sum an f64 sum in sample order from +0.0:
+ *       albedo   = Σ_s C_s / n
+ *       normal   = Σ_s H_s.normal / n   (a miss adds (0, 0, 0); the mean of unit normals is not renormalised)
+ *       depth    = Σ_{s hits} H_s.t / hits, +inf for a pixel no sample hits
+ *       coverage = hits / n
+ *       shape    = H_0.index: sample 0's shape, -1 at a miss
+ *   - The features do not depend on max_depth (max_depth = 0 included).
+ *   - The frame itself is the rt_render_start frame bit for bit: rt_render_poll / wait / stop with progressive delivery,
+ *     rt_render_device_frame, rt_render_device_result, rt_assemble_frame and the tone map work unchanged, and
+ *     rt_stats.paths grows as for rt_render_start.  Multi-device handles shard it as rt_render_start does; shard_count > 1
+ *     renders one shard.  Scenes with more than 32 ray-marched shapes (the fused fallback) are rendered too.
+ *   - The frame never continues or seeds a progressive accumulation (rt_render_accumulated_samples reads 0 after it);
+ *     rt_render_pixel_stats behaves as after rt_render_start.
+ * RT_ERR_INVALID before any device work, checked in this order: a NULL scene, camera or params; every parameter
+ * rt_render_start rejects; feature sums of (the shard's owned pixels, tile padding included) 72-byte slots whose size
+ * overflows 64 bits.  A rejected call leaves the last frame and its features as they were. */
+typedef struct rt_feature_sums {   /* one per owned pixel, tile-packed like rt_render_device_result */
+    rt_vec3 albedo, normal;        /* Σ C_s, Σ H_s.normal over the pixel's samples */
+    double depth, hits;            /* Σ H_s.t over the hitting samples, their count */
+    int32_t shape;                 /* sample 0's shape, -1 at a miss */
+    uint32_t pad;                  /* 0 */
+} rt_feature_sums;                 /* 72 bytes; a padding slot of a clipped border tile: zero sums, shape -1 */
+typedef struct rt_feature_planes { /* w * h values each, pixel (x, y) at [x + y * w]; any pointer may be NULL */
+    rt_vec3* albedo;
+    rt_vec3* normal;
+    double* depth;
+    double* coverage;
+    int32_t* shape;
+} rt_feature_planes;
+int rt_render_start_features(rt_scene* scene, const rt_camera* camera, const rt_render_params* params);
+/* After a completed features frame, unsharded, on a single-device or multi-device handle (waits for the frame in
+ * flight).  host (may be NULL): its non-NULL planes receive a copy; device (may be NULL) is filled with the library's
+ * planes on device_ids[0], valid until the next frame starts.  RT_ERR_STATE after any other frame or a shard of one. */
+int rt_render_features(rt_scene* scene, const rt_feature_planes* host, rt_feature_planes* device);
+/* This shard's feature sums after a completed features frame (waits for it): *n_slots = rt_shard_float4_count slots in
+ * the tile-packed owned order of rt_render_device_result.  Valid until the next frame starts.  RT_ERR_STATE on a
+ * multi-device handle (use rt_render_features) and after any other frame. */
+int rt_render_device_features(rt_scene* scene, const rt_feature_sums** d_sums, uint64_t* n_slots);
+/* rt_assemble_frame for the features: d_sums[s] = shard s's sums (rt_render_device_features), DEVICE pointers on the
+ * scene's device; d_out's non-NULL planes (device pointers, w x h each) receive the features, n = params' samples_number.
+ * Runs on `stream` like rt_assemble_frame (NULL = the library's own stream, cudaStreamLegacy = 0x1 the legacy default
+ * stream) and does not synchronise.  RT_ERR_INVALID for a NULL argument, samples_number 0 and what rt_assemble_frame
+ * rejects. */
+int rt_assemble_features(rt_scene* scene, const rt_render_params* params, const void* const* d_sums,
+                         const rt_feature_planes* d_out, void* stream);
+
 /* Device-side result of the last started frame, for callers that gather shards over NCCL:
  * FOUR DOUBLES (r, g, b sums; samples) per owned pixel -- the f64 sums themselves, so that the assembled frame
  * equals the unsharded one bit for bit; they were floats before ABI 4, hence the names -- tile-packed in this

@@ -8,12 +8,12 @@ face with the reference's names.  Importing this package requires the native lib
 from . import _ffi
 from ._ffi import (Camera, ImageParams, Ray, RenderParams, Stats, Vec3, NativeLibraryMissing,
                    RT_ISECT_BRUTE, RT_ISECT_FAST, RT_ISECT_VERIFY, RT_BOUNCE_MISS, RT_BOUNCE_SCATTER, RT_BOUNCE_EMIT)
-from .api import (GpuRenderer, RtError, Scene, camera_new, device_count, group_means, layer_means, make_rays,
-                  measure_peaks, path_levels, save_png, shadow_rays, tonemap_rgba8, trace_paths)
+from .api import (GpuRenderer, RtError, Scene, camera_new, device_count, feature_means, group_means, layer_means,
+                  make_rays, measure_peaks, path_levels, save_png, shadow_rays, tonemap_rgba8, trace_paths)
 
 __all__ = [
     "Camera", "ImageParams", "Ray", "RenderParams", "Stats", "Vec3", "NativeLibraryMissing",
     "RT_ISECT_BRUTE", "RT_ISECT_FAST", "RT_ISECT_VERIFY", "RT_BOUNCE_MISS", "RT_BOUNCE_SCATTER", "RT_BOUNCE_EMIT",
-    "GpuRenderer", "RtError", "Scene", "camera_new", "device_count", "group_means", "layer_means", "make_rays",
-    "measure_peaks", "path_levels", "save_png", "shadow_rays", "tonemap_rgba8", "trace_paths",
+    "GpuRenderer", "RtError", "Scene", "camera_new", "device_count", "feature_means", "group_means", "layer_means",
+    "make_rays", "measure_peaks", "path_levels", "save_png", "shadow_rays", "tonemap_rgba8", "trace_paths",
 ]

@@ -103,6 +103,12 @@ class AdaptiveParams(C.Structure):
     ]
 
 
+class FeaturePlanes(C.Structure):   # rt_feature_planes: w * h values each, NULL = not wanted
+    _fields_ = [("albedo", C.c_void_p), ("normal", C.c_void_p), ("depth", C.c_void_p), ("coverage", C.c_void_p),
+                ("shape", C.c_void_p)]
+
+
+
 class Stats(C.Structure):
     _fields_ = [
         ("kernel_launches", C.c_uint64),
@@ -171,6 +177,11 @@ CORE_SYMBOLS = {
     "rt_render_device_layers": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]),
     "rt_assemble_layers": (C.c_int, [C.c_void_p, C.POINTER(RenderParams), C.c_uint32, C.POINTER(C.c_void_p),
                                      C.POINTER(C.c_void_p), C.c_void_p, C.c_void_p]),
+    "rt_render_start_features": (C.c_int, [C.c_void_p, C.POINTER(Camera), C.POINTER(RenderParams)]),
+    "rt_render_features": (C.c_int, [C.c_void_p, C.POINTER(FeaturePlanes), C.POINTER(FeaturePlanes)]),
+    "rt_render_device_features": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]),
+    "rt_assemble_features": (C.c_int, [C.c_void_p, C.POINTER(RenderParams), C.POINTER(C.c_void_p),
+                                       C.POINTER(FeaturePlanes), C.c_void_p]),
     "rt_render_device_result": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]),
     "rt_shard_float4_count": (C.c_uint64, [C.POINTER(RenderParams), C.c_uint32]),
     "rt_assemble_frame": (C.c_int, [C.c_void_p, C.POINTER(RenderParams), C.POINTER(C.c_void_p), C.c_void_p,

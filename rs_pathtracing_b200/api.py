@@ -502,6 +502,19 @@ class GpuRenderer:
         render_wait(h, frame)
         return frame, render_layers(h)
 
+    def render_features(self, camera: Camera, width: int, height: int, samples_number: int):
+        """A frame with its first-hit features (rt_render_start_features) on this renderer's devices, depth and seed:
+        returns (frame[h, w, 3] float64, features), frame = render(camera, ...) bit for bit and features the dict of
+        render_features: albedo, normal, depth, coverage, shape."""
+        if self.devices and len(self.devices) > 1:
+            h = self.scene.device_scene_multi(self.devices)
+        else:
+            h = self.scene.device_scene(self.device)
+        render_start_features(h, camera, render_params(width, height, samples_number, self.depth, self.seed))
+        frame = np.zeros((height, width, 3), np.float64)
+        render_wait(h, frame)
+        return frame, render_features(h)
+
 
 def tonemap_rgba8(scene: Scene, frame: np.ndarray, device: Optional[int] = None) -> np.ndarray:
     """src/bin/main_raylib.rs:239-247 on the device."""
@@ -943,6 +956,103 @@ def layer_means(radiance, levels, offsets, n_layers: int) -> np.ndarray:
         s[b[r], g] = s[b[r], g] + f[r]
     with np.errstate(invalid="ignore"):
         return s / count[None, :, None]
+
+
+FEATURE_NAMES = ("albedo", "normal", "depth", "coverage", "shape")
+FEATURE_SUMS_DTYPE = np.dtype([("albedo", "<f8", 3), ("normal", "<f8", 3), ("depth", "<f8"), ("hits", "<f8"),
+                               ("shape", "<i4"), ("pad", "<u4")])   # rt_feature_sums, 72 bytes
+
+
+def render_start_features(dev_scene, camera: Camera, params: RenderParams) -> None:
+    """rt_render_start_features: the render_start frame (poll / wait deliver it as for render_start), and with it the
+    first-hit features of every pixel (render_features): albedo, normal, depth, coverage and shape"""
+    _check(_ffi.core().rt_render_start_features(dev_scene, C.byref(camera), C.byref(params)))
+    _started[_handle_key(dev_scene)] = (params.image.height, params.image.width, False)
+
+
+def _feature_planes(ptrs: dict) -> _ffi.FeaturePlanes:
+    unknown = set(ptrs) - set(FEATURE_NAMES)
+    if unknown:
+        raise ValueError(f"unknown feature planes {sorted(unknown)}; the planes are {FEATURE_NAMES}")
+    return _ffi.FeaturePlanes(*(C.c_void_p(ptrs[k]) if ptrs.get(k) else None for k in FEATURE_NAMES))
+
+
+def render_features(dev_scene, device: bool = False, shape=None) -> dict:
+    """rt_render_features after a completed unsharded features frame (waits for the frame in flight): {"albedo": (h, w, 3),
+    "normal": (h, w, 3), "depth": (h, w), "coverage": (h, w) float64, "shape": (h, w) int32} numpy arrays, pixel (x, y)
+    at [y, x].  device=True returns the device pointers of the library's planes on the handle's first device instead
+    (valid until the next frame starts).  shape = (height, width) for a frame not started through this module."""
+    if device:
+        planes = _ffi.FeaturePlanes()
+        _check(_ffi.core().rt_render_features(dev_scene, None, C.byref(planes)))
+        return {k: getattr(planes, k) for k in FEATURE_NAMES}
+    if shape is None:
+        known = _started.get(_handle_key(dev_scene))
+        if known is None:
+            raise ValueError("frame size unknown: pass shape=(height, width)")
+        shape = known[:2]
+    h, w = shape
+    out = {"albedo": np.empty((h, w, 3)), "normal": np.empty((h, w, 3)), "depth": np.empty((h, w)),
+           "coverage": np.empty((h, w)), "shape": np.empty((h, w), np.int32)}
+    host = _feature_planes({k: v.ctypes.data for k, v in out.items()})
+    _check(_ffi.core().rt_render_features(dev_scene, C.byref(host), None))
+    return out
+
+
+def render_device_features(dev_scene):
+    """(device pointer, n) of the shard's feature sums: n rt_feature_sums (FEATURE_SUMS_DTYPE, 72 bytes) in the
+    tile-packed order of render_device_result"""
+    ptr, n = C.c_void_p(), C.c_uint64()
+    _check(_ffi.core().rt_render_device_features(dev_scene, C.byref(ptr), C.byref(n)))
+    return ptr.value, n.value
+
+
+def assemble_features(dev_scene, params: RenderParams, sum_ptrs, out_ptrs: dict, stream: int = 0) -> None:
+    """rt_assemble_features: the gathered feature sums of every shard -> the planes at out_ptrs (a dict of device
+    pointers by FEATURE_NAMES; a missing or zero one is not written), on `stream` (0: the library's stream)"""
+    sums = (C.c_void_p * len(sum_ptrs))(*sum_ptrs)
+    _check(_ffi.core().rt_assemble_features(dev_scene, C.byref(params), sums, C.byref(_feature_planes(out_ptrs)),
+                                            C.c_void_p(stream) if stream else None))
+
+
+def feature_means(index, t, normal, color, offsets) -> dict:
+    """the first-hit features of groups of camera rays as the features frame takes them: group g = rays offsets[g] ..
+    offsets[g+1]-1 (a pixel's samples in sample order), index / t / normal their nearest hit (Scene.closest_hit), color
+    their level-0 colour (Scene.scatter(level=0)["color"]).  f64 sums in ray order from +0.0: albedo = Σ color / n,
+    normal = Σ normal / n (a miss adds zero), depth = Σ t over the hits / hits (+inf without a hit), coverage = hits / n,
+    shape = the index of the group's first ray (-1 for an empty group); an empty group's means are NaN.  Returns
+    {"albedo": (G, 3), "normal": (G, 3), "depth": (G,), "coverage": (G,) float64, "shape": (G,) int32}."""
+    idx = np.asarray(index).reshape(-1)
+    if not np.issubdtype(idx.dtype, np.integer):
+        raise ValueError("index: one integer shape index per ray")
+    n = idx.shape[0]
+    tt = np.asarray(t, dtype=np.float64).reshape(-1)
+    nrm = np.asarray(normal, dtype=np.float64)
+    col = np.asarray(color, dtype=np.float64)
+    if tt.shape != (n,) or nrm.shape != (n, 3) or col.shape != (n, 3):
+        raise ValueError("t (n,), normal (n, 3) and color (n, 3): one entry per ray")
+    off = np.asarray(offsets, dtype=np.int64).reshape(-1)
+    if off.size == 0 or off[0] != 0 or off[-1] != n or (np.diff(off) < 0).any():
+        raise ValueError("offsets must rise from 0 to len(index)")
+    count = np.diff(off)
+    hit = idx >= 0
+    nrm = np.where(hit[:, None], nrm, 0.0)
+    a, nm = np.zeros((count.size, 3)), np.zeros((count.size, 3))
+    d, hits = np.zeros(count.size), np.zeros(count.size)
+    for k in range(int(count.max(initial=0))):   # step k adds ray k of every group that has one: the in-order sums
+        g = np.flatnonzero(count > k)
+        r = off[:-1][g] + k
+        a[g] = a[g] + col[r]
+        nm[g] = nm[g] + nrm[r]
+        gh, rh = g[hit[r]], r[hit[r]]
+        d[gh] = d[gh] + tt[rh]
+        hits[gh] = hits[gh] + 1.0
+    shape = np.full(count.size, -1, np.int32)
+    shape[count > 0] = idx[off[:-1][count > 0]]
+    with np.errstate(invalid="ignore", divide="ignore"):
+        return {"albedo": a / count[:, None], "normal": nm / count[:, None],
+                "depth": np.where(hits > 0, d / np.maximum(hits, 1.0), np.inf), "coverage": hits / count,
+                "shape": shape}
 
 
 def render_pixel_stats(dev_scene, shape=None):

@@ -6,6 +6,7 @@
 //   k_raygen_views      views frames: k_raygen over the stacked image of several views, each with its own camera
 //   k_bounce            one segment of ray_color for every live path: nearest hit, scatter / emit /
 //                       sky, survivors compacted into the next queue (ballot + popc + one atomic per warp)
+//   k_features_path     features frames: the first-hit record (colour, normal, t, shape) of every camera ray of a batch
 //   k_scatter_shade     rt_scatter_batch: the shading half of that segment for caller rays after k_intersect_batch
 //   k_resolve           per-pixel mean (trace_pixel_samples) -> (f64 sums, samples) accumulator + f64 frame
 //   k_load_groups       caller-supplied rays of groups of any size -> level-0 queue + RNG keys (trace_pixel_samples_group)
@@ -16,8 +17,10 @@
 //   k_load_counts       counts frames: level-0 loader, the caller's sample count per pixel -> queue + RNG keys
 //   k_counts_resolve    counts frames: a pixel's sums over its samples, continued across the pieces of a large pixel
 //   k_resolve_layers    layers frames: k_resolve, plus each pixel's f64 sums per ending bounce level
+//   k_features_resolve  features frames: a pixel's first-hit records, summed in sample order -> rt_feature_sums
 //   k_assemble          multi-GPU: gathered tile-packed shards -> frame
 //   k_assemble_layers   layers frames: (gathered) layer sums / the accumulator's n -> layer-major layers
+//   k_assemble_features features frames: (gathered) feature sums -> albedo / normal / depth / coverage / shape planes
 //   k_tonemap           the bins' sqrt / clamp / *256 -> RGBA8
 //   k_scene_scatter     rt_scene_update_transforms: (slot, value) records of a refit into the scene's tables, in place
 // Compile with -fmad=false (see rt_math.cuh).
@@ -303,13 +306,47 @@ k_raygen(RayCasterDev rc, ShardMap map, unsigned long long first_owned, uint32_t
     }
 }
 
+// Features frames (rt_render_start_features): the first hit of a camera ray, one 64-byte record per path of the batch --
+// the colour scatter_or_emit gives there (sky at a miss), the world normal, t, and the shape (-1 at a miss; then the
+// normal and t are zero).  k_features_resolve sums them per pixel.
+struct __align__(16) FeatRec {
+    rt_vec3 albedo, normal;
+    double t;
+    int32_t shape;
+    uint32_t pad;
+};
+static_assert(sizeof(FeatRec) == 64, "FeatRec: 64 bytes per path");
+static_assert(sizeof(rt_feature_sums) == 72, "rt_feature_sums: 72 bytes per pixel");
+// the record of a camera ray (ro, rd) with nearest hit (bi, bt), as rt_intersect_batch and rt_scatter_batch give them
+__device__ __forceinline__ FeatRec feature_record(const DevScene& S, int bi, double bt, D3 ro, D3 rd) {
+    FeatRec f;
+    f.pad = 0;
+    if (bi < 0) {
+        const D3 c = sky(rd);   // renderer/mod.rs:41-43
+        f.albedo = rt_vec3{c.x, c.y, c.z};
+        f.normal = rt_vec3{0.0, 0.0, 0.0};
+        f.t = 0.0;
+        f.shape = -1;
+        return f;
+    }
+    HitRec h;
+    finalize_hit(S, bi, bt, ro, rd, h, material_reads_uv(S, S.materials[S.material[bi]]));
+    const D3 c = material_color(S, h);
+    f.albedo = rt_vec3{c.x, c.y, c.z};
+    f.normal = rt_vec3{h.normal.x, h.normal.y, h.normal.z};
+    f.t = bt;
+    f.shape = bi;
+    return f;
+}
+
 // One segment of ray_color (src/renderer/mod.rs:23-45), iteratively: `level` = number of hits so
 // far, the reference's `depth` argument at this call is max_depth - level.
-template <bool COUNT>
+// FEATURES (level 0 of a features frame only): also the first-hit record of path pid into feat[pid], whatever the depth.
+template <bool COUNT, bool FEATURES>
 __global__ void __launch_bounds__(256)
 k_bounce(DevScene S, bool use_smem, PathQueue in, const uint32_t* __restrict__ count_in, PathQueue out,
          uint32_t* count_out, uint32_t level, uint32_t max_depth, const uint2* __restrict__ path_key, uint32_t k0,
-         uint32_t k1, float4* __restrict__ radiance, DevCounters* g_counters) {
+         uint32_t k1, float4* __restrict__ radiance, DevCounters* g_counters, FeatRec* __restrict__ feat) {
     Staged st = stage_scene(S, use_smem);
     DevCounters c = {};
     const uint32_t n = *count_in;
@@ -327,6 +364,7 @@ k_bounce(DevScene S, bool use_smem, PathQueue in, const uint32_t* __restrict__ c
             double bt;
             int bi;
             nearest_hit_fast<COUNT>(S, st, ro, rd, 0.001, INFINITY, bt, bi, c);  // mod.rs:24
+            if (FEATURES) feat[pid] = feature_record(S, bi, bt, ro, rd);
             D3 L = mk(0.0, 0.0, 0.0);
             if (bi < 0) {
                 L = hadamard(beta, sky(rd));  // :41-43
@@ -638,6 +676,19 @@ k_shade(DevScene S, PathQueue in, const uint32_t* __restrict__ count_in, HitQueu
     }
 }
 
+// K4f: features frames (rt_render_start_features), between the level-0 k_shade and level 1 (which overwrites hq): the
+// first-hit record of every camera ray.  At level 0 slot i of the queue is path i of the batch (k_extend's raygen), and
+// hq holds its final nearest hit -- also at max_depth 0, where a features frame marches the level in full.
+__global__ void __launch_bounds__(256)
+k_features_path(DevScene S, PathQueue in, HitQueue hq, uint32_t n, FeatRec* __restrict__ feat) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const D3 ro = mk(in.ox[i], in.oy[i], in.oz[i]);
+    const D3 rd = mk(in.dx[i], in.dy[i], in.dz[i]);
+    const int bi = hq.index[i];
+    feat[i] = feature_record(S, bi, bi < 0 ? 0.0 : hq.t[i], ro, rd);
+}
+
 // rt_scatter_batch: shade_slot's segment for caller rays whose nearest hit k_intersect_batch already wrote -- sky at a
 // miss, else finalize_hit and scatter_or_emit with the path RNG of (seed; keys[2i], keys[2i+1]) at event level + 1.  No
 // depth rule, no throughput, no queue: the caller multiplies and decides.  The trip count is rounded up to whole warps
@@ -786,6 +837,34 @@ k_resolve_layers(const float4* __restrict__ radiance, uint32_t n_pixels, uint32_
     const double ln = (double)spp;
     accum[first_owned + pl] = Acc{sx, sy, sz, ln};
     frame_owned[first_owned + pl] = rt_vec3{sx / ln, sy / ln, sz / ln};
+}
+
+// K5f: features frames (rt_render_start_features), after k_resolve: one thread per owned pixel of the batch sums its spp
+// first-hit records (path pl * spp + s, written by k_features_path / k_bounce<., true>) in sample order from +0.0 into
+// the pixel's rt_feature_sums.  A miss's record holds a zero normal, which leaves the normal sum as it is (a sum from
+// +0.0 is never -0.0).  Padding pixels of clipped border tiles have no paths: zero sums and shape -1.
+__global__ void __launch_bounds__(256)
+k_features_resolve(const FeatRec* __restrict__ rec, ShardMap map, uint32_t n_pixels, uint32_t spp,
+                   unsigned long long first_owned, rt_feature_sums* __restrict__ sums) {
+    const uint32_t pl = blockIdx.x * blockDim.x + threadIdx.x;
+    if (pl >= n_pixels) return;
+    rt_feature_sums o{};
+    o.shape = -1;
+    uint32_t x, y;
+    if (map.pixel_of(first_owned + pl, x, y)) {
+        const FeatRec* r = rec + (size_t)pl * spp;
+        for (uint32_t s = 0; s < spp; s++) {
+            const FeatRec f = r[s];
+            o.albedo.x += f.albedo.x; o.albedo.y += f.albedo.y; o.albedo.z += f.albedo.z;
+            o.normal.x += f.normal.x; o.normal.y += f.normal.y; o.normal.z += f.normal.z;
+            if (f.shape >= 0) {
+                o.depth += f.t;
+                o.hits += 1.0;
+            }
+            if (s == 0) o.shape = f.shape;
+        }
+    }
+    sums[first_owned + pl] = o;
 }
 
 // ---- adaptive sampling (rt_render_start_adaptive) -------------------------------------------------------------------
@@ -974,6 +1053,29 @@ k_assemble_layers(ShardPtrs shards, LayerPtrs layers, ShardMap map0, uint32_t n_
         const rt_vec3 v = src[b * stride];
         out[b * n_px + i] = rt_vec3{v.x / n, v.y / n, v.z / n};
     }
+}
+
+// K7f: the feature planes of a features frame (rt_render_start_features) from the (gathered) tile-packed feature sums
+// of every shard, k_assemble's tile arithmetic; n = the frame's samples_number.  A NULL plane is not written.
+struct FeaturePtrs {
+    const rt_feature_sums* p[16];
+};
+__global__ void __launch_bounds__(256)
+k_assemble_features(FeaturePtrs shards, ShardMap map0, double n, rt_feature_planes out) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (uint64_t)map0.width * map0.height) return;
+    const uint32_t y = (uint32_t)(i / map0.width), x = (uint32_t)(i - (uint64_t)y * map0.width);
+    uint32_t tx = x / map0.tile_w, ty = y / map0.tile_h;
+    uint32_t rot = ((ty % map0.tiles_x) * map0.skew) % map0.tiles_x;
+    uint32_t k = ty * map0.tiles_x + (tx + map0.tiles_x - rot) % map0.tiles_x;
+    uint32_t s = k % map0.shard_count, j = k / map0.shard_count;
+    size_t q = (size_t)j * map0.tile_pixels() + (size_t)(y % map0.tile_h) * map0.tile_w + (x % map0.tile_w);
+    const rt_feature_sums v = shards.p[s][q];
+    if (out.albedo) out.albedo[i] = rt_vec3{v.albedo.x / n, v.albedo.y / n, v.albedo.z / n};
+    if (out.normal) out.normal[i] = rt_vec3{v.normal.x / n, v.normal.y / n, v.normal.z / n};
+    if (out.depth) out.depth[i] = v.hits > 0.0 ? v.depth / v.hits : INFINITY;
+    if (out.coverage) out.coverage[i] = v.hits / n;
+    if (out.shape) out.shape[i] = v.shape;
 }
 
 // src/bin/main_raylib.rs:239-247
@@ -1458,6 +1560,19 @@ struct rt_scene {
     uint64_t layer_sums_cap = 0, layers_cap = 0;
     std::vector<rt_vec3*> d_peer_layers;
     std::vector<uint64_t> peer_layers_cap;
+    // features frames (rt_render_start_features): whether the frame in flight / last completed is one, each lane's
+    // first-hit records (64 B per path of a batch; allocated by the first features frame only), the feature sums (owned
+    // order), the planes of an unsharded or multi-device frame (one block: albedo, normal, depth, coverage, shape), and
+    // a multi-device handle's staging for the peers' sums
+    bool features_frame = false;
+    FeatRec* d_feat_rec[RT_MAX_LANES] = {};
+    uint64_t feat_rec_cap[RT_MAX_LANES] = {};
+    rt_feature_sums* d_feat_sums = nullptr;
+    uint64_t feat_sums_cap = 0;
+    uint8_t* d_feat_planes = nullptr;
+    uint64_t feat_planes_cap = 0;   // bytes
+    std::vector<rt_feature_sums*> d_peer_feat;
+    std::vector<uint64_t> peer_feat_cap;
     // scene updates (rt_scene_update[_transforms]): the host side of the cull tree the tables were built from (a
     // multi-device handle refits its first device's and applies the records on every device), the pinned staging and
     // the device copy of a refit's records, the event after which the staging may be rewritten, the event of the last
@@ -1637,8 +1752,10 @@ static int build_tables(const rt_scene_desc* d, int n_sm, size_t smem_optin, Sce
         cudaFuncSetAttribute(k_occluded_batch<false, RT_ISECT_FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
         cudaFuncSetAttribute(k_occluded_batch<true, RT_ISECT_FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
         cudaFuncSetAttribute(k_occluded_batch<false, RT_ISECT_VERIFY>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
-        cudaFuncSetAttribute(k_bounce<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
-        cudaFuncSetAttribute(k_bounce<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
+        cudaFuncSetAttribute(k_bounce<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
+        cudaFuncSetAttribute(k_bounce<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
+        cudaFuncSetAttribute(k_bounce<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
+        cudaFuncSetAttribute(k_bounce<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
         cudaFuncSetAttribute(k_extend<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
         cudaFuncSetAttribute(k_extend<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
         cudaFuncSetAttribute(k_extend<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t.smem_bytes);
@@ -1646,7 +1763,7 @@ static int build_tables(const rt_scene_desc* d, int n_sm, size_t smem_optin, Sce
     }
     // persistent grid: a whole number of CTAs per SM
     int per_sm = 0;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_bounce<false>, 256, t.smem_bytes);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_bounce<false, false>, 256, t.smem_bytes);
     if (per_sm < 1) per_sm = 1;
     t.grid = n_sm * per_sm;
     auto occ_grid = [&](auto kernel, int threads, size_t smem) {
@@ -2041,6 +2158,10 @@ void rt_scene_destroy(rt_scene* sc) {
     cudaFree(sc->d_layer_sums);
     cudaFree(sc->d_layers);
     for (rt_vec3* a : sc->d_peer_layers) cudaFree(a);
+    for (FeatRec* a : sc->d_feat_rec) cudaFree(a);
+    cudaFree(sc->d_feat_sums);
+    cudaFree(sc->d_feat_planes);
+    for (rt_feature_sums* a : sc->d_peer_feat) cudaFree(a);
     if (sc->host_stage) cudaFreeHost(sc->host_stage);
     cudaFree(sc->d_scatter);
     bind_lane(sc, 0);
@@ -2416,8 +2537,11 @@ static const int3 march_tune = {8, 8, 8};
 // are done and its 32 rays stay (nearly) in step: k_march -3 % on cornell_box, -4 % on dupin
 static const int3 march_tune0 = {32, 8, 8};
 
-// enqueue the bounce loop for paths already in q[0] (count in d_counts[0]); no host sync
-static void launch_bounces(rt_scene* sc, uint32_t max_depth, uint64_t seed, const RaygenArgs* raygen = nullptr) {
+// enqueue the bounce loop for paths already in q[0] (count in d_counts[0]); no host sync.  feat != NULL (features frames):
+// the first-hit record of every path of the batch goes to feat[path] -- k_features_path after the level-0 k_shade (which
+// needs the primary rays generated in place, `raygen`), or the fused k_bounce's FEATURES instantiation at level 0.
+static void launch_bounces(rt_scene* sc, uint32_t max_depth, uint64_t seed, const RaygenArgs* raygen = nullptr,
+                           FeatRec* feat = nullptr) {
     uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
     for (uint32_t level = 0; level <= max_depth; level++) {
         PathQueue& in = sc->q[level & 1];
@@ -2426,16 +2550,19 @@ static void launch_bounces(rt_scene* sc, uint32_t max_depth, uint64_t seed, cons
         uint32_t* cnt_out = sc->d_counts + level + 1;
         uint32_t* mcount = sc->d_counts + RT_CNT_MARCH + level;
         uint32_t* rcount = sc->d_counts + RT_CNT_REPLAY + level;
+        const bool features = level == 0 && feat != nullptr;
         if (!sc->wavefront) {
             KernelSpan span(sc, RT_KCLASS_EXTEND);
-            if (sc->counters_on)
-                k_bounce<true><<<sc->grid, 256, sc->smem_bytes, sc->stream>>>(sc->ds, sc->use_smem, in, cnt_in, out, cnt_out, level,
-                                                                              max_depth, sc->hq.key, k0, k1, sc->d_radiance,
-                                                                              sc->d_counters);
-            else
-                k_bounce<false><<<sc->grid, 256, sc->smem_bytes, sc->stream>>>(sc->ds, sc->use_smem, in, cnt_in, out, cnt_out, level,
-                                                                               max_depth, sc->hq.key, k0, k1, sc->d_radiance,
-                                                                               sc->d_counters);
+#define RT_LAUNCH_BOUNCE(C_, F_)                                                                                          \
+    k_bounce<C_, F_><<<sc->grid, 256, sc->smem_bytes, sc->stream>>>(sc->ds, sc->use_smem, in, cnt_in, out, cnt_out, level, \
+                                                                    max_depth, sc->hq.key, k0, k1, sc->d_radiance,       \
+                                                                    sc->d_counters, feat)
+            if (sc->counters_on) {
+                if (features) RT_LAUNCH_BOUNCE(true, true); else RT_LAUNCH_BOUNCE(true, false);
+            } else {
+                if (features) RT_LAUNCH_BOUNCE(false, true); else RT_LAUNCH_BOUNCE(false, false);
+            }
+#undef RT_LAUNCH_BOUNCE
             continue;
         }
         {
@@ -2443,9 +2570,11 @@ static void launch_bounces(rt_scene* sc, uint32_t max_depth, uint64_t seed, cons
             const bool gen = level == 0 && raygen != nullptr;   // the frame's primary rays are generated in place
             RaygenArgs rg{};
             if (gen) rg = *raygen;
+            // (the features need the nearest hit of every camera ray, also when level 0 is the last level)
+            const bool any_hit_suffices = level == max_depth && !features;
 #define RT_LAUNCH_EXTEND(C_, G_)                                                                                        \
     k_extend<C_, G_><<<sc->grid_extend, 256, sc->smem_bytes, sc->stream>>>(sc->ds, sc->use_smem, in, cnt_in, sc->hq, mcount, \
-                                                                           rcount, sc->d_counters, level == max_depth, rg)
+                                                                           rcount, sc->d_counters, any_hit_suffices, rg)
             if (sc->counters_on) {
                 if (gen) RT_LAUNCH_EXTEND(true, true); else RT_LAUNCH_EXTEND(true, false);
             } else {
@@ -2500,6 +2629,10 @@ static void launch_bounces(rt_scene* sc, uint32_t max_depth, uint64_t seed, cons
             }
 #undef RT_LAUNCH_SHADE
         }
+        if (features && raygen) {
+            KernelSpan span(sc, RT_KCLASS_SHADE);
+            k_features_path<<<(raygen->n_paths + 255) / 256, 256, 0, sc->stream>>>(sc->ds, in, sc->hq, raygen->n_paths, feat);
+        }
     }
 }
 
@@ -2530,9 +2663,25 @@ static int ensure_path_buffers(rt_scene* sc, uint64_t need_paths) {
 }
 
 static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_render_params* p,
-                               const rt_adaptive_params* ap = nullptr, uint32_t n_views = 0, uint32_t n_layers = 0);
+                               const rt_adaptive_params* ap = nullptr, uint32_t n_views = 0, uint32_t n_layers = 0,
+                               bool features = false);
 static int render_start_multi(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const uint32_t* counts = nullptr,
-                              uint32_t n_views = 0, uint32_t n_layers = 0);
+                              uint32_t n_views = 0, uint32_t n_layers = 0, bool features = false);
+
+// the feature planes of n pixels in one block (grown on demand): albedo, normal, depth, coverage, shape
+static const uint64_t RT_FEATURE_PLANE_BYTES = 2 * sizeof(rt_vec3) + 2 * sizeof(double) + sizeof(int32_t);
+static int ensure_feature_planes(rt_scene* sc, uint64_t n) {
+    return ensure_device_array(sc->d_feat_planes, sc->feat_planes_cap, n * RT_FEATURE_PLANE_BYTES);
+}
+static rt_feature_planes feature_planes(uint8_t* base, uint64_t n) {
+    rt_feature_planes f;
+    f.albedo = (rt_vec3*)base;
+    f.normal = (rt_vec3*)(base + n * sizeof(rt_vec3));
+    f.depth = (double*)(base + 2 * n * sizeof(rt_vec3));
+    f.coverage = (double*)(base + 2 * n * sizeof(rt_vec3) + n * sizeof(double));
+    f.shape = (int32_t*)(base + 2 * n * sizeof(rt_vec3) + 2 * n * sizeof(double));
+    return f;
+}
 static int render_start_counts_single(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const uint32_t* counts);
 
 int rt_render_start(rt_scene* sc, const rt_camera* cam, const rt_render_params* p) {
@@ -2594,7 +2743,7 @@ static int ensure_frame_buffers(rt_scene* sc) {
 // n_views > 0: a views frame (rt_render_start_views, validated there): `cam` points to n_views cameras and p is the
 // stacked image; level 0 of every batch is k_raygen_views, then the bounce loop runs without raygen.
 static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const rt_adaptive_params* ap,
-                               uint32_t n_views, uint32_t n_layers) {
+                               uint32_t n_views, uint32_t n_layers, bool features) {
     if (!sc || !cam || !p) return fail(RT_ERR_INVALID, "null argument");
     int rc = check_frame_params(p);
     if (rc != RT_OK) return rc;
@@ -2605,7 +2754,7 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
     // progressive accumulation: this frame adds its samples to the previous ones when it is the same frame
     // (image, sharding, depth, seed, camera) and nothing was abandoned; otherwise it starts afresh
     uint32_t sample_base = 0;
-    if (!ap && !n_views && !n_layers && sc->accumulate && sc->accumulated_spp > 0 && sc->wavefront && memcmp(&sc->accum_cam, cam, sizeof *cam) == 0 &&
+    if (!ap && !n_views && !n_layers && !features && sc->accumulate && sc->accumulated_spp > 0 && sc->wavefront && memcmp(&sc->accum_cam, cam, sizeof *cam) == 0 &&
         sc->accum_rp.image.width == p->image.width && sc->accum_rp.image.height == p->image.height &&
         sc->accum_rp.max_depth == p->max_depth && sc->accum_rp.seed == p->seed &&
         (sc->accum_rp.shard_count ? sc->accum_rp.shard_count : 1) == shard_count &&
@@ -2617,6 +2766,7 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
     sc->adaptive_frame = false;
     sc->views_frame = n_views > 0;
     sc->n_layers = n_layers;
+    sc->features_frame = features;
     sc->rp = *p;
     sc->rp.shard_count = shard_count;
     sc->map = make_shard_map(sc->rp, p->shard_index);
@@ -2657,6 +2807,7 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
     for (int l = 0; l < lanes_used && rc == RT_OK; l++) {
         bind_lane(sc, l);
         rc = ensure_path_buffers(sc, std::max<uint64_t>(px_per_batch * spp, refine_paths));
+        if (rc == RT_OK && features) rc = ensure_device_array(sc->d_feat_rec[l], sc->feat_rec_cap[l], px_per_batch * spp);
     }
     bind_lane(sc, 0);
     if (rc != RT_OK) return rc;
@@ -2665,6 +2816,10 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
         if ((rc = ensure_device_array(sc->d_layer_sums, sc->layer_sums_cap, n_layers * sc->owned_pixels)) != RT_OK) return rc;
         if (shard_count == 1 && (rc = ensure_device_array(sc->d_layers, sc->layers_cap, n_layers * sc->owned_pixels)) != RT_OK)
             return rc;
+    }
+    if (features) {   // the feature sums; an unsharded frame also keeps its planes
+        if ((rc = ensure_device_array(sc->d_feat_sums, sc->feat_sums_cap, sc->owned_pixels)) != RT_OK) return rc;
+        if (shard_count == 1 && (rc = ensure_feature_planes(sc, sc->owned_pixels)) != RT_OK) return rc;
     }
     if (ap) {
         if ((rc = ensure_device_array(sc->d_moments, sc->moments_cap, sc->owned_pixels)) != RT_OK) return rc;
@@ -2697,6 +2852,7 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
         for (uint64_t first = 0; first < sc->owned_pixels; first += px_per_batch, batch_no++) {
             bind_lane(sc, (int)(batch_no % (uint64_t)lanes_used));
             uint32_t npx = (uint32_t)std::min<uint64_t>(px_per_batch, sc->owned_pixels - first);
+            FeatRec* const feat = features ? sc->d_feat_rec[sc->cur_lane] : nullptr;
             CU(cudaMemsetAsync(sc->d_counts, 0, RT_CNT_WORDS * sizeof(uint32_t), sc->stream));
             if (n_views) {
                 {
@@ -2709,13 +2865,13 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
                 RaygenArgs rg;
                 rg.rc = rcd; rg.map = sc->map; rg.first_owned = first; rg.n_paths = npx * spp; rg.spp = spp;
                 rg.k0 = k0; rg.k1 = k1; rg.sample_base = sample_base; rg.radiance = sc->d_radiance; rg.count_out = sc->d_counts;
-                launch_bounces(sc, p->max_depth, p->seed, &rg);
+                launch_bounces(sc, p->max_depth, p->seed, &rg, feat);
             } else {
                 {
                     KernelSpan span(sc, RT_KCLASS_RAYGEN);
                     k_raygen<<<sc->grid, 256, 0, sc->stream>>>(rcd, sc->map, first, npx, spp, k0, k1, sc->q[0], sc->d_counts, sc->d_radiance, sc->hq.key, sample_base);
                 }
-                launch_bounces(sc, p->max_depth, p->seed);
+                launch_bounces(sc, p->max_depth, p->seed, nullptr, feat);
             }
             {
                 KernelSpan span(sc, RT_KCLASS_RESOLVE);
@@ -2729,6 +2885,10 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
                 else
                     k_resolve<false><<<(npx + 255) / 256, 256, 0, sc->stream>>>(sc->d_radiance, npx, spp, first, sc->d_accum,
                                                                               sc->d_frame, sample_base != 0, nullptr);
+            }
+            if (features) {
+                KernelSpan span(sc, RT_KCLASS_RESOLVE);
+                k_features_resolve<<<(npx + 255) / 256, 256, 0, sc->stream>>>(feat, sc->map, npx, spp, first, sc->d_feat_sums);
             }
             if (ap) continue;   // an adaptive frame is delivered whole, after its last pass
             Batch b;
@@ -2792,6 +2952,13 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
             k_assemble_layers<<<(unsigned)((sc->owned_pixels + 255) / 256), 256, 0, sc->stream>>>(accs, lp, sc->map, n_layers,
                                                                                                   sc->d_layers);
         }
+        if (features && shard_count == 1) {   // the planes of an unsharded frame (owned order is x + y*width)
+            KernelSpan span(sc, RT_KCLASS_RESOLVE);
+            FeaturePtrs fp{};
+            fp.p[0] = sc->d_feat_sums;
+            k_assemble_features<<<(unsigned)((sc->owned_pixels + 255) / 256), 256, 0, sc->stream>>>(
+                fp, sc->map, (double)spp, feature_planes(sc->d_feat_planes, sc->owned_pixels));
+        }
         if (ap) {   // one delivery unit: the whole frame, once the last pass has resolved
             Batch b;
             b.first_owned = 0;
@@ -2819,7 +2986,7 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
         for (const RefinePass& P : refine) sc->adaptive_m.push_back(P.m);
         return RT_OK;
     }
-    if (n_layers) return RT_OK;   // the frame neither continues nor seeds an accumulation
+    if (n_layers || features) return RT_OK;   // the frame neither continues nor seeds an accumulation
     if (sc->accumulate && sc->wavefront) {  // (enqueued work always runs to completion: rt_render_stop drains it)
         sc->accumulated_spp = sample_base + spp;
         sc->accum_rp = *p;
@@ -2836,7 +3003,7 @@ static int render_start_single(rt_scene* sc, const rt_camera* cam, const rt_rend
 // (rt_render_start_counts, validated there), every shard reading the whole map.  n_views > 0: a views frame
 // (rt_render_start_views, validated there; p is the stacked image), every shard uploading the whole camera table.
 static int render_start_multi(rt_scene* sc, const rt_camera* cam, const rt_render_params* p, const uint32_t* counts,
-                              uint32_t n_views, uint32_t n_layers) {
+                              uint32_t n_views, uint32_t n_layers, bool features) {
     if (p->image.width == 0 || p->image.height == 0 || p->samples_number == 0)
         return fail(RT_ERR_INVALID, "empty image or zero samples");
     const uint32_t n_dev = (uint32_t)sc->peers.size() + 1;
@@ -2875,22 +3042,36 @@ static int render_start_multi(rt_scene* sc, const rt_camera* cam, const rt_rende
         int rc = ensure_device_array(sc->d_layers, sc->layers_cap, n_layers * n_px);
         if (rc != RT_OK) return rc;
     }
+    if (features) {   // the peers' feature sums and the planes, on this device
+        sc->d_peer_feat.resize(n_dev - 1, nullptr);
+        sc->peer_feat_cap.resize(n_dev - 1, 0);
+        for (uint32_t k = 1; k < n_dev; k++) {
+            int rc = ensure_device_array(sc->d_peer_feat[k - 1], sc->peer_feat_cap[k - 1], rt_shard_float4_count(&sp, k));
+            if (rc != RT_OK) return rc;
+        }
+        int rc = ensure_feature_planes(sc, n_px);
+        if (rc != RT_OK) return rc;
+    }
     // enqueue every shard (the peers first: the first device also assembles)
     for (uint32_t k = 1; k < n_dev; k++) {
         rt_scene* peer = sc->peers[k - 1];
         sp.shard_index = k;
         int rc = counts ? render_start_counts_single(peer, cam, &sp, counts)
-                        : render_start_single(peer, cam, &sp, nullptr, n_views, n_layers);
+                        : render_start_single(peer, cam, &sp, nullptr, n_views, n_layers, features);
         if (rc != RT_OK) return rc;
         const uint64_t cnt = rt_shard_float4_count(&sp, k);
         if (cnt) CU(cudaMemcpyPeerAsync(sc->d_peer_acc[k - 1], sc->device, peer->d_accum, peer->device, cnt * sizeof(Acc), peer->stream));
         if (cnt && n_layers)
             CU(cudaMemcpyPeerAsync(sc->d_peer_layers[k - 1], sc->device, peer->d_layer_sums, peer->device,
                                    n_layers * cnt * sizeof(rt_vec3), peer->stream));
+        if (cnt && features)
+            CU(cudaMemcpyPeerAsync(sc->d_peer_feat[k - 1], sc->device, peer->d_feat_sums, peer->device,
+                                   cnt * sizeof(rt_feature_sums), peer->stream));
         CU(cudaEventRecord(sc->ev_peer[k - 1], peer->stream));
     }
     sp.shard_index = 0;
-    int rc = counts ? render_start_counts_single(sc, cam, &sp, counts) : render_start_single(sc, cam, &sp, nullptr, n_views, n_layers);
+    int rc = counts ? render_start_counts_single(sc, cam, &sp, counts)
+                    : render_start_single(sc, cam, &sp, nullptr, n_views, n_layers, features);
     if (rc != RT_OK) return rc;
     CU(cudaSetDevice(sc->device));
     for (uint32_t k = 1; k < n_dev; k++) CU(cudaStreamWaitEvent(sc->stream, sc->ev_peer[k - 1], 0));
@@ -2906,6 +3087,13 @@ static int render_start_multi(rt_scene* sc, const rt_camera* cam, const rt_rende
             lp.stride[k] = rt_shard_float4_count(&sp, k);
         }
         k_assemble_layers<<<(unsigned)((n_px + 255) / 256), 256, 0, sc->stream>>>(ptrs, lp, m0, n_layers, sc->d_layers);
+        sc->launches++;
+    }
+    if (features) {
+        FeaturePtrs fp{};
+        for (uint32_t k = 0; k < n_dev; k++) fp.p[k] = k == 0 ? sc->d_feat_sums : sc->d_peer_feat[k - 1];
+        k_assemble_features<<<(unsigned)((n_px + 255) / 256), 256, 0, sc->stream>>>(fp, m0, (double)p->samples_number,
+                                                                                    feature_planes(sc->d_feat_planes, n_px));
         sc->launches++;
     }
     CU(cudaEventRecord(sc->ev_multi_done, sc->stream));
@@ -3423,6 +3611,7 @@ static int render_start_counts_single(rt_scene* sc, const rt_camera* cam, const 
     sc->adaptive_frame = false;
     sc->views_frame = false;
     sc->n_layers = 0;
+    sc->features_frame = false;
     sc->rp = rp;
     sc->map = map;
     sc->owned_pixels = owned;
@@ -3619,6 +3808,98 @@ int rt_assemble_layers(rt_scene* sc, const rt_render_params* p, uint32_t n_layer
     }
     cudaStream_t st = stream ? (cudaStream_t)stream : sc->stream;
     k_assemble_layers<<<(unsigned)((n_px + 255) / 256), 256, 0, st>>>(accs, lp, m, n_layers, d_out);
+    sc->launches++;
+    CU(cudaGetLastError());
+    return RT_OK;
+}
+
+// ---- first-hit feature buffers (rt_render_start_features) ---------------------------------------------------------
+// The rt_render_start frame, plus the first-hit record of every camera ray (k_features_path after the level-0 k_shade,
+// or the fused k_bounce at level 0) and k_features_resolve after k_resolve.  Pixels are never split over batches in a
+// uniform frame, so each pixel's sums are written by one thread of one batch.
+int rt_render_start_features(rt_scene* sc, const rt_camera* cam, const rt_render_params* p) {
+    if (!sc || !cam || !p) return fail(RT_ERR_INVALID, "null argument");
+    int rc = check_frame_params(p);
+    if (rc != RT_OK) return rc;
+    // (rt_render_start rejects this once it has dropped the last frame; checked here so that the last frame stays)
+    if (p->samples_number > 0xFFFFFFF0u) return fail(RT_ERR_INVALID, "samples_number too large for one batch");
+    // the shard's owned pixels include the padding of its border tiles, which a thin image with tall tiles makes huge
+    rt_render_params pp = *p;
+    pp.shard_count = p->shard_count ? p->shard_count : 1;
+    const ShardMap m = make_shard_map(pp, p->shard_index);
+    const uint64_t owned = owned_tiles(m) * m.tile_pixels();
+    if (owned > UINT64_MAX / sizeof(rt_feature_sums)) return fail(RT_ERR_INVALID, "feature sums of the owned pixels overflow");
+    if (!sc->peers.empty() && p->shard_count <= 1) return render_start_multi(sc, cam, p, nullptr, 0, 0, true);
+    sc->multi_active = false;
+    return render_start_single(sc, cam, p, nullptr, 0, 0, true);
+}
+
+int rt_render_features(rt_scene* sc, const rt_feature_planes* host, rt_feature_planes* device) {
+    if (!sc) return fail(RT_ERR_INVALID, "null scene");
+    if (sc->rendering) {
+        int rc = rt_render_wait(sc, nullptr);
+        if (rc != RT_OK) return rc;
+    }
+    if (!sc->frame_complete) return fail(RT_ERR_STATE, "no completed frame");
+    if (!sc->features_frame) return fail(RT_ERR_STATE, "the last frame was not a features frame (rt_render_start_features)");
+    uint64_t n_px;
+    if (sc->multi_active) {
+        n_px = (uint64_t)sc->multi_rp.image.width * sc->multi_rp.image.height;
+    } else {
+        if (sc->map.shard_count != 1)
+            return fail(RT_ERR_STATE, "the last frame was one shard of a frame: use rt_render_device_features + rt_assemble_features");
+        n_px = (uint64_t)sc->map.width * sc->map.height;
+    }
+    const rt_feature_planes d = feature_planes(sc->d_feat_planes, n_px);
+    CU(cudaSetDevice(sc->device));
+    if (host) {
+        if (host->albedo) CU(cudaMemcpyAsync(host->albedo, d.albedo, n_px * sizeof(rt_vec3), cudaMemcpyDeviceToHost, sc->copy_stream));
+        if (host->normal) CU(cudaMemcpyAsync(host->normal, d.normal, n_px * sizeof(rt_vec3), cudaMemcpyDeviceToHost, sc->copy_stream));
+        if (host->depth) CU(cudaMemcpyAsync(host->depth, d.depth, n_px * sizeof(double), cudaMemcpyDeviceToHost, sc->copy_stream));
+        if (host->coverage)
+            CU(cudaMemcpyAsync(host->coverage, d.coverage, n_px * sizeof(double), cudaMemcpyDeviceToHost, sc->copy_stream));
+        if (host->shape) CU(cudaMemcpyAsync(host->shape, d.shape, n_px * sizeof(int32_t), cudaMemcpyDeviceToHost, sc->copy_stream));
+        const cudaError_t e = cudaStreamSynchronize(sc->copy_stream);
+        if (e != cudaSuccess) return fail(RT_ERR_CUDA, std::string("features: ") + cudaGetErrorString(e));
+    }
+    if (device) *device = d;
+    return RT_OK;
+}
+
+int rt_render_device_features(rt_scene* sc, const rt_feature_sums** d_sums, uint64_t* n_slots) {
+    if (!sc || !d_sums || !n_slots) return fail(RT_ERR_INVALID, "null argument");
+    if (sc->multi_active) return fail(RT_ERR_STATE, "a multi-device handle delivers the assembled features: rt_render_features");
+    if (sc->rendering) {
+        CU(cudaSetDevice(sc->device));
+        CU(cudaStreamSynchronize(sc->stream));
+        int done = 0;
+        int rc = rt_render_poll(sc, nullptr, &done);
+        if (rc != RT_OK) return rc;
+    }
+    if (!sc->frame_complete) return fail(RT_ERR_STATE, "no completed frame");
+    if (!sc->features_frame) return fail(RT_ERR_STATE, "the last frame was not a features frame (rt_render_start_features)");
+    *d_sums = sc->d_feat_sums;
+    *n_slots = sc->owned_pixels;
+    return RT_OK;
+}
+
+int rt_assemble_features(rt_scene* sc, const rt_render_params* p, const void* const* d_sums, const rt_feature_planes* d_out,
+                         void* stream) {
+    if (!sc || !p || !d_sums || !d_out) return fail(RT_ERR_INVALID, "null argument");
+    if (p->samples_number == 0) return fail(RT_ERR_INVALID, "zero samples");
+    uint32_t shard_count = p->shard_count ? p->shard_count : 1;
+    if (shard_count > 16) return fail(RT_ERR_INVALID, "at most 16 shards");
+    const uint64_t n_px = (uint64_t)p->image.width * p->image.height;
+    if (n_px == 0 || n_px > 0xFFFFFFFFull) return fail(RT_ERR_INVALID, "empty or too large image");
+    rt_render_params pp = *p;
+    pp.shard_count = shard_count;
+    ShardMap m = make_shard_map(pp, 0);
+    if (!tile_fits(m)) return fail(RT_ERR_INVALID, "tile_width * tile_height >= 2^32");
+    CU(cudaSetDevice(sc->device));
+    FeaturePtrs fp{};
+    for (uint32_t s = 0; s < shard_count; s++) fp.p[s] = (const rt_feature_sums*)d_sums[s];
+    cudaStream_t st = stream ? (cudaStream_t)stream : sc->stream;
+    k_assemble_features<<<(unsigned)((n_px + 255) / 256), 256, 0, st>>>(fp, m, (double)p->samples_number, *d_out);
     sc->launches++;
     CU(cudaGetLastError());
     return RT_OK;

@@ -624,6 +624,22 @@ __device__ inline bool scatter_or_emit(const DevScene& S, const HitRec& h, D3 rd
     }
 }
 
+// The `atten` scatter_or_emit gives for the hit, without its random draws (the colour depends on the hit only):
+// features frames record it.  A separate switch, so that scatter_or_emit's callers keep their generated code.
+__device__ __forceinline__ D3 material_color(const DevScene& S, const HitRec& h) {
+    const rt_material m = S.materials[S.material[h.shape]];
+    switch (m.kind) {
+        case RT_MAT_LAMBERTIAN:
+        case RT_MAT_METAL:
+        case RT_MAT_DIFFUSE_LIGHT:
+            return texture_value(S, m.texture, h.u, h.v, h.point);
+        case RT_MAT_DIELECTRIC:
+            return mk(1.0, 1.0, 1.0);
+        default:
+            return mk(0.0, 0.0, 0.0);
+    }
+}
+
 // Scene::background, src/world/mod.rs:199-202
 __device__ __forceinline__ D3 sky(D3 rd) {
     double t = 0.5 * (rd.y + 1.0);

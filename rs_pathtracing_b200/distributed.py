@@ -104,6 +104,7 @@ class DistributedRenderer:
         self._host2 = [None, None]
         self._dev_scene_b = None           # a second rt_scene on the same device: two frames of a sequence in flight
         self._layer_bufs = None            # rank 0: the gathered layer sums of layers frames
+        self._feature_bufs = None          # rank 0: the gathered feature sums of features frames
 
     def _params(self, w, h, spp, shard):
         return api.render_params(w, h, spp, self.depth, self.seed, self.world, shard, tile=self.tile)
@@ -137,9 +138,20 @@ class DistributedRenderer:
         return self._render_shard(lambda p: api.render_start_layers(self.dev_scene, camera, p, n_layers),
                                   width, height, samples_number, n_layers)
 
-    def _render_shard(self, start, width: int, height: int, samples_number: int, n_layers: int = 0):
+    def render_features_device(self, camera: Camera, width: int, height: int, samples_number: int):
+        """render_device of a features frame (rt_render_start_features): every rank renders its tiles, and its feature
+        sums (72 bytes per owned pixel) travel to rank 0 in one more exchange.  Returns (frame h x w x 3 float64,
+        features) on rank 0 -- features a dict of device tensors as api.render_features gives them: albedo, normal
+        (h, w, 3), depth, coverage (h, w) float64, shape (h, w) int32 -- each equal to the unsharded features frame's
+        bit for bit, None elsewhere."""
+        return self._render_shard(lambda p: api.render_start_features(self.dev_scene, camera, p),
+                                  width, height, samples_number, features=True)
+
+    def _render_shard(self, start, width: int, height: int, samples_number: int, n_layers: int = 0,
+                      features: bool = False):
         """start(params) this rank's shard of a width x height frame, gather, assemble on rank 0 (n_layers > 0: a
-        layers frame, whose layers are gathered and assembled too: (frame, layers) on rank 0)"""
+        layers frame, whose layers are gathered and assembled too: (frame, layers) on rank 0; features: a features
+        frame, (frame, features) on rank 0)"""
         torch, dist = self.torch, self.dist
         p = self._params(width, height, samples_number, self.rank)
         # The library renders on its own non-blocking streams, the exchange runs on torch's / NCCL's: the
@@ -159,6 +171,11 @@ class DistributedRenderer:
             mine_l = torch.as_tensor(api.DevicePointer(lptr, (ln, 3), "<f8", owner=self), device=f"cuda:{self.device}")
             layer_shards = exchange_to_rank0(dist, mine_l, [n_layers * c for c in counts], self.rank, self.world,
                                              self._layer_bufs)
+        feature_shards = None
+        if features:   # the second exchange: every rank's feature sums, 72 bytes (moved as 9 doubles) per owned pixel
+            fptr, fn = api.render_device_features(self.dev_scene)
+            mine_f = torch.as_tensor(api.DevicePointer(fptr, (fn, 9), "<f8", owner=self), device=f"cuda:{self.device}")
+            feature_shards = exchange_to_rank0(dist, mine_f, counts, self.rank, self.world, self._feature_bufs)
         if self._exchanged is None:
             self._exchanged = torch.cuda.Event()
         self._exchanged.record()   # (the current stream waits for the NCCL work: req.wait() in exchange_to_rank0)
@@ -168,6 +185,8 @@ class DistributedRenderer:
             self._gather_bufs = shards
             if n_layers:
                 self._layer_bufs = layer_shards
+            if features:
+                self._feature_bufs = feature_shards
         if self._frame is None or tuple(self._frame.shape) != (height, width, 3):
             self._frame = torch.empty((height, width, 3), dtype=torch.float64, device=mine.device)
         # (2) k_assemble must run after the receives, i.e. on torch's current stream, and the host copy of
@@ -183,7 +202,18 @@ class DistributedRenderer:
                                 [int(s.data_ptr()) for s in shards], [int(s.data_ptr()) for s in layer_shards],
                                 int(layers.data_ptr()),
                                 stream=int(torch.cuda.current_stream().cuda_stream) or CUDA_STREAM_LEGACY)
+        if features:
+            new = lambda shape, dt: torch.empty(shape, dtype=dt, device=mine.device)
+            feats = {"albedo": new((height, width, 3), torch.float64), "normal": new((height, width, 3), torch.float64),
+                     "depth": new((height, width), torch.float64), "coverage": new((height, width), torch.float64),
+                     "shape": new((height, width), torch.int32)}
+            api.assemble_features(self.dev_scene, self._params(width, height, samples_number, 0),
+                                  [int(s.data_ptr()) for s in feature_shards],
+                                  {k: int(v.data_ptr()) for k, v in feats.items()},
+                                  stream=int(torch.cuda.current_stream().cuda_stream) or CUDA_STREAM_LEGACY)
         self._exchanged.record()   # rank 0's own accumulator is read by k_assemble when it is the only shard
+        if features:
+            return self._frame, feats
         return (self._frame, layers) if n_layers else self._frame
 
     # ---- pipelined sequences: frame n's exchange and assembly overlap frame n+1's render ---------------------------
@@ -368,6 +398,15 @@ class DistributedRenderer:
             return None
         frame, layers = out
         return frame.cpu().numpy(), layers.cpu().numpy()
+
+    def render_features(self, camera: Camera, width: int, height: int, samples_number: int):
+        """render_features_device with everything copied to the host on rank 0: (frame (h, w, 3) float64, features dict
+        of numpy arrays), arrays of their own, None elsewhere"""
+        out = self.render_features_device(camera, width, height, samples_number)
+        if out is None:
+            return None
+        frame, feats = out
+        return frame.cpu().numpy(), {k: v.cpu().numpy() for k, v in feats.items()}
 
     def _to_host(self, frame):
         if frame is None:

@@ -68,6 +68,11 @@ pub const RT_BOUNCE_EMIT: u8 = 2;
     pub shard_count: u32, pub shard_index: u32, pub tile_width: u32, pub tile_height: u32 }
 #[repr(C)] #[derive(Clone, Copy, Debug)] pub struct rt_adaptive_params {
     pub min_samples: u32, pub rel_error: f64, pub abs_error: f64 }
+#[repr(C)] #[derive(Clone, Copy, Default, Debug)] pub struct rt_feature_sums {
+    pub albedo: rt_vec3, pub normal: rt_vec3, pub depth: f64, pub hits: f64, pub shape: i32, pub pad: u32 }
+#[repr(C)] #[derive(Clone, Copy, Debug)] pub struct rt_feature_planes {
+    pub albedo: *mut rt_vec3, pub normal: *mut rt_vec3, pub depth: *mut f64, pub coverage: *mut f64,
+    pub shape: *mut i32 }
 #[repr(C)] #[derive(Clone, Copy, Default, Debug)] pub struct rt_stats {
     pub kernel_launches: u64, pub paths: u64, pub segments: u64, pub shape_tests: u64, pub cull_tests: u64,
     pub march_steps: u64, pub march_rays: u64, pub march_long_rays: u64, pub march_max_evals: u64,
@@ -125,6 +130,14 @@ extern "C" {
     pub fn rt_assemble_layers(scene: *mut rt_scene, params: *const rt_render_params, n_layers: u32,
         d_accs: *const *const c_void, d_layer_sums: *const *const c_void, d_out: *mut rt_vec3,
         stream: *mut c_void) -> c_int;
+    pub fn rt_render_start_features(scene: *mut rt_scene, camera: *const rt_camera,
+        params: *const rt_render_params) -> c_int;
+    pub fn rt_render_features(scene: *mut rt_scene, host: *const rt_feature_planes,
+        device: *mut rt_feature_planes) -> c_int;
+    pub fn rt_render_device_features(scene: *mut rt_scene, d_sums: *mut *const rt_feature_sums,
+        n_slots: *mut u64) -> c_int;
+    pub fn rt_assemble_features(scene: *mut rt_scene, params: *const rt_render_params, d_sums: *const *const c_void,
+        d_out: *const rt_feature_planes, stream: *mut c_void) -> c_int;
     pub fn rt_render_device_result(scene: *mut rt_scene, d_accum: *mut *const c_void, n_float4: *mut u64) -> c_int;
     pub fn rt_shard_float4_count(params: *const rt_render_params, shard_index: u32) -> u64;
     pub fn rt_assemble_frame(scene: *mut rt_scene, params: *const rt_render_params, d_shards: *const *const c_void,

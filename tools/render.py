@@ -3,12 +3,18 @@
   python tools/render.py scenes/cornell_box.json out.png --size 1024 1024 --spp 256 [--depth 8] [--seed 1]
       [--adaptive REL [--min-samples N] [--abs-error A] [--heatmap counts.png]]
       [--counts MAP.npy [--heatmap counts.png]]
-      [--orbit N] [--animate N [--step S]] [--inspect X Y] [--layers N]
+      [--orbit N] [--animate N [--step S]] [--inspect X Y] [--layers N] [--features]
 
 With --layers N, the frame and its N bounce layers (rt_render_start_layers): layer b holds the light of the paths that
 ended on bounce level b (the last layer: on level N-1 or deeper); layer b goes to OUT_Lb.png (out_L00.png, ... for
 out.png), tone-mapped like the frame, and each layer's share of the frame's mean luminance is printed -- what depth is
 enough for the scene.
+
+With --features, the frame and the first-hit features of its samples' camera rays (rt_render_start_features), the inputs
+a denoiser takes beside the colour: OUT_albedo.png (the hit's material colour, sky at a miss, clamped to [0, 1]),
+OUT_normal.png (0.5 n + 0.5 of the mean world normal), OUT_depth.png (mean hit distance, near = white, normalised over
+the finite values; no hit = black) and OUT_shape.png (a hashed colour per shape id of sample 0, miss = black); the mean
+coverage (the share of samples that hit something) is printed.
 
 Scene::from_json -> GpuRenderer (Renderer trait: start_rendering / render_step until done) ->
 rt_tonemap_rgba8 (sqrt, clamp(0, 0.999) * 256, on the device) -> PNG.  With --adaptive, an adaptive frame
@@ -47,6 +53,7 @@ ap.add_argument("--orbit", type=int, default=None, metavar="N", help="N views ar
 ap.add_argument("--animate", type=int, default=None, metavar="N", help="N frames of the random spheres on a random walk")
 ap.add_argument("--step", type=float, default=0.05, help="--animate: random-walk step per axis and frame")
 ap.add_argument("--layers", type=int, default=None, metavar="N", help="N bounce layers, one PNG per layer")
+ap.add_argument("--features", action="store_true", help="albedo, normal, depth and shape PNGs of the first hits")
 ap.add_argument("--inspect", type=int, nargs=2, default=None, metavar=("X", "Y"),
                 help="print each sample's path of pixel (X, Y) and check their mean against the frame")
 a = ap.parse_args()
@@ -62,6 +69,9 @@ if a.animate is not None and (a.animate < 1 or a.orbit is not None or a.adaptive
 if a.layers is not None and (not 1 <= a.layers <= 63 or a.orbit is not None or a.animate is not None
                              or a.adaptive is not None or a.counts is not None or a.inspect is not None):
     ap.error("--layers needs 1 <= N <= 63 and excludes --orbit, --animate, --adaptive, --counts and --inspect")
+if a.features and (a.layers is not None or a.orbit is not None or a.animate is not None or a.adaptive is not None
+                   or a.counts is not None or a.inspect is not None):
+    ap.error("--features excludes --layers, --orbit, --animate, --adaptive, --counts and --inspect")
 if a.heatmap and a.adaptive is None and a.counts is None:
     ap.error("--heatmap needs --adaptive or --counts")
 if a.adaptive is not None and a.counts is not None:
@@ -89,6 +99,29 @@ if a.layers is not None:
         share = y(layers[b]) / total if total else 0.0
         last = "+" if b == a.layers - 1 and a.layers <= a.depth else " "
         print(f"  level {b:2d}{last} {100.0 * share:8.4f} % of the mean luminance  -> {stem}_L{b:02d}{ext or '.png'}")
+    sys.exit(0)
+if a.features:
+    frame, f = r.render_features(cam, w, h, a.spp)
+    dt = time.perf_counter() - t0
+    stem, ext = os.path.splitext(a.out)
+    rt.save_png(a.out, rt.tonemap_rgba8(sc, frame))
+    rgba = lambda c: np.concatenate([np.clip(np.nan_to_num(c) * 255.0 + 0.5, 0, 255).astype(np.uint8),
+                                     np.full(c.shape[:2] + (1,), 255, np.uint8)], axis=2)
+    d = f["depth"]
+    finite = np.isfinite(d)
+    lo, hi = (float(d[finite].min()), float(d[finite].max())) if finite.any() else (0.0, 1.0)
+    near = np.where(finite, 1.0 - (d - lo) / (hi - lo if hi > lo else 1.0), 0.0)
+    ids = f["shape"].astype(np.uint32)
+    hashed = [((ids * np.uint32(0x9E3779B1)) >> np.uint32(s)) & np.uint32(255) for s in (8, 16, 24)]
+    shape_rgb = np.where((f["shape"] >= 0)[..., None], np.stack(hashed, 2) / 255.0, 0.0)
+    outs = {"albedo": f["albedo"], "normal": 0.5 * f["normal"] + 0.5, "depth": np.repeat(near[..., None], 3, 2),
+            "shape": shape_rgb}
+    print(f"{a.scene}: {w}x{h}x{a.spp}, depth {a.depth}, features in {dt * 1e3:.1f} ms -> {a.out}; "
+          f"coverage {100.0 * float(f['coverage'].mean()):.4f} % of the samples hit a shape")
+    for k, img in outs.items():
+        path = f"{stem}_{k}{ext or '.png'}"
+        rt.save_png(path, rgba(img))
+        print(f"  {k:6s} -> {path}")
     sys.exit(0)
 if a.orbit is not None:
     views = r.render_views(rt.api.orbit_cameras(cam, a.orbit), w, h, a.spp)
